@@ -1,13 +1,17 @@
 #!/usr/bin/env python
 """bench.py -- population env-steps/s of the signal-gated market-making rollout on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one full population rollout (BASELINE.json configs[1]: P = 4096 individuals per GPU x
 T = 14 400 bars = 60 synthetic 510300-shaped days, H = 32, no fee, phi = 1e-4): every individual's
 policy MLP + quantisation + FPT env step for every bar, fitness and trade count out.  At N > 1 the
 population is sharded by contiguous global index (weak scaling: 4096 individuals per GPU) and each
 step ends with the ONE all-gather of the packed fitness / trade block that a sharded GA generation performs.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned -- fitness and trade count of the
+whole population, for the exact rollout and for each tensor-core precision -- as DIR/<name>.npy in float64.  The inputs
+are seeded, so two builds of the project can be compared array for array.
 
   value   whole-job env-steps/s, genomes and bars resident in HBM, CUDA-event timed per step
   e2e     the same through the host-buffer C-ABI entries: pinned host genomes H2D + kernel + fitness/trades D2H
@@ -326,6 +330,12 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    def last_outputs(prefix=""):
+        """Fitness and trades of the whole population as the last device step left them in the gathered block."""
+        rows = gather.view(world, blk)
+        return {prefix + "fitness": rows[:, :P_PER_GPU * 8].contiguous().view(torch.float64).flatten().cpu().numpy(),
+                prefix + "trades": rows[:, P_PER_GPU * 8:].contiguous().view(torch.int32).flatten().cpu().numpy().astype(np.float64)}
+
     def time_device(fn, steps):
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         barrier()
@@ -357,6 +367,7 @@ def run_ours(args):
     step_ms = time_device(step_device, K)
     t_wall1 = time.perf_counter()
     checksum = float(fit_view.sum().item())
+    outputs = last_outputs()
     # ---- end-to-end steps (host buffers, copies inside the timed region) ----------------------
     barrier()
     t0 = time.perf_counter()
@@ -372,6 +383,7 @@ def run_ours(args):
     for mode, _ in TC_MODES:
         ms = time_device(lambda m=mode: step_device(m), K)
         csum = float(fit_view.sum().item())
+        outputs.update(last_outputs(f"tensor_core_{mode}_"))
         barrier()
         t0 = time.perf_counter()
         for _ in range(K):
@@ -594,6 +606,10 @@ def run_ours(args):
         guarded("sharded_ga_bit_identical", sharded_identity)
 
     if rank == 0:
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         steps_per_step = p_total * T
         value = steps_per_step * K / (dev_ms * 1e-3)
         kernel_s = (dev_ms / K) * 1e-3                       # the rollout kernel is the whole device step
@@ -722,7 +738,13 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the CUDA path's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,22 +1,19 @@
-"""GPU (-m gpu): BASELINE.json configs[2..4] at their full sizes, the live unmodified reference, and the round-2
+"""GPU (-m gpu): BASELINE.json configs[2..4] at their full sizes, the unmodified reference's outputs, and the round-2
 entry points (H = 256 GA, pipelined host entry, sharding through DRLEngine's building blocks).
 
 Everything goes through the C ABI.  Integer work and every fp32 / fp64 quantity of the exact path are compared BIT-EXACTLY
-with the oracle; against the reference's own Python (oracle/_ref, run in a separate process) the tolerance is the one
+with the oracle; against the reference's own Python (its outputs recorded in tests/golden/ref_long.npz) the tolerance is the one
 BASELINE.json states: trades identical, fitness within 1e-5 relative, and a differing trajectory is excused only when the
 oracle's own raw*5 comes within NEAR_TIE_TICKS of a rounding boundary somewhere along it (MKL's fp32 summation order is
 not the SGMM-F32 order; the difference is ~1e-7 relative and flips a rounding only at such near-ties).
 """
 import os
-import subprocess
-import sys
-import tempfile
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import GOLDEN
 
 pytestmark = pytest.mark.gpu
 
@@ -165,28 +162,23 @@ def test_h256_f16_accumulator_envelope(sg, orc):
 
 
 # ----------------------------------------------------------------------------------------------
-# the live, unmodified reference (oracle/_ref) at config-2 length
+# the unmodified reference at config-2 length
 # ----------------------------------------------------------------------------------------------
-def _run_reference(bundle, stats, genomes, adv, fee, use_arl):
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    try:
-        import stage_ref
-        ok = stage_ref.staged()
-    finally:
-        sys.path.pop(0)
-    if not ok:
-        pytest.skip("oracle/_ref is not staged on this box (__graft_entry__.build() stages it where /root/reference exists; it is "
-                    "git-ignored but travels with the snapshot); the same episodes are pinned by tests/golden/ref_long.npz")
-    with tempfile.TemporaryDirectory() as d:
-        keys = ("s1", "s2", "mid_next", "best_ask", "best_bid", "buy_max", "sell_min")
-        extra = {"adv": adv} if adv is not None else {}
-        np.savez(os.path.join(d, "in.npz"), **dict(zip(keys, bundle)), s1_m=stats["s1_m"], s1_s=stats["s1_s"],
-                 s2_m=stats["s2_m"], s2_s=stats["s2_s"], genomes=genomes, phi=1e-4, tick=0.001, fee=fee, use_arl=use_arl, **extra)
-        subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "run_ref.py"), "--in", os.path.join(d, "in.npz"),
-                        "--out", os.path.join(d, "out.npz"), "--mode", "pool", "--procs", str(min(8, os.cpu_count() or 8)),
-                        "--torch-threads", "1"], check=True, timeout=600, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-        o = np.load(os.path.join(d, "out.npz"))
-        return o["fitness"].copy(), o["trades"].copy()
+def _reference_outputs(bundle, genomes, adv, fee, use_arl):
+    """The reference's own fitness and trades on these episodes, as oracle/make_golden_long.py recorded them (its
+    evaluate_individual in a Pool, run by oracle/run_ref.py) into tests/golden/ref_long.npz."""
+    from sgmm_b200 import synthetic
+    g = np.load(os.path.join(GOLDEN, "ref_long.npz"))
+    P = genomes.shape[0]
+    _, want = synthetic.policy_like_genomes(int(g["P"]), seed=int(g["genome_seed"]), out_scale=float(g["out_scale"]),
+                                            out_bias=tuple(g["out_bias"]))
+    assert np.array_equal(want, genomes) and len(bundle[0]) == 240 * int(g["days"]), "not the recorded episodes"
+    if use_arl:
+        assert np.array_equal(adv, (np.random.default_rng(int(g["adv_seed"])).standard_normal((P, 1250))
+                                    * float(g["adv_scale"])).astype(np.float32)), "not the recorded adversaries"
+    name = {(False, 0.0): "plain", (True, 0.0): "arl", (False, 3e-4): "fee", (True, 3e-4): "arl_fee"}[(use_arl, fee)]
+    assert bool(g[f"{name}.use_arl"]) == use_arl and float(g[f"{name}.fee"]) == fee
+    return g[f"{name}.fitness"].copy(), g[f"{name}.trades"].copy()
 
 
 @pytest.mark.parametrize("use_arl,fee", [(False, 0.0), (True, 0.0), (False, 3e-4), (True, 3e-4)])
@@ -197,7 +189,7 @@ def test_cuda_vs_live_reference_8_individuals_14400_bars(sg, orc, use_arl, fee):
     P = 8
     _, genomes = synthetic.policy_like_genomes(P, seed=12, out_scale=5.0, out_bias=(0.1, 0.1))
     adv = (np.random.default_rng(13).standard_normal((P, 1250)) * 0.5).astype(np.float32) if use_arl else None
-    f_ref, t_ref = _run_reference(bundle, stats, genomes, adv, fee, use_arl)
+    f_ref, t_ref = _reference_outputs(bundle, genomes, adv, fee, use_arl)
     bun = sg.Bundle.from_arrays(bundle, stats, 0.001)
     fit, trd = sg.rollout_population(bun, genomes, adv, phi=1e-4, fee_rate=fee)            # host entry (numpy in / out)
     z1, z2 = orc.normalise(bundle, stats)
@@ -213,7 +205,7 @@ def test_cuda_vs_live_reference_8_individuals_14400_bars(sg, orc, use_arl, fee):
         margin = float(np.min(np.abs(np.abs(q - np.floor(q)) - 0.5)))
         assert margin <= NEAR_TIE_TICKS, (i, trd[i], t_ref[i], fit[i], f_ref[i], margin)
         excused += 1
-    print(f"use_arl={use_arl} fee={fee}: {P - excused}/{P} trajectories identical to the live reference "
+    print(f"use_arl={use_arl} fee={fee}: {P - excused}/{P} trajectories identical to the reference "
           f"(trades equal, fitness within {REL_TOL_VS_REFERENCE} relative); {excused} excused at a logged near-tie")
     assert excused <= 2
     assert t_ref.min() > 100

@@ -279,19 +279,30 @@ def test_adversary_genome_lengths_accepted():
         _as_adv_matrix(torch.zeros(73))
 
 
-def test_reference_staging_recipe():
-    """oracle/_ref holds byte-identical copies of the reference's three hot-path files (staged by build() where
-    /root/reference exists); the manifest detects any edit."""
+def test_reference_staging_recipe(tmp_path):
+    """stage() copies the reference's hot-path files byte for byte and the manifest detects any edit; where oracle/_ref is
+    staged, it holds byte-identical copies of the reference's files."""
     import sys
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     try:
         import stage_ref
     finally:
         sys.path.pop(0)
-    if not os.path.exists(os.path.join(stage_ref.DST, "MANIFEST.json")):
-        pytest.skip("oracle/_ref not staged in this checkout")
-    assert stage_ref.staged()
-    if os.path.isdir(stage_ref.REF):
+    src, dst = tmp_path / "reference", tmp_path / "staged"
+    for k, rel in enumerate(stage_ref.FILES):
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_bytes(f"# stand-in {k}\n".encode() + bytes(range(256)))
+    manifest = stage_ref.stage(ref=str(src), dst=str(dst))
+    assert set(manifest["files"]) == set(stage_ref.FILES) and stage_ref.staged(str(dst))
+    for rel in stage_ref.FILES:
+        assert (dst / rel).read_bytes() == (src / rel).read_bytes()
+    (dst / stage_ref.FILES[0]).write_bytes(b"edited\n")
+    assert not stage_ref.staged(str(dst))
+    (dst / stage_ref.FILES[-1]).unlink()
+    assert not stage_ref.staged(str(dst))
+    if os.path.exists(os.path.join(stage_ref.DST, "MANIFEST.json")):
+        assert stage_ref.staged()
+    if os.path.isdir(stage_ref.REF) and os.path.isdir(stage_ref.DST):
         for rel in stage_ref.FILES:
             assert open(os.path.join(stage_ref.REF, rel), "rb").read() == open(os.path.join(stage_ref.DST, rel), "rb").read()
     tracked = __import__("subprocess").run(["git", "ls-files", "oracle/_ref"], cwd=ROOT, capture_output=True, text=True).stdout
