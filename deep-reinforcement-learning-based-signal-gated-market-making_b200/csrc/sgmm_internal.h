@@ -14,8 +14,9 @@ struct __align__(32) BarSig {
     float z1, z2;        // normalised SGU1 / SGU2 signals (drl_engine.py:33-34), fp32
     float tha, thb;      // float fill thresholds on q = raw*5 (BEFORE rounding):
                          //   fill_sell <=> q_a < tha, fill_buy <=> q_b < thb   (-inf never, +inf always)
-                         // tha = Ka + 0.5 nudged one ulp up when Ka is even, so that the strict
-                         // compare reproduces round-half-even followed by off <= Ka
+                         // tha = Ka + 0.5 nudged one ulp up when Ka is even (|Ka| >= 2^23: the float
+                         // after the largest float <= Ka), so that the strict compare reproduces
+                         // round-half-even followed by off <= Ka
     int32_t ka1, kb1;    // integer thresholds + 1: fill_sell <=> off_a < ka1 (used when the adversary
     int32_t pad0, pad1;  // displaces the rounded offsets); INT32_MIN never, INT32_MAX always
 };
@@ -29,7 +30,6 @@ struct __align__(32) BarPx {
 constexpr int32_t K_NEVER = INT32_MIN;
 constexpr int32_t K_ALWAYS = INT32_MAX;
 constexpr int32_t K_CLAMP = 1 << 30;
-constexpr int32_t K_FLOAT_EXACT = 1 << 22;   // |threshold| below which Ka+0.5 is exact in fp32
 
 }  // namespace sgmm
 

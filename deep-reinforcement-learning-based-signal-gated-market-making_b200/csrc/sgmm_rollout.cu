@@ -88,7 +88,8 @@ __device__ int32_t fill_threshold_plus1(double best, double tick, double bound)
     // the quote is monotone in k (IEEE rounding is monotone), so {k : touch} is a down-set
     if (!touch<ASK>(best, -K_CLAMP, tick, bound)) return K_NEVER;     // includes NaN bounds
     if (touch<ASK>(best, K_CLAMP, tick, bound)) return K_ALWAYS;
-    int lo = -K_CLAMP, hi = K_CLAMP;                                   // touch(lo) true, touch(hi) false
+    // touch(lo) true, touch(hi) false; 64-bit because hi - lo spans 2^31 before the search narrows it
+    int64_t lo = -K_CLAMP, hi = K_CLAMP;
     // warm start: the real-arithmetic solution is within a few ticks of the answer
     const double est = ASK ? (bound - best) / tick : (best - bound) / tick;
     if (est > -1.0e9 && est < 1.0e9) {
@@ -97,22 +98,24 @@ __device__ int32_t fill_threshold_plus1(double best, double tick, double bound)
         if (e + 4 < hi && !touch<ASK>(best, e + 4, tick, bound)) hi = e + 4;
     }
     while (hi - lo > 1) {
-        const int mid = lo + (hi - lo) / 2;
-        if (touch<ASK>(best, mid, tick, bound)) lo = mid; else hi = mid;
+        const int64_t mid = lo + (hi - lo) / 2;
+        if (touch<ASK>(best, (int)mid, tick, bound)) lo = mid; else hi = mid;
     }
-    return lo + 1;
+    return (int32_t)(lo + 1);
 }
 
 // fill <=> rint_half_even(q) <= K  <=>  q < K + 0.5, or q == K + 0.5 exactly and K is even (the tie
 // rounds down to K).  Folding the tie into a strict compare: threshold = K + 0.5, moved one ulp up
-// when K is even.  Exact for |K| < 2^22; beyond that the threshold saturates (documented limit).
+// when K is even -- for -2^23 <= K < 2^23, where K + 0.5 is exact in fp32.  Beyond, the q that can
+// round to the far side of K are fp32 numbers of magnitude >= 2^23, all integers: fill <=> q <= K
+// <=> q < the next float above the largest float <= K.  Exact for every threshold the prologue
+// derives (|K| <= K_CLAMP).
 __device__ __forceinline__ float float_threshold(int32_t k_plus1)
 {
     if (k_plus1 == K_NEVER) return -INFINITY;
     if (k_plus1 == K_ALWAYS) return INFINITY;
     const int32_t K = k_plus1 - 1;
-    if (K >= K_FLOAT_EXACT) return INFINITY;
-    if (K <= -K_FLOAT_EXACT) return -INFINITY;
+    if (K < -(1 << 23) || K >= (1 << 23)) return nextafterf(__int2float_rd(K), INFINITY);
     const float t = (float)K + 0.5f;                  // exact
     return (K & 1) == 0 ? nextafterf(t, INFINITY) : t;
 }

@@ -60,24 +60,32 @@ def test_fill_thresholds_match_exact_fp64_quotes(sg):
     assert (ka == np.iinfo(np.int32).min).sum() == np.isnan(bmax).sum()
 
 
+# exact-touch grids: (first price, step, decimals, tick) -- the 3.400-3.599 grid of SURVEY 7.4-2, the reference's default tick
+# 0.01 on the same 3-decimal prices, 2-decimal prices near 35, 4-decimal prices near 0.9 and 1-decimal prices near 3800
+EXACT_TOUCH_GRIDS = [(3.400, 0.001, 3, 0.001), (3.400, 0.001, 3, 0.01), (34.00, 0.01, 2, 0.01), (0.8800, 0.0001, 4, 0.0001),
+                     (3800.0, 0.2, 1, 0.2)]
+
+
 def test_fill_thresholds_adversarial_grid(sg):
     """SURVEY 7.4-2: on a 3.400-3.599 grid ~10 % of exact-touch cases differ between
-    fl(p +- fl(k*tick)) and the fused/real-arithmetic value; the thresholds must follow the former."""
-    p = np.round(np.arange(3.400, 3.600, 0.001), 3)
-    ks = np.arange(-12, 13)
-    ask = np.repeat(p, ks.size)
-    k = np.tile(ks, p.size)
-    bound_a = np.round(ask + k * 0.001, 3)            # "exact touch" bounds on the 3-dp grid
-    bound_b = np.round(ask - k * 0.001, 3)
-    z = np.zeros(ask.size, np.float32)
-    b = sg.Bundle(z, z, ask, ask, ask, bound_a, bound_b, 0.001)
-    ka, kb = b.thresholds()
-    kk = np.arange(-40, 41)
-    for i in range(ask.size):
-        assert ka[i] == kk[(ask[i] + kk * 0.001) <= bound_a[i]].max()
-        assert kb[i] == kk[(ask[i] - kk * 0.001) >= bound_b[i]].max()
-    naive = np.round((bound_a - ask) / 0.001).astype(int)
-    assert (naive != ka).sum() > 0, "grid should contain cases where the naive integer engine is wrong"
+    fl(p +- fl(k*tick)) and the fused/real-arithmetic value; the thresholds must follow the former.
+    The same holds on every price grid and tick in EXACT_TOUCH_GRIDS."""
+    for first, step, dec, tick in EXACT_TOUCH_GRIDS:
+        p = np.round(first + np.arange(200) * step, dec)
+        ks = np.arange(-12, 13)
+        ask = np.repeat(p, ks.size)
+        k = np.tile(ks, p.size)
+        bound_a = np.round(ask + k * tick, dec)            # "exact touch" bounds on the price grid
+        bound_b = np.round(ask - k * tick, dec)
+        z = np.zeros(ask.size, np.float32)
+        b = sg.Bundle(z, z, ask, ask, ask, bound_a, bound_b, tick)
+        ka, kb = b.thresholds()
+        kk = np.arange(-40, 41)
+        for i in range(ask.size):
+            assert ka[i] == kk[(ask[i] + kk * tick) <= bound_a[i]].max(), (tick, i)
+            assert kb[i] == kk[(ask[i] - kk * tick) >= bound_b[i]].max(), (tick, i)
+        naive = np.round((bound_a - ask) / tick).astype(int)
+        assert (naive != ka).sum() > 0, "grid should contain cases where the naive integer engine is wrong"
     # infinities
     z1 = np.zeros(4, np.float32)
     b2 = sg.Bundle(z1, z1, np.ones(4), np.ones(4), np.ones(4), np.array([np.inf, -np.inf, np.nan, 1.0]),
@@ -293,7 +301,7 @@ def test_seeded_children_match_oracle(sg, orc, use_adv):
 # ----------------------------------------------------------------------------------------------
 # GA on the device vs the same GA composed from oracle pieces
 # ----------------------------------------------------------------------------------------------
-def _oracle_ga(orc, train_bz, val_bz, master, adv_master, *, pop, sigma, phi, fee, use_arl, seed, gens, patience):
+def _oracle_ga(orc, train_bz, val_bz, master, adv_master, *, pop, sigma, phi, tick, fee, use_arl, seed, gens, patience):
     FLIP = 0x8000000000000000
     master = master.copy()
     adv_master = None if adv_master is None else adv_master.copy()
@@ -302,7 +310,7 @@ def _oracle_ga(orc, train_bz, val_bz, master, adv_master, *, pop, sigma, phi, fe
     best_master = master.copy()
     hist = {k: [] for k in ("train_f", "val_f", "train_trades", "val_trades", "sigma")}
     for gen in range(gens):
-        fit, trd = orc.rollout_population(train_bz, phi, 0.001, fee, master=master, sigma=float(s_mm),
+        fit, trd = orc.rollout_population(train_bz, phi, tick, fee, master=master, sigma=float(s_mm),
                                           adv_master=adv_master, adv_sigma=float(s_adv), use_adv=use_arl,
                                           seed=seed, generation=gen, count=pop, nthreads=4)
         best = int(np.argmax(fit))                                        # model.py:74
@@ -310,7 +318,7 @@ def _oracle_ga(orc, train_bz, val_bz, master, adv_master, *, pop, sigma, phi, fe
         if use_arl:
             abest = int(np.argmax(-fit))                                  # drl_engine.py:124-125
             adv_master = orc.mutate(adv_master, float(s_adv), seed ^ FLIP, gen, abest)
-        vf, vt = orc.rollout(master, None, val_bz, phi, 0.001, fee)      # drl_engine.py:129-140
+        vf, vt = orc.rollout(master, None, val_bz, phi, tick, fee)      # drl_engine.py:129-140
         hist["train_f"].append(fit[best]); hist["train_trades"].append(trd[best])
         hist["val_f"].append(vf); hist["val_trades"].append(vt); hist["sigma"].append(s_mm)
         if vf > best_val:
@@ -325,28 +333,31 @@ def _oracle_ga(orc, train_bz, val_bz, master, adv_master, *, pop, sigma, phi, fe
     return hist, master, adv_master, best_master, best_val, float(s_mm)
 
 
-@pytest.mark.parametrize("use_arl", [False, True])
-def test_device_ga_matches_oracle_ga(sg, orc, use_arl):
+@pytest.mark.parametrize("use_arl,phi,tick", [pytest.param(False, 1e-4, 0.001, id="False"), pytest.param(True, 1e-4, 0.001, id="True"),
+                                              pytest.param(False, 0.01, 0.01, id="False-reference_defaults"),
+                                              pytest.param(True, 0.01, 0.01, id="True-reference_defaults")])
+def test_device_ga_matches_oracle_ga(sg, orc, use_arl, phi, tick):
+    """phi = 0.01, tick 0.01: DRLEngine's and FTPEnv's own defaults (Env/drl_engine.py, Env/market_env.py)."""
     from sgmm_b200 import synthetic
     from sgmm_b200.engine import DeviceGA
     tb = synthetic.synthetic_bundle(2, first_day=50)
     vb = synthetic.synthetic_bundle(1, first_day=52)
     stats = synthetic.train_stats_of(tb)
-    train = sg.Bundle.from_arrays(tb, stats, 0.001)
-    val = sg.Bundle.from_arrays(vb, stats, 0.001)
+    train = sg.Bundle.from_arrays(tb, stats, tick)
+    val = sg.Bundle.from_arrays(vb, stats, tick)
     tz = orc.normalise(tb, stats) + tb[2:]
     vz = orc.normalise(vb, stats) + vb[2:]
     master, _ = synthetic.policy_like_genomes(1, seed=21, out_scale=1.0)
     adv_master = (np.random.default_rng(4).standard_normal(1250) * 0.5).astype(np.float32) if use_arl else None
     gens, pop, patience = 9, 24, 3
-    ga = DeviceGA(master, adv_master, pop_size=pop, sigma=0.05, phi=1e-4, fee_rate=0.0, use_arl=use_arl, seed=77,
+    ga = DeviceGA(master, adv_master, pop_size=pop, sigma=0.05, phi=phi, fee_rate=0.0, use_arl=use_arl, seed=77,
                   max_generations=gens, patience=patience)
     for _ in range(gens):
         ga.generation(train, val)
     h = ga.history(gens)
     st = ga.status()
     mm, adv, best = ga.masters()
-    ho, m_o, a_o, b_o, bv_o, s_o = _oracle_ga(orc, tz, vz, master, adv_master, pop=pop, sigma=0.05, phi=1e-4, fee=0.0,
+    ho, m_o, a_o, b_o, bv_o, s_o = _oracle_ga(orc, tz, vz, master, adv_master, pop=pop, sigma=0.05, phi=phi, tick=tick, fee=0.0,
                                                use_arl=use_arl, seed=77, gens=gens, patience=patience)
     assert np.array_equal(bits64(h["train_f"]), bits64(ho["train_f"]))
     assert np.array_equal(bits64(h["val_f"]), bits64(ho["val_f"]))

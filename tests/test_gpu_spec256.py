@@ -88,7 +88,7 @@ def test_ragged_lengths_and_many_individuals(sg, orc, T):
 
 @pytest.mark.parametrize("out_scale,fee", [(300.0, 0.0), (40000.0, 3e-4)])
 def test_large_offsets_through_the_step_codes(sg, orc, out_scale, fee):
-    """Offsets of hundreds to tens of thousands of ticks (both signs, both sides filling in one bar): the 24-bit offset
+    """Offsets of hundreds to tens of thousands of ticks (both signs, both sides filling in one bar): the two int32 offset
     fields of the step code and the accounting kernel reproduce the oracle's env bit for bit on the kernel's actions."""
     bundle, bz, bun, genomes = _setup(sg, orc, 1, 93, 9, seed=3, T=333, out_scale=out_scale)
     fit, trd, raw, act = sg.rollout_spec256_audit(bun, genomes, phi=1e-4, fee_rate=fee)
