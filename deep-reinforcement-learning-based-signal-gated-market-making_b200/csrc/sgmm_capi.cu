@@ -196,12 +196,12 @@ static int check_rollout_args(const sgmm_bundle* bundle, const sgmm_population* 
 {
     if (!bundle || !mm || !params) { set_error("NULL bundle / mm / params"); return SGMM_ERR_INVALID; }
     if (mm->count > 0 && (!fitness || !trades)) { set_error("NULL output array"); return SGMM_ERR_INVALID; }
-    if (params->precision != SGMM_PRECISION_F32 && params->precision != SGMM_PRECISION_BF16 && params->precision != SGMM_PRECISION_TF32 && params->precision != SGMM_PRECISION_F16) { set_error("unknown precision %d", params->precision); return SGMM_ERR_INVALID; }
+    if (params->precision != SGMM_PRECISION_F32 && params->precision != SGMM_PRECISION_BF16 && params->precision != SGMM_PRECISION_TF32 && params->precision != SGMM_PRECISION_F16 && params->precision != SGMM_PRECISION_EXACT) { set_error("unknown precision %d", params->precision); return SGMM_ERR_INVALID; }
     if (mm->hidden == 256) {
-        if (params->precision != SGMM_PRECISION_BF16) { set_error("hidden=256 runs on the tensor cores in bf16: pass precision=SGMM_PRECISION_BF16 (the bit-exact SGMM-F32 path and the tf32 path are built for H=32)"); return SGMM_ERR_UNSUPPORTED; }
-        if (adv) { set_error("the H=256 tensor-core rollout has no adversary path"); return SGMM_ERR_UNSUPPORTED; }
+        if (params->precision != SGMM_PRECISION_BF16 && params->precision != SGMM_PRECISION_EXACT) { set_error("hidden=256: pass precision=SGMM_PRECISION_EXACT (bit-exact SGMM-F32 order) or SGMM_PRECISION_BF16 (tensor cores); F32 and TF32 are H=32 paths"); return SGMM_ERR_UNSUPPORTED; }
+        if (adv && params->precision != SGMM_PRECISION_EXACT) { set_error("the H=256 tensor-core rollout has no adversary path (SGMM_PRECISION_EXACT has one)"); return SGMM_ERR_UNSUPPORTED; }
     } else if (mm->hidden == 32) {
-    } else if (params->precision != SGMM_PRECISION_F32) { set_error("the tensor-core precisions need hidden=32 (BF16 / TF32) or hidden=256 (BF16)"); return SGMM_ERR_UNSUPPORTED; }
+    } else if (params->precision != SGMM_PRECISION_F32) { set_error("precision %d needs hidden=32 or hidden=256 (EXACT, BF16) or hidden=32 (TF32, F16)", params->precision); return SGMM_ERR_UNSUPPORTED; }
     if (adv && adv->count != mm->count) { set_error("adv.count (%lld) != mm.count (%lld): MM i meets adversary i (Env/drl_engine.py:115)", (long long)adv->count, (long long)mm->count); return SGMM_ERR_INVALID; }
     if (adv && adv->hidden != 32) { set_error("adversary genomes are 1250-float TradingPolicy(32) genomes (models/model.py:63)"); return SGMM_ERR_INVALID; }
     return SGMM_OK;
@@ -215,9 +215,12 @@ int sgmm_rollout_population(const sgmm_bundle* bundle, const sgmm_population* mm
     if (int rc = fill_pop(mm, "mm", pm, genome_len(mm->hidden))) return rc;
     if (adv) if (int rc = fill_pop(adv, "adv", pa, 1250)) return rc;
     DeviceGuard guard(bundle->device);
+    const int prec = normalise_precision(params->precision, mm->hidden);
+    if (mm->hidden == 256 && prec == SGMM_PRECISION_EXACT)
+        return launch_exact256(bundle, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, fitness, trades, (cudaStream_t)stream);
     if (mm->hidden == 256)
         return launch_spec256(bundle, pm, params->phi, params->fee_rate, fitness, trades, nullptr, nullptr, (cudaStream_t)stream);
-    if (params->precision != SGMM_PRECISION_F32)
+    if (prec != SGMM_PRECISION_F32)
         return launch_tc32(bundle, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, params->units_per_lane, fitness, trades, nullptr, nullptr,
                            (cudaStream_t)stream, tc32_mode_of(params->precision));
     return launch_rollout(bundle, pm, adv ? &pa : nullptr, mm->hidden, params->phi, params->fee_rate,
@@ -229,7 +232,7 @@ int sgmm_rollout_tc_audit(const sgmm_bundle* bundle, const sgmm_population* mm, 
                           int32_t* act_trace, void* stream)
 {
     if (int rc = check_rollout_args(bundle, mm, adv, params, fitness, trades)) return rc;
-    if (params->precision == SGMM_PRECISION_F32) { set_error("audit entry is for the tensor-core paths (precision BF16 / TF32 / F16)"); return SGMM_ERR_INVALID; }
+    if (params->precision == SGMM_PRECISION_F32 || params->precision == SGMM_PRECISION_EXACT) { set_error("audit entry is for the tensor-core paths (precision BF16 / TF32 / F16)"); return SGMM_ERR_INVALID; }
     PopArgs pm, pa;
     if (int rc = fill_pop(mm, "mm", pm, genome_len(mm->hidden))) return rc;
     if (adv) if (int rc = fill_pop(adv, "adv", pa, 1250)) return rc;
@@ -271,9 +274,12 @@ static int enqueue_host_rollout(sgmm_bundle* b, int slot, const sgmm_population*
         if (int rc = check_cuda(cudaMemcpyAsync(d_adv, asrc, (size_t)(adv->genomes ? P * GA : GA) * sizeof(float), cudaMemcpyHostToDevice, st), "H2D adversary genomes")) return rc;
         if (adv->genomes) pa.genomes = d_adv; else pa.master = d_adv;
     }
-    if (mm->hidden == 256) {
+    const int prec = normalise_precision(params->precision, mm->hidden);
+    if (mm->hidden == 256 && prec == SGMM_PRECISION_EXACT) {
+        if (int rc = launch_exact256(b, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, d_fit, d_trd, st)) return rc;
+    } else if (mm->hidden == 256) {
         if (int rc = launch_spec256(b, pm, params->phi, params->fee_rate, d_fit, d_trd, nullptr, nullptr, st)) return rc;
-    } else if (params->precision != SGMM_PRECISION_F32) {
+    } else if (prec != SGMM_PRECISION_F32) {
         if (int rc = launch_tc32(b, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, params->units_per_lane, d_fit, d_trd, nullptr, nullptr, st,
                                  tc32_mode_of(params->precision))) return rc;
     } else if (int rc = launch_rollout(b, pm, adv ? &pa : nullptr, mm->hidden, params->phi, params->fee_rate,

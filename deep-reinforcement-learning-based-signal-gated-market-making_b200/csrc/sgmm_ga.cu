@@ -166,9 +166,9 @@ int sgmm_ga_create(sgmm_ga** out, const sgmm_ga_config* cfg, const float* mm_mas
     if (!out || !cfg || !mm_master) { set_error("NULL argument"); return SGMM_ERR_INVALID; }
     *out = nullptr;
     if (cfg->hidden != 32 && cfg->hidden != 256) { set_error("hidden=%d: GA rollouts are built for H=32 and H=256", cfg->hidden); return SGMM_ERR_UNSUPPORTED; }
-    if (cfg->hidden == 256 && cfg->precision == SGMM_PRECISION_F32) { set_error("hidden=256 runs on the tensor cores only: pass precision=SGMM_PRECISION_BF16 (the bit-exact SGMM-F32 kernel is built for H=32)"); return SGMM_ERR_UNSUPPORTED; }
-    if (cfg->precision != SGMM_PRECISION_F32 && cfg->precision != SGMM_PRECISION_BF16 && cfg->precision != SGMM_PRECISION_TF32 && cfg->precision != SGMM_PRECISION_F16) { set_error("unknown precision %d", cfg->precision); return SGMM_ERR_INVALID; }
-    if (cfg->hidden == 256 && cfg->use_arl) { set_error("the H=256 tensor-core rollout has no adversary path"); return SGMM_ERR_UNSUPPORTED; }
+    if (cfg->hidden == 256 && cfg->precision == SGMM_PRECISION_F32) { set_error("hidden=256: pass precision=SGMM_PRECISION_EXACT (bit-exact SGMM-F32 order) or SGMM_PRECISION_BF16 (tensor cores)"); return SGMM_ERR_UNSUPPORTED; }
+    if (cfg->precision != SGMM_PRECISION_F32 && cfg->precision != SGMM_PRECISION_BF16 && cfg->precision != SGMM_PRECISION_TF32 && cfg->precision != SGMM_PRECISION_F16 && cfg->precision != SGMM_PRECISION_EXACT) { set_error("unknown precision %d", cfg->precision); return SGMM_ERR_INVALID; }
+    if (cfg->hidden == 256 && cfg->use_arl && cfg->precision != SGMM_PRECISION_EXACT) { set_error("the H=256 tensor-core rollout has no adversary path (SGMM_PRECISION_EXACT has one)"); return SGMM_ERR_UNSUPPORTED; }
     if (cfg->pop_size <= 0 || cfg->shard_first < 0 || cfg->shard_count < 0 ||
         cfg->shard_first + cfg->shard_count > cfg->pop_size) { set_error("bad population / shard bounds"); return SGMM_ERR_INVALID; }
     const int64_t stride = cfg->shard_stride > 0 ? cfg->shard_stride : cfg->pop_size;
@@ -262,10 +262,14 @@ int sgmm_ga_evaluate(sgmm_ga* ga, const sgmm_bundle* train, void* stream)
     mm.first_index = c.shard_first; mm.count = c.shard_count; mm.first_index_dev = nullptr;
     PopArgs adv = mm;
     adv.master = ga->adv_master; adv.sigma_dev = &ga->st->adv_sigma; adv.seed = c.seed ^ ADV_SEED_FLIP;
+    const int prec = normalise_precision(c.precision, c.hidden);
+    if (c.hidden == 256 && prec == SGMM_PRECISION_EXACT)         // bit-exact H=256: policy tables + walks, in batches
+        return launch_exact256(train, mm, c.use_arl ? &adv : nullptr, c.phi, c.fee_rate, ga->my_fit(), ga->my_trd(),
+                               (cudaStream_t)stream);
     if (c.hidden == 256)                                        // BASELINE config 4: spec256_kernel + account_kernel
         return launch_spec256(train, mm, c.phi, c.fee_rate, ga->my_fit(), ga->my_trd(),
                               nullptr, nullptr, (cudaStream_t)stream);
-    if (c.precision != SGMM_PRECISION_F32)                      // tensor-core population evaluation (no adversary path)
+    if (prec != SGMM_PRECISION_F32)                             // tensor-core population evaluation
         return launch_tc32(train, mm, c.use_arl ? &adv : nullptr, c.phi, c.fee_rate, 0, ga->my_fit(), ga->my_trd(),
                            nullptr, nullptr, (cudaStream_t)stream, tc32_mode_of(c.precision));
     return launch_rollout(train, mm, c.use_arl ? &adv : nullptr, c.hidden, c.phi, c.fee_rate, 0, 0,
@@ -284,7 +288,9 @@ int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
     if (int rc = check_cuda(cudaGetLastError(), "ga_tell_kernel launch")) return rc;
     PopArgs one{};
     one.genomes = ga->mm_master; one.master = nullptr; one.count = 1;          // the new master IS the best child
-    if (c.hidden == 256) {                                                     // no exact kernel at this width: same tensor-core path
+    if (c.hidden == 256 && c.precision == SGMM_PRECISION_EXACT) {              // exact population: exact validation
+        if (int rc = launch_exact256(val, one, nullptr, c.phi, c.fee_rate, ga->val_fit, ga->val_trd, st)) return rc;
+    } else if (c.hidden == 256) {                                              // tensor-core population: same tensor-core path
         if (int rc = launch_spec256(val, one, c.phi, c.fee_rate, ga->val_fit, ga->val_trd, nullptr, nullptr, st)) return rc;
     } else if (int rc = launch_rollout(val, one, nullptr, c.hidden, c.phi, c.fee_rate, 0, 0, ga->val_fit, ga->val_trd, st)) return rc;
     // (one individual, adversary off: launch_rollout takes the small-population path of sgmm_one.cu -- policy for every

@@ -123,6 +123,13 @@ constexpr int64_t SMALL_POP_MAX = 400;      // measured break-even against the s
 constexpr int64_t SMALL_POP_MAX_ADV = 148;  // with the adversary (one 512-thread CTA per individual and SM)
 int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
                          cudaStream_t st);
+// the walk + fp64 half of the policy-table path over tables code [P][T][5] / next [P][T][8] (sgmm_one.cu)
+int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const PopArgs* adv, double phi, double fee,
+                double* fitness, int32_t* trades, cudaStream_t st);
+// bit-exact H = 256 (sgmm_exact256.cu): batches of policy table + walk; and the raw-output table of one genome for the trace
+int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
+                    cudaStream_t st);
+int launch_exact256_raw(const sgmm_bundle* b, const float* genome, float2* out, float* stage_buf, cudaStream_t st);
 int launch_trace(const sgmm_bundle* b, const float* mm_genome, int hidden, const float* adv_genome,
                  const int32_t* forced, const int32_t* table, double phi, double fee, const sgmm_trace* tr,
                  double* fitness, int32_t* trades, cudaStream_t st);
@@ -130,6 +137,8 @@ int launch_spec256(const sgmm_bundle* b, const PopArgs& mm, double phi, double f
                    float* raw_table, int32_t* act_trace, cudaStream_t st);
 int launch_tc32(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, int group, double* fitness, int32_t* trades,
                 float* raw_table, int32_t* act_trace, cudaStream_t st, int mode = 0);   // mode: 0 bf16, 1 tf32, 2 f16
+// SGMM_PRECISION_EXACT is SGMM_PRECISION_F32 at H = 32
+inline int normalise_precision(int precision, int hidden) { return (precision == SGMM_PRECISION_EXACT && hidden == 32) ? SGMM_PRECISION_F32 : precision; }
 inline int tc32_mode_of(int precision) { return precision == SGMM_PRECISION_TF32 ? 1 : (precision == SGMM_PRECISION_F16 ? 2 : 0); }
 int launch_tc32_prologue(sgmm_bundle* b, cudaStream_t st);
 int launch_account(const sgmm_bundle* b, const uint64_t* codes, int64_t count, double phi, double fee, double* fitness,

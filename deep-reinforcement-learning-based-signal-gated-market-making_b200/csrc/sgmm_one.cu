@@ -433,13 +433,21 @@ int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs*
         policy_table_kernel<<<(unsigned)(blocks < 1 ? 1 : blocks), PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, adv ? 1 : 0, code, next);
         if (int rc = check_cuda(cudaGetLastError(), "policy_table_kernel launch")) return rc;
     }
+    if (int rc = launch_walk(b, P, code, next, adv, phi, fee, fitness, trades, st)) return rc;
+    return release_codes(b, st);
+}
+
+int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const PopArgs* adv, double phi, double fee,
+                double* fitness, int32_t* trades, cudaStream_t st)
+{
+    using namespace one;
+    const int64_t T = b->T;
     int sms2 = 148;
     cudaDeviceGetAttribute(&sms2, cudaDevAttrMultiProcessorCount, b->device);
     if (adv) walk_account_adv_kernel<512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, *adv, b->tick, phi, fee, fitness, trades);
     else if (P <= sms2) walk_account_kernel<1024><<<(unsigned)P, 1024, 0, st>>>(b->px, T, code, next, b->tick, phi, fee, fitness, trades);
     else walk_account_kernel<512><<<(unsigned)P, 512, 0, st>>>(b->px, T, code, next, b->tick, phi, fee, fitness, trades);
-    if (int rc = check_cuda(cudaGetLastError(), "walk_account_kernel launch")) return rc;
-    return release_codes(b, st);
+    return check_cuda(cudaGetLastError(), "walk_account_kernel launch");
 }
 
 }  // namespace sgmm

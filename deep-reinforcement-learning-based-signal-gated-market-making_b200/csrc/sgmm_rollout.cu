@@ -569,6 +569,7 @@ struct TraceArgs {
     const BarSig* sig; const BarPx* px; const double* bmax; const double* smin;
     int64_t T; double tick, phi, fee;
     const float* mm; const float* adv; const int32_t* forced; const int32_t* table;
+    const float2* raw;       // [T][5] raw policy outputs of every (bar, inventory) (H = 256: sgmm_exact256.cu)
     sgmm_trace tr; double* fitness; int32_t* trades;
 };
 
@@ -607,7 +608,12 @@ __global__ void __launch_bounds__(32, 1) trace_kernel_h32(const TraceArgs a)
         float ra = 0.0f, rb = 0.0f; int ka, kb;
         if (a.forced) { ka = a.forced[2 * t]; kb = a.forced[2 * t + 1]; }
         else if (a.table) { const int64_t r = (t * 5 + (int)env.inventory + 2) * 2; ka = a.table[r]; kb = a.table[r + 1]; }
-        else {
+        else if (a.raw) {
+            const float2 r = a.raw[t * 5 + (int)env.inventory + 2];
+            ra = r.x; rb = r.y;
+            ka = __float2int_rn(__fmul_rn(ra, 5.0f));
+            kb = __float2int_rn(__fmul_rn(rb, 5.0f));
+        } else {
             float v = __fmaf_rn(w1x, sg.z1, b1);
             v = __fmaf_rn(w1y, sg.z2, v);
             v = __fmaf_rn(w1i, inv2, v);
@@ -680,13 +686,31 @@ int launch_trace(const sgmm_bundle* b, const float* mm_genome, int hidden, const
                  const int32_t* forced, const int32_t* table, double phi, double fee, const sgmm_trace* tr,
                  double* fitness, int32_t* trades, cudaStream_t st)
 {
-    if (hidden != 32) { set_error("hidden=%d: the trace kernel is built for H=32", hidden); return SGMM_ERR_UNSUPPORTED; }
+    if (hidden != 32 && hidden != 256) { set_error("hidden=%d: the trace is built for H=32 and H=256", hidden); return SGMM_ERR_UNSUPPORTED; }
     if (!mm_genome && !forced && !table) { set_error("trace needs a genome, forced actions or an inventory table"); return SGMM_ERR_INVALID; }
     TraceArgs a;
     a.sig = b->sig; a.px = b->px; a.bmax = b->bmax; a.smin = b->smin; a.T = b->T;
     a.tick = b->tick; a.phi = phi; a.fee = fee; a.mm = mm_genome; a.adv = adv_genome; a.forced = forced; a.table = table;
+    a.raw = nullptr;
     if (tr) a.tr = *tr; else { sgmm_trace z = {}; a.tr = z; }
     a.fitness = fitness; a.trades = trades;
+    if (hidden == 256) {
+        // the policy of every (bar, inventory) first (exact H = 256 table, raw outputs), then the same trace kernel on it
+        a.mm = nullptr;
+        if (mm_genome && !forced && !table) {
+            uint64_t* buf = nullptr;
+            const int64_t words = 5 * b->T + genome_len(256) / 2;               // float2[T][5] + room for one staged genome, reserved
+                                                                                 // whether or not the genome needs staging (269 KB)
+            if (int rc = reserve_codes(b, b->T > 0 ? (words + b->T - 1) / b->T : 1, st, &buf)) return rc;
+            float2* raw = reinterpret_cast<float2*>(buf);
+            if (b->T > 0)
+                if (int rc = launch_exact256_raw(b, mm_genome, raw, reinterpret_cast<float*>(buf + 5 * b->T), st)) return rc;
+            a.raw = raw;
+            trace_kernel_h32<<<1, 32, 0, st>>>(a);
+            if (int rc = check_cuda(cudaGetLastError(), "trace_kernel_h32 launch")) return rc;
+            return release_codes(b, st);
+        }
+    }
     trace_kernel_h32<<<1, 32, 0, st>>>(a);
     return check_cuda(cudaGetLastError(), "trace_kernel_h32 launch");
 }

@@ -29,14 +29,18 @@ def _stream(device):
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
-PRECISION_F32, PRECISION_BF16, PRECISION_TF32, PRECISION_F16 = 0, 1, 2, 3
+PRECISION_F32, PRECISION_BF16, PRECISION_TF32, PRECISION_F16, PRECISION_EXACT = 0, 1, 2, 3, 4
 
 
 def _precision(precision, hidden):
     """None -> the default of the width: hidden=32 bit-exact SGMM-F32 path, hidden=256 tcgen05 path.
-    "bf16" with hidden=32 selects the tensor-core rollout of sgmm_tc32.cu (all three layers on tcgen05)."""
+    "bf16" with hidden=32 selects the tensor-core rollout of sgmm_tc32.cu (all three layers on tcgen05).
+    "exact" is SGMM-F32 order at any width the library builds: the F32 path at hidden=32, the CUDA-core policy-table
+    path of sgmm_exact256.cu at hidden=256."""
     if precision is None:
         return PRECISION_BF16 if hidden == 256 else PRECISION_F32
+    if precision in ("exact", PRECISION_EXACT):
+        return PRECISION_F32 if hidden == 32 else PRECISION_EXACT
     if precision in ("f32", "fp32", PRECISION_F32):
         return PRECISION_F32
     if precision in ("bf16", "tensor", PRECISION_BF16):
@@ -238,7 +242,8 @@ _TRACE_F32 = ("raw_a", "raw_b")
 def rollout_trace(bundle: Bundle, genome=None, adv_genome=None, forced_actions=None, *, phi,
                   fee_rate=0.0, hidden=32):
     """Per-step trace of one individual: the recorder row contract (Env/recorder.py:8-36,
-    main.py:74-90).  ``forced_actions`` int32[T,2] replaces the policy (teacher-forced replay).
+    main.py:74-90) at hidden 32 or 256, policy in SGMM-F32 order.  ``forced_actions`` int32[T,2] replaces the policy
+    (teacher-forced replay).
     Returns ``(fitness, trades, dict of numpy arrays of length T)``."""
     dev = torch.device(f"cuda:{bundle.device}")
     T = bundle.T
@@ -332,15 +337,23 @@ def _cached_bundle(bundle, train_stats, tick_size, device=None) -> Bundle:
     return b
 
 
+_HIDDEN_OF_LEN = {genome_len(32): 32, genome_len(256): 256}
+
+
 def evaluate_individual(mm_weights, adv_weights, bundle, phi, tick_size, fee_rate, train_stats,
                         use_arl=False):
-    """Drop-in for Env/drl_engine.py:9-67 -> ``(np.float64 total_reward, int trades)``."""
+    """Drop-in for Env/drl_engine.py:9-67 -> ``(np.float64 total_reward, int trades)``.  The policy width follows from
+    the genome length, as the reference's ``TradingPolicy.set_weights`` of the matching width does (1250 floats: H=32,
+    67 330: H=256); both are evaluated in SGMM-F32 order, bit-identical to the reference's fp32 arithmetic."""
     dev_bundle = _cached_bundle(bundle, train_stats, tick_size)
     adv = adv_weights if (use_arl and adv_weights is not None) else None      # :17-21
     mm = torch.as_tensor(mm_weights, dtype=torch.float32).reshape(1, -1).cpu()
+    hidden = _HIDDEN_OF_LEN.get(mm.shape[1])
+    if hidden is None:
+        raise ValueError(f"genome length {mm.shape[1]} is neither {genome_len(32)} (hidden 32) nor {genome_len(256)} (hidden 256)")
     if adv is not None:
         adv = torch.as_tensor(adv, dtype=torch.float32).reshape(1, -1).cpu()
-    fit, trd = rollout_population(dev_bundle, mm, adv, phi=phi, fee_rate=fee_rate)
+    fit, trd = rollout_population(dev_bundle, mm, adv, phi=phi, fee_rate=fee_rate, hidden=hidden, precision="exact")
     return np.float64(fit[0]), int(trd[0])
 
 
@@ -443,7 +456,8 @@ class DRLEngine:
       reference's unseeded ``torch.randn``, models/model.py:69; an integer = reproducible, with the ``train`` call count
       folded in), ``device``, ``patience`` (15, :155), ``hidden_dim`` (32 or 256, models/model.py:7), ``precision``
       (``None`` / "f32": bit-exact population evaluation at hidden 32; "tf32" / "f16" / "bf16": tensor-core rollout;
-      hidden 256 always runs the tensor-core path).
+      ``None`` at hidden 256 runs the tensor-core path, "exact" runs population, validation and adversary bit-exact at
+      hidden 32 and 256).
     * When ``torch.distributed`` is initialised with more than one rank, ``train`` shards the population over the ranks
       (:class:`dist.ShardedGA`: one NCCL all-gather of fitness + trades per generation) -- the multi-GPU replacement of
       the ``Pool(8).starmap`` of drl_engine.py:91,115.  Every rank returns the identical policy and history; rank 0

@@ -61,6 +61,14 @@ extern "C" {
 #define SGMM_PRECISION_F16   3      /* H=32 only: f16 operands AND f16 accumulators for layers 1-2 (read back  */
                                     /* packed, ReLU on f16 pairs, no conversion), fp32 for layer 3             */
 
+#define SGMM_PRECISION_EXACT 4      /* SGMM-F32 order at every width the library builds (H=32 and H=256): bit-identical  */
+                                    /* to the oracle, with or without the adversary.  H=32: the same route as F32.       */
+                                    /* H=256: fp32 CUDA-core policy table of every (bar, inventory) + the automaton walk */
+                                    /* (sgmm_exact256.cu), ~55x the time of the BF16 path.  Populations run in batches   */
+                                    /* whose scratch (48 B per individual and bar, + 269 KB per seeded child) stays under */
+                                    /* the byte budget SGMM_EXACT256_BATCH_BYTES (environment, read on every call;        */
+                                    /* default 2 GiB).  F32 (0) with H=256 stays SGMM_ERR_UNSUPPORTED.                    */
+
 /* rollout flags */
 #define SGMM_FLAG_NONE       0
 
@@ -140,7 +148,8 @@ typedef struct {
  * H = 32 rollouts of more than 400 individuals are one kernel with no per-rollout scratch.  SMALL populations (up to 400
  * individuals, 148 with an adversary; exact precision, default launch geometry) take the policy-table path instead (the
  * exact policy for every (bar, inventory) in parallel + a prefix scan over the inventory automaton, bit-identical results):
- * its table ([count][T] x 48 B) lives in the same grow-only code buffer of the bundle, so the same two rules apply to them.
+ * its table ([count][T] x 48 B) lives in the same grow-only code buffer of the bundle, so the same two rules apply to them,
+ * and to every SGMM_PRECISION_EXACT rollout at H = 256 (the same table path, in batches).
  * The tensor-core precisions with an adversary read a per-(bundle, fee_rate) table of the reference's exact fp64 P&L legs
  * (144 B per bar), built on the first such rollout: that first rollout must not run under a stream capture either. */
 int sgmm_rollout_population(const sgmm_bundle* bundle, const sgmm_population* mm,
@@ -164,7 +173,8 @@ int sgmm_rollout_population_host_async(const sgmm_bundle* bundle, const sgmm_pop
                                        double* fitness, int32_t* trades, int32_t* ticket);
 int sgmm_rollout_wait(const sgmm_bundle* bundle, int32_t ticket);
 
-/* Audit variant of the tensor-core paths (hidden = 32 or 256, SGMM_PRECISION_BF16): same kernel, plus
+/* Audit variant of the tensor-core paths (hidden = 32 or 256, SGMM_PRECISION_BF16; F32 and EXACT are refused with
+ * SGMM_ERR_INVALID): same kernel, plus
  *   raw_table  DEVICE float[count][T][5][2]  policy outputs for every (bar, inventory -2..2)
  *   act_trace  DEVICE int32[count][T][2]     the offsets actually taken along the walked trajectory
  * (either may be NULL).  Used to state the bf16 tolerance against the fp32 oracle and to replay the
@@ -184,6 +194,8 @@ int sgmm_rollout_tc_audit(const sgmm_bundle* bundle, const sgmm_population* mm, 
  * main.py:74-90).  Every pointer is a DEVICE array of length T and may be NULL.
  * forced_actions (DEVICE int32[T,2], may be NULL) replaces the policy: teacher-forced replay of
  * recorded actions through the step core (bit-exact integer work given identical actions).
+ * hidden = 32 or 256, both in SGMM-F32 order (H = 256: the exact policy table of sgmm_exact256.cu first, then the same
+ * trace kernel; it uses the bundle's code buffer like an H = 256 population rollout).
  * ------------------------------------------------------------------------------------------- */
 typedef struct {
     int32_t* off_a; int32_t* off_b;      /* MM action (before the adversary's displacement)      */
@@ -267,11 +279,12 @@ typedef struct {
     uint64_t seed;
     int32_t max_generations;  /* history capacity                                                */
     int32_t precision;        /* SGMM_PRECISION_* of the POPULATION evaluation (0 = F32, bit-exact;  */
-                              /* BF16 / TF32 / F16 = tensor-core rollout).  hidden = 32: the         */
-                              /* validation rollout of the best child always runs the exact F32      */
-                              /* kernel.  hidden = 256 (BASELINE config 4): precision must be a      */
-                              /* tensor-core one, population AND validation run spec256_kernel,      */
-                              /* use_arl must be 0.                                                  */
+                              /* BF16 / TF32 / F16 = tensor-core rollout; EXACT = F32 at H=32).      */
+                              /* hidden = 32: the validation rollout of the best child always runs   */
+                              /* the exact F32 kernel.  hidden = 256 (BASELINE config 4): with a     */
+                              /* tensor-core precision population AND validation run spec256_kernel  */
+                              /* and use_arl must be 0; with EXACT both run the bit-exact H=256 path */
+                              /* (sgmm_exact256.cu), use_arl allowed.  F32 is refused at H=256.      */
 } sgmm_ga_config;
 
 typedef struct {
