@@ -5,7 +5,8 @@
 // 74 146 with back-to-back N=256 MMAs) -- integer, shared-memory and shuffle instructions are unaffected.  The
 // reference's accounting is fp64 by definition (Env/market_env.py:30-58, Env/drl_engine.py:54), so the tensor-core
 // kernels do only the INTEGER half of the env step (offsets, fills, inventory) and record, per bar actually visited,
-// a 64-bit code; this kernel turns the codes into rewards and sums them in the reference's order:
+// a 64-bit code; this kernel turns the codes into rewards (the fp64 step arithmetic of sgmm_step_core.h: quotes, legs,
+// penalty, the no-trade rule) and sums them in the reference's order:
 //     code = (fill_sell ? off_a : SGMM_CODE_NOFILL) | (fill_buy ? off_b : SGMM_CODE_NOFILL) << 32      (two int32)
 // (an offset is only needed on a side that filled; the inventory is re-derived here as the running sum of the fills).
 // The exact H=32 kernel (sgmm_rollout.cu) uses the same split INSIDE one kernel: its compute warps hand the step
@@ -44,7 +45,7 @@ __global__ void __launch_bounds__(ACC_THREADS) account_kernel(const uint64_t* __
         const bool live = ind < count;
         const uint64_t* c = codes + (live ? ind : 0) * T;
         int ntr = 0, inv = 0;                                        // market_env.py:17 (reset)
-        const double pen0 = mul_rn(phi, 0.0), pen1 = mul_rn(phi, 1.0), pen2 = mul_rn(phi, 2.0);
+        const PenaltyTable pen = penalty_table(phi);
         const uint64_t none = FLT ? 0xFFFFFFFFFFFFFFFFull : 0x8000000080000000ull;            // no fills beyond T
         uint64_t code_n = (live && lane < T) ? __ldcs(c + lane) : none;                       // window 0
         // the bars' prices are loaded unconditionally one window ahead (L1/L2-resident: every individual reads the same
@@ -72,21 +73,14 @@ __global__ void __launch_bounds__(ACC_THREADS) account_kernel(const uint64_t* __
             if (traded) {
                 if (fb) {
                     if (FLT) kb = __float2int_rn(__int_as_float(kb));                   // drl_engine.py:39 (np.round, half to even)
-                    const double my_bid = sub_rn(ab.y, mul_rn((double)kb, tick));       // :31
-                    double leg_b = sub_rn(mid, my_bid);
-                    if (FEE) leg_b = sub_rn(leg_b, mul_rn(my_bid, fee));                // :46,:48
-                    pnl = add_rn(pnl, leg_b);
+                    pnl = add_rn(pnl, buy_leg<FEE>(quote_bid(ab.y, kb, tick), mid, fee));
                 }
                 if (fs) {
                     if (FLT) ka = __float2int_rn(__int_as_float(ka));
-                    const double my_ask = add_rn(ab.x, mul_rn((double)ka, tick));       // :30
-                    double leg_s = sub_rn(my_ask, mid);
-                    if (FEE) leg_s = sub_rn(leg_s, mul_rn(my_ask, fee));                // :52,:54
-                    pnl = add_rn(pnl, leg_s);
+                    pnl = add_rn(pnl, sell_leg<FEE>(quote_ask(ab.x, ka, tick), mid, fee));
                 }
             }
-            const double pen = ai == 0 ? pen0 : (ai == 1 ? pen1 : pen2);                 // :57
-            tile[w & 1][warp][lane] = sub_rn(pnl, pen);                                 // :58
+            tile[w & 1][warp][lane] = sub_rn(pnl, penalty(pen, ai));                    // market_env.py:58
             __syncthreads();                                                            // tile w complete; tile w-1 consumed
         }
         if (lane == 0) s_trades[warp] = ntr;
@@ -110,8 +104,7 @@ __global__ void __launch_bounds__(ACC_THREADS) account_kernel(const uint64_t* __
         const int64_t ind = ind0 + lane;
         if (lane < ACC_IND && ind < count) {
             const int ntr = s_trades[lane];
-            if (ntr == 0) total = sub_rn(total, 50.0);                                  // drl_engine.py:64-65
-            fitness[ind] = total;
+            fitness[ind] = episode_fitness(total, ntr);
             trades[ind] = ntr;
         }
     }

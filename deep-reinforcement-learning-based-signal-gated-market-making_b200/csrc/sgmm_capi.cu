@@ -41,15 +41,29 @@ static int ensure_workspace(sgmm_bundle* b, int slot, size_t bytes)
     return SGMM_OK;
 }
 
-static int fill_pop(const sgmm_population* p, const char* name, PopArgs& out, int64_t G)
+static int fill_pop(const sgmm_population* p, const char* name, PopArgs& out)
 {
     if (p->count < 0) { set_error("%s.count < 0", name); return SGMM_ERR_INVALID; }
     if (p->count > 0 && !p->genomes && !p->master) { set_error("%s: neither genomes nor master given", name); return SGMM_ERR_INVALID; }
-    (void)G;
     out.genomes = p->genomes; out.master = p->master; out.first_index_dev = nullptr;
     out.sigma = p->sigma; out.sigma_dev = nullptr; out.seed = p->seed; out.generation = p->generation;
     out.generation_dev = nullptr; out.first_index = p->first_index; out.count = p->count;
     return SGMM_OK;
+}
+
+static int tc32_mode_of(int precision) { return precision == SGMM_PRECISION_TF32 ? 1 : (precision == SGMM_PRECISION_F16 ? 2 : 0); }
+
+int launch_population(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int hidden, int precision, double phi, double fee,
+                      int units_per_lane, int warps_per_cta, double* fitness, int32_t* trades, cudaStream_t st)
+{
+    if (precision == SGMM_PRECISION_EXACT && hidden == 32) precision = SGMM_PRECISION_F32;     // EXACT at H = 32 is the F32 route
+    if (hidden == 256 && precision == SGMM_PRECISION_EXACT)         // bit-exact H = 256: policy tables + walks, in batches
+        return launch_exact256(b, mm, adv, phi, fee, fitness, trades, st);
+    if (hidden == 256)                                              // BASELINE config 4: spec256_kernel + account_kernel
+        return launch_spec256(b, mm, phi, fee, fitness, trades, nullptr, nullptr, st);
+    if (precision != SGMM_PRECISION_F32)                            // tensor cores at H = 32
+        return launch_tc32(b, mm, adv, phi, fee, units_per_lane, fitness, trades, nullptr, nullptr, st, tc32_mode_of(precision));
+    return launch_rollout(b, mm, adv, hidden, phi, fee, units_per_lane, warps_per_cta, fitness, trades, st);
 }
 
 }  // namespace sgmm
@@ -212,19 +226,11 @@ int sgmm_rollout_population(const sgmm_bundle* bundle, const sgmm_population* mm
 {
     if (int rc = check_rollout_args(bundle, mm, adv, params, fitness, trades)) return rc;
     PopArgs pm, pa;
-    if (int rc = fill_pop(mm, "mm", pm, genome_len(mm->hidden))) return rc;
-    if (adv) if (int rc = fill_pop(adv, "adv", pa, 1250)) return rc;
+    if (int rc = fill_pop(mm, "mm", pm)) return rc;
+    if (adv) if (int rc = fill_pop(adv, "adv", pa)) return rc;
     DeviceGuard guard(bundle->device);
-    const int prec = normalise_precision(params->precision, mm->hidden);
-    if (mm->hidden == 256 && prec == SGMM_PRECISION_EXACT)
-        return launch_exact256(bundle, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, fitness, trades, (cudaStream_t)stream);
-    if (mm->hidden == 256)
-        return launch_spec256(bundle, pm, params->phi, params->fee_rate, fitness, trades, nullptr, nullptr, (cudaStream_t)stream);
-    if (prec != SGMM_PRECISION_F32)
-        return launch_tc32(bundle, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, params->units_per_lane, fitness, trades, nullptr, nullptr,
-                           (cudaStream_t)stream, tc32_mode_of(params->precision));
-    return launch_rollout(bundle, pm, adv ? &pa : nullptr, mm->hidden, params->phi, params->fee_rate,
-                          params->units_per_lane, params->warps_per_cta, fitness, trades, (cudaStream_t)stream);
+    return launch_population(bundle, pm, adv ? &pa : nullptr, mm->hidden, params->precision, params->phi, params->fee_rate,
+                             params->units_per_lane, params->warps_per_cta, fitness, trades, (cudaStream_t)stream);
 }
 
 int sgmm_rollout_tc_audit(const sgmm_bundle* bundle, const sgmm_population* mm, const sgmm_population* adv,
@@ -234,8 +240,8 @@ int sgmm_rollout_tc_audit(const sgmm_bundle* bundle, const sgmm_population* mm, 
     if (int rc = check_rollout_args(bundle, mm, adv, params, fitness, trades)) return rc;
     if (params->precision == SGMM_PRECISION_F32 || params->precision == SGMM_PRECISION_EXACT) { set_error("audit entry is for the tensor-core paths (precision BF16 / TF32 / F16)"); return SGMM_ERR_INVALID; }
     PopArgs pm, pa;
-    if (int rc = fill_pop(mm, "mm", pm, genome_len(mm->hidden))) return rc;
-    if (adv) if (int rc = fill_pop(adv, "adv", pa, 1250)) return rc;
+    if (int rc = fill_pop(mm, "mm", pm)) return rc;
+    if (adv) if (int rc = fill_pop(adv, "adv", pa)) return rc;
     DeviceGuard guard(bundle->device);
     if (mm->hidden == 32)
         return launch_tc32(bundle, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, params->units_per_lane, fitness, trades, raw_table,
@@ -264,26 +270,18 @@ static int enqueue_host_rollout(sgmm_bundle* b, int slot, const sgmm_population*
     float* d_mm = (float*)base; float* d_adv = (float*)(base + mm_bytes);
     double* d_fit = (double*)(base + mm_bytes + adv_bytes); int32_t* d_trd = (int32_t*)(base + mm_bytes + adv_bytes + fit_bytes);
     PopArgs pm, pa;
-    if (int rc = fill_pop(mm, "mm", pm, G)) return rc;
+    if (int rc = fill_pop(mm, "mm", pm)) return rc;
     const float* hsrc = mm->genomes ? mm->genomes : mm->master;
     if (int rc = check_cuda(cudaMemcpyAsync(d_mm, hsrc, (size_t)(mm->genomes ? P * G : G) * sizeof(float), cudaMemcpyHostToDevice, st), "H2D genomes")) return rc;
     if (mm->genomes) pm.genomes = d_mm; else pm.master = d_mm;
     if (adv) {
-        if (int rc = fill_pop(adv, "adv", pa, GA)) return rc;
+        if (int rc = fill_pop(adv, "adv", pa)) return rc;
         const float* asrc = adv->genomes ? adv->genomes : adv->master;
         if (int rc = check_cuda(cudaMemcpyAsync(d_adv, asrc, (size_t)(adv->genomes ? P * GA : GA) * sizeof(float), cudaMemcpyHostToDevice, st), "H2D adversary genomes")) return rc;
         if (adv->genomes) pa.genomes = d_adv; else pa.master = d_adv;
     }
-    const int prec = normalise_precision(params->precision, mm->hidden);
-    if (mm->hidden == 256 && prec == SGMM_PRECISION_EXACT) {
-        if (int rc = launch_exact256(b, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, d_fit, d_trd, st)) return rc;
-    } else if (mm->hidden == 256) {
-        if (int rc = launch_spec256(b, pm, params->phi, params->fee_rate, d_fit, d_trd, nullptr, nullptr, st)) return rc;
-    } else if (prec != SGMM_PRECISION_F32) {
-        if (int rc = launch_tc32(b, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, params->units_per_lane, d_fit, d_trd, nullptr, nullptr, st,
-                                 tc32_mode_of(params->precision))) return rc;
-    } else if (int rc = launch_rollout(b, pm, adv ? &pa : nullptr, mm->hidden, params->phi, params->fee_rate,
-                                       params->units_per_lane, params->warps_per_cta, d_fit, d_trd, st)) return rc;
+    if (int rc = launch_population(b, pm, adv ? &pa : nullptr, mm->hidden, params->precision, params->phi, params->fee_rate,
+                                   params->units_per_lane, params->warps_per_cta, d_fit, d_trd, st)) return rc;
     if (int rc = check_cuda(cudaMemcpyAsync(fitness, d_fit, (size_t)P * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H fitness")) return rc;
     return check_cuda(cudaMemcpyAsync(trades, d_trd, (size_t)P * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "D2H trades");
 }

@@ -262,18 +262,8 @@ int sgmm_ga_evaluate(sgmm_ga* ga, const sgmm_bundle* train, void* stream)
     mm.first_index = c.shard_first; mm.count = c.shard_count; mm.first_index_dev = nullptr;
     PopArgs adv = mm;
     adv.master = ga->adv_master; adv.sigma_dev = &ga->st->adv_sigma; adv.seed = c.seed ^ ADV_SEED_FLIP;
-    const int prec = normalise_precision(c.precision, c.hidden);
-    if (c.hidden == 256 && prec == SGMM_PRECISION_EXACT)         // bit-exact H=256: policy tables + walks, in batches
-        return launch_exact256(train, mm, c.use_arl ? &adv : nullptr, c.phi, c.fee_rate, ga->my_fit(), ga->my_trd(),
-                               (cudaStream_t)stream);
-    if (c.hidden == 256)                                        // BASELINE config 4: spec256_kernel + account_kernel
-        return launch_spec256(train, mm, c.phi, c.fee_rate, ga->my_fit(), ga->my_trd(),
-                              nullptr, nullptr, (cudaStream_t)stream);
-    if (prec != SGMM_PRECISION_F32)                             // tensor-core population evaluation
-        return launch_tc32(train, mm, c.use_arl ? &adv : nullptr, c.phi, c.fee_rate, 0, ga->my_fit(), ga->my_trd(),
-                           nullptr, nullptr, (cudaStream_t)stream, tc32_mode_of(c.precision));
-    return launch_rollout(train, mm, c.use_arl ? &adv : nullptr, c.hidden, c.phi, c.fee_rate, 0, 0,
-                          ga->my_fit(), ga->my_trd(), (cudaStream_t)stream);
+    return launch_population(train, mm, c.use_arl ? &adv : nullptr, c.hidden, c.precision, c.phi, c.fee_rate, 0, 0,
+                             ga->my_fit(), ga->my_trd(), (cudaStream_t)stream);
 }
 
 int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
@@ -288,13 +278,11 @@ int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
     if (int rc = check_cuda(cudaGetLastError(), "ga_tell_kernel launch")) return rc;
     PopArgs one{};
     one.genomes = ga->mm_master; one.master = nullptr; one.count = 1;          // the new master IS the best child
-    if (c.hidden == 256 && c.precision == SGMM_PRECISION_EXACT) {              // exact population: exact validation
-        if (int rc = launch_exact256(val, one, nullptr, c.phi, c.fee_rate, ga->val_fit, ga->val_trd, st)) return rc;
-    } else if (c.hidden == 256) {                                              // tensor-core population: same tensor-core path
-        if (int rc = launch_spec256(val, one, c.phi, c.fee_rate, ga->val_fit, ga->val_trd, nullptr, nullptr, st)) return rc;
-    } else if (int rc = launch_rollout(val, one, nullptr, c.hidden, c.phi, c.fee_rate, 0, 0, ga->val_fit, ga->val_trd, st)) return rc;
-    // (one individual, adversary off: launch_rollout takes the small-population path of sgmm_one.cu -- policy for every
-    //  (bar, inventory) in parallel, automaton scan, reference-order sum; bit-identical to the sequential kernel)
+    // H = 256: the population's own route (exact, or the same tensor-core path).  H = 32: always exact -- one individual,
+    // adversary off, so launch_rollout takes the small-population path of sgmm_one.cu (policy for every (bar, inventory)
+    // in parallel, automaton scan, reference-order sum; bit-identical to the sequential kernel)
+    const int val_precision = c.hidden == 32 ? SGMM_PRECISION_F32 : c.precision;
+    if (int rc = launch_population(val, one, nullptr, c.hidden, val_precision, c.phi, c.fee_rate, 0, 0, ga->val_fit, ga->val_trd, st)) return rc;
     ga_update_kernel<<<1, 256, 0, st>>>(ga->st, ga->val_fit, ga->val_trd, ga->mm_master, ga->best_master, ga->G,
                                         c.patience, c.use_arl, c.max_generations, ga->h_train_f, ga->h_val_f,
                                         ga->h_train_t, ga->h_val_t, ga->h_sigma);

@@ -137,9 +137,10 @@ int launch_spec256(const sgmm_bundle* b, const PopArgs& mm, double phi, double f
                    float* raw_table, int32_t* act_trace, cudaStream_t st);
 int launch_tc32(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, int group, double* fitness, int32_t* trades,
                 float* raw_table, int32_t* act_trace, cudaStream_t st, int mode = 0);   // mode: 0 bf16, 1 tf32, 2 f16
-// SGMM_PRECISION_EXACT is SGMM_PRECISION_F32 at H = 32
-inline int normalise_precision(int precision, int hidden) { return (precision == SGMM_PRECISION_EXACT && hidden == 32) ? SGMM_PRECISION_F32 : precision; }
-inline int tc32_mode_of(int precision) { return precision == SGMM_PRECISION_TF32 ? 1 : (precision == SGMM_PRECISION_F16 ? 2 : 0); }
+// the rollout of a population on the kernel that serves (hidden, precision, adversary) (sgmm_capi.cu); units_per_lane is
+// the tensor-core group size at H = 32 in BF16 / TF32 / F16.  The arguments are checked by the caller.
+int launch_population(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int hidden, int precision, double phi, double fee,
+                      int units_per_lane, int warps_per_cta, double* fitness, int32_t* trades, cudaStream_t st);
 int launch_tc32_prologue(sgmm_bundle* b, cudaStream_t st);
 int launch_account(const sgmm_bundle* b, const uint64_t* codes, int64_t count, double phi, double fee, double* fitness,
                    int32_t* trades, cudaStream_t st, bool float_offsets = false);

@@ -11,10 +11,11 @@
 //                           EVERY (bar, inventory) pair -- 5 T independent evaluations spread over the whole GPU, one pair
 //                           per thread with the weights broadcast from shared memory -- and the integer half of the env
 //                           step of the pair: fills, next inventory, 8-byte step code;
-//   2. walk_account_kernel  one CTA: the walk through the 5-state automaton as a parallel prefix scan over function
+//   2. walk_account_kernel<Walk5>  one CTA: the walk through the 5-state automaton as a parallel prefix scan over function
 //                           composition (every bar is a map {0..4} -> {0..4}; composition is associative), then the fp64
 //                           half for the visited pairs in parallel, and the one thing that is inherently serial -- the
 //                           reference-order fp64 reward sum (drl_engine.py:54) -- by one thread, chunk by chunk.
+//                           With the adversary the same kernel walks a 20-state automaton (walk_account_kernel<Walk20>).
 // 5x the policy FLOPs of the sequential walk, ~10x less time; results bit-identical to rollout_kernel_h32
 // (tests/test_gpu_configs.py compares both with the oracle; the GA parity tests compare whole histories).  One CTA of
 // walk_account_kernel per individual; the launcher takes this path below SMALL_POP_MAX individuals (measured break-even
@@ -159,6 +160,15 @@ __global__ void __launch_bounds__(PT_THREADS) policy_table_kernel(const BarSig* 
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// The walk (walk_account_kernel below) runs over one of two automata; each gives its map type, the map of bar t and the
+// step of bar t from a state:
+//   Walk5   no adversary: the state is the inventory index 0..4, the map of a bar comes from the table's `next` bytes.
+//   Walk20  with the adversary (drl_engine.py:42-48) the walk has 20 states (fill_sell_prev, fill_buy_prev, inventory):
+//           the policy table holds the raw q = raw*5 of every (bar, inventory) pair, every bar is a map {0..19} -> {0..19}
+//           built from it, the bar's integer thresholds and the individual's 20-entry displacement table.
+// ---------------------------------------------------------------------------------------------
+
 // maps {0..4} -> {0..4} packed 3 bits per entry
 __device__ __forceinline__ uint32_t map_of(const uint8_t* n) { return n[0] | (n[1] << 3) | (n[2] << 6) | (n[3] << 9) | (n[4] << 12); }
 __device__ __forceinline__ uint32_t map_at(uint32_t m, uint32_t e) { return (m >> (3u * e)) & 7u; }
@@ -170,99 +180,34 @@ __device__ __forceinline__ uint32_t map_then(uint32_t f, uint32_t g)
 }
 constexpr uint32_t MAP_ID = 0u | (1u << 3) | (2u << 6) | (3u << 9) | (4u << 12);
 
-// WALK_THREADS = 1024 (one individual per SM: shortest latency, populations up to the SM count) or 512 (three per SM: the
-// serial reward sum of one individual hides behind the others)
-template <int WALK_THREADS>
-__global__ void __launch_bounds__(WALK_THREADS, WALK_THREADS == 1024 ? 1 : 3) walk_account_kernel(const BarPx* __restrict__ px, int64_t T, const float2* __restrict__ code_all,
-                                                                         const uint8_t* __restrict__ next_all, double tick, double phi, double fee,
-                                                                         double* __restrict__ fitness, int32_t* __restrict__ trades)
-{
-    const float2* code = code_all + (int64_t)blockIdx.x * T * 5;          // one CTA per individual
-    const uint8_t* next = next_all + (int64_t)blockIdx.x * T * 8;
-    __shared__ uint32_t s_warp[32];                         // (WALK_THREADS / 32 entries used)
-    __shared__ int s_trades;
-    __shared__ double s_rew[SUM_CHUNK];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0) s_trades = 0;
-    // ---- 1. every thread composes the maps of its contiguous segment of bars ----
-    const int64_t L = (T + WALK_THREADS - 1) / WALK_THREADS;
-    const int64_t t_lo = (int64_t)tid * L < T ? (int64_t)tid * L : T, t_hi = t_lo + L < T ? t_lo + L : T;
-    uint32_t m = MAP_ID;
-    for (int64_t t = t_lo; t < t_hi; ++t) m = map_then(m, map_of(next + t * 8));
-    // ---- 2. exclusive scan over the segments (composition is associative, not commutative: earlier bars first) ----
-    uint32_t inc = m;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t o = __shfl_up_sync(0xffffffffu, inc, d);
-        if (lane >= d) inc = map_then(o, inc);
+struct Walk5 {
+    using Map = uint32_t;
+    static constexpr int STATES = 5, SCAN_UNROLL = 5;
+    struct Step { float2 q; bool fb, fs; uint32_t next; };
+    const float2* code;                    // this individual's [T][5] q of each side that filled, NaN marker otherwise
+    const uint8_t* next;                   // [T][8] next inventory index
+    __device__ Walk5(const BarSig*, const float2* code_all, const uint8_t* next_all, const PopArgs&, int64_t ind, int64_t T)
+        : code(code_all + ind * T * 5), next(next_all + ind * T * 8) {}
+    __device__ static Map identity() { return MAP_ID; }
+    __device__ static Map then(Map f, Map g) { return map_then(f, g); }
+    __device__ static Map shfl_up(Map m, int d) { return __shfl_up_sync(0xffffffffu, m, d); }
+    __device__ static uint32_t at(Map m, uint32_t s) { return map_at(m, s); }
+    __device__ static int inventory_index(uint32_t s) { return (int)s; }
+    __device__ Map bar_map(int64_t t) const { return map_of(next + t * 8); }
+    __device__ Step step(uint32_t iv, int64_t t) const
+    {
+        Step r;
+        r.q = code[t * 5 + iv];
+        r.fs = __float_as_int(r.q.x) != SGMM_CODE_NOFILL_F;
+        r.fb = __float_as_int(r.q.y) != SGMM_CODE_NOFILL_F;
+        r.next = next[t * 8 + iv];
+        return r;
     }
-    if (lane == 31) s_warp[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-        uint32_t w = lane < WALK_THREADS / 32 ? s_warp[lane] : MAP_ID;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const uint32_t o = __shfl_up_sync(0xffffffffu, w, d);
-            if (lane >= d) w = map_then(o, w);
-        }
-        s_warp[lane] = w;                                   // inclusive over warps
-    }
-    __syncthreads();
-    uint32_t before = __shfl_up_sync(0xffffffffu, inc, 1);   // everything before this thread inside its warp
-    if (lane == 0) before = MAP_ID;
-    if (warp > 0) before = map_then(s_warp[warp - 1], before);
-    uint32_t iv = map_at(before, 2);                        // the episode starts flat: inventory 0 = index 2 (market_env.py:17)
-    // ---- 3. the fp64 half for the visited pairs, chunk by chunk; one thread sums each chunk in bar order ----
-    const double pen0 = mul_rn(phi, 0.0), pen1 = mul_rn(phi, 1.0), pen2 = mul_rn(phi, 2.0);       // market_env.py:57
-    int ntr = 0;
-    double total = 0.0;                                     // thread 0 only (drl_engine.py:26)
-    for (int64_t c0 = 0; c0 < T; c0 += SUM_CHUNK) {
-        const int64_t c1 = c0 + SUM_CHUNK < T ? c0 + SUM_CHUNK : T;
-        const int64_t a = t_lo > c0 ? t_lo : c0, b = t_hi < c1 ? t_hi : c1;       // this thread's bars inside the chunk
-        for (int64_t t = a; t < b; ++t) {
-            const float2 q = code[t * 5 + iv];
-            int ka = __float_as_int(q.x), kb = __float_as_int(q.y);
-            const bool fs = ka != SGMM_CODE_NOFILL_F, fb = kb != SGMM_CODE_NOFILL_F;
-            const uint32_t niv = next[t * 8 + iv];
-            ntr += (fb || fs) ? 1 : 0;                                             // drl_engine.py:60-61
-            double pnl = 0.0;                                                      // market_env.py:40
-            if (fb || fs) {
-                const BarPx p = px[t];
-                ka = __float2int_rn(q.x); kb = __float2int_rn(q.y);                // drl_engine.py:39
-                const double my_ask = add_rn(p.ask, mul_rn((double)ka, tick));     // market_env.py:30
-                const double my_bid = sub_rn(p.bid, mul_rn((double)kb, tick));     // :31
-                double leg_b = sub_rn(p.mid_next, my_bid), leg_s = sub_rn(my_ask, p.mid_next);
-                leg_b = sub_rn(leg_b, mul_rn(my_bid, fee));                        // :46,:48 (fee terms evaluated as the reference does, fee_rate 0 included)
-                leg_s = sub_rn(leg_s, mul_rn(my_ask, fee));                        // :52,:54
-                pnl = fb ? add_rn(pnl, leg_b) : pnl;
-                pnl = fs ? add_rn(pnl, leg_s) : pnl;
-            }
-            const int ai = niv < 2u ? 2 - (int)niv : (int)niv - 2;
-            s_rew[t - c0] = sub_rn(pnl, ai == 0 ? pen0 : (ai == 1 ? pen1 : pen2));                 // :57-58
-            iv = niv;
-        }
-        __syncthreads();
-        if (tid == 0) {
-            const int n = (int)(c1 - c0);
-            for (int i = 0; i < n; ++i) total = add_rn(total, s_rew[i]);           // drl_engine.py:54
-        }
-        __syncthreads();
-    }
-    if (ntr) atomicAdd(&s_trades, ntr);
-    __syncthreads();
-    if (tid == 0) {
-        const int n = s_trades;
-        if (n == 0) total = sub_rn(total, 50.0);                                   // drl_engine.py:64-65
-        fitness[blockIdx.x] = total; trades[blockIdx.x] = n;
-    }
-}
+    // the offsets of a bar that traded (drl_engine.py:39)
+    __device__ static int2 offsets(const Step& r) { return make_int2(__float2int_rn(r.q.x), __float2int_rn(r.q.y)); }
+};
 
-// ---------------------------------------------------------------------------------------------
-// With the adversary (drl_engine.py:42-48) the walk has 20 states (fill_sell_prev, fill_buy_prev, inventory): the policy
-// table holds the raw q = raw*5 of every (bar, inventory) pair, every bar is a map {0..19} -> {0..19} built from it, the
-// bar's integer thresholds and the individual's 20-entry displacement table, and the same prefix scan applies.
-// Maps: 20 entries of 5 bits, six per 32-bit word.
-// ---------------------------------------------------------------------------------------------
+// Maps {0..19} -> {0..19}: 20 entries of 5 bits, six per 32-bit word.
 struct Map20 { uint32_t w[4]; };
 __device__ __forceinline__ uint32_t m20_at(const Map20& m, uint32_t e)          // dynamic index
 {
@@ -309,83 +254,108 @@ __device__ __forceinline__ void bar_map_rec(Map20& m, const float2* __restrict__
     if constexpr (S < 20) { m20_set<S>(m, adv_step((uint32_t)S, code_t, k1, at0, at1, at2).next); bar_map_rec<S + 1>(m, code_t, k1, at0, at1, at2); }
 }
 
-template <int WALK_THREADS>
-__global__ void __launch_bounds__(WALK_THREADS, 1) walk_account_adv_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px, int64_t T,
-                                                                            const float2* __restrict__ code_all, const PopArgs adv_in, double tick, double phi,
-                                                                            double fee, double* __restrict__ fitness, int32_t* __restrict__ trades)
+struct Walk20 {
+    using Map = Map20;
+    static constexpr int STATES = 20, SCAN_UNROLL = 1;
+    using Step = AdvStep;
+    const BarSig* sig;
+    const float2* code;                    // this individual's [T][5] raw q = raw*5
+    uint32_t at0, at1, at2;                // displacement table (sgmm_adversary.cuh)
+    __device__ Walk20(const BarSig* sig_, const float2* code_all, const uint8_t*, const PopArgs& adv_in, int64_t ind, int64_t T)
+        : sig(sig_), code(code_all + ind * T * 5)
+    {
+        __shared__ uint32_t s_adv[3];
+        const int tid = threadIdx.x;
+        if (tid < 3) s_adv[tid] = 0u;
+        __syncthreads();
+        if (tid < 20) {                                     // the individual's adversary as its displacement table
+            const PopArgs advp = resolve(adv_in);
+            const uint32_t e = adversary_entry(make_source(advp, ind, (int64_t)1250), tid);
+            atomicOr(&s_adv[tid >> 3], e << ((tid & 7) * 4));
+        }
+        __syncthreads();
+        at0 = s_adv[0]; at1 = s_adv[1]; at2 = s_adv[2];
+    }
+    __device__ static Map identity() { return m20_identity(); }
+    __device__ static Map then(const Map& f, const Map& g) { return m20_then(f, g); }
+    __device__ static Map shfl_up(const Map& m, int d) { return m20_shfl_up(m, d); }
+    __device__ static uint32_t at(const Map& m, uint32_t s) { return m20_at(m, s); }
+    __device__ static int inventory_index(uint32_t s) { return (int)(s % 5u); }
+    __device__ int2 k1(int64_t t) const { return __ldg(reinterpret_cast<const int2*>(&sig[t].ka1)); }
+    __device__ Map bar_map(int64_t t) const
+    {
+        Map20 m = {{0u, 0u, 0u, 0u}};
+        bar_map_rec(m, code + t * 5, k1(t), at0, at1, at2);
+        return m;
+    }
+    __device__ Step step(uint32_t st, int64_t t) const { return adv_step(st, code + t * 5, k1(t), at0, at1, at2); }
+    __device__ static int2 offsets(const Step& r) { return make_int2(r.oa, r.ob); }
+};
+
+// One CTA per individual.  WALK_THREADS = 1024 (one individual per SM: shortest latency, populations up to the SM count) or
+// 512 (three per SM without the adversary: the serial reward sum of one individual hides behind the others)
+template <class A, int WALK_THREADS>
+__global__ void __launch_bounds__(WALK_THREADS, (WALK_THREADS == 1024 || A::STATES == 20) ? 1 : 3)
+walk_account_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px, int64_t T, const float2* __restrict__ code_all,
+                    const uint8_t* __restrict__ next_all, const PopArgs adv, double tick, double phi, double fee,
+                    double* __restrict__ fitness, int32_t* __restrict__ trades)
 {
-    const float2* code = code_all + (int64_t)blockIdx.x * T * 5;          // one CTA per individual
-    __shared__ Map20 s_warp[32];
-    __shared__ uint32_t s_adv[3];
+    using Map = typename A::Map;
+    __shared__ Map s_warp[32];                              // (WALK_THREADS / 32 entries used)
     __shared__ int s_trades;
     __shared__ double s_rew[SUM_CHUNK];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) s_trades = 0;
-    if (tid < 3) s_adv[tid] = 0u;
-    __syncthreads();
-    if (tid < 20) {                                         // the individual's adversary as its displacement table (sgmm_adversary.cuh)
-        const PopArgs advp = resolve(adv_in);
-        const uint32_t e = adversary_entry(make_source(advp, blockIdx.x, (int64_t)1250), tid);
-        atomicOr(&s_adv[tid >> 3], e << ((tid & 7) * 4));
-    }
-    __syncthreads();
-    const uint32_t at0 = s_adv[0], at1 = s_adv[1], at2 = s_adv[2];
+    const A w(sig, code_all, next_all, adv, blockIdx.x, T);
     // ---- 1. every thread composes the maps of its contiguous segment of bars ----
     const int64_t L = (T + WALK_THREADS - 1) / WALK_THREADS;
     const int64_t t_lo = (int64_t)tid * L < T ? (int64_t)tid * L : T, t_hi = t_lo + L < T ? t_lo + L : T;
-    Map20 m = m20_identity();
-    for (int64_t t = t_lo; t < t_hi; ++t) {
-        Map20 bm = {{0u, 0u, 0u, 0u}};
-        bar_map_rec(bm, code + t * 5, __ldg(reinterpret_cast<const int2*>(&sig[t].ka1)), at0, at1, at2);
-        m = m20_then(m, bm);
-    }
-    // ---- 2. exclusive scan over the segments ----
-    Map20 inc = m;
-#pragma unroll 1
+    Map m = A::identity();
+    for (int64_t t = t_lo; t < t_hi; ++t) m = A::then(m, w.bar_map(t));
+    // ---- 2. exclusive scan over the segments (composition is associative, not commutative: earlier bars first) ----
+    Map inc = m;
+#pragma unroll A::SCAN_UNROLL
     for (int d = 1; d < 32; d <<= 1) {
-        const Map20 o = m20_shfl_up(inc, d);
-        if (lane >= d) inc = m20_then(o, inc);
+        const Map o = A::shfl_up(inc, d);
+        if (lane >= d) inc = A::then(o, inc);
     }
     if (lane == 31) s_warp[warp] = inc;
     __syncthreads();
     if (warp == 0) {
-        Map20 w = lane < WALK_THREADS / 32 ? s_warp[lane] : m20_identity();
-#pragma unroll 1
+        Map v = lane < WALK_THREADS / 32 ? s_warp[lane] : A::identity();
+#pragma unroll A::SCAN_UNROLL
         for (int d = 1; d < 32; d <<= 1) {
-            const Map20 o = m20_shfl_up(w, d);
-            if (lane >= d) w = m20_then(o, w);
+            const Map o = A::shfl_up(v, d);
+            if (lane >= d) v = A::then(o, v);
         }
-        s_warp[lane] = w;                                   // inclusive over warps
+        s_warp[lane] = v;                                   // inclusive over warps
     }
     __syncthreads();
-    Map20 before = m20_shfl_up(inc, 1);
-    if (lane == 0) before = m20_identity();
-    if (warp > 0) before = m20_then(s_warp[warp - 1], before);
-    uint32_t st = m20_at(before, 2u);                       // flat, no previous fills (market_env.py:17, drl_engine.py:29)
+    Map before = A::shfl_up(inc, 1);                        // everything before this thread inside its warp
+    if (lane == 0) before = A::identity();
+    if (warp > 0) before = A::then(s_warp[warp - 1], before);
+    uint32_t st = A::at(before, 2u);                        // flat, no previous fills: state 2 (market_env.py:17, drl_engine.py:29)
     // ---- 3. the fp64 half for the visited states, chunk by chunk; one thread sums each chunk in bar order ----
-    const double pen0 = mul_rn(phi, 0.0), pen1 = mul_rn(phi, 1.0), pen2 = mul_rn(phi, 2.0);       // market_env.py:57
+    const PenaltyTable pen = penalty_table(phi);
     int ntr = 0;
-    double total = 0.0;
+    double total = 0.0;                                     // thread 0 only (drl_engine.py:26)
     for (int64_t c0 = 0; c0 < T; c0 += SUM_CHUNK) {
         const int64_t c1 = c0 + SUM_CHUNK < T ? c0 + SUM_CHUNK : T;
-        const int64_t a = t_lo > c0 ? t_lo : c0, b = t_hi < c1 ? t_hi : c1;
+        const int64_t a = t_lo > c0 ? t_lo : c0, b = t_hi < c1 ? t_hi : c1;       // this thread's bars inside the chunk
         for (int64_t t = a; t < b; ++t) {
-            const AdvStep r = adv_step(st, code + t * 5, __ldg(reinterpret_cast<const int2*>(&sig[t].ka1)), at0, at1, at2);
+            const typename A::Step r = w.step(st, t);
             ntr += (r.fb || r.fs) ? 1 : 0;                                         // drl_engine.py:60-61
             double pnl = 0.0;                                                      // market_env.py:40
             if (r.fb || r.fs) {
                 const BarPx p = px[t];
-                const double my_ask = add_rn(p.ask, mul_rn((double)r.oa, tick));   // :30
-                const double my_bid = sub_rn(p.bid, mul_rn((double)r.ob, tick));   // :31
-                double leg_b = sub_rn(p.mid_next, my_bid), leg_s = sub_rn(my_ask, p.mid_next);
-                leg_b = sub_rn(leg_b, mul_rn(my_bid, fee));                        // :46,:48
-                leg_s = sub_rn(leg_s, mul_rn(my_ask, fee));                        // :52,:54
+                const int2 k = A::offsets(r);
+                const double my_ask = quote_ask(p.ask, k.x, tick), my_bid = quote_bid(p.bid, k.y, tick);         // :30-31
+                // fee terms evaluated as the reference does, fee_rate 0 included
+                const double leg_b = buy_leg(my_bid, p.mid_next, fee), leg_s = sell_leg(my_ask, p.mid_next, fee);
                 pnl = r.fb ? add_rn(pnl, leg_b) : pnl;
                 pnl = r.fs ? add_rn(pnl, leg_s) : pnl;
             }
-            const int niv = (int)(r.next % 5u);
-            const int ai = niv < 2 ? 2 - niv : niv - 2;
-            s_rew[t - c0] = sub_rn(pnl, ai == 0 ? pen0 : (ai == 1 ? pen1 : pen2));                 // :57-58
+            s_rew[t - c0] = sub_rn(pnl, penalty(pen, abs(A::inventory_index(r.next) - 2)));      // :57-58
             st = r.next;
         }
         __syncthreads();
@@ -399,8 +369,7 @@ __global__ void __launch_bounds__(WALK_THREADS, 1) walk_account_adv_kernel(const
     __syncthreads();
     if (tid == 0) {
         const int n = s_trades;
-        if (n == 0) total = sub_rn(total, 50.0);                                   // drl_engine.py:64-65
-        fitness[blockIdx.x] = total; trades[blockIdx.x] = n;
+        fitness[blockIdx.x] = episode_fitness(total, n); trades[blockIdx.x] = n;
     }
 }
 
@@ -444,9 +413,10 @@ int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8
     const int64_t T = b->T;
     int sms2 = 148;
     cudaDeviceGetAttribute(&sms2, cudaDevAttrMultiProcessorCount, b->device);
-    if (adv) walk_account_adv_kernel<512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, *adv, b->tick, phi, fee, fitness, trades);
-    else if (P <= sms2) walk_account_kernel<1024><<<(unsigned)P, 1024, 0, st>>>(b->px, T, code, next, b->tick, phi, fee, fitness, trades);
-    else walk_account_kernel<512><<<(unsigned)P, 512, 0, st>>>(b->px, T, code, next, b->tick, phi, fee, fitness, trades);
+    const PopArgs none = {};
+    if (adv) walk_account_kernel<Walk20, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, nullptr, *adv, b->tick, phi, fee, fitness, trades);
+    else if (P <= sms2) walk_account_kernel<Walk5, 1024><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, T, code, next, none, b->tick, phi, fee, fitness, trades);
+    else walk_account_kernel<Walk5, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, next, none, b->tick, phi, fee, fitness, trades);
     return check_cuda(cudaGetLastError(), "walk_account_kernel launch");
 }
 

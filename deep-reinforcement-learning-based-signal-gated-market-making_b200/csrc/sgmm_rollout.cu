@@ -215,7 +215,7 @@ rollout_kernel_h32(const RolloutArgs a)
         const int64_t indj = first + lane;
         const bool livej = lane < live_warps * NI && indj < a.mm.count;
         const double tick = a.tick, fee = a.fee;
-        const double pen0 = mul_rn(a.phi, 0.0), pen1 = mul_rn(a.phi, 1.0), pen2 = mul_rn(a.phi, 2.0);   // market_env.py:57
+        const PenaltyTable pen = penalty_table(a.phi);
         double total = 0.0;                                              // drl_engine.py:26
         int ntr = 0, inv = 0;                                            // market_env.py:17
         int64_t next_load = 0;
@@ -255,26 +255,17 @@ rollout_kernel_h32(const RolloutArgs a)
                     const double2 ab = *reinterpret_cast<const double2*>(&pxs[i].ask);
                     const double mid = pxs[i].mid_next;
                     if (!ADV) { ka = __float2int_rn(__int_as_float(ka)); kb = __float2int_rn(__int_as_float(kb)); }   // drl_engine.py:39
-                    const double my_ask = add_rn(ab.x, mul_rn((double)ka, tick));       // market_env.py:30
-                    const double my_bid = sub_rn(ab.y, mul_rn((double)kb, tick));       // :31
-                    double leg_b = sub_rn(mid, my_bid), leg_s = sub_rn(my_ask, mid);
-                    if (FEE) {
-                        leg_b = sub_rn(leg_b, mul_rn(my_bid, fee));                     // :46,:48
-                        leg_s = sub_rn(leg_s, mul_rn(my_ask, fee));                     // :52,:54
-                    }
+                    const double my_ask = quote_ask(ab.x, ka, tick), my_bid = quote_bid(ab.y, kb, tick);      // market_env.py:30-31
+                    const double leg_b = buy_leg<FEE>(my_bid, mid, fee), leg_s = sell_leg<FEE>(my_ask, mid, fee);
                     pnl = fb ? add_rn(pnl, leg_b) : pnl;
                     pnl = fs ? add_rn(pnl, leg_s) : pnl;
                 }
-                const double pen = ai == 0 ? pen0 : (ai == 1 ? pen1 : pen2);            // :57
-                total = add_rn(total, sub_rn(pnl, pen));                                // :58, drl_engine.py:54
+                total = add_rn(total, sub_rn(pnl, penalty(pen, ai)));                   // market_env.py:58, drl_engine.py:54
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(&sm.rec_empty[r]);
         }
-        if (livej) {
-            if (ntr == 0) total = sub_rn(total, 50.0);                                  // drl_engine.py:64-65
-            a.fitness[indj] = total; a.trades[indj] = ntr;
-        }
+        if (livej) { a.fitness[indj] = episode_fitness(total, ntr); a.trades[indj] = ntr; }
         return;
     }
     if (warp >= live_warps) return;
@@ -675,7 +666,7 @@ __global__ void __launch_bounds__(32, 1) trace_kernel_h32(const TraceArgs a)
             if (tr.unrealized_pnl) tr.unrealized_pnl[t] = unreal;
         }
     }
-    if (trades == 0) total = sub_rn(total, 50.0);
+    total = episode_fitness(total, trades);
     if (lane == 0) {
         if (a.fitness) *a.fitness = total;
         if (a.trades) *a.trades = trades;

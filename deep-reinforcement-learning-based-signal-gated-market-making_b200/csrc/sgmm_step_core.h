@@ -51,6 +51,35 @@ SGMM_HD double quote_bid(double best_bid, int64_t off_b, double tick) { return q
 SGMM_HD double quote_ask(double best_ask, int off_a, double tick) { return quote_ask(best_ask, (double)off_a, tick); }
 SGMM_HD double quote_bid(double best_bid, int off_b, double tick) { return quote_bid(best_bid, (double)off_b, tick); }
 
+// market_env.py:46,48 and :52,54 -- the P&L leg of one filled side at its quoted price, fee term included.  FEE = false
+// drops the fee term, for callers that have checked fee_rate == 0.
+template <bool FEE = true>
+SGMM_HD double buy_leg(double my_bid, double mid_next, double fee_rate)
+{
+    const double leg = sub_rn(mid_next, my_bid);
+    return FEE ? sub_rn(leg, mul_rn(my_bid, fee_rate)) : leg;
+}
+template <bool FEE = true>
+SGMM_HD double sell_leg(double my_ask, double mid_next, double fee_rate)
+{
+    const double leg = sub_rn(my_ask, mid_next);
+    return FEE ? sub_rn(leg, mul_rn(my_ask, fee_rate)) : leg;
+}
+
+// market_env.py:57 -- phi * |inventory| for the three values |inventory| takes in the reference's env (i_max = -i_min = 2)
+struct PenaltyTable { double p0, p1, p2; };
+SGMM_HD PenaltyTable penalty_table(double phi) { return {mul_rn(phi, 0.0), mul_rn(phi, 1.0), mul_rn(phi, 2.0)}; }
+// (The copies make the select one over values, which keeps the branch layout the hot loops were tuned with; nvcc lays out
+// a select over struct members differently.)
+SGMM_HD double penalty(const PenaltyTable& pen, int abs_inventory)
+{
+    const double p0 = pen.p0, p1 = pen.p1, p2 = pen.p2;
+    return abs_inventory == 0 ? p0 : (abs_inventory == 1 ? p1 : p2);
+}
+
+// drl_engine.py:64-65 -- an episode without a single trade loses 50
+SGMM_HD double episode_fitness(double total, int trades) { return trades == 0 ? sub_rn(total, 50.0) : total; }
+
 // market_env.py:22-67.  off_a/off_b already include the adversary's displacement (:25-28).  Off = int64_t or double.
 template <typename Off>
 SGMM_HD void env_step(sgmm_env_state& e, Off off_a, Off off_b,
@@ -68,14 +97,14 @@ SGMM_HD void env_step(sgmm_env_state& e, Off off_a, Off off_b,
         e.inventory += 1;
         const double fee = mul_rn(my_bid, e.fee_rate);
         e.cash = sub_rn(e.cash, add_rn(my_bid, fee));
-        pnl = add_rn(pnl, sub_rn(sub_rn(mid_next, my_bid), fee));
+        pnl = add_rn(pnl, buy_leg(my_bid, mid_next, e.fee_rate));
         fee_paid = add_rn(fee_paid, fee);
     }
     if (fill_sell) {                                               // :50-55
         e.inventory -= 1;
         const double fee = mul_rn(my_ask, e.fee_rate);
         e.cash = add_rn(e.cash, sub_rn(my_ask, fee));
-        pnl = add_rn(pnl, sub_rn(sub_rn(my_ask, mid_next), fee));
+        pnl = add_rn(pnl, sell_leg(my_ask, mid_next, e.fee_rate));
         fee_paid = add_rn(fee_paid, fee);
     }
     const int64_t ai = e.inventory < 0 ? -e.inventory : e.inventory;

@@ -443,17 +443,13 @@ __device__ __forceinline__ double int_to_double(int k)
     return __dadd_rn(__hiloint2double(0x43300000, k ^ (int)0x80000000), -4503601774854144.0);
 }
 
-// The P&L leg of one filled side, the slow way: literal market_env.py:30-31,46-48,52-54 for an offset outside the bar's
-// leg table (more than LEG_N - 1 ticks inside the fill threshold, or an always-filling bar).
+// The P&L leg of one filled side, the slow way: computed from the quote for an offset outside the bar's leg table (more
+// than LEG_N - 1 ticks inside the fill threshold, or an always-filling bar).
 __device__ __noinline__ double slow_leg(bool sell, const BarPx* px, int k, double tick, double fee)
 {
     const double best = sell ? px->ask : px->bid, mid = px->mid_next;
-    if (sell) {
-        const double my_ask = add_rn(best, mul_rn(int_to_double(k), tick));
-        return sub_rn(sub_rn(my_ask, mid), mul_rn(my_ask, fee));
-    }
-    const double my_bid = sub_rn(best, mul_rn(int_to_double(k), tick));
-    return sub_rn(sub_rn(mid, my_bid), mul_rn(my_bid, fee));
+    if (sell) return sell_leg(quote_ask(best, int_to_double(k), tick), mid, fee);
+    return buy_leg(quote_bid(best, int_to_double(k), tick), mid, fee);
 }
 
 // One 25-bar chunk of one individual's walk through the table.
@@ -855,13 +851,8 @@ __device__ __noinline__ void e3_role_plain(const Ctx& cx, uint32_t e3set)
                 // speculative env step of (bar t, inventory iv-2)  (market_env.py:30-58)
                 const bool fb = (inv < 2) && (kb < kth.y);                   // :34,:37
                 const bool fs = (inv > -2) && (ka < kth.x);                  // :35,:38
-                const double my_ask = add_rn(ab.x, mul_rn(int_to_double(ka), tick));
-                const double my_bid = sub_rn(ab.y, mul_rn(int_to_double(kb), tick));
-                double leg_b = sub_rn(mid, my_bid), leg_s = sub_rn(my_ask, mid);
-                if (FEE) {
-                    leg_b = sub_rn(leg_b, mul_rn(my_bid, fee));
-                    leg_s = sub_rn(leg_s, mul_rn(my_ask, fee));
-                }
+                const double leg_s = sell_leg<FEE>(quote_ask(ab.x, int_to_double(ka), tick), mid, fee);
+                const double leg_b = buy_leg<FEE>(quote_bid(ab.y, int_to_double(kb), tick), mid, fee);
                 double pnl = 0.0;
                 pnl = fb ? add_rn(pnl, leg_b) : pnl;
                 pnl = fs ? add_rn(pnl, leg_s) : pnl;
@@ -946,8 +937,7 @@ __device__ __noinline__ void walker_role_plain(const Ctx& cx)
     }
     if (live) {
         trades >>= 3;                                                  // walk_chunk_plain counts in units of 8
-        if (trades == 0) total = sub_rn(total, 50.0);                 // drl_engine.py:64-65
-        cx.fitness[ind] = total; cx.trades[ind] = trades;
+        cx.fitness[ind] = episode_fitness(total, trades); cx.trades[ind] = trades;
     }
 }
 
@@ -957,7 +947,7 @@ __device__ __noinline__ void walker_role_plain(const Ctx& cx)
 // leg table (market_env.py:30-31,44-55) and reward = pnl - phi*|inventory| (:57-58), stored as a double over the bar's
 // first row of the offset table (dead by now) for the walker's bar-order sum.
 template <bool ADV>
-__device__ __forceinline__ void account_chunk(const Ctx& cx, uint32_t c, const double (&pens)[3])
+__device__ __forceinline__ void account_chunk(const Ctx& cx, uint32_t c, const PenaltyTable& pen)
 {
     Smem& sm = *cx.sm;
     const uint32_t q = cx.gc + c, cbuf = q % 3u;
@@ -1007,9 +997,7 @@ __device__ __forceinline__ void account_chunk(const Ctx& cx, uint32_t c, const d
         }
         // pnl = 0.0 (+ leg_b) (+ leg_s) in the reference's order (:40,:48,:54); 0.0 + leg == leg (a leg is never -0.0)
         const double pnl = fb ? (fs ? add_rn(lb, ls) : lb) : ls;
-        const int ai = abs(niv - 2);
-        const double pen = ai == 0 ? pens[0] : (ai == 1 ? pens[1] : pens[2]);
-        *reinterpret_cast<double*>(&sm.tab_k[cbuf][g][s * 5]) = sub_rn(pnl, pen);      // :58
+        *reinterpret_cast<double*>(&sm.tab_k[cbuf][g][s * 5]) = sub_rn(pnl, penalty(pen, abs(niv - 2)));      // :58
     }
     __syncwarp();
     if (cx.lane == 0) mbar_arrive_a(BAR(rew_full, cbuf));
@@ -1044,7 +1032,7 @@ __device__ __noinline__ void e3_role(const Ctx& cx, uint32_t e3set)
     const int inv = iv - 2;
     const bool leader = lane == 0;
     const bool can_buy = inv < 2, can_sell = inv > -2;                          // market_env.py:34-35
-    const double pens[3] = {mul_rn(cx.phi, 0.0), mul_rn(cx.phi, 1.0), mul_rn(cx.phi, 2.0)};       // phi * |inventory|, market_env.py:57
+    const PenaltyTable pen = penalty_table(cx.phi);
     if (nchunks > 0) load_bar(0, kth_n);
 #pragma unroll 1
     for (uint32_t c = 0; c < nchunks; ++c) {
@@ -1052,7 +1040,7 @@ __device__ __noinline__ void e3_role(const Ctx& cx, uint32_t e3set)
         if (c + 1 < nchunks) load_bar(c + 1, kth_n);                            // prefetch the next chunk's thresholds
         uint32_t up = e3set >= base3 ? e3set - base3 : e3set + NBUF - base3;    // first unit of the chunk that is ours
         base3 += ug3; if (base3 >= NBUF) base3 -= NBUF;
-        if (up >= UG) { if (c >= 1) account_chunk<ADV>(cx, c - 1, pens); continue; }     // (groups of 2 or 4: not every chunk has a unit of ours)
+        if (up >= UG) { if (c >= 1) account_chunk<ADV>(cx, c - 1, pen); continue; }     // (groups of 2 or 4: not every chunk has a unit of ours)
         const uint32_t q = gc + c, cbuf = q % 3u;
         const bool valid = row_ok && ((int64_t)c * TILE_BARS + tl < T);
         mbar_wait_a_(cx, BAR(tab_empty, cbuf), ((q / 3u) & 1u) ^ 1u);                // walker has left this table buffer
@@ -1127,9 +1115,9 @@ __device__ __noinline__ void e3_role(const Ctx& cx, uint32_t e3set)
             if (leader) mbar_arrive_a(tab_full);
         }
         // the fp64 half of the PREVIOUS chunk's visited rows (the walker has marked them by now), all E3 warps
-        if (c >= 1) account_chunk<ADV>(cx, c - 1, pens);
+        if (c >= 1) account_chunk<ADV>(cx, c - 1, pen);
     }
-    if (nchunks >= 1) account_chunk<ADV>(cx, nchunks - 1, pens);
+    if (nchunks >= 1) account_chunk<ADV>(cx, nchunks - 1, pen);
     // pad units of the group (at most two, one per set): drain the accumulator so that the barrier phases stay in step
     for (uint32_t it = cx.nunits; it < cx.nunits_p; ++it) {
         if (it % NBUF != e3set) continue;
@@ -1199,10 +1187,7 @@ __device__ __noinline__ void walker_role(const Ctx& cx)
         if (c >= 1) sum_chunk(c - 1);
     }
     if (nchunks >= 1) sum_chunk(nchunks - 1);
-    if (live) {
-        if (trades == 0) total = sub_rn(total, 50.0);                 // drl_engine.py:64-65
-        cx.fitness[ind] = total; cx.trades[ind] = trades;
-    }
+    if (live) { cx.fitness[ind] = episode_fitness(total, trades); cx.trades[ind] = trades; }
 }
 
 template <bool ADV, bool FEE, int MODE>
@@ -1374,13 +1359,8 @@ __global__ void tc32_legs_kernel(int64_t T, const BarSig* __restrict__ sig, cons
         const long long k = (long long)k1 - 1 - j;
         if (k >= -(long long)K_CLAMP - 1 && k <= (long long)K_CLAMP + 1) {
             const BarPx p = px[t];
-            if (side == 0) {
-                const double my_ask = add_rn(p.ask, mul_rn(int_to_double((int)k), tick));          // market_env.py:30
-                leg = sub_rn(sub_rn(my_ask, p.mid_next), mul_rn(my_ask, fee));                     // :52,:54
-            } else {
-                const double my_bid = sub_rn(p.bid, mul_rn(int_to_double((int)k), tick));          // :31
-                leg = sub_rn(sub_rn(p.mid_next, my_bid), mul_rn(my_bid, fee));                     // :46,:48
-            }
+            if (side == 0) leg = sell_leg(quote_ask(p.ask, int_to_double((int)k), tick), p.mid_next, fee);
+            else leg = buy_leg(quote_bid(p.bid, int_to_double((int)k), tick), p.mid_next, fee);
         }
     }
     (side == 0 ? legs[t].leg_s : legs[t].leg_b)[j] = leg;
