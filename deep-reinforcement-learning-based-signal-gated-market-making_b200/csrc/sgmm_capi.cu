@@ -59,6 +59,8 @@ int launch_population(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* ad
     if (precision == SGMM_PRECISION_EXACT && hidden == 32) precision = SGMM_PRECISION_F32;     // EXACT at H = 32 is the F32 route
     if (hidden == 256 && precision == SGMM_PRECISION_EXACT)         // bit-exact H = 256: policy tables + walks, in batches
         return launch_exact256(b, mm, adv, phi, fee, fitness, trades, st);
+    if (hidden == 256 && adv && precision == SGMM_PRECISION_BF16)   // spec256 q tables + walk_account_kernel<Walk20>, in batches
+        return launch_spec256_adv(b, mm, *adv, phi, fee, fitness, trades, nullptr, nullptr, st);
     if (hidden == 256)                                              // BASELINE config 4: spec256_kernel + account_kernel
         return launch_spec256(b, mm, phi, fee, fitness, trades, nullptr, nullptr, st);
     if (precision != SGMM_PRECISION_F32)                            // tensor cores at H = 32
@@ -213,7 +215,6 @@ static int check_rollout_args(const sgmm_bundle* bundle, const sgmm_population* 
     if (params->precision != SGMM_PRECISION_F32 && params->precision != SGMM_PRECISION_BF16 && params->precision != SGMM_PRECISION_TF32 && params->precision != SGMM_PRECISION_F16 && params->precision != SGMM_PRECISION_EXACT) { set_error("unknown precision %d", params->precision); return SGMM_ERR_INVALID; }
     if (mm->hidden == 256) {
         if (params->precision != SGMM_PRECISION_BF16 && params->precision != SGMM_PRECISION_EXACT) { set_error("hidden=256: pass precision=SGMM_PRECISION_EXACT (bit-exact SGMM-F32 order) or SGMM_PRECISION_BF16 (tensor cores); F32 and TF32 are H=32 paths"); return SGMM_ERR_UNSUPPORTED; }
-        if (adv && params->precision != SGMM_PRECISION_EXACT) { set_error("the H=256 tensor-core rollout has no adversary path (SGMM_PRECISION_EXACT has one)"); return SGMM_ERR_UNSUPPORTED; }
     } else if (mm->hidden == 32) {
     } else if (params->precision != SGMM_PRECISION_F32) { set_error("precision %d needs hidden=32 or hidden=256 (EXACT, BF16) or hidden=32 (TF32, F16)", params->precision); return SGMM_ERR_UNSUPPORTED; }
     if (adv && adv->count != mm->count) { set_error("adv.count (%lld) != mm.count (%lld): MM i meets adversary i (Env/drl_engine.py:115)", (long long)adv->count, (long long)mm->count); return SGMM_ERR_INVALID; }
@@ -246,6 +247,8 @@ int sgmm_rollout_tc_audit(const sgmm_bundle* bundle, const sgmm_population* mm, 
     if (mm->hidden == 32)
         return launch_tc32(bundle, pm, adv ? &pa : nullptr, params->phi, params->fee_rate, params->units_per_lane, fitness, trades, raw_table,
                            act_trace, (cudaStream_t)stream, tc32_mode_of(params->precision));
+    if (adv)
+        return launch_spec256_adv(bundle, pm, pa, params->phi, params->fee_rate, fitness, trades, raw_table, act_trace, (cudaStream_t)stream);
     return launch_spec256(bundle, pm, params->phi, params->fee_rate, fitness, trades, raw_table, act_trace, (cudaStream_t)stream);
 }
 

@@ -277,6 +277,17 @@ bool needs_stage(const PopArgs& mm) { return mm.genomes == nullptr || (reinterpr
 
 }  // namespace x256
 
+int reserve_batches(const sgmm_bundle* b, int64_t P, int64_t per_ind, cudaStream_t st, int64_t* nb, uint64_t** buf)
+{
+    const int64_t T = b->T;
+    int64_t n = x256::batch_bytes() / (per_ind * 8 > 0 ? per_ind * 8 : 1);
+    if (n < 1) n = 1;
+    if (n > P) n = P;
+    *nb = n;
+    const int64_t units = T > 0 ? (n * per_ind + T - 1) / T + 1 : 1;           // reserve_codes counts in units of T words
+    return reserve_codes(b, units, st, buf);
+}
+
 // Episodes at H = 256 in SGMM-F32 order (with or without the adversary): batches of individuals, each batch = (staged
 // genomes,) policy table, walk.  The table ([n][T] x 48 B) and the staged genomes ([n] x 269 KB; seeded children, or
 // explicit rows not 8-byte aligned) live in the bundle's grow-only code buffer (sgmm_account.cu), under the byte budget of
@@ -289,35 +300,21 @@ int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv,
     const int64_t T = b->T, P = mm.count;
     if (P == 0) return SGMM_OK;
     const bool stage = T > 0 && needs_stage(mm);
-    const int64_t per_ind = 6 * T + (stage ? G / 2 : 0);                       // 8-byte words per individual
-    int64_t nb = batch_bytes() / (per_ind * 8 > 0 ? per_ind * 8 : 1);
-    if (nb < 1) nb = 1;
-    if (nb > P) nb = P;
+    int64_t nb = 0;
     uint64_t* buf = nullptr;
-    const int64_t units = T > 0 ? (nb * per_ind + T - 1) / T + 1 : 1;          // reserve_codes counts in units of T words
-    if (int rc = reserve_codes(b, units, st, &buf)) return rc;
+    if (int rc = reserve_batches(b, P, 6 * T + (stage ? G / 2 : 0), st, &nb, &buf)) return rc;
     float2* code = reinterpret_cast<float2*>(buf);
     uint8_t* next = reinterpret_cast<uint8_t*>(code + nb * T * 5);
     float* staged = reinterpret_cast<float*>(buf + nb * T * 6);
-    for (int64_t b0 = 0; b0 < P; b0 += nb) {
-        const int64_t n = P - b0 < nb ? P - b0 : nb;
-        PopArgs pm = mm;
-        if (pm.genomes) pm.genomes += b0 * G; else pm.first_index += b0;
-        pm.count = n;
+    const int rc = walk_batches(b, mm, adv, nb, code, next, phi, fee, fitness, trades, st, [&](const PopArgs& pm, const PopArgs*, int64_t) {
         const float* rows = pm.genomes;
         if (stage) {
-            if (int rc = launch_stage(b, pm, n, staged, st)) return rc;
+            if (int rc = launch_stage(b, pm, pm.count, staged, st)) return rc;
             rows = staged;
         }
-        if (int rc = launch_table(b, rows, n, adv ? 1 : 0, code, next, st)) return rc;
-        PopArgs pa{};
-        if (adv) {
-            pa = *adv;
-            if (pa.genomes) pa.genomes += b0 * 1250; else pa.first_index += b0;
-            pa.count = n;
-        }
-        if (int rc = launch_walk(b, n, code, next, adv ? &pa : nullptr, phi, fee, fitness + b0, trades + b0, st)) return rc;
-    }
+        return launch_table(b, rows, pm.count, adv ? 1 : 0, code, next, st);
+    });
+    if (rc) return rc;
     return release_codes(b, st);
 }
 

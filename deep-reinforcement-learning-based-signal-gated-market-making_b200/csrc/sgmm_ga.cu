@@ -168,7 +168,7 @@ int sgmm_ga_create(sgmm_ga** out, const sgmm_ga_config* cfg, const float* mm_mas
     if (cfg->hidden != 32 && cfg->hidden != 256) { set_error("hidden=%d: GA rollouts are built for H=32 and H=256", cfg->hidden); return SGMM_ERR_UNSUPPORTED; }
     if (cfg->hidden == 256 && cfg->precision == SGMM_PRECISION_F32) { set_error("hidden=256: pass precision=SGMM_PRECISION_EXACT (bit-exact SGMM-F32 order) or SGMM_PRECISION_BF16 (tensor cores)"); return SGMM_ERR_UNSUPPORTED; }
     if (cfg->precision != SGMM_PRECISION_F32 && cfg->precision != SGMM_PRECISION_BF16 && cfg->precision != SGMM_PRECISION_TF32 && cfg->precision != SGMM_PRECISION_F16 && cfg->precision != SGMM_PRECISION_EXACT) { set_error("unknown precision %d", cfg->precision); return SGMM_ERR_INVALID; }
-    if (cfg->hidden == 256 && cfg->use_arl && cfg->precision != SGMM_PRECISION_EXACT) { set_error("the H=256 tensor-core rollout has no adversary path (SGMM_PRECISION_EXACT has one)"); return SGMM_ERR_UNSUPPORTED; }
+    if (cfg->hidden == 256 && cfg->use_arl && cfg->precision != SGMM_PRECISION_EXACT && cfg->precision != SGMM_PRECISION_BF16) { set_error("use_arl at hidden=256: pass precision=SGMM_PRECISION_BF16 (tensor cores) or SGMM_PRECISION_EXACT"); return SGMM_ERR_UNSUPPORTED; }
     if (cfg->pop_size <= 0 || cfg->shard_first < 0 || cfg->shard_count < 0 ||
         cfg->shard_first + cfg->shard_count > cfg->pop_size) { set_error("bad population / shard bounds"); return SGMM_ERR_INVALID; }
     const int64_t stride = cfg->shard_stride > 0 ? cfg->shard_stride : cfg->pop_size;

@@ -99,6 +99,8 @@ struct RolloutArgs {
 void set_error(const char* fmt, ...);
 int check_cuda(cudaError_t e, const char* what);
 
+inline int64_t genome_len(int H) { return (int64_t)H * H + 7 * (int64_t)H + 2; }
+
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a PER-DEVICE attribute of a kernel: opt in once per (kernel, device).
 // `mask` is one static word per kernel instantiation, bit d = configured on device d (the calling thread's current
 // device).  Devices >= 64 simply re-apply the attribute on every launch.  Safe from concurrent host threads: a lost
@@ -126,6 +128,35 @@ int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs*
 // the walk + fp64 half of the policy-table path over tables code [P][T][5] / next [P][T][8] (sgmm_one.cu)
 int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const PopArgs* adv, double phi, double fee,
                 double* fitness, int32_t* trades, cudaStream_t st);
+// the market maker's offsets before the adversary's displacement along the Walk20 walk of q tables [P][T][5] (audit, sgmm_one.cu)
+int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, const PopArgs& adv, int32_t* act_trace, cudaStream_t st);
+// H = 256 populations as batches of policy table + walk (sgmm_exact256.cu, and sgmm_spec256.cu with the adversary).  The
+// scratch of a batch, `per_ind` 8-byte words per individual, is the bundle's code buffer (ordered rollouts per bundle; the
+// first rollout of a size must not run under a stream capture) and stays under the byte budget SGMM_EXACT256_BATCH_BYTES
+// (environment, read on every call; default 2 GiB): *nb individuals per batch.
+int reserve_batches(const sgmm_bundle* b, int64_t P, int64_t per_ind, cudaStream_t st, int64_t* nb, uint64_t** buf);
+// Batches of at most nb individuals: table(pm, pa, b0) enqueues the policy table (code / next) of individuals b0 .. b0+n-1,
+// pm / pa being those individuals of mm / adv (pa nullptr without the adversary); the walk then writes their fitness / trades.
+template <class Table>
+int walk_batches(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int64_t nb, const float2* code, const uint8_t* next,
+                 double phi, double fee, double* fitness, int32_t* trades, cudaStream_t st, Table table)
+{
+    for (int64_t b0 = 0; b0 < mm.count; b0 += nb) {
+        const int64_t n = mm.count - b0 < nb ? mm.count - b0 : nb;
+        PopArgs pm = mm;
+        if (pm.genomes) pm.genomes += b0 * genome_len(256); else pm.first_index += b0;
+        pm.count = n;
+        PopArgs pa{};
+        if (adv) {
+            pa = *adv;
+            if (pa.genomes) pa.genomes += b0 * 1250; else pa.first_index += b0;
+            pa.count = n;
+        }
+        if (int rc = table(pm, adv ? &pa : nullptr, b0)) return rc;
+        if (int rc = launch_walk(b, n, code, next, adv ? &pa : nullptr, phi, fee, fitness + b0, trades + b0, st)) return rc;
+    }
+    return SGMM_OK;
+}
 // bit-exact H = 256 (sgmm_exact256.cu): batches of policy table + walk; and the raw-output table of one genome for the trace
 int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
                     cudaStream_t st);
@@ -135,6 +166,9 @@ int launch_trace(const sgmm_bundle* b, const float* mm_genome, int hidden, const
                  double* fitness, int32_t* trades, cudaStream_t st);
 int launch_spec256(const sgmm_bundle* b, const PopArgs& mm, double phi, double fee, double* fitness, int32_t* trades,
                    float* raw_table, int32_t* act_trace, cudaStream_t st);
+// H = 256 on the tensor cores with the adversary: spec256 q tables walked by walk_account_kernel<Walk20>, in batches
+int launch_spec256_adv(const sgmm_bundle* b, const PopArgs& mm, const PopArgs& adv, double phi, double fee, double* fitness,
+                       int32_t* trades, float* raw_table, int32_t* act_trace, cudaStream_t st);
 int launch_tc32(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, int group, double* fitness, int32_t* trades,
                 float* raw_table, int32_t* act_trace, cudaStream_t st, int mode = 0);   // mode: 0 bf16, 1 tf32, 2 f16
 // the rollout of a population on the kernel that serves (hidden, precision, adversary) (sgmm_capi.cu); units_per_lane is
@@ -155,7 +189,5 @@ int launch_bundle_windows(int64_t E, const double* ask1, const double* bid1, con
                           double* buy_max, double* sell_min, cudaStream_t st);
 int launch_analytics(int64_t B, int64_t T, const double* wealth, const double* cash, const double* mid,
                      const int32_t* inventory, const uint8_t* is_trade, double* scratch, double* out, cudaStream_t st);
-
-inline int64_t genome_len(int H) { return (int64_t)H * H + 7 * (int64_t)H + 2; }
 
 }  // namespace sgmm

@@ -233,6 +233,8 @@ __device__ __forceinline__ Map20 m20_shfl_up(const Map20& m, int d)
     return o;
 }
 
+// the market maker's offset of one side, before the adversary's displacement (drl_engine.py:39, clamped to +-K_CLAMP)
+__device__ __forceinline__ int mm_offset(float q) { return max(min(__float2int_rn(q), K_CLAMP), -K_CLAMP); }
 // one bar's step from state st: displaced offsets, fills against the integer thresholds, next state
 struct AdvStep { int oa, ob; bool fb, fs; uint32_t next; };
 __device__ __forceinline__ AdvStep adv_step(uint32_t st, const float2* __restrict__ code_t, int2 k1, uint32_t at0, uint32_t at1, uint32_t at2)
@@ -241,8 +243,8 @@ __device__ __forceinline__ AdvStep adv_step(uint32_t st, const float2* __restric
     const float2 q = code_t[iv];
     const uint32_t e = table_lookup(at0, at1, at2, (int)st);
     AdvStep r;
-    r.oa = max(min(__float2int_rn(q.x), K_CLAMP), -K_CLAMP) + (int)(e & 3u) - 1;          // drl_engine.py:39, market_env.py:26-28
-    r.ob = max(min(__float2int_rn(q.y), K_CLAMP), -K_CLAMP) + (int)(e >> 2) - 1;
+    r.oa = mm_offset(q.x) + (int)(e & 3u) - 1;                                              // market_env.py:26-28
+    r.ob = mm_offset(q.y) + (int)(e >> 2) - 1;
     r.fb = (iv < 4u) && (r.ob < k1.y);                                                     // :34,:37
     r.fs = (iv > 0u) && (r.oa < k1.x);                                                     // :35,:38
     r.next = (r.fs ? 10u : 0u) + (r.fb ? 5u : 0u) + iv + (r.fb ? 1u : 0u) - (r.fs ? 1u : 0u);
@@ -252,6 +254,21 @@ template <int S = 0>
 __device__ __forceinline__ void bar_map_rec(Map20& m, const float2* __restrict__ code_t, int2 k1, uint32_t at0, uint32_t at1, uint32_t at2)
 {
     if constexpr (S < 20) { m20_set<S>(m, adv_step((uint32_t)S, code_t, k1, at0, at1, at2).next); bar_map_rec<S + 1>(m, code_t, k1, at0, at1, at2); }
+}
+
+// the individual's adversary as its displacement table (sgmm_adversary.cuh), built in s_adv[3] (shared memory) by the
+// first 20 threads; every thread of the block calls it
+__device__ __forceinline__ void build_adv_table(const PopArgs& adv_in, int64_t ind, uint32_t* s_adv)
+{
+    const int tid = threadIdx.x;
+    if (tid < 3) s_adv[tid] = 0u;
+    __syncthreads();
+    if (tid < 20) {
+        const PopArgs advp = resolve(adv_in);
+        const uint32_t e = adversary_entry(make_source(advp, ind, (int64_t)1250), tid);
+        atomicOr(&s_adv[tid >> 3], e << ((tid & 7) * 4));
+    }
+    __syncthreads();
 }
 
 struct Walk20 {
@@ -265,15 +282,7 @@ struct Walk20 {
         : sig(sig_), code(code_all + ind * T * 5)
     {
         __shared__ uint32_t s_adv[3];
-        const int tid = threadIdx.x;
-        if (tid < 3) s_adv[tid] = 0u;
-        __syncthreads();
-        if (tid < 20) {                                     // the individual's adversary as its displacement table
-            const PopArgs advp = resolve(adv_in);
-            const uint32_t e = adversary_entry(make_source(advp, ind, (int64_t)1250), tid);
-            atomicOr(&s_adv[tid >> 3], e << ((tid & 7) * 4));
-        }
-        __syncthreads();
+        build_adv_table(adv_in, ind, s_adv);
         at0 = s_adv[0]; at1 = s_adv[1]; at2 = s_adv[2];
     }
     __device__ static Map identity() { return m20_identity(); }
@@ -373,6 +382,24 @@ walk_account_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px
     }
 }
 
+// Audit of a walk over q tables: the market maker's offsets before the displacement at the state walk_account_kernel<Walk20>
+// visits, bar after bar on one thread (the offsets tests replay through the oracle; not a hot path).  One CTA per individual.
+__global__ void __launch_bounds__(32) adv_offsets_kernel(const BarSig* __restrict__ sig, int64_t T, const float2* __restrict__ code_all,
+                                                         const PopArgs adv, int32_t* __restrict__ act_trace)
+{
+    __shared__ uint32_t s_adv[3];                           // its own: sharing Walk20's static table would move walk_account_kernel's shared layout
+    build_adv_table(adv, blockIdx.x, s_adv);
+    if (threadIdx.x != 0) return;
+    const float2* code = code_all + (int64_t)blockIdx.x * T * 5;
+    int32_t* act = act_trace + (int64_t)blockIdx.x * T * 2;
+    uint32_t st = 2u;                                       // flat, no previous fills
+    for (int64_t t = 0; t < T; ++t) {
+        const float2 q = code[t * 5 + st % 5u];
+        act[2 * t] = mm_offset(q.x); act[2 * t + 1] = mm_offset(q.y);
+        st = adv_step(st, code + t * 5, __ldg(reinterpret_cast<const int2*>(&sig[t].ka1)), s_adv[0], s_adv[1], s_adv[2]).next;
+    }
+}
+
 }  // namespace one
 
 // Episodes of a small population on `b` (H = 32, exact SGMM-F32 order, with or without the adversary) through the kernels above.  The
@@ -418,6 +445,13 @@ int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8
     else if (P <= sms2) walk_account_kernel<Walk5, 1024><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, T, code, next, none, b->tick, phi, fee, fitness, trades);
     else walk_account_kernel<Walk5, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, next, none, b->tick, phi, fee, fitness, trades);
     return check_cuda(cudaGetLastError(), "walk_account_kernel launch");
+}
+
+int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, const PopArgs& adv, int32_t* act_trace, cudaStream_t st)
+{
+    if (P == 0) return SGMM_OK;
+    one::adv_offsets_kernel<<<(unsigned)P, 32, 0, st>>>(b->sig, b->T, code, adv, act_trace);
+    return check_cuda(cudaGetLastError(), "adv_offsets_kernel launch");
 }
 
 }  // namespace sgmm

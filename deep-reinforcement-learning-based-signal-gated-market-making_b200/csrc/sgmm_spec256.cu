@@ -32,6 +32,10 @@
 //                         reference order), trades; fitness / trade count out (Env/drl_engine.py:54-67)
 // W2 (f16, 128 KB, swizzled K-major B operand) stays resident in shared memory for the episode.
 //
+// With the adversary (q-table mode, QTAB = true) the next state of a bar depends on the previous bar's fills as well, a
+// 20-state automaton (sgmm_one.cu, Walk20): E3 writes q = raw*5 of every (bar, inventory) row to global memory instead
+// of step codes, the walker warp idles, and walk_account_kernel<Walk20> walks the table afterwards (launch_spec256_adv).
+//
 // Precision: h1, W2 and the layer-2 accumulator are f16 (11 significand bits), the output layer accumulates in fp32;
 // tests/test_gpu_spec256.py states the tolerance against the fp32 oracle (0.05 tick; measured 0.008), checks that no
 // rounding flips where the oracle's margin exceeds it, and checks that GIVEN the kernel's actions
@@ -267,9 +271,10 @@ struct Args {
     double* fitness; int32_t* trades;
     float* raw_table;        // optional audit output [P][T][5][2]
     int32_t* act_trace;      // optional audit output [P][T][2] : actions actually taken
+    float2* qtab;            // q-table mode: q = raw*5 of every (bar, inventory) [P][T][5] (Walk20's table)
 };
 
-template <bool FEE>
+template <bool FEE, bool QTAB = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1) spec256_kernel(const Args a)
 {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -406,7 +411,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) spec256_kernel(const Args a)
                 const bool valid = (row < TILE_BARS * 5) && (t < T);
                 const int64_t tc_ = valid ? t : 0;
                 int2 kth = make_int2(0, 0);
-                if (T > 0) kth = __ldg(reinterpret_cast<const int2*>(&a.sig[tc_].ka1));
+                if (!QTAB && T > 0) kth = __ldg(reinterpret_cast<const int2*>(&a.sig[tc_].ka1));
                 mbar_wait(&sm.l3_done[buf], use & 1u);
                 tc_fence_after();
                 if (warp == 0) TR(5);
@@ -424,19 +429,25 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) spec256_kernel(const Args a)
                 // speculative env step of (bar t, inventory iv-2)  (market_env.py:30-58)
                 uint64_t code = 0; uint32_t nxt = (uint32_t)iv;
                 if (valid) {
-                    // the INTEGER half of the env step (market_env.py:34-38, 45, 51); quotes, P&L and the penalty are
-                    // fp64 and belong to the accounting pass
-                    const int inv = iv - 2;
-                    const bool fb = (inv < 2) && (kb < kth.y);               // :34,:37
-                    const bool fs = (inv > -2) && (ka < kth.x);              // :35,:38
-                    const int ninv = inv + (fb ? 1 : 0) - (fs ? 1 : 0);
-                    code = (uint64_t)(uint32_t)(fs ? ka : SGMM_CODE_NOFILL) | ((uint64_t)(uint32_t)(fb ? kb : SGMM_CODE_NOFILL) << 32);
-                    nxt = (uint32_t)(ninv + 2) | ((fb || fs) ? 8u : 0u);
+                    if constexpr (QTAB) {
+                        // the row's q, as fl(raw*5) above; the 125 rows of a tile are contiguous: coalesced stores
+                        a.qtab[((int64_t)ind * T + t) * 5 + iv] = make_float2(__fmul_rn(ra, 5.0f), __fmul_rn(rb, 5.0f));
+                    } else {
+                        // the INTEGER half of the env step (market_env.py:34-38, 45, 51); quotes, P&L and the penalty are
+                        // fp64 and belong to the accounting pass
+                        const int inv = iv - 2;
+                        const bool fb = (inv < 2) && (kb < kth.y);               // :34,:37
+                        const bool fs = (inv > -2) && (ka < kth.x);              // :35,:38
+                        const int ninv = inv + (fb ? 1 : 0) - (fs ? 1 : 0);
+                        code = (uint64_t)(uint32_t)(fs ? ka : SGMM_CODE_NOFILL) | ((uint64_t)(uint32_t)(fb ? kb : SGMM_CODE_NOFILL) << 32);
+                        nxt = (uint32_t)(ninv + 2) | ((fb || fs) ? 8u : 0u);
+                    }
                     if (a.raw_table) {
                         float* o = a.raw_table + (((int64_t)ind * T + t) * 5 + iv) * 2;
                         o[0] = ra; o[1] = rb;
                     }
                 }
+                if constexpr (QTAB) return;                // no tile table: t_full / t_empty stay untouched in this mode
                 // publish the tile's table
                 if (warp == 0) TR(13);
                 mbar_wait(&sm.t_empty[buf], (use & 1u) ^ 1u);
@@ -588,8 +599,8 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) spec256_kernel(const Args a)
             }
             if (ntiles > 0) issue_l3(ntiles - 1);
         } else {
-            // =========================== WALKER ================================================
-            if (lane == 0) {
+            // =========================== WALKER (idle in q-table mode) ==========================
+            if (!QTAB && lane == 0) {
                 int iv = 2;                                                   // inventory 0
                 uint64_t* codes = a.codes + (int64_t)ind * T;
                 for (int64_t it = 0; it < ntiles; ++it) {
@@ -638,6 +649,20 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) spec256_kernel(const Args a)
     }
 }
 
+// one persistent CTA per SM, at most one per individual
+template <bool FEE, bool QTAB>
+int launch_kernel(const sgmm_bundle* b, const Args& a, cudaStream_t st)
+{
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
+    const int grid = (int)(a.mm.count < sms ? a.mm.count : sms);
+    const size_t smem = sizeof(Smem) + 1024;
+    static std::atomic<uint64_t> configured{0};       // per instantiation, one bit per device
+    if (int rc = opt_in_smem(spec256_kernel<FEE, QTAB>, smem, configured, "cudaFuncSetAttribute(spec256 smem)")) return rc;
+    spec256_kernel<FEE, QTAB><<<grid, NUM_THREADS, smem, st>>>(a);
+    return check_cuda(cudaGetLastError(), "spec256_kernel launch");
+}
+
 }  // namespace s256
 
 int launch_spec256(const sgmm_bundle* b, const PopArgs& mm, double phi, double fee, double* fitness, int32_t* trades,
@@ -645,21 +670,39 @@ int launch_spec256(const sgmm_bundle* b, const PopArgs& mm, double phi, double f
 {
     using namespace s256;
     if (mm.count == 0) return SGMM_OK;
-    Args a;
+    Args a{};
     a.sig = b->sig; a.px = b->px; a.T = b->T; a.tick = b->tick; a.phi = phi; a.fee = fee;
     a.mm = mm; a.fitness = fitness; a.trades = trades; a.raw_table = raw_table; a.act_trace = act_trace;
     if (int rc = reserve_codes(b, mm.count, st, &a.codes)) return rc;
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
-    const int grid = (int)(mm.count < sms ? mm.count : sms);
-    const size_t smem = sizeof(Smem) + 1024;
-    static std::atomic<uint64_t> configured[2];       // per variant, one bit per device (zero-initialised)
-    const bool has_fee = fee != 0.0;
-    auto kern = has_fee ? spec256_kernel<true> : spec256_kernel<false>;
-    if (int rc = opt_in_smem(kern, smem, configured[has_fee], "cudaFuncSetAttribute(spec256 smem)")) return rc;
-    kern<<<grid, NUM_THREADS, smem, st>>>(a);
-    if (int rc = check_cuda(cudaGetLastError(), "spec256_kernel launch")) return rc;
+    if (int rc = fee != 0.0 ? launch_kernel<true, false>(b, a, st) : launch_kernel<false, false>(b, a, st)) return rc;
     if (int rc = launch_account(b, a.codes, mm.count, phi, fee, fitness, trades, st)) return rc;   // the fp64 half, after the tensor-core kernel
+    return release_codes(b, st);
+}
+
+// With the adversary: batches of (spec256_kernel<false, true> -> q table [n][T][5], 40 B per individual and bar, in the
+// bundle's code buffer under the budget of batch_bytes(); walk_account_kernel<Walk20> over it).  Seeded children need no
+// staging: the kernel regenerates them.  Audit: raw_table comes from the same kernel, act_trace (the market maker's offsets
+// before the displacement) from a replay of the walk over the table (launch_adv_offsets).
+int launch_spec256_adv(const sgmm_bundle* b, const PopArgs& mm, const PopArgs& adv, double phi, double fee, double* fitness,
+                       int32_t* trades, float* raw_table, int32_t* act_trace, cudaStream_t st)
+{
+    using namespace s256;
+    const int64_t T = b->T;
+    if (mm.count == 0) return SGMM_OK;
+    int64_t nb = 0;
+    uint64_t* buf = nullptr;
+    if (int rc = reserve_batches(b, mm.count, 5 * T, st, &nb, &buf)) return rc;
+    float2* q = reinterpret_cast<float2*>(buf);
+    Args a{};
+    a.sig = b->sig; a.px = b->px; a.T = T; a.tick = b->tick; a.phi = phi; a.fee = fee; a.qtab = q;
+    const int rc = walk_batches(b, mm, &adv, nb, q, nullptr, phi, fee, fitness, trades, st,
+                                [&](const PopArgs& pm, const PopArgs* pa, int64_t b0) {
+        a.mm = pm;
+        a.raw_table = raw_table ? raw_table + b0 * T * 10 : nullptr;
+        if (int rc = launch_kernel<false, true>(b, a, st)) return rc;      // FEE is not read by the kernel body
+        return act_trace ? launch_adv_offsets(b, pm.count, q, *pa, act_trace + b0 * T * 2, st) : SGMM_OK;
+    });
+    if (rc) return rc;
     return release_codes(b, st);
 }
 

@@ -201,14 +201,14 @@ def rollout_seeded(bundle: Bundle, master, *, count, sigma, seed, generation, fi
     return fit, trd
 
 
-TC_ADVERSARY = True          # the H=32 tensor-core rollout carries the adversary (sgmm_tc32.cu, 20-state automaton)
+TC_ADVERSARY = True          # the tensor-core rollouts carry the adversary (20-state automaton; H=256: q tables + walk)
 
 
 def rollout_tc_audit(bundle: Bundle, genomes, adv_genomes=None, *, phi, fee_rate=0.0, hidden=32, group=0, precision="bf16"):
     """Tensor-core rollout (hidden=32: sgmm_tc32.cu, hidden=256: sgmm_spec256.cu) with its audit
     outputs: returns ``(fitness, trades, raw_table float32[P,T,5,2], act_trace int32[P,T,2])`` as
     CUDA tensors -- the policy outputs for every (bar, inventory) and the offsets actually taken (the market maker's,
-    before the adversary's displacement when ``adv_genomes`` is given; hidden=32 only)."""
+    before the adversary's displacement when ``adv_genomes`` is given, at hidden 32 and 256)."""
     g = _as_f32_matrix(genomes, genome_len(hidden)).to(f"cuda:{bundle.device}")
     P, T = g.shape[0], bundle.T
     fit = torch.empty(P, dtype=torch.float64, device=g.device)
@@ -456,8 +456,8 @@ class DRLEngine:
       reference's unseeded ``torch.randn``, models/model.py:69; an integer = reproducible, with the ``train`` call count
       folded in), ``device``, ``patience`` (15, :155), ``hidden_dim`` (32 or 256, models/model.py:7), ``precision``
       (``None`` / "f32": bit-exact population evaluation at hidden 32; "tf32" / "f16" / "bf16": tensor-core rollout;
-      ``None`` at hidden 256 runs the tensor-core path, "exact" runs population, validation and adversary bit-exact at
-      hidden 32 and 256).
+      ``None`` at hidden 256 runs the tensor-core path, with ``use_arl`` too; "exact" runs population, validation and
+      adversary bit-exact at hidden 32 and 256).
     * When ``torch.distributed`` is initialised with more than one rank, ``train`` shards the population over the ranks
       (:class:`dist.ShardedGA`: one NCCL all-gather of fitness + trades per generation) -- the multi-GPU replacement of
       the ``Pool(8).starmap`` of drl_engine.py:91,115.  Every rank returns the identical policy and history; rank 0

@@ -43,7 +43,8 @@ extern "C" {
 /* precision of the policy MLP */
 #define SGMM_PRECISION_F32   0      /* SGMM-F32 order on CUDA cores: bit-identical to the oracle (H=32) */
                                     /* The adversary (adv != NULL) runs on every H=32 path, tensor-core ones  */
-                                    /* included (a 20-state automaton instead of a 5-state one).              */
+                                    /* included (a 20-state automaton instead of a 5-state one), and at H=256 */
+                                    /* with BF16 and EXACT.                                                    */
 #define SGMM_PRECISION_BF16  1      /* policy layers on tcgen05 tensor cores, bf16 x bf16 -> fp32 in  */
                                     /* TMEM, all 5 inventories of every bar evaluated at once:        */
                                     /*   H=32  all three layers as GEMMs chained through TMEM         */
@@ -51,6 +52,10 @@ extern "C" {
                                     /*         CTA group, even, 0 = auto)                             */
                                     /*   H=256 hidden and output layer (sgmm_spec256.cu: f16 operands,*/
                                     /*         f16 layer-2 accumulator, whatever tensor mode is asked)*/
+                                    /*         With an adversary the kernel writes q = raw*5 of every */
+                                    /*         (bar, inventory) and the 20-state walk of the exact    */
+                                    /*         path runs over it, in batches of 40 B per individual   */
+                                    /*         and bar under SGMM_EXACT256_BATCH_BYTES (see EXACT)    */
                                     /* policy outputs within a stated tolerance of the fp32 oracle;   */
                                     /* the env step given the offsets stays bit-exact                 */
 
@@ -182,9 +187,10 @@ int sgmm_rollout_wait(const sgmm_bundle* bundle, int32_t ticket);
 int sgmm_rollout_spec256_audit(const sgmm_bundle* bundle, const sgmm_population* mm,
                                const sgmm_rollout_params* params, double* fitness, int32_t* trades,
                                float* raw_table, int32_t* act_trace, void* stream);
-/* The same with an adversary population (hidden = 32 only; adv may be NULL): act_trace holds the market maker's offsets
+/* The same with an adversary population (hidden = 32 or 256; adv may be NULL): act_trace holds the market maker's offsets
  * BEFORE the adversary's displacement (the recorder's off_a / off_b, Env/recorder.py:12), so that replaying them through
- * the reference's env together with the adversary genome reproduces the episode. */
+ * the reference's env together with the adversary genome reproduces the episode.  At hidden = 256 with an adversary the
+ * rollout runs in batches in the bundle's code buffer, like an SGMM_PRECISION_EXACT rollout at H = 256. */
 int sgmm_rollout_tc_audit(const sgmm_bundle* bundle, const sgmm_population* mm, const sgmm_population* adv,
                           const sgmm_rollout_params* params, double* fitness, int32_t* trades,
                           float* raw_table, int32_t* act_trace, void* stream);
@@ -282,9 +288,11 @@ typedef struct {
                               /* BF16 / TF32 / F16 = tensor-core rollout; EXACT = F32 at H=32).      */
                               /* hidden = 32: the validation rollout of the best child always runs   */
                               /* the exact F32 kernel.  hidden = 256 (BASELINE config 4): with a     */
-                              /* tensor-core precision population AND validation run spec256_kernel  */
-                              /* and use_arl must be 0; with EXACT both run the bit-exact H=256 path */
-                              /* (sgmm_exact256.cu), use_arl allowed.  F32 is refused at H=256.      */
+                              /* tensor-core precision population AND validation run spec256_kernel; */
+                              /* use_arl needs BF16 (the population's q tables walked by the exact   */
+                              /* 20-state walk; validation stays without adversary).  With EXACT     */
+                              /* both run the bit-exact H=256 path (sgmm_exact256.cu), use_arl       */
+                              /* allowed.  F32 is refused at H=256.                                  */
 } sgmm_ga_config;
 
 typedef struct {
