@@ -10,9 +10,9 @@ from ._lib import SgmmError, SgmmLibraryError, lib  # noqa: F401
 from .env import FTPEnv  # noqa: F401
 from .policy import AdversaryPolicy, NeuroEvolution, TradingPolicy, genome_len  # noqa: F401
 from .bundle import Bundle, normalise, bundle_windows, day_bundle, concat_days  # noqa: F401
-from .analytics import StrategyAnalytics, population_summary  # noqa: F401
+from .analytics import StrategyAnalytics, backtest_population, population_summary  # noqa: F401
 from .engine import (DRLEngine, evaluate_individual, rollout_population, rollout_population_async, rollout_seeded,  # noqa: F401
-                     rollout_trace, rollout_table, rollout_spec256_audit, rollout_tc_audit, measure_fp32_peak)
+                     rollout_trace, rollout_trace_population, rollout_table, rollout_spec256_audit, rollout_tc_audit, measure_fp32_peak)
 from .recorder import StrategyRecorder  # noqa: F401
 from .benchmarks import FOICPolicy, GLFTPolicy  # noqa: F401
 from . import synthetic  # noqa: F401

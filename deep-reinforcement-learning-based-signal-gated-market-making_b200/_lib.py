@@ -103,6 +103,8 @@ SIGNATURES = {
     "sgmm_rollout_trace": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                      C.POINTER(RolloutParams), C.POINTER(Trace), C.c_void_p, C.c_void_p,
                                      C.c_void_p]),
+    "sgmm_rollout_trace_population": (C.c_int, [C.c_void_p, C.POINTER(Population), C.POINTER(Population), C.POINTER(RolloutParams),
+                                                C.POINTER(Trace), C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_rollout_table": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(RolloutParams), C.POINTER(Trace), C.c_void_p,
                                      C.c_void_p, C.c_void_p]),
     "sgmm_env_init": (C.c_int, [C.POINTER(EnvState), C.c_double, C.c_double, C.c_double]),

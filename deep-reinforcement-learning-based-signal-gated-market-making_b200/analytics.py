@@ -1,7 +1,8 @@
 """StrategyAnalytics (analytics/mm_analyzer.py:5-56) as device reductions.
 
 ``StrategyAnalytics(df)`` keeps the reference's properties and ``summary_dict``; ``population_summary`` does the
-same for a whole batch of traces in one launch (one warp per trace).  The float64 reductions follow pandas /
+same for a whole batch of traces in one launch (one warp per trace), and ``backtest_population`` traces a whole population
+and summarises it without leaving the device.  The float64 reductions follow pandas /
 numpy's pairwise summation order, so every figure -- the trade Sharpe ratio included -- is bit-identical to the
 reference's.  Plotting (BacktestVisualizer) is out of scope.
 """
@@ -32,6 +33,30 @@ def population_summary(wealth, inventory, is_trade, device=None):
     p = (lambda a: C.c_void_p(a.ctypes.data) if a.size else None)
     _lib.check(_lib.lib().sgmm_trace_analytics_host(B, T, p(w), p(iv), p(tr), C.c_void_p(out.ctypes.data), int(device), st))
     return out
+
+
+def backtest_population(bundle, genomes=None, adv_genomes=None, *, master=None, count=None, sigma=None, seed=None, generation=0,
+                        first_index=0, adv_master=None, adv_sigma=None, phi, fee_rate=0.0, hidden=32):
+    """Backtest and risk analytics of a whole population: the population arguments of
+    :func:`engine.rollout_trace_population` -> ``(fitness float64[P], trades int32[P], summary float64[P, 6])``, CUDA
+    tensors, summary columns in ``KEYS`` order.  Row i equals
+    ``StrategyAnalytics(StrategyRecorder.from_trace(rollout_trace(...)[2], bundle).to_dataframe()).summary_dict`` of
+    individual i.  Only wealth, inventory and the fills are traced; nothing goes through the host."""
+    from .engine import rollout_trace_population, _stream
+    fit, trd, cols = rollout_trace_population(bundle, genomes, adv_genomes, master=master, count=count, sigma=sigma, seed=seed,
+                                              generation=generation, first_index=first_index, adv_master=adv_master,
+                                              adv_sigma=adv_sigma, phi=phi, fee_rate=fee_rate, hidden=hidden,
+                                              columns=("wealth", "inventory", "fill_buy", "fill_sell"))
+    P, T = cols["wealth"].shape
+    out = torch.empty(P, 6, dtype=torch.float64, device=fit.device)
+    if P == 0:
+        return fit, trd, out
+    is_trade = (cols["fill_buy"] | cols["fill_sell"]).to(torch.uint8)          # the recorder's is_trade: fill_buy or fill_sell
+    scratch = torch.empty(P, T, dtype=torch.float64, device=fit.device)
+    p = (lambda x: x.data_ptr() if x.numel() else None)
+    _lib.check(_lib.lib().sgmm_trace_analytics(P, T, p(cols["wealth"]), None, None, p(cols["inventory"]), p(is_trade),
+                                               p(scratch), out.data_ptr(), _stream(bundle.device)))
+    return fit, trd, out
 
 
 class StrategyAnalytics:

@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsgmm_b200.so")
-SOURCES = ["sgmm_capi.cu", "sgmm_rollout.cu", "sgmm_spec256.cu", "sgmm_tc32.cu", "sgmm_ga.cu", "sgmm_peak.cu", "sgmm_prep.cu", "sgmm_account.cu", "sgmm_one.cu", "sgmm_exact256.cu"]
+SOURCES = ["sgmm_capi.cu", "sgmm_rollout.cu", "sgmm_spec256.cu", "sgmm_tc32.cu", "sgmm_ga.cu", "sgmm_peak.cu", "sgmm_prep.cu", "sgmm_account.cu", "sgmm_one.cu", "sgmm_exact256.cu", "sgmm_trace_pop.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -344,6 +344,27 @@ int sgmm_rollout_trace(const sgmm_bundle* bundle, const float* mm_genome, int32_
                         trace, fitness, trades, (cudaStream_t)stream);
 }
 
+int sgmm_rollout_trace_population(const sgmm_bundle* bundle, const sgmm_population* mm, const sgmm_population* adv,
+                                  const sgmm_rollout_params* params, const sgmm_trace* trace, double* fitness, int32_t* trades,
+                                  void* stream)
+{
+    if (!params) { set_error("NULL bundle / mm / params"); return SGMM_ERR_INVALID; }
+    if (params->precision == SGMM_PRECISION_BF16 || params->precision == SGMM_PRECISION_TF32 || params->precision == SGMM_PRECISION_F16) {
+        set_error("the population trace runs in SGMM-F32 order: pass precision SGMM_PRECISION_F32 or SGMM_PRECISION_EXACT (tensor-core traces are not built)");
+        return SGMM_ERR_UNSUPPORTED;
+    }
+    sgmm_rollout_params exact = *params;                    // F32 and EXACT are the same trace at either width
+    if (exact.precision == SGMM_PRECISION_F32) exact.precision = SGMM_PRECISION_EXACT;
+    if (int rc = check_rollout_args(bundle, mm, adv, &exact, fitness, trades)) return rc;
+    if (mm->count == 0) return SGMM_OK;
+    PopArgs pm, pa;
+    if (int rc = fill_pop(mm, "mm", pm)) return rc;
+    if (adv) if (int rc = fill_pop(adv, "adv", pa)) return rc;
+    DeviceGuard guard(bundle->device);
+    return launch_trace_population(bundle, pm, adv ? &pa : nullptr, mm->hidden, params->phi, params->fee_rate, trace, fitness, trades,
+                                   (cudaStream_t)stream);
+}
+
 int sgmm_rollout_table(const sgmm_bundle* bundle, const int32_t* table, const sgmm_rollout_params* params,
                        const sgmm_trace* trace, double* fitness, int32_t* trades, void* stream)
 {

@@ -125,6 +125,9 @@ constexpr int64_t SMALL_POP_MAX = 400;      // measured break-even against the s
 constexpr int64_t SMALL_POP_MAX_ADV = 148;  // with the adversary (one 512-thread CTA per individual and SM)
 int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
                          cudaStream_t st);
+// the policy table of the small-population path for mm.count individuals (sgmm_one.cu), in the format of `mode`: 0 step code
+// + next inventory, 1 q = raw*5 per (bar, inventory) (adversary walk), 2 raw outputs per (bar, inventory) (population trace)
+int launch_policy_table(const sgmm_bundle* b, const PopArgs& mm, int mode, float2* code, uint8_t* next, cudaStream_t st);
 // the walk + fp64 half of the policy-table path over tables code [P][T][5] / next [P][T][8] (sgmm_one.cu)
 int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const PopArgs* adv, double phi, double fee,
                 double* fitness, int32_t* trades, cudaStream_t st);
@@ -135,16 +138,15 @@ int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, cons
 // first rollout of a size must not run under a stream capture) and stays under the byte budget SGMM_EXACT256_BATCH_BYTES
 // (environment, read on every call; default 2 GiB): *nb individuals per batch.
 int reserve_batches(const sgmm_bundle* b, int64_t P, int64_t per_ind, cudaStream_t st, int64_t* nb, uint64_t** buf);
-// Batches of at most nb individuals: table(pm, pa, b0) enqueues the policy table (code / next) of individuals b0 .. b0+n-1,
-// pm / pa being those individuals of mm / adv (pa nullptr without the adversary); the walk then writes their fitness / trades.
-template <class Table>
-int walk_batches(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int64_t nb, const float2* code, const uint8_t* next,
-                 double phi, double fee, double* fitness, int32_t* trades, cudaStream_t st, Table table)
+// Batches of at most nb individuals of genome length G: fn(pm, pa, b0) gets individuals b0 .. b0+n-1 of mm / adv as pm / pa
+// (pa nullptr without the adversary).
+template <class Fn>
+int for_each_batch(const PopArgs& mm, const PopArgs* adv, int64_t nb, int64_t G, Fn fn)
 {
     for (int64_t b0 = 0; b0 < mm.count; b0 += nb) {
         const int64_t n = mm.count - b0 < nb ? mm.count - b0 : nb;
         PopArgs pm = mm;
-        if (pm.genomes) pm.genomes += b0 * genome_len(256); else pm.first_index += b0;
+        if (pm.genomes) pm.genomes += b0 * G; else pm.first_index += b0;
         pm.count = n;
         PopArgs pa{};
         if (adv) {
@@ -152,18 +154,38 @@ int walk_batches(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, in
             if (pa.genomes) pa.genomes += b0 * 1250; else pa.first_index += b0;
             pa.count = n;
         }
-        if (int rc = table(pm, adv ? &pa : nullptr, b0)) return rc;
-        if (int rc = launch_walk(b, n, code, next, adv ? &pa : nullptr, phi, fee, fitness + b0, trades + b0, st)) return rc;
+        if (int rc = fn(pm, adv ? &pa : nullptr, b0)) return rc;
     }
     return SGMM_OK;
+}
+// Batches of at most nb individuals: table(pm, pa, b0) enqueues the policy table (code / next) of individuals b0 .. b0+n-1,
+// pm / pa being those individuals of mm / adv (pa nullptr without the adversary); the walk then writes their fitness / trades.
+template <class Table>
+int walk_batches(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int64_t nb, const float2* code, const uint8_t* next,
+                 double phi, double fee, double* fitness, int32_t* trades, cudaStream_t st, Table table)
+{
+    return for_each_batch(mm, adv, nb, genome_len(256), [&](const PopArgs& pm, const PopArgs* pa, int64_t b0) {
+        if (int rc = table(pm, pa, b0)) return rc;
+        return launch_walk(b, pm.count, code, next, pa, phi, fee, fitness + b0, trades + b0, st);
+    });
 }
 // bit-exact H = 256 (sgmm_exact256.cu): batches of policy table + walk; and the raw-output table of one genome for the trace
 int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
                     cudaStream_t st);
+namespace x256 {
+// the exact H = 256 policy table of `count` 8-byte aligned genome rows (modes as launch_policy_table), and the staging of
+// seeded children or unaligned rows into such rows (sgmm_exact256.cu)
+int launch_table(const sgmm_bundle* b, const float* rows, int64_t count, int mode, float2* code, uint8_t* next, cudaStream_t st);
+int launch_stage(const sgmm_bundle* b, const PopArgs& mm, int64_t count, float* out, cudaStream_t st);
+bool needs_stage(const PopArgs& mm);
+}
 int launch_exact256_raw(const sgmm_bundle* b, const float* genome, float2* out, float* stage_buf, cudaStream_t st);
 int launch_trace(const sgmm_bundle* b, const float* mm_genome, int hidden, const float* adv_genome,
                  const int32_t* forced, const int32_t* table, double phi, double fee, const sgmm_trace* tr,
                  double* fitness, int32_t* trades, cudaStream_t st);
+// recorder traces of a population, H = 32 or 256 in SGMM-F32 order, [count][T] per column (sgmm_trace_pop.cu)
+int launch_trace_population(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int hidden, double phi, double fee,
+                            const sgmm_trace* tr, double* fitness, int32_t* trades, cudaStream_t st);
 int launch_spec256(const sgmm_bundle* b, const PopArgs& mm, double phi, double fee, double* fitness, int32_t* trades,
                    float* raw_table, int32_t* act_trace, cudaStream_t st);
 // H = 256 on the tensor cores with the adversary: spec256 q tables walked by walk_account_kernel<Walk20>, in batches

@@ -24,6 +24,7 @@
 #include "sgmm_rng.cuh"
 #include "sgmm_adversary.cuh"
 #include "sgmm_step_core.h"
+#include "sgmm_walk.cuh"
 
 namespace sgmm {
 
@@ -56,7 +57,10 @@ struct PtSmem {
 // hidden unit 2.5x slower, one pair per thread 1.15x slower than this).  Same operations in the same order as trace_kernel_h32 (SGMM-F32
 // order): layer 1 fma chain from b1; layer 2 four chains over k mod 4 from (b2, 0, 0, 0), combined (c0+c2)+(c1+c3); layer 3
 // products summed by the xor-butterfly tree 16, 8, 4, 2, 1 (written out serially: s[l] = s[l] + s[l + m]) plus b3.
-__global__ void __launch_bounds__(PT_THREADS) policy_table_kernel(const BarSig* __restrict__ sig, int64_t T, const PopArgs mm_in, int64_t pairs_per_task,
+// RAW_OUT: the table holds the raw outputs before x5 (the population trace, sgmm_trace_pop.cu), and `raw` is ignored; its
+// launch bound lets ptxas take 180 registers instead of spilling two words at 168.
+template <bool RAW_OUT>
+__global__ void __launch_bounds__(PT_THREADS, RAW_OUT ? 1 : 0) policy_table_kernel(const BarSig* __restrict__ sig, int64_t T, const PopArgs mm_in, int64_t pairs_per_task,
                                                                    int raw, float2* __restrict__ code, uint8_t* __restrict__ next)
 {
     __shared__ PtSmem sm;
@@ -147,8 +151,9 @@ __global__ void __launch_bounds__(PT_THREADS) policy_table_kernel(const BarSig* 
                 if (r == 1 && !ok1) break;
                 const int64_t p = pp[r], t = tt[r];
                 const int iv = ivv[r];
-                const float qa = __fmul_rn(__fadd_rn(pa[r][0], sm.b3[0]), 5.0f);              // raw*5.0 (drl_engine.py:39)
-                const float qb = __fmul_rn(__fadd_rn(pb[r][0], sm.b3[1]), 5.0f);
+                const float ra = __fadd_rn(pa[r][0], sm.b3[0]), rb = __fadd_rn(pb[r][0], sm.b3[1]);
+                if constexpr (RAW_OUT) { codei[p] = make_float2(ra, rb); continue; }
+                const float qa = __fmul_rn(ra, 5.0f), qb = __fmul_rn(rb, 5.0f);               // raw*5.0 (drl_engine.py:39)
                 if (raw) { codei[p] = make_float2(qa, qb); continue; }                        // adversary: the fills depend on the walk's state
                 // ---- integer half of the env step: rounding folded into the per-bar float thresholds, as rollout_kernel_h32 ----
                 const bool fb = (inv2[r] < 1.0f) && (qb < sg[r].w);                           // market_env.py:34,37
@@ -168,17 +173,6 @@ __global__ void __launch_bounds__(PT_THREADS) policy_table_kernel(const BarSig* 
 //           the policy table holds the raw q = raw*5 of every (bar, inventory) pair, every bar is a map {0..19} -> {0..19}
 //           built from it, the bar's integer thresholds and the individual's 20-entry displacement table.
 // ---------------------------------------------------------------------------------------------
-
-// maps {0..4} -> {0..4} packed 3 bits per entry
-__device__ __forceinline__ uint32_t map_of(const uint8_t* n) { return n[0] | (n[1] << 3) | (n[2] << 6) | (n[3] << 9) | (n[4] << 12); }
-__device__ __forceinline__ uint32_t map_at(uint32_t m, uint32_t e) { return (m >> (3u * e)) & 7u; }
-// (g after f)[e] = g[f[e]]
-__device__ __forceinline__ uint32_t map_then(uint32_t f, uint32_t g)
-{
-    return map_at(g, map_at(f, 0)) | (map_at(g, map_at(f, 1)) << 3) | (map_at(g, map_at(f, 2)) << 6) | (map_at(g, map_at(f, 3)) << 9) |
-           (map_at(g, map_at(f, 4)) << 12);
-}
-constexpr uint32_t MAP_ID = 0u | (1u << 3) | (2u << 6) | (3u << 9) | (4u << 12);
 
 struct Walk5 {
     using Map = uint32_t;
@@ -206,70 +200,6 @@ struct Walk5 {
     // the offsets of a bar that traded (drl_engine.py:39)
     __device__ static int2 offsets(const Step& r) { return make_int2(__float2int_rn(r.q.x), __float2int_rn(r.q.y)); }
 };
-
-// Maps {0..19} -> {0..19}: 20 entries of 5 bits, six per 32-bit word.
-struct Map20 { uint32_t w[4]; };
-__device__ __forceinline__ uint32_t m20_at(const Map20& m, uint32_t e)          // dynamic index
-{
-    const uint32_t hi = e >= 12u, w = hi ? (e >= 18u ? m.w[3] : m.w[2]) : (e >= 6u ? m.w[1] : m.w[0]);
-    const uint32_t base = hi ? (e >= 18u ? 18u : 12u) : (e >= 6u ? 6u : 0u);
-    return (w >> (5u * (e - base))) & 31u;
-}
-template <int S> __device__ __forceinline__ uint32_t m20_get(const Map20& m) { return (m.w[S / 6] >> (5 * (S % 6))) & 31u; }
-template <int S> __device__ __forceinline__ void m20_set(Map20& m, uint32_t v) { m.w[S / 6] |= v << (5 * (S % 6)); }
-template <int S = 0>
-__device__ __forceinline__ void m20_then_rec(const Map20& f, const Map20& g, Map20& out)     // out[s] = g[f[s]]
-{
-    if constexpr (S < 20) { m20_set<S>(out, m20_at(g, m20_get<S>(f))); m20_then_rec<S + 1>(f, g, out); }
-}
-__device__ __forceinline__ Map20 m20_then(const Map20& f, const Map20& g) { Map20 o = {{0u, 0u, 0u, 0u}}; m20_then_rec(f, g, o); return o; }
-template <int S = 0> __device__ __forceinline__ void m20_id_rec(Map20& m) { if constexpr (S < 20) { m20_set<S>(m, (uint32_t)S); m20_id_rec<S + 1>(m); } }
-__device__ __forceinline__ Map20 m20_identity() { Map20 m = {{0u, 0u, 0u, 0u}}; m20_id_rec(m); return m; }
-__device__ __forceinline__ Map20 m20_shfl_up(const Map20& m, int d)
-{
-    Map20 o;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) o.w[i] = __shfl_up_sync(0xffffffffu, m.w[i], d);
-    return o;
-}
-
-// the market maker's offset of one side, before the adversary's displacement (drl_engine.py:39, clamped to +-K_CLAMP)
-__device__ __forceinline__ int mm_offset(float q) { return max(min(__float2int_rn(q), K_CLAMP), -K_CLAMP); }
-// one bar's step from state st: displaced offsets, fills against the integer thresholds, next state
-struct AdvStep { int oa, ob; bool fb, fs; uint32_t next; };
-__device__ __forceinline__ AdvStep adv_step(uint32_t st, const float2* __restrict__ code_t, int2 k1, uint32_t at0, uint32_t at1, uint32_t at2)
-{
-    const uint32_t iv = st % 5u;
-    const float2 q = code_t[iv];
-    const uint32_t e = table_lookup(at0, at1, at2, (int)st);
-    AdvStep r;
-    r.oa = mm_offset(q.x) + (int)(e & 3u) - 1;                                              // market_env.py:26-28
-    r.ob = mm_offset(q.y) + (int)(e >> 2) - 1;
-    r.fb = (iv < 4u) && (r.ob < k1.y);                                                     // :34,:37
-    r.fs = (iv > 0u) && (r.oa < k1.x);                                                     // :35,:38
-    r.next = (r.fs ? 10u : 0u) + (r.fb ? 5u : 0u) + iv + (r.fb ? 1u : 0u) - (r.fs ? 1u : 0u);
-    return r;
-}
-template <int S = 0>
-__device__ __forceinline__ void bar_map_rec(Map20& m, const float2* __restrict__ code_t, int2 k1, uint32_t at0, uint32_t at1, uint32_t at2)
-{
-    if constexpr (S < 20) { m20_set<S>(m, adv_step((uint32_t)S, code_t, k1, at0, at1, at2).next); bar_map_rec<S + 1>(m, code_t, k1, at0, at1, at2); }
-}
-
-// the individual's adversary as its displacement table (sgmm_adversary.cuh), built in s_adv[3] (shared memory) by the
-// first 20 threads; every thread of the block calls it
-__device__ __forceinline__ void build_adv_table(const PopArgs& adv_in, int64_t ind, uint32_t* s_adv)
-{
-    const int tid = threadIdx.x;
-    if (tid < 3) s_adv[tid] = 0u;
-    __syncthreads();
-    if (tid < 20) {
-        const PopArgs advp = resolve(adv_in);
-        const uint32_t e = adversary_entry(make_source(advp, ind, (int64_t)1250), tid);
-        atomicOr(&s_adv[tid >> 3], e << ((tid & 7) * 4));
-    }
-    __syncthreads();
-}
 
 struct Walk20 {
     using Map = Map20;
@@ -415,22 +345,30 @@ int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs*
     if (int rc = reserve_codes(b, P * 6 + 1, st, &buf)) return rc;               // 48 B per (individual, bar) + slack for T == 0
     float2* code = reinterpret_cast<float2*>(buf);
     uint8_t* next = reinterpret_cast<uint8_t*>(code + P * T * 5);
-    if (T > 0) {
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
-        // task = (individual, range of pairs): ranges of whole 128-pair rounds, sized so that the GPU gets ~8 blocks per SM
-        const int64_t want_blocks = (int64_t)sms * 8;
-        int64_t ppt = (P * T * 5 + want_blocks - 1) / want_blocks;
-        ppt = (ppt + 2 * PT_THREADS - 1) / (2 * PT_THREADS) * (2 * PT_THREADS);
-        const int64_t ppt_min = mm.genomes ? 2 * PT_THREADS : 4 * PT_THREADS;      // seeded children: staging costs ~10 Philox calls per thread
-        if (ppt < ppt_min) ppt = ppt_min;
-        const int64_t ntasks = P * ((T * 5 + ppt - 1) / ppt);
-        const int64_t blocks = ntasks < want_blocks * 2 ? ntasks : want_blocks * 2;
-        policy_table_kernel<<<(unsigned)(blocks < 1 ? 1 : blocks), PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, adv ? 1 : 0, code, next);
-        if (int rc = check_cuda(cudaGetLastError(), "policy_table_kernel launch")) return rc;
-    }
+    if (int rc = launch_policy_table(b, mm, adv ? 1 : 0, code, next, st)) return rc;
     if (int rc = launch_walk(b, P, code, next, adv, phi, fee, fitness, trades, st)) return rc;
     return release_codes(b, st);
+}
+
+int launch_policy_table(const sgmm_bundle* b, const PopArgs& mm, int mode, float2* code, uint8_t* next, cudaStream_t st)
+{
+    using namespace one;
+    const int64_t T = b->T, P = mm.count;
+    if (T == 0 || P == 0) return SGMM_OK;
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
+    // task = (individual, range of pairs): ranges of whole 128-pair rounds, sized so that the GPU gets ~8 blocks per SM
+    const int64_t want_blocks = (int64_t)sms * 8;
+    int64_t ppt = (P * T * 5 + want_blocks - 1) / want_blocks;
+    ppt = (ppt + 2 * PT_THREADS - 1) / (2 * PT_THREADS) * (2 * PT_THREADS);
+    const int64_t ppt_min = mm.genomes ? 2 * PT_THREADS : 4 * PT_THREADS;      // seeded children: staging costs ~10 Philox calls per thread
+    if (ppt < ppt_min) ppt = ppt_min;
+    const int64_t ntasks = P * ((T * 5 + ppt - 1) / ppt);
+    const int64_t blocks = ntasks < want_blocks * 2 ? ntasks : want_blocks * 2;
+    const unsigned grid = (unsigned)(blocks < 1 ? 1 : blocks);
+    if (mode == 2) policy_table_kernel<true><<<grid, PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, 0, code, next);
+    else policy_table_kernel<false><<<grid, PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, mode, code, next);
+    return check_cuda(cudaGetLastError(), "policy_table_kernel launch");
 }
 
 int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const PopArgs* adv, double phi, double fee,

@@ -31,7 +31,9 @@ class StrategyRecorder:
     # -- device trace -> rows (main.py:74-90 layout: ask/bid keys, fills, signals) ----------------
     @classmethod
     def from_trace(cls, trace, bundle):
-        """``trace``: dict from :func:`engine.rollout_trace`; ``bundle``: the host 7-tuple."""
+        """``trace``: dict from :func:`engine.rollout_trace`, or row i of a population trace moved to numpy
+        (``{k: v[i].cpu().numpy() for k, v in engine.rollout_trace_population(...)[2].items()}``, all columns);
+        ``bundle``: the host 7-tuple."""
         s1, s2, mid, ask, bid = (np.asarray(bundle[i]) for i in range(5))
         rec = cls()
         T = len(mid)

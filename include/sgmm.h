@@ -225,6 +225,24 @@ int sgmm_rollout_trace(const sgmm_bundle* bundle, const float* mm_genome, int32_
                        const sgmm_rollout_params* params, const sgmm_trace* trace,
                        double* fitness, int32_t* trades, void* stream);
 
+/* Recorder traces of a whole population in one call (a backtest of many agents on one bundle: the top children of a
+ * generation, several checkpoints, a phi / fee sweep, market maker and adversary pairs side by side).
+ *   mm     the population as for sgmm_rollout_population: explicit genomes or seeded children (genomes == NULL: master +
+ *          sigma * Philox from first_index on); hidden = 32 or 256.  adv may be NULL; otherwise adv->count == mm->count.
+ *   trace  each non-NULL column is a DEVICE array [mm->count][T], row-major; row i holds exactly what sgmm_rollout_trace
+ *          writes for individual i alone.  NULL columns are not written (trace itself may be NULL), and the work only they
+ *          need is skipped.
+ *   fitness / trades  DEVICE [mm->count], always written: bit-identical to the exact rollout (sgmm_rollout_population with
+ *          SGMM_PRECISION_F32 at hidden 32, SGMM_PRECISION_EXACT at hidden 256).
+ * The trace is in SGMM-F32 order whatever the width: params->precision must be SGMM_PRECISION_F32 or SGMM_PRECISION_EXACT
+ * (BF16 / TF32 / F16: SGMM_ERR_UNSUPPORTED).  count == 0 writes nothing.  The raw policy table of a batch (40 B per
+ * individual and bar, plus 269 KB per seeded or unaligned genome at hidden 256) lives in the bundle's code buffer, in batches
+ * under SGMM_EXACT256_BATCH_BYTES: calls on one bundle must be ordered, and the first call of a size must not run under a
+ * stream capture (as for sgmm_rollout_population above). */
+int sgmm_rollout_trace_population(const sgmm_bundle* bundle, const sgmm_population* mm, const sgmm_population* adv,
+                                  const sgmm_rollout_params* params, const sgmm_trace* trace,
+                                  double* fitness, int32_t* trades, void* stream);
+
 /* Inventory-table policies (benchmarks FOIC / GLFT, Env/benchmarks.py:3-40 driven by main.py:99-132):
  * the action at bar t is table[t][inv+2][{a,b}] (DEVICE int32[T,5,2]); same step core, same trace. */
 int sgmm_rollout_table(const sgmm_bundle* bundle, const int32_t* table, const sgmm_rollout_params* params,
