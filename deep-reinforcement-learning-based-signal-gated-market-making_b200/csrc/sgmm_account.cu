@@ -124,8 +124,9 @@ int launch_account(const sgmm_bundle* b, const uint64_t* codes, int64_t count, d
     return check_cuda(cudaGetLastError(), "account_kernel launch");
 }
 
-// The code buffer of a bundle: [count][T] 64-bit codes, grow-only.  It is scratch of ONE rollout at a time: rollouts of
-// the tensor-core kernels on the same bundle must be ordered on one stream (or serialised by the caller).
+// The code buffer of a bundle: [count][T] 64-bit codes, grown on demand.  It is scratch of ONE rollout at a time: an eager
+// rollout arriving on another stream than the last user waits for the last user's event; captured rollouts of one bundle
+// must stay on one stream.  An outgrown buffer is freed, unless a capture has used the bundle's buffer (then retired).
 int reserve_codes(const sgmm_bundle* cb, int64_t count, cudaStream_t st, uint64_t** out)
 {
     sgmm_bundle* b = const_cast<sgmm_bundle*>(cb);
@@ -157,18 +158,33 @@ int reserve_codes(const sgmm_bundle* cb, int64_t count, cudaStream_t st, uint64_
     return SGMM_OK;
 }
 
-int release_codes(const sgmm_bundle* cb, cudaStream_t st)
+namespace {
+
+// release_codes; `report` = false leaves the thread's error message alone (an error exit keeps its own message)
+int release(const sgmm_bundle* cb, cudaStream_t st, bool report)
 {
     sgmm_bundle* b = const_cast<sgmm_bundle*>(cb);
     std::lock_guard<std::mutex> lock(b->codes_mutex);
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     if (st) cudaStreamIsCapturing(st, &cap);
     if (cap != cudaStreamCaptureStatusNone) return SGMM_OK;
+    auto ck = [report](cudaError_t e, const char* what) {
+        return report ? check_cuda(e, what) : (e == cudaSuccess ? SGMM_OK : SGMM_ERR_CUDA);
+    };
     if (!b->codes_done)
-        if (int rc = check_cuda(cudaEventCreateWithFlags(&b->codes_done, cudaEventDisableTiming), "cudaEventCreate(code buffer)")) return rc;
-    if (int rc = check_cuda(cudaEventRecord(b->codes_done, st), "cudaEventRecord(code buffer)")) return rc;
+        if (int rc = ck(cudaEventCreateWithFlags(&b->codes_done, cudaEventDisableTiming), "cudaEventCreate(code buffer)")) return rc;
+    if (int rc = ck(cudaEventRecord(b->codes_done, st), "cudaEventRecord(code buffer)")) return rc;
     b->codes_stream = st; b->codes_busy = true;
     return SGMM_OK;
+}
+
+}  // namespace
+
+int release_codes(const sgmm_bundle* b, cudaStream_t st) { return release(b, st, true); }
+
+CodesRelease::~CodesRelease()
+{
+    if (pending) release(b, st, false);
 }
 
 }  // namespace sgmm

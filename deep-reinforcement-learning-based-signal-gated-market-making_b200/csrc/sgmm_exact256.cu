@@ -303,6 +303,7 @@ int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv,
     int64_t nb = 0;
     uint64_t* buf = nullptr;
     if (int rc = reserve_batches(b, P, 6 * T + (stage ? G / 2 : 0), st, &nb, &buf)) return rc;
+    CodesRelease release(b, st);
     float2* code = reinterpret_cast<float2*>(buf);
     uint8_t* next = reinterpret_cast<uint8_t*>(code + nb * T * 5);
     float* staged = reinterpret_cast<float*>(buf + nb * T * 6);
@@ -315,7 +316,7 @@ int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv,
         return launch_table(b, rows, pm.count, adv ? 1 : 0, code, next, st);
     });
     if (rc) return rc;
-    return release_codes(b, st);
+    return release.done();
 }
 
 // raw policy outputs (before x5) of ONE explicit genome for every (bar, inventory): out = float2[T][5].  `stage_buf` holds

@@ -202,6 +202,19 @@ int launch_account(const sgmm_bundle* b, const uint64_t* codes, int64_t count, d
                    int32_t* trades, cudaStream_t st, bool float_offsets = false);
 int reserve_codes(const sgmm_bundle* b, int64_t count, cudaStream_t st, uint64_t** out);
 int release_codes(const sgmm_bundle* b, cudaStream_t st);      // after the last kernel that reads the codes was enqueued
+// Scope guard of a successful reserve_codes / reserve_batches: done() is release_codes on the success path; any other exit
+// (an error return after some kernels were enqueued) still records the bundle's event on `st`, so that the next user on
+// another stream waits for the work already enqueued.  The error message of that exit is kept.
+struct CodesRelease {
+    const sgmm_bundle* b;
+    cudaStream_t st;
+    bool pending = true;
+    CodesRelease(const sgmm_bundle* bundle, cudaStream_t stream) : b(bundle), st(stream) {}
+    CodesRelease(const CodesRelease&) = delete;
+    CodesRelease& operator=(const CodesRelease&) = delete;
+    int done() { pending = false; return release_codes(b, st); }
+    ~CodesRelease();
+};
 size_t tc32_a1_bytes(int64_t T);
 int launch_prologue(sgmm_bundle* b, const float* z1, const float* z2, const double* mid,
                     const double* ask, const double* bid, cudaStream_t st);

@@ -343,11 +343,12 @@ int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs*
     if (P == 0) return SGMM_OK;
     uint64_t* buf = nullptr;
     if (int rc = reserve_codes(b, P * 6 + 1, st, &buf)) return rc;               // 48 B per (individual, bar) + slack for T == 0
+    CodesRelease release(b, st);
     float2* code = reinterpret_cast<float2*>(buf);
     uint8_t* next = reinterpret_cast<uint8_t*>(code + P * T * 5);
     if (int rc = launch_policy_table(b, mm, adv ? 1 : 0, code, next, st)) return rc;
     if (int rc = launch_walk(b, P, code, next, adv, phi, fee, fitness, trades, st)) return rc;
-    return release_codes(b, st);
+    return release.done();
 }
 
 int launch_policy_table(const sgmm_bundle* b, const PopArgs& mm, int mode, float2* code, uint8_t* next, cudaStream_t st)

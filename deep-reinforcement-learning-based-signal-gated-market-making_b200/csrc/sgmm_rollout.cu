@@ -693,13 +693,14 @@ int launch_trace(const sgmm_bundle* b, const float* mm_genome, int hidden, const
             const int64_t words = 5 * b->T + genome_len(256) / 2;               // float2[T][5] + room for one staged genome, reserved
                                                                                  // whether or not the genome needs staging (269 KB)
             if (int rc = reserve_codes(b, b->T > 0 ? (words + b->T - 1) / b->T : 1, st, &buf)) return rc;
+            CodesRelease release(b, st);
             float2* raw = reinterpret_cast<float2*>(buf);
             if (b->T > 0)
                 if (int rc = launch_exact256_raw(b, mm_genome, raw, reinterpret_cast<float*>(buf + 5 * b->T), st)) return rc;
             a.raw = raw;
             trace_kernel_h32<<<1, 32, 0, st>>>(a);
             if (int rc = check_cuda(cudaGetLastError(), "trace_kernel_h32 launch")) return rc;
-            return release_codes(b, st);
+            return release.done();
         }
     }
     trace_kernel_h32<<<1, 32, 0, st>>>(a);

@@ -674,9 +674,10 @@ int launch_spec256(const sgmm_bundle* b, const PopArgs& mm, double phi, double f
     a.sig = b->sig; a.px = b->px; a.T = b->T; a.tick = b->tick; a.phi = phi; a.fee = fee;
     a.mm = mm; a.fitness = fitness; a.trades = trades; a.raw_table = raw_table; a.act_trace = act_trace;
     if (int rc = reserve_codes(b, mm.count, st, &a.codes)) return rc;
+    CodesRelease release(b, st);
     if (int rc = fee != 0.0 ? launch_kernel<true, false>(b, a, st) : launch_kernel<false, false>(b, a, st)) return rc;
     if (int rc = launch_account(b, a.codes, mm.count, phi, fee, fitness, trades, st)) return rc;   // the fp64 half, after the tensor-core kernel
-    return release_codes(b, st);
+    return release.done();
 }
 
 // With the adversary: batches of (spec256_kernel<false, true> -> q table [n][T][5], 40 B per individual and bar, in the
@@ -692,6 +693,7 @@ int launch_spec256_adv(const sgmm_bundle* b, const PopArgs& mm, const PopArgs& a
     int64_t nb = 0;
     uint64_t* buf = nullptr;
     if (int rc = reserve_batches(b, mm.count, 5 * T, st, &nb, &buf)) return rc;
+    CodesRelease release(b, st);
     float2* q = reinterpret_cast<float2*>(buf);
     Args a{};
     a.sig = b->sig; a.px = b->px; a.T = T; a.tick = b->tick; a.phi = phi; a.fee = fee; a.qtab = q;
@@ -703,7 +705,7 @@ int launch_spec256_adv(const sgmm_bundle* b, const PopArgs& mm, const PopArgs& a
         return act_trace ? launch_adv_offsets(b, pm.count, q, *pa, act_trace + b0 * T * 2, st) : SGMM_OK;
     });
     if (rc) return rc;
-    return release_codes(b, st);
+    return release.done();
 }
 
 }  // namespace sgmm

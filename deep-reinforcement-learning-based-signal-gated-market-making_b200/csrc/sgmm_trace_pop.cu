@@ -283,6 +283,7 @@ int launch_trace_population(const sgmm_bundle* b, const PopArgs& mm, const PopAr
     int64_t nb = 0;
     uint64_t* buf = nullptr;
     if (int rc = reserve_batches(b, P, 5 * T + (stage ? G / 2 : 0), st, &nb, &buf)) return rc;
+    CodesRelease release(b, st);
     float2* raw = reinterpret_cast<float2*>(buf);
     float* staged = reinterpret_cast<float*>(buf + nb * T * 5);
     sgmm_trace none = {};
@@ -315,7 +316,7 @@ int launch_trace_population(const sgmm_bundle* b, const PopArgs& mm, const PopAr
         return pa ? tpop::launch_kernel<tpop::RawWalk20>(args, pm.count, st) : tpop::launch_kernel<tpop::RawWalk5>(args, pm.count, st);
     });
     if (rc) return rc;
-    return release_codes(b, st);
+    return release.done();
 }
 
 }  // namespace sgmm

@@ -147,16 +147,22 @@ typedef struct {
  * and writes one 8-byte step code per bar into a grow-only scratch buffer OF THE BUNDLE ([count][T] codes); an
  * accounting kernel then does the reference's fp64 arithmetic (an FP64 instruction issued while tcgen05.mma executes
  * waits ~80x longer).  Consequences for the caller of H = 256 rollouts:
- *   - rollouts on one bundle must be ordered (one stream, or serialised): they share the scratch;
+ *   - rollouts on one bundle share the scratch.  Eager calls on different streams are ordered by the library: a call on
+ *     another stream than the last user of the buffer waits for that user's event.  Captured calls do not wait on
+ *     events: the captures of one bundle must stay on one stream, and replays of a captured graph are ordered by the caller;
  *   - the first rollout of a given size allocates and therefore must not run under a stream capture (run one eagerly,
- *     then capture; a buffer that has been handed out is never freed before sgmm_bundle_destroy).
+ *     then capture: under a capture a buffer too small is refused with SGMM_ERR_INVALID).  An outgrown buffer is freed
+ *     (cudaFree, after every enqueued user) unless a capture has used the bundle's buffer: from then on outgrown buffers
+ *     stay allocated until sgmm_bundle_destroy, so that a captured graph never holds a freed address.
  * H = 32 rollouts of more than 400 individuals are one kernel with no per-rollout scratch.  SMALL populations (up to 400
  * individuals, 148 with an adversary; exact precision, default launch geometry) take the policy-table path instead (the
  * exact policy for every (bar, inventory) in parallel + a prefix scan over the inventory automaton, bit-identical results):
  * its table ([count][T] x 48 B) lives in the same grow-only code buffer of the bundle, so the same two rules apply to them,
  * and to every SGMM_PRECISION_EXACT rollout at H = 256 (the same table path, in batches).
  * The tensor-core precisions with an adversary read a per-(bundle, fee_rate) table of the reference's exact fp64 P&L legs
- * (144 B per bar), built on the first such rollout: that first rollout must not run under a stream capture either. */
+ * (144 B per bar), built on the first such rollout: that first rollout must not run under a stream capture either (refused
+ * with SGMM_ERR_INVALID).  Eager users on other streams wait for the build.  Fee rates are keyed by their bits (-0.0 and 0.0
+ * are two tables); a bundle holds at most 64 of them, the 65th fee rate is SGMM_ERR_NOMEM. */
 int sgmm_rollout_population(const sgmm_bundle* bundle, const sgmm_population* mm,
                             const sgmm_population* adv, const sgmm_rollout_params* params,
                             double* fitness, int32_t* trades, void* stream);
