@@ -75,6 +75,11 @@ class GaStatus(C.Structure):
                 ("best_val", C.c_double), ("last_best_index", C.c_int64)]
 
 
+class GaRun(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("phi", C.c_double), ("fee_rate", C.c_double),
+                ("sigma", C.c_float), ("patience", C.c_int32)]
+
+
 # every symbol include/sgmm.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "sgmm_version": (C.c_int, []),
@@ -124,6 +129,12 @@ SIGNATURES = {
     "sgmm_ga_master_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_ga_history_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sgmm_ga_create_sweep": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(GaConfig), C.c_int32, C.POINTER(GaRun), C.c_void_p,
+                                       C.c_void_p, C.c_int, C.c_void_p]),
+    "sgmm_ga_run_status_host": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(GaStatus), C.c_void_p]),
+    "sgmm_ga_run_master_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sgmm_ga_run_history_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_bundle_windows": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_bundle_windows_host": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
@@ -158,12 +169,40 @@ def lib():
                 raise SgmmLibraryError(f"{LIB_PATH} does not export {name}") from e
             fn.restype = res
             fn.argtypes = args
-        for which, struct in enumerate((Population, RolloutParams, Trace, EnvState, StepInfo, GaConfig, GaStatus)):
+        for which, struct in enumerate((Population, RolloutParams, Trace, EnvState, StepInfo, GaConfig, GaStatus, GaRun)):
             if L.sgmm_abi_sizeof(which) != C.sizeof(struct):
                 raise SgmmLibraryError(f"{LIB_PATH}: sizeof({struct.__name__}) is {L.sgmm_abi_sizeof(which)} in the library, "
                                        f"{C.sizeof(struct)} in the ctypes mirror -- rebuild the library (stale .so?)")
         _lib = L
     return _lib
+
+
+_DEFERRED = []          # (destroy entry, handle) released while a CUDA graph was being captured
+
+
+def _capturing() -> bool:
+    try:
+        import torch
+        return torch.cuda.is_available() and torch.cuda.is_current_stream_capturing()
+    except Exception:
+        return False
+
+
+def release(destroy: str, handle) -> None:
+    """Destroy a bundle or GA handle (``destroy`` names its entry: sgmm_bundle_destroy, sgmm_ga_destroy).  The destroy entries
+    free device memory and synchronise, which a stream capture in progress on this thread does not allow: the capture would
+    be invalidated.  A handle released while the current stream captures a CUDA graph (typically an object the garbage
+    collector finalises in the middle of ``torch.cuda.graph``) is therefore kept and destroyed at the next release outside
+    a capture."""
+    h = handle.value if isinstance(handle, C.c_void_p) else handle
+    if h:
+        _DEFERRED.append((destroy, h))
+    if not _DEFERRED or _capturing():
+        return
+    L = lib()
+    while _DEFERRED:
+        name, p = _DEFERRED.pop()
+        getattr(L, name)(C.c_void_p(p))
 
 
 def check(code: int):

@@ -73,8 +73,8 @@ class Bundle:
 
     def close(self):
         if getattr(self, "_h", None):
-            _lib.lib().sgmm_bundle_destroy(self._h)
-            self._h = C.c_void_p()
+            h, self._h = self._h, C.c_void_p()
+            _lib.release("sgmm_bundle_destroy", h)
 
     def __del__(self):
         try:

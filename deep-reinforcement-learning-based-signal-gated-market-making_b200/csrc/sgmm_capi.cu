@@ -87,6 +87,7 @@ int sgmm_abi_sizeof(int which)
         case 4: return (int)sizeof(sgmm_step_info);
         case 5: return (int)sizeof(sgmm_ga_config);
         case 6: return (int)sizeof(sgmm_ga_status);
+        case 7: return (int)sizeof(sgmm_ga_run);
         default: return SGMM_ERR_INVALID;
     }
 }

@@ -85,6 +85,33 @@ struct PopArgs {
     int64_t count;
 };
 
+// Device state of one GA run (sgmm_ga.cu); a sweep of K runs keeps K of them, contiguous.  seed / patience / phi / fee are
+// set at creation and read by the sweep's table and walk kernels (sgmm_one.cu) and by ga_tell_kernel / ga_update_kernel.
+struct GaDev {
+    int32_t generation;
+    int32_t stale;
+    float sigma, adv_sigma;
+    double best_val;
+    int64_t best_idx, adv_best_idx;
+    double train_f; int32_t train_trades; int32_t patience;
+    uint64_t seed;
+    double phi, fee;             // the walk reads the fee as stored: -0.0 and 0.0 stay distinct
+};
+
+constexpr uint64_t ADV_SEED_FLIP = 0x8000000000000000ull;   // adversary noise stream (same as the oracle)
+
+// The seeded children of a GA sweep (K runs of lambda children each, one launch): individual i of a launch is g = first + i
+// of the sweep, child g % lambda of run r = g / lambda, regenerated from row r of `master` with run r's device sigma
+// (adv_sigma when `adv`), generation and seed (seed ^ ADV_SEED_FLIP when `adv`) -- the child a solo GA of that run draws.
+// The sweep's walks read run r's phi and fee from st[r].  With lambda = 1 and master = nullptr it only indexes the runs
+// (validation of the K masters).
+struct SweepPop {
+    const float* master;       // [K][G] (G = 1250: the market makers' or the adversaries' masters)
+    const GaDev* st;           // [K]
+    int64_t lambda, first, count;
+    int adv;
+};
+
 struct RolloutArgs {
     const BarSig* sig;
     const BarPx* px;
@@ -138,22 +165,31 @@ int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, cons
 // first rollout of a size must not run under a stream capture) and stays under the byte budget SGMM_EXACT256_BATCH_BYTES
 // (environment, read on every call; default 2 GiB): *nb individuals per batch.
 int reserve_batches(const sgmm_bundle* b, int64_t P, int64_t per_ind, cudaStream_t st, int64_t* nb, uint64_t** buf);
+// individuals b0 .. b0+n-1 of a population of genome length G
+inline PopArgs batch_of(const PopArgs& p, int64_t b0, int64_t n, int64_t G)
+{
+    PopArgs r = p;
+    if (r.genomes) r.genomes += b0 * G; else r.first_index += b0;
+    r.count = n;
+    return r;
+}
+inline SweepPop batch_of(const SweepPop& p, int64_t b0, int64_t n, int64_t)
+{
+    SweepPop r = p;
+    r.first += b0;                                  // a batch may start inside a run: the kernels split first + i into (run, child)
+    r.count = n;
+    return r;
+}
 // Batches of at most nb individuals of genome length G: fn(pm, pa, b0) gets individuals b0 .. b0+n-1 of mm / adv as pm / pa
-// (pa nullptr without the adversary).
-template <class Fn>
-int for_each_batch(const PopArgs& mm, const PopArgs* adv, int64_t nb, int64_t G, Fn fn)
+// (pa nullptr without the adversary).  Pop: PopArgs, or SweepPop (the children of a GA sweep).
+template <class Pop, class Fn>
+int for_each_batch(const Pop& mm, const Pop* adv, int64_t nb, int64_t G, Fn fn)
 {
     for (int64_t b0 = 0; b0 < mm.count; b0 += nb) {
         const int64_t n = mm.count - b0 < nb ? mm.count - b0 : nb;
-        PopArgs pm = mm;
-        if (pm.genomes) pm.genomes += b0 * G; else pm.first_index += b0;
-        pm.count = n;
-        PopArgs pa{};
-        if (adv) {
-            pa = *adv;
-            if (pa.genomes) pa.genomes += b0 * 1250; else pa.first_index += b0;
-            pa.count = n;
-        }
+        const Pop pm = batch_of(mm, b0, n, G);
+        Pop pa{};
+        if (adv) pa = batch_of(*adv, b0, n, (int64_t)1250);
         if (int rc = fn(pm, adv ? &pa : nullptr, b0)) return rc;
     }
     return SGMM_OK;
@@ -169,6 +205,14 @@ int walk_batches(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, in
         return launch_walk(b, pm.count, code, next, pa, phi, fee, fitness + b0, trades + b0, st);
     });
 }
+// GA sweeps at H = 32, exact (sgmm_one.cu).  launch_sweep_population: the mm.count seeded children of mm (and adv) on the
+// policy-table path at every size, in batches under SGMM_EXACT256_BATCH_BYTES in the bundle's code buffer; every walk CTA
+// takes its run's phi and fee.  launch_sweep_validation: K explicit masters [K][1250] (adversary off), walk CTA r with run
+// r's phi and fee.
+int launch_sweep_population(const sgmm_bundle* b, const SweepPop& mm, const SweepPop* adv, double* fitness, int32_t* trades,
+                            cudaStream_t st);
+int launch_sweep_validation(const sgmm_bundle* b, const float* masters, const GaDev* runs, int64_t K, double* fitness,
+                            int32_t* trades, cudaStream_t st);
 // bit-exact H = 256 (sgmm_exact256.cu): batches of policy table + walk; and the raw-output table of one genome for the trace
 int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
                     cudaStream_t st);

@@ -59,12 +59,14 @@ struct PtSmem {
 // products summed by the xor-butterfly tree 16, 8, 4, 2, 1 (written out serially: s[l] = s[l] + s[l + m]) plus b3.
 // RAW_OUT: the table holds the raw outputs before x5 (the population trace, sgmm_trace_pop.cu), and `raw` is ignored; its
 // launch bound lets ptxas take 180 registers instead of spilling two words at 168.
-template <bool RAW_OUT>
-__global__ void __launch_bounds__(PT_THREADS, RAW_OUT ? 1 : 0) policy_table_kernel(const BarSig* __restrict__ sig, int64_t T, const PopArgs mm_in, int64_t pairs_per_task,
+// Pop: PopArgs (a population), or SweepPop (the children of a GA sweep: individual i of the launch is child
+// (mm.first + i) % lambda of run (mm.first + i) / lambda).
+template <bool RAW_OUT, class Pop>
+__global__ void __launch_bounds__(PT_THREADS, RAW_OUT ? 1 : 0) policy_table_kernel(const BarSig* __restrict__ sig, int64_t T, const Pop mm_in, int64_t pairs_per_task,
                                                                    int raw, float2* __restrict__ code, uint8_t* __restrict__ next)
 {
     __shared__ PtSmem sm;
-    const PopArgs mm = resolve(mm_in);
+    const Pop mm = resolve(mm_in);
     constexpr int64_t G = (int64_t)H * H + 7 * H + 2;
     const int64_t pairs = T * 5, tasks_per_ind = (pairs + pairs_per_task - 1) / pairs_per_task, ntasks = mm.count * tasks_per_ind;
     int64_t loaded = -1;
@@ -180,7 +182,8 @@ struct Walk5 {
     struct Step { float2 q; bool fb, fs; uint32_t next; };
     const float2* code;                    // this individual's [T][5] q of each side that filled, NaN marker otherwise
     const uint8_t* next;                   // [T][8] next inventory index
-    __device__ Walk5(const BarSig*, const float2* code_all, const uint8_t* next_all, const PopArgs&, int64_t ind, int64_t T)
+    template <class Pop>
+    __device__ Walk5(const BarSig*, const float2* code_all, const uint8_t* next_all, const Pop&, int64_t ind, int64_t T)
         : code(code_all + ind * T * 5), next(next_all + ind * T * 8) {}
     __device__ static Map identity() { return MAP_ID; }
     __device__ static Map then(Map f, Map g) { return map_then(f, g); }
@@ -208,7 +211,8 @@ struct Walk20 {
     const BarSig* sig;
     const float2* code;                    // this individual's [T][5] raw q = raw*5
     uint32_t at0, at1, at2;                // displacement table (sgmm_adversary.cuh)
-    __device__ Walk20(const BarSig* sig_, const float2* code_all, const uint8_t*, const PopArgs& adv_in, int64_t ind, int64_t T)
+    template <class Pop>
+    __device__ Walk20(const BarSig* sig_, const float2* code_all, const uint8_t*, const Pop& adv_in, int64_t ind, int64_t T)
         : sig(sig_), code(code_all + ind * T * 5)
     {
         __shared__ uint32_t s_adv[3];
@@ -231,12 +235,26 @@ struct Walk20 {
     __device__ static int2 offsets(const Step& r) { return make_int2(r.oa, r.ob); }
 };
 
+// phi and fee of this CTA's episode: the launch's (a population), or those of its individual's run (a GA sweep)
+__device__ __forceinline__ double cta_phi(const PopArgs&, double phi) { return phi; }
+__device__ __forceinline__ double cta_fee(const PopArgs&, double fee) { return fee; }
+__device__ __forceinline__ const GaDev* cta_run(const SweepPop& p) { return p.st + (p.first + (int64_t)blockIdx.x) / p.lambda; }
+__device__ __forceinline__ double cta_phi(const SweepPop& p, double) { return cta_run(p)->phi; }
+__device__ __forceinline__ double cta_fee(const SweepPop& p, double) { return cta_run(p)->fee; }
+
+// CTAs per SM of the 512-thread walk without the adversary: 3 (40 registers); a sweep's CTA also keeps its run's phi / fee
+// and takes 2, so that it runs in 64 registers without spilling
+template <class Pop> constexpr int walk_ctas_per_sm() { return 3; }
+template <> constexpr int walk_ctas_per_sm<SweepPop>() { return 2; }
+
 // One CTA per individual.  WALK_THREADS = 1024 (one individual per SM: shortest latency, populations up to the SM count) or
-// 512 (three per SM without the adversary: the serial reward sum of one individual hides behind the others)
-template <class A, int WALK_THREADS>
-__global__ void __launch_bounds__(WALK_THREADS, (WALK_THREADS == 1024 || A::STATES == 20) ? 1 : 3)
+// 512 (three per SM without the adversary: the serial reward sum of one individual hides behind the others).
+// Pop: PopArgs (phi_arg / fee_arg apply to every CTA), or SweepPop (a GA sweep: CTA i walks individual adv.first + i of the
+// sweep with its run's phi and fee; with the adversary, adv gives the individual's seeded adversary).
+template <class A, int WALK_THREADS, class Pop>
+__global__ void __launch_bounds__(WALK_THREADS, (WALK_THREADS == 1024 || A::STATES == 20) ? 1 : walk_ctas_per_sm<Pop>())
 walk_account_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px, int64_t T, const float2* __restrict__ code_all,
-                    const uint8_t* __restrict__ next_all, const PopArgs adv, double tick, double phi, double fee,
+                    const uint8_t* __restrict__ next_all, const Pop adv, double tick, double phi_arg, double fee_arg,
                     double* __restrict__ fitness, int32_t* __restrict__ trades)
 {
     using Map = typename A::Map;
@@ -275,7 +293,7 @@ walk_account_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px
     if (warp > 0) before = A::then(s_warp[warp - 1], before);
     uint32_t st = A::at(before, 2u);                        // flat, no previous fills: state 2 (market_env.py:17, drl_engine.py:29)
     // ---- 3. the fp64 half for the visited states, chunk by chunk; one thread sums each chunk in bar order ----
-    const PenaltyTable pen = penalty_table(phi);
+    const PenaltyTable pen = penalty_table(cta_phi(adv, phi_arg));
     int ntr = 0;
     double total = 0.0;                                     // thread 0 only (drl_engine.py:26)
     for (int64_t c0 = 0; c0 < T; c0 += SUM_CHUNK) {
@@ -290,6 +308,7 @@ walk_account_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px
                 const int2 k = A::offsets(r);
                 const double my_ask = quote_ask(p.ask, k.x, tick), my_bid = quote_bid(p.bid, k.y, tick);         // :30-31
                 // fee terms evaluated as the reference does, fee_rate 0 included
+                const double fee = cta_fee(adv, fee_arg);
                 const double leg_b = buy_leg(my_bid, p.mid_next, fee), leg_s = sell_leg(my_ask, p.mid_next, fee);
                 pnl = r.fb ? add_rn(pnl, leg_b) : pnl;
                 pnl = r.fs ? add_rn(pnl, leg_s) : pnl;
@@ -351,22 +370,46 @@ int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs*
     return release.done();
 }
 
+namespace one {
+// grid and pairs per task of policy_table_kernel for P individuals: task = (individual, range of pairs), ranges of whole
+// 128-pair rounds, sized so that the GPU gets ~8 blocks per SM
+static unsigned policy_table_grid(const sgmm_bundle* b, int64_t P, bool seeded, int64_t* pairs_per_task)
+{
+    const int64_t T = b->T;
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
+    const int64_t want_blocks = (int64_t)sms * 8;
+    int64_t ppt = (P * T * 5 + want_blocks - 1) / want_blocks;
+    ppt = (ppt + 2 * PT_THREADS - 1) / (2 * PT_THREADS) * (2 * PT_THREADS);
+    const int64_t ppt_min = seeded ? 4 * PT_THREADS : 2 * PT_THREADS;          // seeded children: staging costs ~10 Philox calls per thread
+    if (ppt < ppt_min) ppt = ppt_min;
+    const int64_t ntasks = P * ((T * 5 + ppt - 1) / ppt);
+    const int64_t blocks = ntasks < want_blocks * 2 ? ntasks : want_blocks * 2;
+    *pairs_per_task = ppt;
+    return (unsigned)(blocks < 1 ? 1 : blocks);
+}
+
+// the walk of P individuals over tables code / next: adversary off (Walk5) or on (Walk20, the adversaries from runs); CTA i
+// takes the phi and fee of the run of sweep individual runs.first + i
+static int launch_sweep_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const SweepPop& runs, bool adv,
+                             double* fitness, int32_t* trades, cudaStream_t st)
+{
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
+    if (adv) walk_account_kernel<Walk20, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, b->T, code, nullptr, runs, b->tick, 0.0, 0.0, fitness, trades);
+    else if (P <= sms) walk_account_kernel<Walk5, 1024><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, b->T, code, next, runs, b->tick, 0.0, 0.0, fitness, trades);
+    else walk_account_kernel<Walk5, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, b->T, code, next, runs, b->tick, 0.0, 0.0, fitness, trades);
+    return check_cuda(cudaGetLastError(), "walk_account_kernel launch (sweep)");
+}
+}  // namespace one
+
 int launch_policy_table(const sgmm_bundle* b, const PopArgs& mm, int mode, float2* code, uint8_t* next, cudaStream_t st)
 {
     using namespace one;
     const int64_t T = b->T, P = mm.count;
     if (T == 0 || P == 0) return SGMM_OK;
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
-    // task = (individual, range of pairs): ranges of whole 128-pair rounds, sized so that the GPU gets ~8 blocks per SM
-    const int64_t want_blocks = (int64_t)sms * 8;
-    int64_t ppt = (P * T * 5 + want_blocks - 1) / want_blocks;
-    ppt = (ppt + 2 * PT_THREADS - 1) / (2 * PT_THREADS) * (2 * PT_THREADS);
-    const int64_t ppt_min = mm.genomes ? 2 * PT_THREADS : 4 * PT_THREADS;      // seeded children: staging costs ~10 Philox calls per thread
-    if (ppt < ppt_min) ppt = ppt_min;
-    const int64_t ntasks = P * ((T * 5 + ppt - 1) / ppt);
-    const int64_t blocks = ntasks < want_blocks * 2 ? ntasks : want_blocks * 2;
-    const unsigned grid = (unsigned)(blocks < 1 ? 1 : blocks);
+    int64_t ppt = 0;
+    const unsigned grid = policy_table_grid(b, P, mm.genomes == nullptr, &ppt);
     if (mode == 2) policy_table_kernel<true><<<grid, PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, 0, code, next);
     else policy_table_kernel<false><<<grid, PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, mode, code, next);
     return check_cuda(cudaGetLastError(), "policy_table_kernel launch");
@@ -384,6 +427,54 @@ int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8
     else if (P <= sms2) walk_account_kernel<Walk5, 1024><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, T, code, next, none, b->tick, phi, fee, fitness, trades);
     else walk_account_kernel<Walk5, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, next, none, b->tick, phi, fee, fitness, trades);
     return check_cuda(cudaGetLastError(), "walk_account_kernel launch");
+}
+
+// The K*lambda children of a GA sweep take the policy-table path whatever their number (a solo GA of more than
+// SMALL_POP_MAX children runs rollout_kernel_h32, which gives the same bits).  The table ([n][T] x 48 B) lives in the
+// bundle's code buffer, in batches of n individuals under SGMM_EXACT256_BATCH_BYTES; a batch may start inside a run.
+int launch_sweep_population(const sgmm_bundle* b, const SweepPop& mm, const SweepPop* adv, double* fitness, int32_t* trades,
+                            cudaStream_t st)
+{
+    using namespace one;
+    const int64_t T = b->T, P = mm.count;
+    if (P == 0) return SGMM_OK;
+    int64_t nb = 0;
+    uint64_t* buf = nullptr;
+    if (int rc = reserve_batches(b, P, 6 * T, st, &nb, &buf)) return rc;
+    CodesRelease release(b, st);
+    float2* code = reinterpret_cast<float2*>(buf);
+    uint8_t* next = reinterpret_cast<uint8_t*>(code + nb * T * 5);
+    const int rc = for_each_batch(mm, adv, nb, genome_len(32), [&](const SweepPop& pm, const SweepPop* pa, int64_t b0) {
+        if (T > 0) {
+            int64_t ppt = 0;
+            const unsigned grid = policy_table_grid(b, pm.count, true, &ppt);
+            policy_table_kernel<false><<<grid, PT_THREADS, 0, st>>>(b->sig, T, pm, ppt, pa ? 1 : 0, code, next);
+            if (int rc = check_cuda(cudaGetLastError(), "policy_table_kernel launch (sweep)")) return rc;
+        }
+        return launch_sweep_walk(b, pm.count, code, next, pa ? *pa : pm, pa != nullptr, fitness + b0, trades + b0, st);
+    });
+    if (rc) return rc;
+    return release.done();
+}
+
+// The K masters of a sweep, contiguous [K][1250] rows, as one explicit population: one table, K walk CTAs with per-run phi
+// and fee, adversary off (as the validation of a solo GA)
+int launch_sweep_validation(const sgmm_bundle* b, const float* masters, const GaDev* runs, int64_t K, double* fitness,
+                            int32_t* trades, cudaStream_t st)
+{
+    using namespace one;
+    if (K == 0) return SGMM_OK;
+    uint64_t* buf = nullptr;
+    if (int rc = reserve_codes(b, K * 6 + 1, st, &buf)) return rc;              // 48 B per (individual, bar) + slack for T == 0
+    CodesRelease release(b, st);
+    float2* code = reinterpret_cast<float2*>(buf);
+    uint8_t* next = reinterpret_cast<uint8_t*>(code + K * b->T * 5);
+    PopArgs pm{};
+    pm.genomes = masters; pm.count = K;
+    if (int rc = launch_policy_table(b, pm, 0, code, next, st)) return rc;
+    const SweepPop all{nullptr, runs, 1, 0, K, 0};
+    if (int rc = launch_sweep_walk(b, K, code, next, all, false, fitness, trades, st)) return rc;
+    return release.done();
 }
 
 int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, const PopArgs& adv, int32_t* act_trace, cudaStream_t st)

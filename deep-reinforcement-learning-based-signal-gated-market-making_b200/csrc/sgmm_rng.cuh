@@ -131,4 +131,26 @@ __device__ __forceinline__ GenomeSource make_source(const PopArgs& p, int64_t i,
     return g;
 }
 
+// a GA sweep's children (SweepPop, sgmm_internal.h): individual i of the launch is child (first + i) % lambda of run
+// (first + i) / lambda, drawn exactly as the solo GA of that run draws it
+__device__ __forceinline__ SweepPop resolve(const SweepPop& p) { return p; }
+
+__device__ __forceinline__ GenomeSource make_source(const SweepPop& p, int64_t i, int64_t G)
+{
+    const int64_t g = p.first + i, r = g / p.lambda;
+    const GaDev* s = p.st + r;
+    GenomeSource src;
+    src.seeded = true;
+    src.row = p.master + r * G;
+    src.sigma = p.adv ? s->adv_sigma : s->sigma;
+    src.seed = p.adv ? s->seed ^ ADV_SEED_FLIP : s->seed;
+    src.generation = (uint64_t)s->generation;
+    src.individual = (uint64_t)(g - r * p.lambda);
+    return src;
+}
+
+// the source of individual i of a launch, device scalars resolved
+template <class Pop>
+__device__ __forceinline__ GenomeSource source_of(const Pop& p, int64_t i, int64_t G) { return make_source(resolve(p), i, G); }
+
 }  // namespace sgmm

@@ -74,15 +74,15 @@ __device__ __forceinline__ void bar_map_rec(Map20& m, const float2* __restrict__
 }
 
 // the individual's adversary as its displacement table (sgmm_adversary.cuh), built in s_adv[3] (shared memory) by the
-// first 20 threads; every thread of the block calls it
-__device__ __forceinline__ void build_adv_table(const PopArgs& adv_in, int64_t ind, uint32_t* s_adv)
+// first 20 threads; every thread of the block calls it.  Pop: PopArgs, or SweepPop (a GA sweep's adversaries)
+template <class Pop>
+__device__ __forceinline__ void build_adv_table(const Pop& adv_in, int64_t ind, uint32_t* s_adv)
 {
     const int tid = threadIdx.x;
     if (tid < 3) s_adv[tid] = 0u;
     __syncthreads();
     if (tid < 20) {
-        const PopArgs advp = resolve(adv_in);
-        const uint32_t e = adversary_entry(make_source(advp, ind, (int64_t)1250), tid);
+        const uint32_t e = adversary_entry(source_of(adv_in, ind, (int64_t)1250), tid);
         atomicOr(&s_adv[tid >> 3], e << ((tid & 7) * 4));
     }
     __syncthreads();

@@ -429,7 +429,64 @@ def evaluate_individual(mm_weights, adv_weights, bundle, phi, tick_size, fee_rat
 # ------------------------------------------------------------------------------------------------
 # DRLEngine
 # ------------------------------------------------------------------------------------------------
-class DeviceGA:
+class _GAHandle:
+    """What every ``sgmm_ga`` handle offers: the generation phases, graph capture, the per-run read-backs and close."""
+
+    def evaluate(self, train: Bundle):
+        _lib.check(_lib.lib().sgmm_ga_evaluate(self._h, train.handle, _stream(self.device)))
+
+    def select(self, val: Bundle):
+        _lib.check(_lib.lib().sgmm_ga_select(self._h, val.handle, _stream(self.device)))
+
+    def generation(self, train: Bundle, val: Bundle):
+        _lib.check(_lib.lib().sgmm_ga_generation(self._h, train.handle, val.handle, _stream(self.device)))
+
+    def capture(self, train: Bundle, val: Bundle):
+        """Capture one generation (ask + rollout + tell + validation rollout + select: 4 kernels, no
+        host round trip) into a CUDA graph; ``graph.replay()`` then advances the GA by one generation.
+        Call :meth:`generation` once before capturing (first launches configure the kernels)."""
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            self.generation(train, val)
+        return g
+
+    def _status(self, run):
+        s = _lib.GaStatus()
+        _lib.check(_lib.lib().sgmm_ga_run_status_host(self._h, int(run), C.byref(s), _stream(self.device)))
+        return {"generation": s.generation, "stale": s.stale, "sigma": s.sigma, "adv_sigma": s.adv_sigma,
+                "best_val": s.best_val, "last_best_index": s.last_best_index}
+
+    def _masters(self, run):
+        mm = np.empty(self.G, np.float32)
+        adv = np.empty(1250, np.float32)
+        best = np.empty(self.G, np.float32)
+        _lib.check(_lib.lib().sgmm_ga_run_master_host(self._h, int(run), mm.ctypes.data, adv.ctypes.data, best.ctypes.data,
+                                                      _stream(self.device)))
+        return mm, adv, best
+
+    def _history(self, run, n):
+        n = self._status(run)["generation"] if n is None else int(n)
+        n = max(0, min(n, self.max_generations))
+        tf, vf = np.empty(n, np.float64), np.empty(n, np.float64)
+        tt, vt = np.empty(n, np.int32), np.empty(n, np.int32)
+        sg = np.empty(n, np.float32)
+        _lib.check(_lib.lib().sgmm_ga_run_history_host(self._h, int(run), n, tf.ctypes.data, vf.ctypes.data, tt.ctypes.data,
+                                                       vt.ctypes.data, sg.ctypes.data, _stream(self.device)))
+        return {"train_f": tf, "val_f": vf, "train_trades": tt, "val_trades": vt, "sigma": sg}
+
+    def close(self):
+        if getattr(self, "_h", None):
+            h, self._h = self._h, C.c_void_p()
+            _lib.release("sgmm_ga_destroy", h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class DeviceGA(_GAHandle):
     """Thin owner of a ``sgmm_ga`` handle (include/sgmm.h): ask/evaluate/tell/validate/select on
     the device, one call per generation, no host round trip."""
 
@@ -459,59 +516,76 @@ class DeviceGA:
         _lib.check(_lib.lib().sgmm_ga_buffers(self._h, *[C.byref(x) for x in p], C.byref(bb), C.byref(nb), C.byref(mb)))
         return p[0].value, p[1].value, p[2].value, bb.value, nb.value, mb.value
 
-    def evaluate(self, train: Bundle):
-        _lib.check(_lib.lib().sgmm_ga_evaluate(self._h, train.handle, _stream(self.device)))
-
-    def select(self, val: Bundle):
-        _lib.check(_lib.lib().sgmm_ga_select(self._h, val.handle, _stream(self.device)))
-
-    def generation(self, train: Bundle, val: Bundle):
-        _lib.check(_lib.lib().sgmm_ga_generation(self._h, train.handle, val.handle, _stream(self.device)))
-
-    def capture(self, train: Bundle, val: Bundle):
-        """Capture one generation (ask + rollout + tell + validation rollout + select: 4 kernels, no
-        host round trip) into a CUDA graph; ``graph.replay()`` then advances the GA by one generation.
-        Call :meth:`generation` once before capturing (first launches configure the kernels)."""
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g):
-            self.generation(train, val)
-        return g
-
     def status(self):
-        s = _lib.GaStatus()
-        _lib.check(_lib.lib().sgmm_ga_status_host(self._h, C.byref(s), _stream(self.device)))
-        return {"generation": s.generation, "stale": s.stale, "sigma": s.sigma, "adv_sigma": s.adv_sigma,
-                "best_val": s.best_val, "last_best_index": s.last_best_index}
+        return self._status(0)
 
     def masters(self):
-        mm = np.empty(self.G, np.float32)
-        adv = np.empty(1250, np.float32)
-        best = np.empty(self.G, np.float32)
-        _lib.check(_lib.lib().sgmm_ga_master_host(self._h, mm.ctypes.data, adv.ctypes.data, best.ctypes.data,
-                                                  _stream(self.device)))
-        return mm, adv, best
+        return self._masters(0)
 
     def history(self, n=None):
         """History columns of the first ``n`` generations (default: the generations completed so far)."""
-        n = self.status()["generation"] if n is None else int(n)
-        n = max(0, min(n, self.max_generations))
-        tf, vf = np.empty(n, np.float64), np.empty(n, np.float64)
-        tt, vt = np.empty(n, np.int32), np.empty(n, np.int32)
-        sg = np.empty(n, np.float32)
-        _lib.check(_lib.lib().sgmm_ga_history_host(self._h, n, tf.ctypes.data, vf.ctypes.data, tt.ctypes.data,
-                                                   vt.ctypes.data, sg.ctypes.data, _stream(self.device)))
-        return {"train_f": tf, "val_f": vf, "train_trades": tt, "val_trades": vt, "sigma": sg}
+        return self._history(0, n)
 
-    def close(self):
-        if getattr(self, "_h", None):
-            _lib.lib().sgmm_ga_destroy(self._h)
-            self._h = C.c_void_p()
 
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
+_RUN_DEFAULTS = {"fee_rate": 0.0, "sigma": 0.05, "patience": 15}
+
+
+class DeviceGASweep(_GAHandle):
+    """K independent GA runs advanced by the same launches (``sgmm_ga_create_sweep``): a phi / fee / seed sweep at the
+    reference's scale without K sequential GAs.  ``runs`` is a list of dicts ``{seed, phi, fee_rate, sigma, patience}``
+    (``fee_rate`` 0, ``sigma`` 0.05, ``patience`` 15 when left out); ``masters`` [K, 1250] (or one [1250] master for
+    every run), ``adv_masters`` likewise when ``use_arl``.  ``pop_size`` is lambda PER RUN.  Run r is bit-identical to
+    ``DeviceGA(masters[r], adv_masters[r], precision="exact", **runs[r])``.  Hidden width 32, exact precision, one
+    device.  Read-backs take the run: ``status(r)``, ``masters(r)``, ``history(r)``."""
+
+    def __init__(self, masters, adv_masters=None, *, runs, pop_size, use_arl, max_generations, device=None):
+        self.device = torch.cuda.current_device() if device is None else int(device)
+        K = len(runs)
+        if K == 0:
+            raise ValueError("a sweep needs at least one run")
+        unknown = [k for r in runs for k in r if k not in ("seed", "phi", "fee_rate", "sigma", "patience")]
+        if unknown:
+            raise ValueError(f"unknown run keys {sorted(set(unknown))}")
+        arr = (_lib.GaRun * K)()
+        for i, r in enumerate(runs):
+            r = {**_RUN_DEFAULTS, **r}
+            arr[i] = _lib.GaRun(int(r["seed"]) & 0xFFFFFFFFFFFFFFFF, float(r["phi"]), float(r["fee_rate"]), float(r["sigma"]),
+                                int(r["patience"]))
+
+        def rows(x, what):
+            x = torch.as_tensor(x).detach().cpu().to(torch.float32)
+            x = x.reshape(1, -1) if x.dim() == 1 else x
+            if x.shape[0] == 1 and K > 1:
+                x = x.expand(K, -1)
+            if x.shape[0] != K:
+                raise ValueError(f"{what}: {x.shape[0]} rows for {K} runs")
+            return x
+        m = np.ascontiguousarray(rows(masters, "masters").numpy(), np.float32)
+        if m.shape[1] != genome_len(32):
+            raise ValueError(f"master length {m.shape[1]} != {genome_len(32)} (a sweep runs hidden 32)")
+        a = None
+        if use_arl:
+            if adv_masters is None:
+                raise ValueError("use_arl needs adversary masters")
+            a = np.ascontiguousarray(_as_adv_matrix(rows(adv_masters, "adv_masters")).numpy(), np.float32)
+        cfg = _lib.GaConfig(32, int(bool(use_arl)), int(pop_size), 0, int(pop_size), 0, 0.0, 0, 0.0, 0.0, 0,
+                            int(max_generations), PRECISION_F32)
+        self.G, self.runs = genome_len(32), K
+        self.pop_size, self.max_generations = int(pop_size), int(max_generations)
+        self._h = C.c_void_p()
+        _lib.check(_lib.lib().sgmm_ga_create_sweep(C.byref(self._h), C.byref(cfg), K, arr, m.ctypes.data,
+                                                   None if a is None else a.ctypes.data, self.device, _stream(self.device)))
+
+    def status(self, run):
+        return self._status(run)
+
+    def masters(self, run):
+        """``(mm_master, adv_master, best_val_master)`` of run ``run`` as numpy arrays."""
+        return self._masters(run)
+
+    def history(self, run, n=None):
+        """History columns of run ``run`` over its first ``n`` generations (default: the generations completed so far)."""
+        return self._history(run, n)
 
 
 class DRLEngine:
@@ -643,3 +717,89 @@ class DRLEngine:
         # generation and is loaded back into the returned policy
         self.mm_evolver.master_policy.set_weights(torch.from_numpy(best if improved else mm))
         return self.mm_evolver.master_policy, history
+
+    def train_sweep(self, train_bundle, val_bundle, train_stats, generations=100, *, phis=None, fee_rates=None, seeds=None,
+                    output_prefix="agent", log_every=5, verbose=True):
+        """Train K independent runs with the same launches (:class:`DeviceGASweep`): run r is what ``train`` would do with
+        phi ``phis[r]``, fee rate ``fee_rates[r]`` and seed ``seeds[r]``.  Each argument is a scalar, ``None`` (the
+        engine's own value; ``seeds=None`` draws one key per run as ``train`` does per call) or a list of length K.
+        Every run starts from the engine's current masters and ``mm_evolver.sigma``; the evolvers are left as they are.
+        Run r saves its best-on-validation master to ``{save_dir}/{output_prefix}_run{r}_best_val_{phi_r}.pth`` at the
+        polls where it improved.  Returns a list of ``(policy, history)``, one per run.  Hidden width 32, exact
+        precision, one device."""
+        import torch.distributed as tdist
+        if self.hidden_dim != 32:
+            raise ValueError(f"train_sweep runs hidden_dim=32 only (this engine: {self.hidden_dim}); use train()")
+        if _precision(self.precision, 32) != PRECISION_F32:
+            raise ValueError(f"train_sweep runs the exact path only (this engine: precision={self.precision!r}); use train()")
+        if tdist.is_available() and tdist.is_initialized() and tdist.get_world_size(self.group) > 1:
+            raise ValueError("train_sweep runs on one rank; a multi-rank run shards one GA with train()")
+        given = {k: v for k, v in (("phis", phis), ("fee_rates", fee_rates), ("seeds", seeds)) if isinstance(v, (list, tuple))}
+        lengths = {len(v) for v in given.values()}
+        if len(lengths) > 1:
+            raise ValueError(f"sweep lists of different lengths: { {k: len(v) for k, v in given.items()} }")
+        K = lengths.pop() if lengths else 1
+        if K == 0:
+            raise ValueError("empty sweep lists")
+
+        def per_run(x, default):
+            if isinstance(x, (list, tuple)):
+                return list(x)
+            return [default if x is None else x] * K
+        phi_r = per_run(phis, self.phi)
+        fee_r = per_run(fee_rates, self.fee_rate)
+        seed_r = list(seeds) if isinstance(seeds, (list, tuple)) else (
+            [self._run_seed() for _ in range(K)] if seeds is None else [seeds] * K)
+        dev = torch.cuda.current_device() if self.device is None else int(self.device)
+        train = _cached_bundle(train_bundle, train_stats, self.tick_size, dev)
+        val = _cached_bundle(val_bundle, train_stats, self.tick_size, dev)
+        runs = [{"seed": int(seed_r[r]), "phi": float(phi_r[r]), "fee_rate": float(fee_r[r]), "sigma": float(self.mm_evolver.sigma),
+                 "patience": int(self.patience)} for r in range(K)]
+        ga = DeviceGASweep(self.mm_evolver.master_policy.get_weights(),
+                           self.adv_evolver.master_policy.get_weights() if self.use_arl else None,
+                           runs=runs, pop_size=self.mm_evolver.pop_size, use_arl=self.use_arl,
+                           max_generations=max(1, generations), device=dev)
+        save_paths = [os.path.join(self.save_dir, f"{output_prefix}_run{r}_best_val_{phi_r[r]}.pth") for r in range(K)]
+        saved_val = [-np.inf] * K
+
+        def checkpoint(r, best_val):
+            """as train(): at every poll that saw an improvement, the best-on-validation master of run r"""
+            if best_val > saved_val[r]:
+                saved_val[r] = best_val
+                _, _, best = ga.masters(r)
+                snap = TradingPolicy(hidden_dim=32)
+                snap.set_weights(torch.from_numpy(best))
+                torch.save(snap.state_dict(), save_paths[r])
+
+        out = []
+        try:
+            for gen in range(generations):
+                ga.generation(train, val)                       # K runs: ask + evaluate + tell + validate + select
+                if gen % log_every == 0:
+                    for r in range(K):
+                        h = ga.history(r, gen + 1)
+                        best_so_far = np.maximum.accumulate(h["val_f"])
+                        checkpoint(r, float(best_so_far[gen]))
+                        if verbose:
+                            tag = "*" if (gen == 0 or h["val_f"][gen] > best_so_far[gen - 1]) else ""
+                            arl = "ARL:ON" if self.use_arl else "ARL:OFF"
+                            print(f"Run {r:02d} phi={phi_r[r]} | Gen {gen:03d} | {arl} | Best Train: {h['train_f'][gen]:.2f} | "
+                                  f"Val: {h['val_f'][gen]:.2f}{tag}")
+            for r in range(K):
+                h = ga.history(r, generations)
+                st = ga.status(r)
+                mm, _, best = ga.masters(r)
+                improved = generations > 0 and st["best_val"] > -np.inf
+                if improved:
+                    checkpoint(r, float(st["best_val"]))
+                policy = TradingPolicy(hidden_dim=32)
+                policy.set_weights(torch.from_numpy(best if improved else mm))
+                history = {'gen': list(range(generations)),
+                           'train_f': [np.float64(x) for x in h["train_f"]],
+                           'val_f': [np.float64(x) for x in h["val_f"]],
+                           'train_trades': [int(x) for x in h["train_trades"]],
+                           'val_trades': [int(x) for x in h["val_trades"]]}
+                out.append((policy, history))
+        finally:
+            ga.close()
+        return out

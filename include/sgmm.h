@@ -356,6 +356,41 @@ int sgmm_ga_history_host(sgmm_ga* ga, int32_t n, double* train_f, double* val_f,
                          int32_t* train_trades, int32_t* val_trades, float* sigma, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * A sweep of independent GA runs advanced by the same launches (a phi / fee / seed sweep at the reference's scale,
+ * lambda = 50 on a few days of bars, leaves most of the GPU idle when run one GA at a time).  Every run has its own
+ * initial masters, seed, phi, fee_rate, sigma_0 and patience; use_arl, lambda (cfg.pop_size, PER RUN),
+ * max_generations and the bundles are shared.  Run r is bit-identical to the solo GA (sgmm_ga_create) of its
+ * parameters: its children are drawn from its own master, sigma and seed, every walk CTA applies its run's phi and
+ * fee_rate, and tell / select are one block per run.
+ *   evaluate  the runs*lambda seeded children on the policy-table path (H = 32, exact) at every size, in batches under
+ *             SGMM_EXACT256_BATCH_BYTES in the train bundle's code buffer (ordered per bundle; the first generation
+ *             allocates and must not run under a stream capture -- capture after one eager generation)
+ *   select    tell per run, the runs new masters validated as one population, update per run
+ * Scope: hidden 32, precision SGMM_PRECISION_F32 / SGMM_PRECISION_EXACT (others: SGMM_ERR_UNSUPPORTED), one rank
+ * (a sharded cfg: SGMM_ERR_INVALID).  sgmm_ga_generation / _evaluate / _select / _destroy drive the sweep;
+ * sgmm_ga_buffers and the run-less status / master / history entries refuse a handle of more than one run
+ * (SGMM_ERR_INVALID) -- read it back per run.  The run_* entries accept run 0 of any GA.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+    uint64_t seed;            /* Philox key of the run (adversary: seed ^ 1<<63)                 */
+    double phi, fee_rate;     /* the run's inventory penalty and fee rate (fee_rate bits kept: -0.0 != 0.0) */
+    float sigma;              /* sigma_0 of market maker and adversary                           */
+    int32_t patience;         /* stale generations before sigma halves                           */
+} sgmm_ga_run;
+
+/* cfg gives hidden (32), use_arl, pop_size (lambda PER RUN), max_generations, precision (F32 / EXACT) and an unsharded
+ * layout (shard_first 0, shard_count = pop_size, shard_stride 0); its seed / phi / fee_rate / sigma / patience are not
+ * read.  run: HOST [runs].  mm_masters HOST float[runs][1250], adv_masters HOST float[runs][1250] (NULL without use_arl). */
+int sgmm_ga_create_sweep(sgmm_ga** out, const sgmm_ga_config* cfg, int32_t runs, const sgmm_ga_run* run,
+                         const float* mm_masters, const float* adv_masters, int device, void* stream);
+/* synchronising read-backs of run `run` (0 <= run < runs), HOST pointers as the run-less entries above */
+int sgmm_ga_run_status_host(sgmm_ga* ga, int32_t run, sgmm_ga_status* status, void* stream);
+int sgmm_ga_run_master_host(sgmm_ga* ga, int32_t run, float* mm_master, float* adv_master, float* best_val_master,
+                            void* stream);
+int sgmm_ga_run_history_host(sgmm_ga* ga, int32_t run, int32_t n, double* train_f, double* val_f,
+                             int32_t* train_trades, int32_t* val_trades, float* sigma, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Upstream of the rollout: the per-day window loop of load_signals_bundle
  * (pipeline/agent_trainer.py:47-73).  Inputs are one day's event frame columns (loader2.event_df:
  * askprice1, bidprice1, p_buy_max, p_sell_min; n_events rows, NaN allowed in the last two) and
@@ -393,7 +428,7 @@ int sgmm_trace_analytics_host(int64_t n_traces, int64_t n_steps, const double* w
 
 /* sizeof() of the public structs as this library was compiled, for foreign-function bindings to verify their
  * mirrors: which = 0 sgmm_population, 1 sgmm_rollout_params, 2 sgmm_trace, 3 sgmm_env_state, 4 sgmm_step_info,
- * 5 sgmm_ga_config, 6 sgmm_ga_status; negative for an unknown index. */
+ * 5 sgmm_ga_config, 6 sgmm_ga_status, 7 sgmm_ga_run; negative for an unknown index. */
 int sgmm_abi_sizeof(int which);
 
 /* ---------------------------------------------------------------------------------------------
