@@ -124,46 +124,22 @@ int launch_account(const sgmm_bundle* b, const uint64_t* codes, int64_t count, d
     return check_cuda(cudaGetLastError(), "account_kernel launch");
 }
 
-// The code buffer of a bundle: [count][T] 64-bit codes, grown on demand.  It is scratch of ONE rollout at a time: an eager
-// rollout arriving on another stream than the last user waits for the last user's event; captured rollouts of one bundle
-// must stay on one stream.  An outgrown buffer is freed, unless a capture has used the bundle's buffer (then retired).
-int reserve_codes(const sgmm_bundle* cb, int64_t count, cudaStream_t st, uint64_t** out)
-{
-    sgmm_bundle* b = const_cast<sgmm_bundle*>(cb);
-    std::lock_guard<std::mutex> lock(b->codes_mutex);
-    const size_t want = (size_t)count * (size_t)b->T;
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    if (st) cudaStreamIsCapturing(st, &cap);
-    // another stream used the buffer last: order this rollout after its accounting kernel (a capture cannot wait on an
-    // event recorded outside it -- captured rollouts of one bundle must stay on one stream, as the header says)
-    if (b->codes_busy && b->codes_stream != st && cap == cudaStreamCaptureStatusNone && b->codes_done)
-        if (int rc = check_cuda(cudaStreamWaitEvent(st, b->codes_done, 0), "cudaStreamWaitEvent(code buffer)")) return rc;
-    if (cap != cudaStreamCaptureStatusNone) b->codes_captured = true;
-    if (b->codes_cap < want) {
-        if (cap != cudaStreamCaptureStatusNone) {
-            set_error("the code buffer of the bundle holds %zu codes, this rollout needs %zu: run one rollout of this size outside "
-                      "the stream capture first", b->codes_cap, want);
-            return SGMM_ERR_INVALID;
-        }
-        // a captured CUDA graph may hold the old buffer's address: once any capture has used this bundle's code buffer the
-        // outgrown buffers stay alive until the bundle is destroyed; otherwise cudaFree (which synchronises the device,
-        // so every enqueued user is done) returns the memory now -- no unbounded growth when population sizes vary
-        if (b->codes) { if (b->codes_captured) b->codes_retired.push_back(b->codes); else cudaFree(b->codes); }
-        b->codes = nullptr; b->codes_cap = 0;
-        const size_t grow = want + want / 4;
-        if (int rc = check_cuda(cudaMalloc(&b->codes, grow * sizeof(uint64_t)), "cudaMalloc(code buffer)")) return rc;
-        b->codes_cap = grow;
-    }
-    *out = b->codes;
-    return SGMM_OK;
-}
-
 namespace {
 
-// release_codes; `report` = false leaves the thread's error message alone (an error exit keeps its own message)
-int release(const sgmm_bundle* cb, cudaStream_t st, bool report)
+constexpr int64_t DEFAULT_BATCH_BYTES = (int64_t)2 << 30;
+
+// bytes of scratch a batch may use: SGMM_EXACT256_BATCH_BYTES (read on every call), else 2 GiB
+int64_t batch_bytes()
 {
-    sgmm_bundle* b = const_cast<sgmm_bundle*>(cb);
+    const char* e = getenv("SGMM_EXACT256_BATCH_BYTES");
+    const long long v = e ? atoll(e) : 0;
+    return v > 0 ? (int64_t)v : DEFAULT_BATCH_BYTES;
+}
+
+// records the buffer's event on `st` (not under a capture); `report` = false leaves the thread's error message alone (an
+// error exit keeps its own message)
+int release(sgmm_bundle* b, cudaStream_t st, bool report)
+{
     std::lock_guard<std::mutex> lock(b->codes_mutex);
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     if (st) cudaStreamIsCapturing(st, &cap);
@@ -180,11 +156,61 @@ int release(const sgmm_bundle* cb, cudaStream_t st, bool report)
 
 }  // namespace
 
-int release_codes(const sgmm_bundle* b, cudaStream_t st) { return release(b, st, true); }
-
-CodesRelease::~CodesRelease()
+// The code buffer of a bundle grows in whole rows of T words ([count][T] step codes), so a reservation is rounded up to
+// them.  It is scratch of ONE call at a time: an eager call arriving on another stream than the last user waits for the
+// last user's event; captured calls of one bundle must stay on one stream.  An outgrown buffer is freed, unless a capture
+// has used the bundle's buffer (then retired).
+int ScratchLease::reserve(int64_t words, uint64_t** out)
 {
-    if (pending) release(b, st, false);
+    std::lock_guard<std::mutex> lock(b_->codes_mutex);
+    const int64_t T = b_->T;
+    const size_t want = T > 0 ? (size_t)((words + T - 1) / T) * (size_t)T : 0;
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    if (st_) cudaStreamIsCapturing(st_, &cap);
+    // another stream used the buffer last: order this call after its last kernel (a capture cannot wait on an event
+    // recorded outside it -- captured calls of one bundle must stay on one stream, as the header says)
+    if (b_->codes_busy && b_->codes_stream != st_ && cap == cudaStreamCaptureStatusNone && b_->codes_done)
+        if (int rc = check_cuda(cudaStreamWaitEvent(st_, b_->codes_done, 0), "cudaStreamWaitEvent(code buffer)")) return rc;
+    if (cap != cudaStreamCaptureStatusNone) b_->codes_captured = true;
+    if (b_->codes_cap < want) {
+        if (cap != cudaStreamCaptureStatusNone) {
+            set_error("the code buffer of the bundle holds %zu codes, this rollout needs %zu: run one rollout of this size outside "
+                      "the stream capture first", b_->codes_cap, want);
+            return SGMM_ERR_INVALID;
+        }
+        // a captured CUDA graph may hold the old buffer's address: once any capture has used this bundle's code buffer the
+        // outgrown buffers stay alive until the bundle is destroyed; otherwise cudaFree (which synchronises the device,
+        // so every enqueued user is done) returns the memory now -- no unbounded growth when population sizes vary
+        if (b_->codes) { if (b_->codes_captured) b_->codes_retired.push_back(b_->codes); else cudaFree(b_->codes); }
+        b_->codes = nullptr; b_->codes_cap = 0;
+        const size_t grow = want + want / 4;
+        if (int rc = check_cuda(cudaMalloc(&b_->codes, grow * sizeof(uint64_t)), "cudaMalloc(code buffer)")) return rc;
+        b_->codes_cap = grow;
+    }
+    *out = b_->codes;
+    pending_ = true;
+    return SGMM_OK;
+}
+
+// nb individuals per batch as the budget allows (at least one, at most P), and T words of slack beyond their nb * per_ind
+int ScratchLease::reserve_in_batches(int64_t P, int64_t per_ind, int64_t* nb, uint64_t** out)
+{
+    int64_t n = batch_bytes() / (per_ind * 8 > 0 ? per_ind * 8 : 1);
+    if (n < 1) n = 1;
+    if (n > P) n = P;
+    *nb = n;
+    return reserve(n * per_ind + b_->T, out);
+}
+
+int ScratchLease::done()
+{
+    pending_ = false;
+    return release(b_, st_, true);
+}
+
+ScratchLease::~ScratchLease()
+{
+    if (pending_) release(b_, st_, false);
 }
 
 }  // namespace sgmm

@@ -25,11 +25,17 @@ int check_cuda(cudaError_t e, const char* what)
     return e == cudaErrorMemoryAllocation ? SGMM_ERR_NOMEM : SGMM_ERR_CUDA;
 }
 
-struct DeviceGuard {
-    int prev = -1; bool ok = false;
-    explicit DeviceGuard(int dev) { if (cudaGetDevice(&prev) == cudaSuccess && cudaSetDevice(dev) == cudaSuccess) ok = true; }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
+int sm_count(int device)
+{
+    static std::atomic<int> cached[64];             // 0 = not asked yet
+    const bool tracked = device >= 0 && device < 64;
+    if (tracked)
+        if (const int n = cached[device].load(std::memory_order_relaxed)) return n;
+    int n = 0;
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || n <= 0) return 148;
+    if (tracked) cached[device].store(n, std::memory_order_relaxed);
+    return n;
+}
 
 static int ensure_workspace(sgmm_bundle* b, int slot, size_t bytes)
 {

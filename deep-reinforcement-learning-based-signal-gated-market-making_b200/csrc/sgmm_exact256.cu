@@ -240,23 +240,12 @@ __global__ void __launch_bounds__(256) stage_genomes_kernel(const PopArgs mm_in,
     }
 }
 
-constexpr int64_t DEFAULT_BATCH_BYTES = (int64_t)2 << 30;
-
-// bytes of scratch a batch may use: SGMM_EXACT256_BATCH_BYTES (read on every call), else 2 GiB
-int64_t batch_bytes()
-{
-    const char* e = getenv("SGMM_EXACT256_BATCH_BYTES");
-    const long long v = e ? atoll(e) : 0;
-    return v > 0 ? (int64_t)v : DEFAULT_BATCH_BYTES;
-}
-
 int launch_table(const sgmm_bundle* b, const float* rows, int64_t count, int mode, float2* code, uint8_t* next, cudaStream_t st)
 {
     if (b->T == 0 || count == 0) return SGMM_OK;
     static std::atomic<uint64_t> configured{0};
     if (int rc = opt_in_smem(exact256_table_kernel, sizeof(Smem), configured, "cudaFuncSetAttribute(exact256 smem)")) return rc;
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
+    const int sms = sm_count(b->device);
     const int64_t tasks = count * ((b->T * 5 + BM - 1) / BM);
     const int64_t blocks = tasks < sms ? tasks : sms;
     exact256_table_kernel<<<(unsigned)blocks, THREADS, sizeof(Smem), st>>>(b->sig, b->T, rows, count, mode, code, next);
@@ -265,10 +254,8 @@ int launch_table(const sgmm_bundle* b, const float* rows, int64_t count, int mod
 
 int launch_stage(const sgmm_bundle* b, const PopArgs& mm, int64_t count, float* out, cudaStream_t st)
 {
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
     const int64_t work = count * ((G + 3) / 4);
-    const int64_t want = (work + 255) / 256, cap = (int64_t)sms * 8;
+    const int64_t want = (work + 255) / 256, cap = (int64_t)sm_count(b->device) * 8;
     stage_genomes_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(mm, count, out);
     return check_cuda(cudaGetLastError(), "stage_genomes_kernel launch");
 }
@@ -277,46 +264,23 @@ bool needs_stage(const PopArgs& mm) { return mm.genomes == nullptr || (reinterpr
 
 }  // namespace x256
 
-int reserve_batches(const sgmm_bundle* b, int64_t P, int64_t per_ind, cudaStream_t st, int64_t* nb, uint64_t** buf)
-{
-    const int64_t T = b->T;
-    int64_t n = x256::batch_bytes() / (per_ind * 8 > 0 ? per_ind * 8 : 1);
-    if (n < 1) n = 1;
-    if (n > P) n = P;
-    *nb = n;
-    const int64_t units = T > 0 ? (n * per_ind + T - 1) / T + 1 : 1;           // reserve_codes counts in units of T words
-    return reserve_codes(b, units, st, buf);
-}
-
 // Episodes at H = 256 in SGMM-F32 order (with or without the adversary): batches of individuals, each batch = (staged
-// genomes,) policy table, walk.  The table ([n][T] x 48 B) and the staged genomes ([n] x 269 KB; seeded children, or
-// explicit rows not 8-byte aligned) live in the bundle's grow-only code buffer (sgmm_account.cu), under the byte budget of
-// x256::batch_bytes(); rollouts sharing the buffer are ordered across streams, and the first rollout of a size allocates
-// and must not run under a stream capture.
+// genomes,) policy table, walk (table_walk_batches).  The table ([n][T] x 48 B) and the staged genomes ([n] x 269 KB; seeded
+// children, or explicit rows not 8-byte aligned) live in the bundle's code buffer.
 int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
                     cudaStream_t st)
 {
     using namespace x256;
-    const int64_t T = b->T, P = mm.count;
-    if (P == 0) return SGMM_OK;
-    const bool stage = T > 0 && needs_stage(mm);
-    int64_t nb = 0;
-    uint64_t* buf = nullptr;
-    if (int rc = reserve_batches(b, P, 6 * T + (stage ? G / 2 : 0), st, &nb, &buf)) return rc;
-    CodesRelease release(b, st);
-    float2* code = reinterpret_cast<float2*>(buf);
-    uint8_t* next = reinterpret_cast<uint8_t*>(code + nb * T * 5);
-    float* staged = reinterpret_cast<float*>(buf + nb * T * 6);
-    const int rc = walk_batches(b, mm, adv, nb, code, next, phi, fee, fitness, trades, st, [&](const PopArgs& pm, const PopArgs*, int64_t) {
+    const bool stage = b->T > 0 && needs_stage(mm);
+    return table_walk_batches(b, mm, adv, mm, G, true, stage ? G / 2 : 0, phi, fee, fitness, trades, st,
+                              [&](const PopArgs& pm, const PopArgs*, int64_t, const BatchScratch& s) {
         const float* rows = pm.genomes;
         if (stage) {
-            if (int rc = launch_stage(b, pm, pm.count, staged, st)) return rc;
-            rows = staged;
+            if (int rc = launch_stage(b, pm, pm.count, reinterpret_cast<float*>(s.extra), st)) return rc;
+            rows = reinterpret_cast<float*>(s.extra);
         }
-        return launch_table(b, rows, pm.count, adv ? 1 : 0, code, next, st);
+        return launch_table(b, rows, pm.count, adv ? 1 : 0, s.code, s.next, st);
     });
-    if (rc) return rc;
-    return release.done();
 }
 
 // raw policy outputs (before x5) of ONE explicit genome for every (bar, inventory): out = float2[T][5].  `stage_buf` holds

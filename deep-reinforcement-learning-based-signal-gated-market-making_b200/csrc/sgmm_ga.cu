@@ -159,16 +159,10 @@ struct sgmm_ga {
 };
 
 namespace {
-struct Guard {
-    int prev = -1;
-    explicit Guard(int d) { cudaGetDevice(&prev); cudaSetDevice(d); }
-    ~Guard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-
 // device buffers of ga->runs runs, initial states `init` [runs] and HOST masters [runs][G] / [runs][1250] (adv may be NULL)
 int ga_allocate(sgmm_ga* ga, const GaDev* init, const float* mm_masters, const float* adv_masters, cudaStream_t st)
 {
-    Guard guard(ga->device);
+    DeviceGuard guard(ga->device);
     const size_t R = (size_t)ga->runs, G = (size_t)ga->G, cap = (size_t)ga->capacity, mg = (size_t)ga->cfg.max_generations;
     int rc = SGMM_OK;
     if (!rc) rc = check_cuda(cudaMalloc(&ga->mm_master, R * G * sizeof(float)), "cudaMalloc");
@@ -301,7 +295,7 @@ int sgmm_ga_destroy(sgmm_ga* ga)
 {
     if (!ga) return SGMM_OK;
     {
-        Guard guard(ga->device);
+        DeviceGuard guard(ga->device);
         cudaFree(ga->mm_master); cudaFree(ga->adv_master); cudaFree(ga->best_master);
         cudaFree(ga->gather.base); cudaFree(ga->val_fit); cudaFree(ga->val_trd);
         cudaFree(ga->st); cudaFree(ga->h_train_f); cudaFree(ga->h_val_f); cudaFree(ga->h_train_t);
@@ -329,7 +323,7 @@ int sgmm_ga_evaluate(sgmm_ga* ga, const sgmm_bundle* train, void* stream)
 {
     if (!ga || !train) { set_error("NULL argument"); return SGMM_ERR_INVALID; }
     if (train->device != ga->device) { set_error("bundle and GA live on different devices"); return SGMM_ERR_INVALID; }
-    Guard guard(ga->device);
+    DeviceGuard guard(ga->device);
     const sgmm_ga_config& c = ga->cfg;
     if (ga->sweep) {                                                // run r's children are individuals [r*lambda, (r+1)*lambda)
         const SweepPop mm{ga->mm_master, ga->st, c.pop_size, 0, (int64_t)ga->runs * c.pop_size, 0};
@@ -351,7 +345,7 @@ int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
 {
     if (!ga || !val) { set_error("NULL argument"); return SGMM_ERR_INVALID; }
     if (val->device != ga->device) { set_error("bundle and GA live on different devices"); return SGMM_ERR_INVALID; }
-    Guard guard(ga->device);
+    DeviceGuard guard(ga->device);
     cudaStream_t st = (cudaStream_t)stream;
     const sgmm_ga_config& c = ga->cfg;
     ga_tell_kernel<<<(unsigned)ga->runs, 256, 0, st>>>(ga->st, ga->gather, c.pop_size, ga->mm_master, ga->G,
@@ -389,7 +383,7 @@ int sgmm_ga_run_status_host(sgmm_ga* ga, int32_t run, sgmm_ga_status* status, vo
 {
     if (!ga || !status) { set_error("NULL argument"); return SGMM_ERR_INVALID; }
     if (int rc = check_run(ga, run)) return rc;
-    Guard guard(ga->device);
+    DeviceGuard guard(ga->device);
     GaDev h;
     cudaStream_t st = (cudaStream_t)stream;
     if (int rc = check_cuda(cudaMemcpyAsync(&h, ga->st + run, sizeof h, cudaMemcpyDeviceToHost, st), "D2H ga state")) return rc;
@@ -403,7 +397,7 @@ int sgmm_ga_run_master_host(sgmm_ga* ga, int32_t run, float* mm_master, float* a
 {
     if (!ga) { set_error("ga is NULL"); return SGMM_ERR_INVALID; }
     if (int rc = check_run(ga, run)) return rc;
-    Guard guard(ga->device);
+    DeviceGuard guard(ga->device);
     cudaStream_t st = (cudaStream_t)stream;
     const size_t G = (size_t)ga->G, r = (size_t)run;
     if (mm_master) if (int rc = check_cuda(cudaMemcpyAsync(mm_master, ga->mm_master + r * G, G * sizeof(float), cudaMemcpyDeviceToHost, st), "D2H master")) return rc;
@@ -418,7 +412,7 @@ int sgmm_ga_run_history_host(sgmm_ga* ga, int32_t run, int32_t n, double* train_
     if (!ga || n < 0) { set_error("bad argument"); return SGMM_ERR_INVALID; }
     if (int rc = check_run(ga, run)) return rc;
     if (n > ga->cfg.max_generations) n = ga->cfg.max_generations;
-    Guard guard(ga->device);
+    DeviceGuard guard(ga->device);
     cudaStream_t st = (cudaStream_t)stream;
     const size_t k = (size_t)n, row = (size_t)run * (size_t)ga->cfg.max_generations;
     if (train_f) if (int rc = check_cuda(cudaMemcpyAsync(train_f, ga->h_train_f + row, k * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H history")) return rc;

@@ -52,7 +52,7 @@ struct sgmm_bundle {
     size_t ws_bytes[SGMM_HOST_SLOTS] = {};
     cudaStream_t slot_stream[SGMM_HOST_SLOTS] = {};
     uint64_t async_next = 0;
-    // [count][T] 64-bit step codes of the tensor-core rollouts (sgmm_account.cu), grow-only
+    // grow-only scratch of one call at a time: [count][T] 64-bit step codes, policy tables (ScratchLease, sgmm_account.cu)
     std::mutex codes_mutex;
     uint64_t* codes = nullptr;
     size_t codes_cap = 0;
@@ -126,6 +126,17 @@ struct RolloutArgs {
 void set_error(const char* fmt, ...);
 int check_cuda(cudaError_t e, const char* what);
 
+// Makes `dev` the calling thread's current device for the scope and restores the previous one; ok = the switch worked
+struct DeviceGuard {
+    int prev = -1; bool ok = false;
+    explicit DeviceGuard(int dev) { if (cudaGetDevice(&prev) == cudaSuccess && cudaSetDevice(dev) == cudaSuccess) ok = true; }
+    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+};
+
+// The SM count of `device`, queried once per device (sgmm_capi.cu).  A failed query is not cached and answers 148 (a B200);
+// its error stays the thread's last CUDA error, so the launch check that follows reports it.
+int sm_count(int device);
+
 inline int64_t genome_len(int H) { return (int64_t)H * H + 7 * (int64_t)H + 2; }
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a PER-DEVICE attribute of a kernel: opt in once per (kernel, device).
@@ -153,18 +164,43 @@ constexpr int64_t SMALL_POP_MAX_ADV = 148;  // with the adversary (one 512-threa
 int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
                          cudaStream_t st);
 // the policy table of the small-population path for mm.count individuals (sgmm_one.cu), in the format of `mode`: 0 step code
-// + next inventory, 1 q = raw*5 per (bar, inventory) (adversary walk), 2 raw outputs per (bar, inventory) (population trace)
-int launch_policy_table(const sgmm_bundle* b, const PopArgs& mm, int mode, float2* code, uint8_t* next, cudaStream_t st);
-// the walk + fp64 half of the policy-table path over tables code [P][T][5] / next [P][T][8] (sgmm_one.cu)
-int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const PopArgs* adv, double phi, double fee,
-                double* fitness, int32_t* trades, cudaStream_t st);
+// + next inventory, 1 q = raw*5 per (bar, inventory) (adversary walk), 2 raw outputs per (bar, inventory) (population trace,
+// PopArgs only).  Pop: PopArgs, or SweepPop (the children of a GA sweep).
+template <class Pop>
+int launch_policy_table(const sgmm_bundle* b, const Pop& mm, int mode, float2* code, uint8_t* next, cudaStream_t st);
+// the walk + fp64 half of the policy-table path over tables code [P][T][5] / next [P][T][8] (sgmm_one.cu).  CTA i walks
+// individual i of `pop`: with `adv` pop holds the adversaries (the 20-state walk over q tables; next unused); a SweepPop
+// gives every CTA its run's phi and fee, a PopArgs takes phi / fee (and is not read without the adversary).
+template <class Pop>
+int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const Pop& pop, bool adv, double phi,
+                double fee, double* fitness, int32_t* trades, cudaStream_t st);
 // the market maker's offsets before the adversary's displacement along the Walk20 walk of q tables [P][T][5] (audit, sgmm_one.cu)
 int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, const PopArgs& adv, int32_t* act_trace, cudaStream_t st);
-// H = 256 populations as batches of policy table + walk (sgmm_exact256.cu, and sgmm_spec256.cu with the adversary).  The
-// scratch of a batch, `per_ind` 8-byte words per individual, is the bundle's code buffer (ordered rollouts per bundle; the
-// first rollout of a size must not run under a stream capture) and stays under the byte budget SGMM_EXACT256_BATCH_BYTES
-// (environment, read on every call; default 2 GiB): *nb individuals per batch.
-int reserve_batches(const sgmm_bundle* b, int64_t P, int64_t per_ind, cudaStream_t st, int64_t* nb, uint64_t** buf);
+
+// Scratch of one call in the bundle's grow-only code buffer (sgmm_account.cu).  Calls on one bundle take turns: an eager call
+// on another stream than the buffer's last user waits for that user's event; under a stream capture the buffer cannot grow
+// (the call is refused), and once a capture has used it an outgrown buffer is retired instead of freed.  Build the lease on
+// (bundle, stream), reserve once, enqueue the kernels that use the scratch, then return done(): it records the event and
+// reports its errors.  Any other exit after a successful reserve records the event in the destructor and keeps the error
+// message of that exit.
+class ScratchLease {
+public:
+    ScratchLease(const sgmm_bundle* b, cudaStream_t st) : b_(const_cast<sgmm_bundle*>(b)), st_(st) {}
+    ScratchLease(const ScratchLease&) = delete;
+    ScratchLease& operator=(const ScratchLease&) = delete;
+    ~ScratchLease();
+    // at least `words` 8-byte words at *out
+    int reserve(int64_t words, uint64_t** out);
+    // P individuals of per_ind words each, in batches under the byte budget SGMM_EXACT256_BATCH_BYTES (environment, read on
+    // every call; default 2 GiB): *nb individuals per batch, nb * per_ind words at *out
+    int reserve_in_batches(int64_t P, int64_t per_ind, int64_t* nb, uint64_t** out);
+    int done();
+private:
+    sgmm_bundle* b_;
+    cudaStream_t st_;
+    bool pending_ = false;
+};
+
 // individuals b0 .. b0+n-1 of a population of genome length G
 inline PopArgs batch_of(const PopArgs& p, int64_t b0, int64_t n, int64_t G)
 {
@@ -194,21 +230,43 @@ int for_each_batch(const Pop& mm, const Pop* adv, int64_t nb, int64_t G, Fn fn)
     }
     return SGMM_OK;
 }
-// Batches of at most nb individuals: table(pm, pa, b0) enqueues the policy table (code / next) of individuals b0 .. b0+n-1,
-// pm / pa being those individuals of mm / adv (pa nullptr without the adversary); the walk then writes their fitness / trades.
-template <class Table>
-int walk_batches(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int64_t nb, const float2* code, const uint8_t* next,
-                 double phi, double fee, double* fitness, int32_t* trades, cudaStream_t st, Table table)
+// The scratch of one table-and-walk batch of n individuals: the policy table code [n][T][5], the next-inventory bytes
+// [n][T][8] of the 5-state walk (nullptr when the table kind has none), then `extra` words per individual for the table
+// callback (staged genomes).
+struct BatchScratch {
+    float2* code;
+    uint8_t* next;
+    uint64_t* extra;
+};
+// Episodes of mm.count individuals of genome length G as batches of policy table + walk in the bundle's code buffer
+// (ScratchLease::reserve_in_batches).  table(pm, pa, b0, s) enqueues into s the table of individuals b0 .. b0+n-1, pm / pa being
+// those individuals of mm / adv (pa nullptr without the adversary); the walk then writes their fitness / trades: over the
+// adversaries pa, or else with individuals b0 .. b0+n-1 of `walk` as its CTAs' population -- mm itself, or the runs of a
+// GA sweep whose phi and fee the CTAs take (launch_walk).
+template <class Pop, class WalkPop, class Table>
+int table_walk_batches(const sgmm_bundle* b, const Pop& mm, const Pop* adv, const WalkPop& walk, int64_t G, bool with_next,
+                       int64_t extra, double phi, double fee, double* fitness, int32_t* trades, cudaStream_t st, Table table)
 {
-    return for_each_batch(mm, adv, nb, genome_len(256), [&](const PopArgs& pm, const PopArgs* pa, int64_t b0) {
-        if (int rc = table(pm, pa, b0)) return rc;
-        return launch_walk(b, pm.count, code, next, pa, phi, fee, fitness + b0, trades + b0, st);
+    if (mm.count == 0) return SGMM_OK;
+    const int64_t T = b->T, table_words = (with_next ? 6 : 5) * T;
+    ScratchLease lease(b, st);
+    int64_t nb = 0;
+    uint64_t* buf = nullptr;
+    if (int rc = lease.reserve_in_batches(mm.count, table_words + extra, &nb, &buf)) return rc;
+    const BatchScratch s{reinterpret_cast<float2*>(buf), with_next ? reinterpret_cast<uint8_t*>(buf + nb * T * 5) : nullptr,
+                         buf + nb * table_words};
+    const int rc = for_each_batch(mm, adv, nb, G, [&](const Pop& pm, const Pop* pa, int64_t b0) {
+        if (int rc = table(pm, pa, b0, s)) return rc;
+        if (pa) return launch_walk(b, pm.count, s.code, nullptr, *pa, true, phi, fee, fitness + b0, trades + b0, st);
+        return launch_walk(b, pm.count, s.code, s.next, batch_of(walk, b0, pm.count, G), false, phi, fee, fitness + b0,
+                           trades + b0, st);
     });
+    if (rc) return rc;
+    return lease.done();
 }
 // GA sweeps at H = 32, exact (sgmm_one.cu).  launch_sweep_population: the mm.count seeded children of mm (and adv) on the
-// policy-table path at every size, in batches under SGMM_EXACT256_BATCH_BYTES in the bundle's code buffer; every walk CTA
-// takes its run's phi and fee.  launch_sweep_validation: K explicit masters [K][1250] (adversary off), walk CTA r with run
-// r's phi and fee.
+// policy-table path at every size, in batches (table_walk_batches); every walk CTA takes its run's phi and fee.
+// launch_sweep_validation: K explicit masters [K][1250] (adversary off), walk CTA r with run r's phi and fee.
 int launch_sweep_population(const sgmm_bundle* b, const SweepPop& mm, const SweepPop* adv, double* fitness, int32_t* trades,
                             cudaStream_t st);
 int launch_sweep_validation(const sgmm_bundle* b, const float* masters, const GaDev* runs, int64_t K, double* fitness,
@@ -244,21 +302,6 @@ int launch_population(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* ad
 int launch_tc32_prologue(sgmm_bundle* b, cudaStream_t st);
 int launch_account(const sgmm_bundle* b, const uint64_t* codes, int64_t count, double phi, double fee, double* fitness,
                    int32_t* trades, cudaStream_t st, bool float_offsets = false);
-int reserve_codes(const sgmm_bundle* b, int64_t count, cudaStream_t st, uint64_t** out);
-int release_codes(const sgmm_bundle* b, cudaStream_t st);      // after the last kernel that reads the codes was enqueued
-// Scope guard of a successful reserve_codes / reserve_batches: done() is release_codes on the success path; any other exit
-// (an error return after some kernels were enqueued) still records the bundle's event on `st`, so that the next user on
-// another stream waits for the work already enqueued.  The error message of that exit is kept.
-struct CodesRelease {
-    const sgmm_bundle* b;
-    cudaStream_t st;
-    bool pending = true;
-    CodesRelease(const sgmm_bundle* bundle, cudaStream_t stream) : b(bundle), st(stream) {}
-    CodesRelease(const CodesRelease&) = delete;
-    CodesRelease& operator=(const CodesRelease&) = delete;
-    int done() { pending = false; return release_codes(b, st); }
-    ~CodesRelease();
-};
 size_t tc32_a1_bytes(int64_t T);
 int launch_prologue(sgmm_bundle* b, const float* z1, const float* z2, const double* mid,
                     const double* ask, const double* bid, cudaStream_t st);

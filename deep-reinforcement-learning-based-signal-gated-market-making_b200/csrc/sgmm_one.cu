@@ -20,6 +20,7 @@
 // (tests/test_gpu_configs.py compares both with the oracle; the GA parity tests compare whole histories).  One CTA of
 // walk_account_kernel per individual; the launcher takes this path below SMALL_POP_MAX individuals (measured break-even
 // against the sequential kernel: profiles/r2_small_population_path.log).
+#include <type_traits>
 #include "sgmm_internal.h"
 #include "sgmm_rng.cuh"
 #include "sgmm_adversary.cuh"
@@ -351,34 +352,13 @@ __global__ void __launch_bounds__(32) adv_offsets_kernel(const BarSig* __restric
 
 }  // namespace one
 
-// Episodes of a small population on `b` (H = 32, exact SGMM-F32 order, with or without the adversary) through the kernels above.  The
-// policy table ([count][T] x 48 B) lives in the bundle's grow-only code buffer (sgmm_account.cu: rollouts sharing it are
-// ordered across streams; the first rollout of a size allocates and must not run under a stream capture).
-int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
-                         cudaStream_t st)
-{
-    using namespace one;
-    const int64_t T = b->T, P = mm.count;
-    if (P == 0) return SGMM_OK;
-    uint64_t* buf = nullptr;
-    if (int rc = reserve_codes(b, P * 6 + 1, st, &buf)) return rc;               // 48 B per (individual, bar) + slack for T == 0
-    CodesRelease release(b, st);
-    float2* code = reinterpret_cast<float2*>(buf);
-    uint8_t* next = reinterpret_cast<uint8_t*>(code + P * T * 5);
-    if (int rc = launch_policy_table(b, mm, adv ? 1 : 0, code, next, st)) return rc;
-    if (int rc = launch_walk(b, P, code, next, adv, phi, fee, fitness, trades, st)) return rc;
-    return release.done();
-}
-
 namespace one {
 // grid and pairs per task of policy_table_kernel for P individuals: task = (individual, range of pairs), ranges of whole
 // 128-pair rounds, sized so that the GPU gets ~8 blocks per SM
 static unsigned policy_table_grid(const sgmm_bundle* b, int64_t P, bool seeded, int64_t* pairs_per_task)
 {
     const int64_t T = b->T;
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
-    const int64_t want_blocks = (int64_t)sms * 8;
+    const int64_t want_blocks = (int64_t)sm_count(b->device) * 8;
     int64_t ppt = (P * T * 5 + want_blocks - 1) / want_blocks;
     ppt = (ppt + 2 * PT_THREADS - 1) / (2 * PT_THREADS) * (2 * PT_THREADS);
     const int64_t ppt_min = seeded ? 4 * PT_THREADS : 2 * PT_THREADS;          // seeded children: staging costs ~10 Philox calls per thread
@@ -389,92 +369,81 @@ static unsigned policy_table_grid(const sgmm_bundle* b, int64_t P, bool seeded, 
     return (unsigned)(blocks < 1 ? 1 : blocks);
 }
 
-// the walk of P individuals over tables code / next: adversary off (Walk5) or on (Walk20, the adversaries from runs); CTA i
-// takes the phi and fee of the run of sweep individual runs.first + i
-static int launch_sweep_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const SweepPop& runs, bool adv,
-                             double* fitness, int32_t* trades, cudaStream_t st)
+static bool seeded(const PopArgs& p) { return p.genomes == nullptr; }
+static bool seeded(const SweepPop&) { return true; }
+
+// the table callback of table_walk_batches on this path: step codes + next inventory, or q tables with the adversary
+inline auto policy_tables(const sgmm_bundle* b, cudaStream_t st)
 {
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
-    if (adv) walk_account_kernel<Walk20, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, b->T, code, nullptr, runs, b->tick, 0.0, 0.0, fitness, trades);
-    else if (P <= sms) walk_account_kernel<Walk5, 1024><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, b->T, code, next, runs, b->tick, 0.0, 0.0, fitness, trades);
-    else walk_account_kernel<Walk5, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, b->T, code, next, runs, b->tick, 0.0, 0.0, fitness, trades);
-    return check_cuda(cudaGetLastError(), "walk_account_kernel launch (sweep)");
+    return [b, st](const auto& pm, const auto* pa, int64_t, const BatchScratch& s) {
+        return launch_policy_table(b, pm, pa ? 1 : 0, s.code, s.next, st);
+    };
 }
 }  // namespace one
 
-int launch_policy_table(const sgmm_bundle* b, const PopArgs& mm, int mode, float2* code, uint8_t* next, cudaStream_t st)
+template <class Pop>
+int launch_policy_table(const sgmm_bundle* b, const Pop& mm, int mode, float2* code, uint8_t* next, cudaStream_t st)
 {
     using namespace one;
     const int64_t T = b->T, P = mm.count;
     if (T == 0 || P == 0) return SGMM_OK;
     int64_t ppt = 0;
-    const unsigned grid = policy_table_grid(b, P, mm.genomes == nullptr, &ppt);
-    if (mode == 2) policy_table_kernel<true><<<grid, PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, 0, code, next);
-    else policy_table_kernel<false><<<grid, PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, mode, code, next);
+    const unsigned grid = policy_table_grid(b, P, seeded(mm), &ppt);
+    if constexpr (std::is_same<Pop, PopArgs>::value)          // raw outputs: the population trace (no sweep instantiation)
+        if (mode == 2) {
+            policy_table_kernel<true><<<grid, PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, 0, code, next);
+            return check_cuda(cudaGetLastError(), "policy_table_kernel launch");
+        }
+    policy_table_kernel<false><<<grid, PT_THREADS, 0, st>>>(b->sig, T, mm, ppt, mode, code, next);
     return check_cuda(cudaGetLastError(), "policy_table_kernel launch");
 }
 
-int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const PopArgs* adv, double phi, double fee,
-                double* fitness, int32_t* trades, cudaStream_t st)
+template <class Pop>
+int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const Pop& pop, bool adv, double phi,
+                double fee, double* fitness, int32_t* trades, cudaStream_t st)
 {
     using namespace one;
     const int64_t T = b->T;
-    int sms2 = 148;
-    cudaDeviceGetAttribute(&sms2, cudaDevAttrMultiProcessorCount, b->device);
-    const PopArgs none = {};
-    if (adv) walk_account_kernel<Walk20, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, nullptr, *adv, b->tick, phi, fee, fitness, trades);
-    else if (P <= sms2) walk_account_kernel<Walk5, 1024><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, T, code, next, none, b->tick, phi, fee, fitness, trades);
-    else walk_account_kernel<Walk5, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, next, none, b->tick, phi, fee, fitness, trades);
+    if (adv) walk_account_kernel<Walk20, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, nullptr, pop, b->tick, phi, fee, fitness, trades);
+    else if (P <= sm_count(b->device)) walk_account_kernel<Walk5, 1024><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, T, code, next, pop, b->tick, phi, fee, fitness, trades);
+    else walk_account_kernel<Walk5, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, next, pop, b->tick, phi, fee, fitness, trades);
     return check_cuda(cudaGetLastError(), "walk_account_kernel launch");
+}
+
+template int launch_policy_table<PopArgs>(const sgmm_bundle*, const PopArgs&, int, float2*, uint8_t*, cudaStream_t);
+template int launch_policy_table<SweepPop>(const sgmm_bundle*, const SweepPop&, int, float2*, uint8_t*, cudaStream_t);
+template int launch_walk<PopArgs>(const sgmm_bundle*, int64_t, const float2*, const uint8_t*, const PopArgs&, bool, double, double,
+                                  double*, int32_t*, cudaStream_t);
+template int launch_walk<SweepPop>(const sgmm_bundle*, int64_t, const float2*, const uint8_t*, const SweepPop&, bool, double, double,
+                                   double*, int32_t*, cudaStream_t);
+
+// Episodes of a small population on `b` (H = 32, exact SGMM-F32 order, with or without the adversary) through the kernels
+// above.  The policy table ([count][T] x 48 B) lives in the bundle's code buffer, as batches of table_walk_batches: one
+// batch at the default budget.
+int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
+                         cudaStream_t st)
+{
+    return table_walk_batches(b, mm, adv, mm, genome_len(32), true, 0, phi, fee, fitness, trades, st, one::policy_tables(b, st));
 }
 
 // The K*lambda children of a GA sweep take the policy-table path whatever their number (a solo GA of more than
 // SMALL_POP_MAX children runs rollout_kernel_h32, which gives the same bits).  The table ([n][T] x 48 B) lives in the
-// bundle's code buffer, in batches of n individuals under SGMM_EXACT256_BATCH_BYTES; a batch may start inside a run.
+// bundle's code buffer, in batches of n individuals; a batch may start inside a run.  phi / fee are the runs'.
 int launch_sweep_population(const sgmm_bundle* b, const SweepPop& mm, const SweepPop* adv, double* fitness, int32_t* trades,
                             cudaStream_t st)
 {
-    using namespace one;
-    const int64_t T = b->T, P = mm.count;
-    if (P == 0) return SGMM_OK;
-    int64_t nb = 0;
-    uint64_t* buf = nullptr;
-    if (int rc = reserve_batches(b, P, 6 * T, st, &nb, &buf)) return rc;
-    CodesRelease release(b, st);
-    float2* code = reinterpret_cast<float2*>(buf);
-    uint8_t* next = reinterpret_cast<uint8_t*>(code + nb * T * 5);
-    const int rc = for_each_batch(mm, adv, nb, genome_len(32), [&](const SweepPop& pm, const SweepPop* pa, int64_t b0) {
-        if (T > 0) {
-            int64_t ppt = 0;
-            const unsigned grid = policy_table_grid(b, pm.count, true, &ppt);
-            policy_table_kernel<false><<<grid, PT_THREADS, 0, st>>>(b->sig, T, pm, ppt, pa ? 1 : 0, code, next);
-            if (int rc = check_cuda(cudaGetLastError(), "policy_table_kernel launch (sweep)")) return rc;
-        }
-        return launch_sweep_walk(b, pm.count, code, next, pa ? *pa : pm, pa != nullptr, fitness + b0, trades + b0, st);
-    });
-    if (rc) return rc;
-    return release.done();
+    return table_walk_batches(b, mm, adv, mm, genome_len(32), true, 0, 0.0, 0.0, fitness, trades, st, one::policy_tables(b, st));
 }
 
-// The K masters of a sweep, contiguous [K][1250] rows, as one explicit population: one table, K walk CTAs with per-run phi
-// and fee, adversary off (as the validation of a solo GA)
+// The K masters of a sweep, contiguous [K][1250] rows, as one explicit population (adversary off, as the validation of a
+// solo GA); the walk's CTA r takes run r's phi and fee
 int launch_sweep_validation(const sgmm_bundle* b, const float* masters, const GaDev* runs, int64_t K, double* fitness,
                             int32_t* trades, cudaStream_t st)
 {
-    using namespace one;
-    if (K == 0) return SGMM_OK;
-    uint64_t* buf = nullptr;
-    if (int rc = reserve_codes(b, K * 6 + 1, st, &buf)) return rc;              // 48 B per (individual, bar) + slack for T == 0
-    CodesRelease release(b, st);
-    float2* code = reinterpret_cast<float2*>(buf);
-    uint8_t* next = reinterpret_cast<uint8_t*>(code + K * b->T * 5);
     PopArgs pm{};
     pm.genomes = masters; pm.count = K;
-    if (int rc = launch_policy_table(b, pm, 0, code, next, st)) return rc;
     const SweepPop all{nullptr, runs, 1, 0, K, 0};
-    if (int rc = launch_sweep_walk(b, K, code, next, all, false, fitness, trades, st)) return rc;
-    return release.done();
+    return table_walk_batches(b, pm, (const PopArgs*)nullptr, all, genome_len(32), true, 0, 0.0, 0.0, fitness, trades, st, one::policy_tables(b, st));
 }
 
 int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, const PopArgs& adv, int32_t* act_trace, cudaStream_t st)

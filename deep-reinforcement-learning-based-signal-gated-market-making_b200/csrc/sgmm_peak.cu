@@ -58,7 +58,7 @@ extern "C" int sgmm_measure_fp32_peak(int device, double* tflops, void* stream)
     if (!tflops) { set_error("tflops is NULL"); return SGMM_ERR_INVALID; }
     int prev = 0; cudaGetDevice(&prev);
     if (int rc = check_cuda(cudaSetDevice(device), "cudaSetDevice")) return rc;
-    int sms = 0; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    const int sms = sm_count(device);
     float* d_out = nullptr;
     int rc = check_cuda(cudaMalloc(&d_out, 256), "cudaMalloc");
     double a = 0.0, b = 0.0;

@@ -495,8 +495,6 @@ static int launch_u(const RolloutArgs& args, bool adv, bool fee, int warps, cuda
     return fee ? launch_variant<U, false, true>(args, warps, st) : launch_variant<U, false, false>(args, warps, st);
 }
 
-static int g_sm_count[64] = {0};
-
 int launch_rollout(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int hidden,
                    double phi, double fee, int units_per_lane, int warps_per_cta,
                    double* fitness, int32_t* trades, cudaStream_t st)
@@ -512,13 +510,7 @@ int launch_rollout(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, 
         if (units_per_lane == 0 && warps_per_cta == 0 && mm.count <= (adv ? adv_max : small_max))
             return launch_rollout_small(b, mm, adv, phi, fee, fitness, trades, st);
     }
-    int dev = b->device;
-    if (dev >= 0 && dev < 64 && g_sm_count[dev] == 0) {
-        int n = 0;
-        if (int rc = check_cuda(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev), "query SM count")) return rc;
-        g_sm_count[dev] = n;
-    }
-    const int sms = (dev >= 0 && dev < 64 && g_sm_count[dev] > 0) ? g_sm_count[dev] : 148;
+    const int sms = sm_count(b->device);
     int U = units_per_lane;
     // auto: a whole warp per individual while that still leaves at most one compute warp per scheduler (the step of a
     // lone warp is latency-bound and shortest with 32 lanes per individual: P = 50 x 14 400 bars 2.49 instead of 2.87 ms,
@@ -689,18 +681,17 @@ int launch_trace(const sgmm_bundle* b, const float* mm_genome, int hidden, const
         // the policy of every (bar, inventory) first (exact H = 256 table, raw outputs), then the same trace kernel on it
         a.mm = nullptr;
         if (mm_genome && !forced && !table) {
+            ScratchLease lease(b, st);
             uint64_t* buf = nullptr;
-            const int64_t words = 5 * b->T + genome_len(256) / 2;               // float2[T][5] + room for one staged genome, reserved
-                                                                                 // whether or not the genome needs staging (269 KB)
-            if (int rc = reserve_codes(b, b->T > 0 ? (words + b->T - 1) / b->T : 1, st, &buf)) return rc;
-            CodesRelease release(b, st);
+            // float2[T][5] + room for one staged genome, reserved whether or not the genome needs staging (269 KB)
+            if (int rc = lease.reserve(5 * b->T + genome_len(256) / 2, &buf)) return rc;
             float2* raw = reinterpret_cast<float2*>(buf);
             if (b->T > 0)
                 if (int rc = launch_exact256_raw(b, mm_genome, raw, reinterpret_cast<float*>(buf + 5 * b->T), st)) return rc;
             a.raw = raw;
             trace_kernel_h32<<<1, 32, 0, st>>>(a);
             if (int rc = check_cuda(cudaGetLastError(), "trace_kernel_h32 launch")) return rc;
-            return release.done();
+            return lease.done();
         }
     }
     trace_kernel_h32<<<1, 32, 0, st>>>(a);

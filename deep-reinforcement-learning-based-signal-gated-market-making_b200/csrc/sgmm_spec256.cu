@@ -653,8 +653,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) spec256_kernel(const Args a)
 template <bool FEE, bool QTAB>
 int launch_kernel(const sgmm_bundle* b, const Args& a, cudaStream_t st)
 {
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
+    const int sms = sm_count(b->device);
     const int grid = (int)(a.mm.count < sms ? a.mm.count : sms);
     const size_t smem = sizeof(Smem) + 1024;
     static std::atomic<uint64_t> configured{0};       // per instantiation, one bit per device
@@ -673,39 +672,32 @@ int launch_spec256(const sgmm_bundle* b, const PopArgs& mm, double phi, double f
     Args a{};
     a.sig = b->sig; a.px = b->px; a.T = b->T; a.tick = b->tick; a.phi = phi; a.fee = fee;
     a.mm = mm; a.fitness = fitness; a.trades = trades; a.raw_table = raw_table; a.act_trace = act_trace;
-    if (int rc = reserve_codes(b, mm.count, st, &a.codes)) return rc;
-    CodesRelease release(b, st);
+    ScratchLease lease(b, st);
+    if (int rc = lease.reserve(mm.count * b->T, &a.codes)) return rc;
     if (int rc = fee != 0.0 ? launch_kernel<true, false>(b, a, st) : launch_kernel<false, false>(b, a, st)) return rc;
     if (int rc = launch_account(b, a.codes, mm.count, phi, fee, fitness, trades, st)) return rc;   // the fp64 half, after the tensor-core kernel
-    return release.done();
+    return lease.done();
 }
 
 // With the adversary: batches of (spec256_kernel<false, true> -> q table [n][T][5], 40 B per individual and bar, in the
-// bundle's code buffer under the budget of batch_bytes(); walk_account_kernel<Walk20> over it).  Seeded children need no
-// staging: the kernel regenerates them.  Audit: raw_table comes from the same kernel, act_trace (the market maker's offsets
-// before the displacement) from a replay of the walk over the table (launch_adv_offsets).
+// bundle's code buffer; walk_account_kernel<Walk20> over it) through table_walk_batches.  Seeded children need no staging:
+// the kernel regenerates them.  Audit: raw_table comes from the same kernel, act_trace (the market maker's offsets before the
+// displacement) from a replay of the walk over the table (launch_adv_offsets).
 int launch_spec256_adv(const sgmm_bundle* b, const PopArgs& mm, const PopArgs& adv, double phi, double fee, double* fitness,
                        int32_t* trades, float* raw_table, int32_t* act_trace, cudaStream_t st)
 {
     using namespace s256;
     const int64_t T = b->T;
-    if (mm.count == 0) return SGMM_OK;
-    int64_t nb = 0;
-    uint64_t* buf = nullptr;
-    if (int rc = reserve_batches(b, mm.count, 5 * T, st, &nb, &buf)) return rc;
-    CodesRelease release(b, st);
-    float2* q = reinterpret_cast<float2*>(buf);
     Args a{};
-    a.sig = b->sig; a.px = b->px; a.T = T; a.tick = b->tick; a.phi = phi; a.fee = fee; a.qtab = q;
-    const int rc = walk_batches(b, mm, &adv, nb, q, nullptr, phi, fee, fitness, trades, st,
-                                [&](const PopArgs& pm, const PopArgs* pa, int64_t b0) {
+    a.sig = b->sig; a.px = b->px; a.T = T; a.tick = b->tick; a.phi = phi; a.fee = fee;
+    return table_walk_batches(b, mm, &adv, mm, genome_len(256), false, 0, phi, fee, fitness, trades, st,
+                              [&](const PopArgs& pm, const PopArgs* pa, int64_t b0, const BatchScratch& s) {
         a.mm = pm;
+        a.qtab = s.code;
         a.raw_table = raw_table ? raw_table + b0 * T * 10 : nullptr;
         if (int rc = launch_kernel<false, true>(b, a, st)) return rc;      // FEE is not read by the kernel body
-        return act_trace ? launch_adv_offsets(b, pm.count, q, *pa, act_trace + b0 * T * 2, st) : SGMM_OK;
+        return act_trace ? launch_adv_offsets(b, pm.count, s.code, *pa, act_trace + b0 * T * 2, st) : SGMM_OK;
     });
-    if (rc) return rc;
-    return release.done();
 }
 
 }  // namespace sgmm

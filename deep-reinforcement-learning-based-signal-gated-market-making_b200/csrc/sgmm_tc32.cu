@@ -1416,8 +1416,7 @@ int launch_tc32(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, dou
     a.sig = b->sig; a.px = b->px; a.a1 = b->a1 + (mode == M_F16 ? tc32_chunks(b->T) * A1_BYTES : 0); a.T = b->T; a.tick = b->tick; a.phi = phi; a.fee = fee;
     a.mm = mm; a.fitness = fitness; a.trades = trades; a.raw_table = raw_table; a.act_trace = act_trace;
     if (adv) a.adv = *adv; else { PopArgs z = {}; a.adv = z; }
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
+    const int sms = sm_count(b->device);
     a.group = (group >= 2 && group <= GMAX && group % 2 == 0) ? group : tc32_group_size(mm.count, sms);
     const int64_t groups = (mm.count + a.group - 1) / a.group;
     const int grid = (int)(groups < sms ? groups : sms);

@@ -270,7 +270,7 @@ int launch_kernel(const Args& args, int64_t n, cudaStream_t st)
 
 }  // namespace tpop
 
-// Traces of mm.count individuals, in batches under the byte budget of x256::batch_bytes(): the raw table ([n][T] x 40 B, plus
+// Traces of mm.count individuals, in batches (ScratchLease::reserve_in_batches): the raw table ([n][T] x 40 B, plus
 // the staged genomes at H = 256 when seeded or unaligned) lives in the bundle's code buffer (rollouts sharing it are ordered
 // across streams; the first call of a size allocates and must not run under a stream capture).  Batch b0 writes rows b0 ...
 // of the caller's columns.
@@ -280,10 +280,10 @@ int launch_trace_population(const sgmm_bundle* b, const PopArgs& mm, const PopAr
     const int64_t T = b->T, P = mm.count, G = genome_len(hidden);
     if (P == 0) return SGMM_OK;
     const bool stage = hidden == 256 && T > 0 && x256::needs_stage(mm);
+    ScratchLease lease(b, st);
     int64_t nb = 0;
     uint64_t* buf = nullptr;
-    if (int rc = reserve_batches(b, P, 5 * T + (stage ? G / 2 : 0), st, &nb, &buf)) return rc;
-    CodesRelease release(b, st);
+    if (int rc = lease.reserve_in_batches(P, 5 * T + (stage ? G / 2 : 0), &nb, &buf)) return rc;
     float2* raw = reinterpret_cast<float2*>(buf);
     float* staged = reinterpret_cast<float*>(buf + nb * T * 5);
     sgmm_trace none = {};
@@ -316,7 +316,7 @@ int launch_trace_population(const sgmm_bundle* b, const PopArgs& mm, const PopAr
         return pa ? tpop::launch_kernel<tpop::RawWalk20>(args, pm.count, st) : tpop::launch_kernel<tpop::RawWalk5>(args, pm.count, st);
     });
     if (rc) return rc;
-    return release.done();
+    return lease.done();
 }
 
 }  // namespace sgmm

@@ -158,7 +158,9 @@ typedef struct {
  * individuals, 148 with an adversary; exact precision, default launch geometry) take the policy-table path instead (the
  * exact policy for every (bar, inventory) in parallel + a prefix scan over the inventory automaton, bit-identical results):
  * its table ([count][T] x 48 B) lives in the same grow-only code buffer of the bundle, so the same two rules apply to them,
- * and to every SGMM_PRECISION_EXACT rollout at H = 256 (the same table path, in batches).
+ * and to every SGMM_PRECISION_EXACT rollout at H = 256 (the same table path).  Both run in batches under the byte budget
+ * SGMM_EXACT256_BATCH_BYTES: a small population is one batch at the default 2 GiB (P <= 400, T up to ~111 000 bars); a
+ * smaller budget may split it, with identical results.
  * The tensor-core precisions with an adversary read a per-(bundle, fee_rate) table of the reference's exact fp64 P&L legs
  * (144 B per bar), built on the first such rollout: that first rollout must not run under a stream capture either (refused
  * with SGMM_ERR_INVALID).  Eager users on other streams wait for the build.  Fee rates are keyed by their bits (-0.0 and 0.0

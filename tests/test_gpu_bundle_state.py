@@ -43,7 +43,7 @@ SEED, GEN, FIRST, SIGMA, ADV_SIGMA = 31, 3, 5, 0.05, 0.1
 #   scratch layouts (words of 8 B the call reserves in the code buffer, default batch budget):
 #     "table"  (6P + 1) T                         small-population path (sgmm_one.cu)
 #     "codes"  P T                                spec256 step codes (sgmm_spec256.cu)
-#     "batch"  (floor((P w + T - 1) / T) + 1) T   reserve_batches with w words per individual (exact256, spec256 + adversary,
+#     "batch"  (floor((P w + T - 1) / T) + 1) T   batches of w words per individual (exact256, spec256 + adversary,
 #                                                 population trace)
 #     "trace"  ceil((5 T + G/2) / T) T            single H = 256 trace (sgmm_rollout.cu)
 ROUTES = {
@@ -70,13 +70,13 @@ def count_of(name, size):
 
 
 def batch_words(name, T):
-    """Words per individual of a batched route (reserve_batches' per_ind)."""
+    """Words per individual of a batched route (ScratchLease::reserve_in_batches' per_ind)."""
     return {"spec256_adv": 5 * T, "exact256": 6 * T, "exact256_seeded_adv": 6 * T + G256 // 2, "tracepop32_adv": 5 * T,
             "tracepop256_seeded": 5 * T + G256 // 2}[name]
 
 
 def footprint(name, size, T, batch_bytes=2 << 30):
-    """8-byte words of the bundle's code buffer a call reserves (sgmm_account.cu reserve_codes, sgmm_exact256.cu reserve_batches)."""
+    """8-byte words of the bundle's code buffer a call reserves (sgmm_account.cu ScratchLease)."""
     P, kind = count_of(name, size), ROUTES[name][5]
     if kind is None:
         return 0
@@ -92,7 +92,7 @@ def footprint(name, size, T, batch_bytes=2 << 30):
 
 
 def capacity(words):
-    return words + words // 4          # reserve_codes allocates 1.25x what it was asked for
+    return words + words // 4          # the lease allocates 1.25x what it was asked for
 
 
 def pair_kind(x, y, case, T):
