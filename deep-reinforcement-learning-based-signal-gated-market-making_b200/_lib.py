@@ -12,6 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libsgmm_b200.so")
 
 OK, ERR_INVALID, ERR_CUDA, ERR_NOMEM, ERR_UNSUPPORTED = 0, -1, -2, -3, -4
+MAX_PARENTS = 1024          # SGMM_MAX_PARENTS
 
 
 class SgmmLibraryError(RuntimeError):
@@ -135,6 +136,9 @@ SIGNATURES = {
     "sgmm_ga_run_master_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_ga_run_history_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                            C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sgmm_ga_set_parents": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
+    "sgmm_ga_run_parents_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sgmm_ga_parents_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_bundle_windows": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_bundle_windows_host": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,

@@ -4,7 +4,8 @@
 //   ask       children are never materialised: the rollout kernel regenerates child i from
 //             (master, sigma, seed, generation, i) with the counter-based noise of sgmm_rng.cuh
 //   tell      argmax with numpy's semantics (first maximum, a NaN wins) -> master <- that child
-//             (model.py:73-76); the adversary is told -fitness (drl_engine.py:123-125)
+//             (model.py:73-76); the adversary is told -fitness (drl_engine.py:123-125).  After sgmm_ga_set_parents:
+//             the mu best children (device top-k) recombined into master + sigma * sum_k w_k eps_k instead
 //   validate  rollout of the new master (== best child, drl_engine.py:129-140) with no adversary
 //   select    keep-best-on-validation snapshot (:144-150), sigma halving after `patience` stale
 //             generations (:155-160), history (:163-167)
@@ -12,7 +13,9 @@
 // table and one walk (sgmm_one.cu), one tell block and one update block per run, the K new masters validated as one
 // population.  Each run's state is its own GaDev (sgmm_internal.h) and history row; run r is bit-identical to the solo GA
 // of its seed, phi, fee, sigma and patience.  A GA from sgmm_ga_create is the one-run case of the same kernels.
+#include <cmath>
 #include <new>
+#include <vector>
 #include "sgmm_internal.h"
 #include "sgmm_rng.cuh"
 
@@ -138,6 +141,182 @@ __global__ void __launch_bounds__(256) ga_update_kernel(GaDev* runs, const doubl
     }
 }
 
+// ---- truncation selection (sgmm_ga_set_parents): the mu best children of a run, in rank order, recombined into the new
+// master m + sigma * sum_k w_k eps_k.  The rank order is ga_tell_kernel's: NaN first, then descending fitness (adversary:
+// descending -fitness), ties to the lower index, -0.0 == +0.0; with mu = 1 parent 0 is block_argmax's child.
+constexpr int SELECT_THREADS = 512;
+constexpr int RECOMBINE_THREADS = 64;
+
+// Order-preserving 64-bit key of a fitness value, larger = ranked first: NaN is the maximum, -0.0 is canonicalised and
+// SIGN = -1 ranks -fitness.  Every real key lies in [0x000F..F, 0xFFF0..0], so 0 is free for padding.
+template <int SIGN>
+__device__ __forceinline__ uint64_t rank_key(double v)
+{
+    if (v != v) return ~0ull;
+    uint64_t b = (uint64_t)__double_as_longlong(v == 0.0 ? 0.0 : v);
+    b = (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+    return SIGN > 0 ? b : ~b;
+}
+
+// Visits the children first .. first+n-1 of the gather buffer in index order, nt at a time, without a division per child:
+// every thread of the block makes every call (the loop bounds are uniform), thread t with child base + t, or with
+// valid == false past the end.  f(i, key, valid) gets the index relative to `first`.
+template <int SIGN, class F>
+__device__ __forceinline__ void for_children(const Gather& g, int64_t first, int64_t n, F&& f)
+{
+    const int64_t end = first + n;
+    for (int64_t b = first / g.stride; b * g.stride < end; ++b) {
+        const int64_t b0 = b * g.stride, lo = max(first, b0), hi = min(end, b0 + g.stride);
+        const double* fb = g.fit_block(b);
+        for (int64_t base = lo; base < hi; base += blockDim.x) {
+            const int64_t gi = base + threadIdx.x;
+            const bool valid = gi < hi;
+            f(gi - first, valid ? rank_key<SIGN>(fb[gi - b0]) : 0ull, valid);
+        }
+    }
+}
+
+struct SelectSmem {
+    uint64_t key[SGMM_MAX_PARENTS];
+    int64_t idx[SGMM_MAX_PARENTS];
+    int hist[256];
+    int warp_ties[SELECT_THREADS / 32];
+    int digit, k, count, ties_seen;
+};
+
+// The first mu children of the rank order of children first .. first+n-1, written to out[0..mu) (indices relative to
+// `first`); returns out[0].  A radix select (8 passes of 8-bit digit histograms) finds the mu-th key; every key above it
+// and the first keys equal to it in index order are kept, then sorted by (key descending, index ascending).
+template <int SIGN>
+__device__ int64_t select_parents(const Gather& f, int64_t first, int64_t n, int mu, SelectSmem& s, int64_t* out)
+{
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    uint64_t prefix = 0, mask = 0;
+    int k = mu;                                                     // rank of the wanted key among those matching prefix
+    for (int shift = 56; shift >= 0; shift -= 8) {
+        for (int i = tid; i < 256; i += blockDim.x) s.hist[i] = 0;
+        __syncthreads();
+        for_children<SIGN>(f, first, n, [&](int64_t, uint64_t key, bool valid) {
+            if (valid && (key & mask) == prefix) atomicAdd(&s.hist[(key >> shift) & 0xFF], 1);
+        });
+        __syncthreads();
+        if (warp == 0) {                                            // lane l holds digits 255-8l .. 248-8l, top down
+            int c[8], sum = 0;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) { c[j] = s.hist[255 - 8 * lane - j]; sum += c[j]; }
+            int incl = sum;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int y = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+                if (lane >= o) incl += y;
+            }
+            int cum = incl - sum;
+            if (cum < k && k <= incl) {
+                bool found = false;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    if (!found && cum + c[j] >= k) { s.digit = 255 - 8 * lane - j; s.k = k - cum; found = true; }
+                    if (!found) cum += c[j];
+                }
+            }
+        }
+        __syncthreads();
+        prefix |= (uint64_t)s.digit << shift; mask |= 0xFFull << shift; k = s.k;
+    }
+    // prefix is the mu-th key; k of the keys equal to it are parents, the first k in index order
+    if (tid == 0) { s.count = 0; s.ties_seen = 0; }
+    __syncthreads();
+    for_children<SIGN>(f, first, n, [&](int64_t i, uint64_t key, bool valid) {
+        const bool tie = valid && key == prefix;
+        const unsigned ties = __ballot_sync(0xFFFFFFFFu, tie);
+        if (lane == 0) s.warp_ties[warp] = __popc(ties);
+        __syncthreads();
+        int before = s.ties_seen + __popc(ties & ((1u << lane) - 1u));
+        for (int w = 0; w < warp; ++w) before += s.warp_ties[w];
+        if ((valid && key > prefix) || (tie && before < k)) {
+            const int slot = atomicAdd(&s.count, 1);
+            s.key[slot] = key; s.idx[slot] = i;
+        }
+        __syncthreads();
+        if (tid == 0) for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s.ties_seen += s.warp_ties[w];
+        __syncthreads();
+    });
+    int S = 1;
+    while (S < mu) S <<= 1;
+    for (int i = mu + tid; i < S; i += blockDim.x) { s.key[i] = 0; s.idx[i] = INT64_MAX; }   // padding sorts last
+    __syncthreads();
+    for (int size = 2; size <= S; size <<= 1) {                     // bitonic sort: (key descending, index ascending)
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int t = tid; t < S / 2; t += blockDim.x) {
+                const int lo = 2 * t - (t & (stride - 1)), hi = lo + stride;
+                const uint64_t kl = s.key[lo], kh = s.key[hi];
+                const int64_t il = s.idx[lo], ih = s.idx[hi];
+                const bool hi_first = kh > kl || (kh == kl && ih < il);
+                if (hi_first == ((lo & size) == 0)) { s.key[lo] = kh; s.key[hi] = kl; s.idx[lo] = ih; s.idx[hi] = il; }
+            }
+            __syncthreads();
+        }
+    }
+    for (int i = tid; i < mu; i += blockDim.x) out[i] = s.idx[i];
+    const int64_t best = s.idx[0];
+    __syncthreads();
+    return best;
+}
+
+// One block per run: run r's parents (rows r of mm_parents / adv_parents [runs][mu]) and its best child's state, as
+// ga_tell_kernel records it.  The masters are left to ga_recombine_kernel.
+__global__ void __launch_bounds__(SELECT_THREADS) ga_select_kernel(GaDev* runs, const Gather fit, int64_t pop, int mu,
+                                                                   int64_t* mm_parents, int64_t* adv_parents, int use_arl)
+{
+    __shared__ SelectSmem s;
+    const int64_t run = blockIdx.x, first = run * pop;
+    GaDev* st = runs + run;
+    const int64_t best = select_parents<+1>(fit, first, pop, mu, s, mm_parents + run * mu);
+    int64_t abest = 0;
+    if (use_arl) abest = select_parents<-1>(fit, first, pop, mu, s, adv_parents + run * mu);
+    if (threadIdx.x == 0) {
+        st->best_idx = best; st->adv_best_idx = abest;
+        st->train_f = fit.fit(first + best); st->train_trades = fit.trd(first + best);
+    }
+}
+
+// Grid (runs, quad blocks): thread q of run r owns elements 4q .. 4q+3 of one master (quad blocks [0, mm_blocks) the
+// market maker's [runs][G], the rest the adversary's [runs][1250]) and regenerates the same normal4 block of every parent:
+//   acc = w0*eps_0;  acc = fma(w_k, eps_k, acc) for k = 1 .. mu-1 in rank order;  m += acc*sigma
+// With w = [1] this is ga_tell_kernel's master + noise*sigma bit for bit.  Each thread updates only its own elements.
+__global__ void __launch_bounds__(RECOMBINE_THREADS) ga_recombine_kernel(const GaDev* runs, int mu, const float* w,
+                                                                         const int64_t* mm_parents, const int64_t* adv_parents,
+                                                                         float* mm_masters, int64_t G, float* adv_masters,
+                                                                         int mm_blocks)
+{
+    const int64_t run = blockIdx.x;
+    const GaDev* st = runs + run;
+    const bool adv = (int)blockIdx.y >= mm_blocks;
+    const int64_t n = adv ? 1250 : G;
+    const int64_t q = (int64_t)(adv ? blockIdx.y - mm_blocks : blockIdx.y) * blockDim.x + threadIdx.x;
+    if (4 * q >= n) return;
+    const int64_t* par = (adv ? adv_parents : mm_parents) + run * mu;
+    float* m = adv ? adv_masters + run * 1250 : mm_masters + run * G;
+    const uint64_t seed = adv ? st->seed ^ ADV_SEED_FLIP : st->seed, gen = (uint64_t)st->generation;
+    const float sigma = adv ? st->adv_sigma : st->sigma;
+    float acc[4];
+    {
+        float e[4]; normal4(seed, gen, (uint64_t)par[0], (uint32_t)q, e);
+        const float w0 = w[0];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) acc[i] = __fmul_rn(w0, e[i]);
+    }
+    for (int k = 1; k < mu; ++k) {
+        float e[4]; normal4(seed, gen, (uint64_t)par[k], (uint32_t)q, e);
+        const float wk = w[k];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) acc[i] = __fmaf_rn(wk, e[i], acc[i]);
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        if (4 * q + i < n) m[4 * q + i] = __fadd_rn(m[4 * q + i], __fmul_rn(acc[i], sigma));
+}
+
 }  // namespace sgmm
 
 using namespace sgmm;
@@ -156,6 +335,11 @@ struct sgmm_ga {
     GaDev* st = nullptr;                                                    // [runs]
     double* h_train_f = nullptr; double* h_val_f = nullptr; int32_t* h_train_t = nullptr; int32_t* h_val_t = nullptr;
     float* h_sigma = nullptr;                                               // [runs][max_generations]
+    // truncation selection (sgmm_ga_set_parents): weights != nullptr selects ga_select_kernel + ga_recombine_kernel
+    int32_t parents = 1;
+    float* weights = nullptr;                                               // [parents]
+    int64_t* mm_parents = nullptr; int64_t* adv_parents = nullptr;          // [runs][parents]
+    bool started = false;                                                   // a generation phase has been enqueued
 };
 
 namespace {
@@ -300,6 +484,7 @@ int sgmm_ga_destroy(sgmm_ga* ga)
         cudaFree(ga->gather.base); cudaFree(ga->val_fit); cudaFree(ga->val_trd);
         cudaFree(ga->st); cudaFree(ga->h_train_f); cudaFree(ga->h_val_f); cudaFree(ga->h_train_t);
         cudaFree(ga->h_val_t); cudaFree(ga->h_sigma);
+        cudaFree(ga->weights); cudaFree(ga->mm_parents); cudaFree(ga->adv_parents);
     }
     delete ga;
     return SGMM_OK;
@@ -324,6 +509,7 @@ int sgmm_ga_evaluate(sgmm_ga* ga, const sgmm_bundle* train, void* stream)
     if (!ga || !train) { set_error("NULL argument"); return SGMM_ERR_INVALID; }
     if (train->device != ga->device) { set_error("bundle and GA live on different devices"); return SGMM_ERR_INVALID; }
     DeviceGuard guard(ga->device);
+    ga->started = true;
     const sgmm_ga_config& c = ga->cfg;
     if (ga->sweep) {                                                // run r's children are individuals [r*lambda, (r+1)*lambda)
         const SweepPop mm{ga->mm_master, ga->st, c.pop_size, 0, (int64_t)ga->runs * c.pop_size, 0};
@@ -348,14 +534,26 @@ int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
     DeviceGuard guard(ga->device);
     cudaStream_t st = (cudaStream_t)stream;
     const sgmm_ga_config& c = ga->cfg;
-    ga_tell_kernel<<<(unsigned)ga->runs, 256, 0, st>>>(ga->st, ga->gather, c.pop_size, ga->mm_master, ga->G,
-                                                       ga->adv_master, c.use_arl);
-    if (int rc = check_cuda(cudaGetLastError(), "ga_tell_kernel launch")) return rc;
-    if (ga->sweep) {                                                // the new masters ARE the best children: [runs][1250] rows
+    ga->started = true;
+    if (!ga->weights) {
+        ga_tell_kernel<<<(unsigned)ga->runs, 256, 0, st>>>(ga->st, ga->gather, c.pop_size, ga->mm_master, ga->G,
+                                                           ga->adv_master, c.use_arl);
+        if (int rc = check_cuda(cudaGetLastError(), "ga_tell_kernel launch")) return rc;
+    } else {
+        ga_select_kernel<<<(unsigned)ga->runs, SELECT_THREADS, 0, st>>>(ga->st, ga->gather, c.pop_size, ga->parents,
+                                                                        ga->mm_parents, ga->adv_parents, c.use_arl);
+        if (int rc = check_cuda(cudaGetLastError(), "ga_select_kernel launch")) return rc;
+        const int64_t quads = RECOMBINE_THREADS * 4;
+        const int mm_blocks = (int)((ga->G + quads - 1) / quads), adv_blocks = c.use_arl ? (int)((1250 + quads - 1) / quads) : 0;
+        ga_recombine_kernel<<<dim3((unsigned)ga->runs, (unsigned)(mm_blocks + adv_blocks)), RECOMBINE_THREADS, 0, st>>>(
+            ga->st, ga->parents, ga->weights, ga->mm_parents, ga->adv_parents, ga->mm_master, ga->G, ga->adv_master, mm_blocks);
+        if (int rc = check_cuda(cudaGetLastError(), "ga_recombine_kernel launch")) return rc;
+    }
+    if (ga->sweep) {                                                // the new masters (best children, or recombined): [runs] rows
         if (int rc = launch_sweep_validation(val, ga->mm_master, ga->st, ga->runs, ga->val_fit, ga->val_trd, st)) return rc;
     } else {
         PopArgs one{};
-        one.genomes = ga->mm_master; one.master = nullptr; one.count = 1;      // the new master IS the best child
+        one.genomes = ga->mm_master; one.master = nullptr; one.count = 1;      // the new master (best child, or recombined)
         // H = 256: the population's own route (exact, or the same tensor-core path).  H = 32: always exact -- one individual,
         // adversary off, so launch_rollout takes the small-population path of sgmm_one.cu (policy for every (bar, inventory)
         // in parallel, automaton scan, reference-order sum; bit-identical to the sequential kernel)
@@ -443,6 +641,79 @@ int sgmm_ga_history_host(sgmm_ga* ga, int32_t n, double* train_f, double* val_f,
     if (!ga || n < 0) { set_error("bad argument"); return SGMM_ERR_INVALID; }
     if (int rc = single_run(ga, "sgmm_ga_history_host")) return rc;
     return sgmm_ga_run_history_host(ga, 0, n, train_f, val_f, train_trades, val_trades, sigma, stream);
+}
+
+int sgmm_ga_set_parents(sgmm_ga* ga, int32_t parents, const float* weights, void* stream)
+{
+    if (!ga) { set_error("ga is NULL"); return SGMM_ERR_INVALID; }
+    if (ga->started) {
+        set_error("sgmm_ga_set_parents: a generation of this GA has already been enqueued; set the parents right after create");
+        return SGMM_ERR_INVALID;
+    }
+    if (parents < 1 || parents > SGMM_MAX_PARENTS || parents > ga->cfg.pop_size) {
+        set_error("parents=%d: need 1 <= parents <= min(pop_size=%lld, %d)", (int)parents, (long long)ga->cfg.pop_size,
+                  SGMM_MAX_PARENTS);
+        return SGMM_ERR_INVALID;
+    }
+    std::vector<float> w((size_t)parents, 1.0f / (float)parents);
+    if (weights) {
+        bool any = false;
+        for (int32_t k = 0; k < parents; ++k) {
+            if (!std::isfinite(weights[k]) || weights[k] < 0.0f) { set_error("weight %d = %g: weights must be finite and >= 0", (int)k, (double)weights[k]); return SGMM_ERR_INVALID; }
+            any = any || weights[k] > 0.0f;
+            w[k] = weights[k];
+        }
+        if (!any) { set_error("every recombination weight is 0"); return SGMM_ERR_INVALID; }
+    }
+    DeviceGuard guard(ga->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaFree(ga->weights); cudaFree(ga->mm_parents); cudaFree(ga->adv_parents);     // a second call before the first generation
+    ga->weights = nullptr; ga->mm_parents = ga->adv_parents = nullptr;
+    const size_t n = (size_t)ga->runs * (size_t)parents;
+    int rc = SGMM_OK;
+    if (!rc) rc = check_cuda(cudaMalloc(&ga->mm_parents, n * sizeof(int64_t)), "cudaMalloc");
+    if (!rc) rc = check_cuda(cudaMalloc(&ga->adv_parents, n * sizeof(int64_t)), "cudaMalloc");
+    if (!rc) rc = check_cuda(cudaMalloc(&ga->weights, (size_t)parents * sizeof(float)), "cudaMalloc");
+    if (!rc) rc = check_cuda(cudaMemsetAsync(ga->mm_parents, 0, n * sizeof(int64_t), st), "memset");
+    if (!rc) rc = check_cuda(cudaMemsetAsync(ga->adv_parents, 0, n * sizeof(int64_t), st), "memset");
+    if (!rc) rc = check_cuda(cudaMemcpyAsync(ga->weights, w.data(), (size_t)parents * sizeof(float), cudaMemcpyHostToDevice, st), "H2D weights");
+    if (!rc) rc = check_cuda(cudaStreamSynchronize(st), "ga_set_parents");
+    if (rc) {                                                       // back to the (1,lambda) GA
+        cudaFree(ga->weights); cudaFree(ga->mm_parents); cudaFree(ga->adv_parents);
+        ga->weights = nullptr; ga->mm_parents = ga->adv_parents = nullptr;
+        return rc;
+    }
+    ga->parents = parents;
+    return SGMM_OK;
+}
+
+int sgmm_ga_run_parents_host(sgmm_ga* ga, int32_t run, int32_t n, int64_t* mm_index, int64_t* adv_index, void* stream)
+{
+    if (!ga || n < 0) { set_error("bad argument"); return SGMM_ERR_INVALID; }
+    if (int rc = check_run(ga, run)) return rc;
+    const size_t k = (size_t)(n < ga->parents ? n : ga->parents), r = (size_t)run;
+    if (k == 0) return SGMM_OK;
+    DeviceGuard guard(ga->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!ga->weights) {                                             // (1,lambda): the best children of the state
+        GaDev h;
+        if (int rc = check_cuda(cudaMemcpyAsync(&h, ga->st + run, sizeof h, cudaMemcpyDeviceToHost, st), "D2H ga state")) return rc;
+        if (int rc = check_cuda(cudaStreamSynchronize(st), "ga_parents")) return rc;
+        if (mm_index) mm_index[0] = h.best_idx;
+        if (adv_index) adv_index[0] = h.adv_best_idx;
+        return SGMM_OK;
+    }
+    const size_t P = (size_t)ga->parents;
+    if (mm_index) if (int rc = check_cuda(cudaMemcpyAsync(mm_index, ga->mm_parents + r * P, k * sizeof(int64_t), cudaMemcpyDeviceToHost, st), "D2H parents")) return rc;
+    if (adv_index) if (int rc = check_cuda(cudaMemcpyAsync(adv_index, ga->adv_parents + r * P, k * sizeof(int64_t), cudaMemcpyDeviceToHost, st), "D2H parents")) return rc;
+    return check_cuda(cudaStreamSynchronize(st), "ga_parents");
+}
+
+int sgmm_ga_parents_host(sgmm_ga* ga, int32_t n, int64_t* mm_index, int64_t* adv_index, void* stream)
+{
+    if (!ga || n < 0) { set_error("bad argument"); return SGMM_ERR_INVALID; }
+    if (int rc = single_run(ga, "sgmm_ga_parents_host")) return rc;
+    return sgmm_ga_run_parents_host(ga, 0, n, mm_index, adv_index, stream);
 }
 
 }  // extern "C"

@@ -429,8 +429,46 @@ def evaluate_individual(mm_weights, adv_weights, bundle, phi, tick_size, fee_rat
 # ------------------------------------------------------------------------------------------------
 # DRLEngine
 # ------------------------------------------------------------------------------------------------
+def _parent_weights(parents, weights, pop_size):
+    """Checks the truncation-selection arguments (``sgmm_ga_set_parents``) without touching a device.  Returns the
+    float32 weights to pass (``None``: equal weights ``fl(1/parents)``), or ``False`` when the GA keeps the (1,lambda) rule
+    (``parents == 1`` and no weights)."""
+    if isinstance(parents, bool) or int(parents) != parents:
+        raise ValueError(f"parents must be an integer, got {parents!r}")
+    parents = int(parents)
+    if not 1 <= parents <= min(int(pop_size), _lib.MAX_PARENTS):
+        raise ValueError(f"parents={parents}: need 1 <= parents <= min(pop_size={pop_size}, {_lib.MAX_PARENTS})")
+    if weights is None:
+        return None if parents != 1 else False
+    w = np.ascontiguousarray(np.asarray(weights, dtype=np.float32).reshape(-1))
+    if w.size != parents:
+        raise ValueError(f"{w.size} weights for {parents} parents")
+    if not np.all(np.isfinite(w)) or np.any(w < 0) or not np.any(w > 0):
+        raise ValueError("weights must be finite, >= 0 and not all 0")
+    return w
+
+
 class _GAHandle:
     """What every ``sgmm_ga`` handle offers: the generation phases, graph capture, the per-run read-backs and close."""
+
+    def _set_parents(self, parents, w):
+        """After create: switch to truncation selection of ``parents`` parents (``w``: from :func:`_parent_weights`)."""
+        self.n_parents = int(parents) if w is not False else 1
+        if w is False:
+            return
+        try:
+            _lib.check(_lib.lib().sgmm_ga_set_parents(self._h, self.n_parents, None if w is None else w.ctypes.data,
+                                                      _stream(self.device)))
+        except Exception:
+            self.close()
+            raise
+
+    def _parents(self, run):
+        mm = np.zeros(self.n_parents, np.int64)
+        adv = np.zeros(self.n_parents, np.int64)
+        _lib.check(_lib.lib().sgmm_ga_run_parents_host(self._h, int(run), self.n_parents, mm.ctypes.data, adv.ctypes.data,
+                                                       _stream(self.device)))
+        return mm, adv
 
     def evaluate(self, train: Bundle):
         _lib.check(_lib.lib().sgmm_ga_evaluate(self._h, train.handle, _stream(self.device)))
@@ -488,10 +526,15 @@ class _GAHandle:
 
 class DeviceGA(_GAHandle):
     """Thin owner of a ``sgmm_ga`` handle (include/sgmm.h): ask/evaluate/tell/validate/select on
-    the device, one call per generation, no host round trip."""
+    the device, one call per generation, no host round trip.
+
+    ``parents`` (mu) > 1 or ``weights`` switch the (1,lambda) rule to truncation selection (``sgmm_ga_set_parents``): the
+    mu best children in rank order are recombined into the new master ``master + sigma * sum_k weights[k] * eps_k``
+    (``weights`` float[mu], used as given; default ``1/mu`` each).  ``parents()`` reads the last generation's parents."""
 
     def __init__(self, mm_master, adv_master=None, *, pop_size, sigma, phi, fee_rate, use_arl, seed,
-                 max_generations, patience=15, hidden=32, device=None, shard=None, precision=None):
+                 max_generations, patience=15, hidden=32, device=None, shard=None, precision=None, parents=1, weights=None):
+        w = _parent_weights(parents, weights, pop_size)
         self.device = torch.cuda.current_device() if device is None else int(device)
         first, count, stride = (0, pop_size, 0) if shard is None else shard
         cfg = _lib.GaConfig(hidden, int(bool(use_arl)), pop_size, first, count, stride, float(sigma), patience,
@@ -507,6 +550,11 @@ class DeviceGA(_GAHandle):
         _lib.check(_lib.lib().sgmm_ga_create(C.byref(self._h), C.byref(cfg), m.ctypes.data,
                                              None if a is None else a.ctypes.data, self.device,
                                              _stream(self.device)))
+        self._set_parents(parents, w)
+
+    def parents(self):
+        """``(mm_index, adv_index)`` int64[mu]: the last generation's parents in rank order (global child indices)."""
+        return self._parents(0)
 
     def buffers(self):
         """``(fitness_slice, trades_slice, gather_base, block_bytes, n_blocks, my_block)``: raw device addresses of
@@ -536,9 +584,12 @@ class DeviceGASweep(_GAHandle):
     (``fee_rate`` 0, ``sigma`` 0.05, ``patience`` 15 when left out); ``masters`` [K, 1250] (or one [1250] master for
     every run), ``adv_masters`` likewise when ``use_arl``.  ``pop_size`` is lambda PER RUN.  Run r is bit-identical to
     ``DeviceGA(masters[r], adv_masters[r], precision="exact", **runs[r])``.  Hidden width 32, exact precision, one
-    device.  Read-backs take the run: ``status(r)``, ``masters(r)``, ``history(r)``."""
+    device.  Read-backs take the run: ``status(r)``, ``masters(r)``, ``history(r)``, ``parents(r)``.  ``parents`` /
+    ``weights`` select truncation selection as for :class:`DeviceGA`, one setting for every run."""
 
-    def __init__(self, masters, adv_masters=None, *, runs, pop_size, use_arl, max_generations, device=None):
+    def __init__(self, masters, adv_masters=None, *, runs, pop_size, use_arl, max_generations, device=None, parents=1,
+                 weights=None):
+        w = _parent_weights(parents, weights, pop_size)
         self.device = torch.cuda.current_device() if device is None else int(device)
         K = len(runs)
         if K == 0:
@@ -575,6 +626,12 @@ class DeviceGASweep(_GAHandle):
         self._h = C.c_void_p()
         _lib.check(_lib.lib().sgmm_ga_create_sweep(C.byref(self._h), C.byref(cfg), K, arr, m.ctypes.data,
                                                    None if a is None else a.ctypes.data, self.device, _stream(self.device)))
+        self._set_parents(parents, w)
+
+    def parents(self, run=0):
+        """``(mm_index, adv_index)`` int64[mu] of run ``run``: its last generation's parents in rank order (indices within
+        the run's lambda children)."""
+        return self._parents(run)
 
     def status(self, run):
         return self._status(run)
@@ -605,11 +662,19 @@ class DRLEngine:
       (:class:`dist.ShardedGA`: one NCCL all-gather of fitness + trades per generation) -- the multi-GPU replacement of
       the ``Pool(8).starmap`` of drl_engine.py:91,115.  Every rank returns the identical policy and history; rank 0
       writes the checkpoint.
+    * ``parents`` (mu) and ``parent_weights`` (float[mu], default ``1/mu`` each) replace the reference's (1,lambda) rule
+      by truncation selection with weighted recombination, in ``train`` (solo and sharded) and ``train_sweep``: the new
+      master is ``master + sigma * sum_k w_k eps_k`` over the mu best children (see :class:`DeviceGA`).  The defaults
+      keep the (1,lambda) rule.  With mu > 1 the master is no longer a child: ``val_f`` in the history, the
+      keep-best-on-validation choice and the checkpoint all belong to the recombined master; ``train_f`` /
+      ``train_trades`` stay those of the best child.
     """
 
     def __init__(self, pop_size=50, sigma=0.05, phi=0.01, tick_size=0.01, fee_rate=0.0, use_arl=False,
                  save_dir="checkpoints/drl", seed=None, device=None, patience=15, precision=None, hidden_dim=32,
-                 group=None):
+                 group=None, parents=1, parent_weights=None):
+        _parent_weights(parents, parent_weights, pop_size)            # argument errors before any side effect
+        self.parents, self.parent_weights = parents, parent_weights
         self.precision = precision
         self.phi = phi
         self.tick_size = tick_size
@@ -659,7 +724,8 @@ class DRLEngine:
                             pop_size=pop, sigma=self.mm_evolver.sigma, phi=self.phi,
                             fee_rate=self.fee_rate, use_arl=self.use_arl, seed=seed,
                             max_generations=max(1, generations), patience=self.patience, device=dev,
-                            precision=self.precision, hidden=self.hidden_dim, shard=shard)
+                            precision=self.precision, hidden=self.hidden_dim, shard=shard,
+                            parents=self.parents, weights=self.parent_weights)
         if sharded:
             from .dist import ShardedGA
             runner = ShardedGA(make, pop, group=self.group)
@@ -758,7 +824,8 @@ class DRLEngine:
         ga = DeviceGASweep(self.mm_evolver.master_policy.get_weights(),
                            self.adv_evolver.master_policy.get_weights() if self.use_arl else None,
                            runs=runs, pop_size=self.mm_evolver.pop_size, use_arl=self.use_arl,
-                           max_generations=max(1, generations), device=dev)
+                           max_generations=max(1, generations), device=dev, parents=self.parents,
+                           weights=self.parent_weights)
         save_paths = [os.path.join(self.save_dir, f"{output_prefix}_run{r}_best_val_{phi_r[r]}.pth") for r in range(K)]
         saved_val = [-np.inf] * K
 

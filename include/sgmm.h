@@ -393,6 +393,30 @@ int sgmm_ga_run_history_host(sgmm_ga* ga, int32_t run, int32_t n, double* train_
                              int32_t* train_trades, int32_t* val_trades, float* sigma, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Truncation selection with weighted recombination, a (mu/mu_w, lambda) evolution strategy, on any GA handle (solo,
+ * sharded or sweep; one setting for every run).  Each generation the children of a run are ranked -- market maker: NaN
+ * first, then descending fitness; adversary (use_arl): NaN first, then ascending fitness; ties to the lower index,
+ * -0.0 == +0.0 (with mu = 1 exactly the (1,lambda) argmax) -- and the first mu are the parents.  The new master is
+ *     acc = w[0]*eps_0;  acc = fmaf(w[k], eps_k, acc), k = 1 .. mu-1 in rank order;  m[e] = m[e] + acc*sigma
+ * per genome element, eps_k the noise of parent k (the adversary's with seed ^ 1<<63 and adv_sigma).  Children are still
+ * master + sigma*eps, so every population route is unchanged.  The history's train_f / train_trades and
+ * status.last_best_index are those of parent 0; validation, keep-best-on-validation and sigma decay act on the
+ * recombined master (val_f and best_val_master are the recombined master's).
+ *   parents   mu, 1 <= mu <= min(pop_size (lambda per run), SGMM_MAX_PARENTS)
+ *   weights   HOST float[parents], used as given (no normalisation): finite, >= 0, not all 0; NULL = fl(1/mu) each.
+ *             w = [1] is bit for bit the (1,lambda) GA, and so is w = [1, 0, ..., 0] for any mu.
+ * Call it after create and before the first evaluate / select / generation of the handle (later: SGMM_ERR_INVALID),
+ * so a captured generation never holds a buffer it reallocates.  Synchronises the stream.  Without this call the GA
+ * runs the (1,lambda) rule of the reference. */
+#define SGMM_MAX_PARENTS 1024
+int sgmm_ga_set_parents(sgmm_ga* ga, int32_t parents, const float* weights, void* stream);
+/* synchronising read-back of the last generation's parents of run `run` in rank order: the first min(n, parents)
+ * entries (indices within the run's lambda children) of each HOST array; either may be NULL.  Without
+ * sgmm_ga_set_parents: the best children (one entry).  The adversary's list reads 0 without use_arl. */
+int sgmm_ga_run_parents_host(sgmm_ga* ga, int32_t run, int32_t n, int64_t* mm_index, int64_t* adv_index, void* stream);
+int sgmm_ga_parents_host(sgmm_ga* ga, int32_t n, int64_t* mm_index, int64_t* adv_index, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Upstream of the rollout: the per-day window loop of load_signals_bundle
  * (pipeline/agent_trainer.py:47-73).  Inputs are one day's event frame columns (loader2.event_df:
  * askprice1, bidprice1, p_buy_max, p_sell_min; n_events rows, NaN allowed in the last two) and
