@@ -495,6 +495,393 @@ static int launch_u(const RolloutArgs& args, bool adv, bool fee, int warps, cuda
     return fee ? launch_variant<U, false, true>(args, warps, st) : launch_variant<U, false, false>(args, warps, st);
 }
 
+// ---------------------------------------------------------------------------------------------
+// the two-chain rollout kernel (H = 32, no adversary)
+// ---------------------------------------------------------------------------------------------
+// rollout_kernel_h32 advances one dependent chain per individual, and two warps per scheduler cannot hide it (§5 of
+// DESIGN.md: ~620 cycles per pair of warp-steps, ~400 of them FMA-pipe time).  Here every warp advances TWO time blocks
+// of its individuals' episodes on the same weight registers.  The episode runs in rounds of ROUND_BARS bars; with a
+// burn-in of B bars and N = (ROUND_BARS + B) / 2:
+//   * chain A steps bars [0, N) of the round from the exact state the previous round left;
+//   * chain B steps bars [N - B, ROUND_BARS) from inventory 0; its first B bars are burn-in.
+// Without the adversary the state entering a bar is the inventory alone, and a step's record is a function of (bar,
+// inventory): once B's inventory equals the true one, B's records are the true records.  At the round's end each
+// individual compares A's inventory entering bar N with B's; where they differ, B's block is stepped again from the
+// true state (warp-uniform loop, lone chain) until the repaired inventory meets B's, or to the round's end.  Cold
+// starts join fast (tools/exact_join_stats.py: median 3 bars; after 8 bars 10 % have not, after 16 bars 2.1 %);
+// the path is exact for a policy that never joins.  A partial last round runs chain A alone.
+// Measured on one B200 (1 000 W, profiles/r8_exact_chains_bench.json): P = 592 (U = 1, one warp per scheduler) 2.16 instead
+// of 2.68 ms; P = 4096 (U = 4, two warps per scheduler) only 4.35 instead of 4.51 ms -- there the two warps already
+// overlap most of each other's chain.  Loading half of the burst's activations after the other chain's stores (which
+// moves its decision in front of the burst in the SASS) was slower: 4.60 ms at P = 4096, 2.68 ms at P = 592.
+// The accounting warp consumes whole validated rounds in bar order: two round buffers of records and bars (the round
+// r + 2 is loaded once round r is accounted), so the fp64 reward sum keeps the reference's order.
+constexpr int ROUND_BARS = 256;
+constexpr int ROLLOUT_BURN_IN = 4;        // default burn-in of chain B (even, < ROUND_BARS): 4.350 ms at the bench shape, 8: 4.379, 16: 4.44, 32: 4.66
+
+struct Ring2Smem {
+    uint64_t full[2];                     // the round's bars landed (TMA)
+    uint64_t rec_full[2];                 // the round's records are validated (one arrival per compute warp)
+    BarSig sig[2][ROUND_BARS];
+    BarPx px[2][ROUND_BARS];              // prices: read by the accounting warp only
+    float hbuf[2][MAX_WARPS][128];        // [chain][warp]: as RingSmem::hbuf
+    float rbuf[2][MAX_WARPS][80];         // [chain][warp]: as RingSmem::rbuf
+    uint64_t rec[2][ROUND_BARS][32];      // one 8-byte step record per (bar of the round, individual of the CTA)
+};
+
+template <int U>
+struct H32Regs {
+    float w1x[U], w1y[U], w1i[U], b1[U], b2[U], w3a[U], w3b[U];
+    float2 w2[U][16];
+    float b3a, b3b;
+};
+
+// layer 1 (bar part + inventory term) + ReLU of one bar, in rollout_kernel_h32's op order
+template <int U>
+__device__ __forceinline__ void h32_layer1(const H32Regs<U>& w, float2 z, float inv2, float h[U])
+{
+#pragma unroll
+    for (int u = 0; u < U; ++u) h[u] = fmaxf(__fmaf_rn(w.w1i[u], inv2, __fmaf_rn(w.w1y[u], z.y, __fmaf_rn(w.w1x[u], z.x, w.b1[u]))), 0.0f);
+}
+template <int U>
+__device__ __forceinline__ void h32_put_h1(float* hb, int g, int l, const float h[U])
+{
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const int j = l + (32 / U) * u;
+        hb[((j >> 2) * U + g) * 4 + (j & 3)] = h[u];
+    }
+}
+template <int U>
+__device__ __forceinline__ void h32_get_h1(const float* hb, int g, float4 h4[8])
+{
+#pragma unroll
+    for (int k = 0; k < 8; ++k) h4[k] = *reinterpret_cast<const float4*>(&hb[(k * U + g) * 4]);
+}
+// layers 2 and 3 up to the lane's partial outputs; for U < 4 the cross-lane butterfly too (shuffles)
+template <int U>
+__device__ __forceinline__ float2 h32_layer23(const H32Regs<U>& w, const float4 h4[8])
+{
+    constexpr int L = 32 / U;
+    float2 P[U], Q[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) { P[u] = make_float2(w.b2[u], 0.0f); Q[u] = make_float2(0.0f, 0.0f); }
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+        const float2 hlo = make_float2(h4[k].x, h4[k].y), hhi = make_float2(h4[k].z, h4[k].w);
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            P[u] = __ffma2_rn(w.w2[u][2 * k], hlo, P[u]);
+            Q[u] = __ffma2_rn(w.w2[u][2 * k + 1], hhi, Q[u]);
+        }
+    }
+    float pa[U], pb[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const float2 S = __fadd2_rn(P[u], Q[u]);
+        const float h2 = fmaxf(__fadd_rn(S.x, S.y), 0.0f);
+        pa[u] = __fmul_rn(w.w3a[u], h2);
+        pb[u] = __fmul_rn(w.w3b[u], h2);
+    }
+    float ra, rb;
+    if (U == 4) {
+        ra = __fadd_rn(__fadd_rn(pa[0], pa[2 % U]), __fadd_rn(pa[1 % U], pa[3 % U]));
+        rb = __fadd_rn(__fadd_rn(pb[0], pb[2 % U]), __fadd_rn(pb[1 % U], pb[3 % U]));
+    } else {
+        if (U == 2) { ra = __fadd_rn(pa[0], pa[1 % U]); rb = __fadd_rn(pb[0], pb[1 % U]); }
+        else { ra = pa[0]; rb = pb[0]; }
+#pragma unroll
+        for (int m = L / 2; m >= 1; m >>= 1) {
+            ra = __fadd_rn(ra, __shfl_xor_sync(0xffffffffu, ra, m));
+            rb = __fadd_rn(rb, __shfl_xor_sync(0xffffffffu, rb, m));
+        }
+    }
+    return make_float2(ra, rb);
+}
+// U = 4: the 8 lanes' partials through shared memory, the same tree as rollout_kernel_h32
+__device__ __forceinline__ void h32_put_partial(float* rbw, int g, int l, float2 r)
+{
+    *reinterpret_cast<float2*>(&rbw[g * 20 + l * 2]) = r;
+}
+__device__ __forceinline__ void h32_get_partials(const float* rbw, int g, float4 r[4])
+{
+#pragma unroll
+    for (int k = 0; k < 4; ++k) r[k] = *reinterpret_cast<const float4*>(&rbw[g * 20 + 4 * k]);
+}
+__device__ __forceinline__ float2 h32_tree(const float4 r[4])
+{
+    const float2 t04 = __fadd2_rn(make_float2(r[0].x, r[0].y), make_float2(r[2].x, r[2].y));
+    const float2 t15 = __fadd2_rn(make_float2(r[0].z, r[0].w), make_float2(r[2].z, r[2].w));
+    const float2 t26 = __fadd2_rn(make_float2(r[1].x, r[1].y), make_float2(r[3].x, r[3].y));
+    const float2 t37 = __fadd2_rn(make_float2(r[1].z, r[1].w), make_float2(r[3].z, r[3].w));
+    return __fadd2_rn(__fadd2_rn(t04, t26), __fadd2_rn(t15, t37));
+}
+// quantise + fill decision against the bar's float thresholds (tha, thb); moves inv2 and returns the step record
+__device__ __forceinline__ float2 h32_decide(float2 r, float b3a, float b3b, float2 th, float& inv2)
+{
+    const float qa = __fmul_rn(__fadd_rn(r.x, b3a), 5.0f);           // raw*5.0 (drl_engine.py:39)
+    const float qb = __fmul_rn(__fadd_rn(r.y, b3b), 5.0f);
+    const bool fb = (inv2 < 1.0f) && (qb < th.y);
+    const bool fs = (inv2 > -1.0f) && (qa < th.x);
+    inv2 = __fadd_rn(inv2, fb ? (fs ? 0.0f : 0.5f) : (fs ? -0.5f : 0.0f));
+    return make_float2(fs ? qa : __int_as_float(SGMM_CODE_NOFILL_F), fb ? qb : __int_as_float(SGMM_CODE_NOFILL_F));
+}
+// the inventory move (in halves) a step record encodes
+__device__ __forceinline__ float h32_record_move(float2 c)
+{
+    const bool fs = __float_as_int(c.x) != SGMM_CODE_NOFILL_F, fb = __float_as_int(c.y) != SGMM_CODE_NOFILL_F;
+    return fb ? (fs ? 0.0f : 0.5f) : (fs ? -0.5f : 0.0f);
+}
+
+template <int U, bool FEE>
+__global__ void __launch_bounds__((max_compute_warps(U) + 1) * 32, 1)
+rollout2_kernel_h32(const RolloutArgs a, const int burn)
+{
+    constexpr int H = 32;
+    constexpr int NI = U;
+    constexpr int L = 32 / U;
+    constexpr int64_t G = (int64_t)H * H + 7 * H + 2;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    Ring2Smem& sm = *reinterpret_cast<Ring2Smem*>(smem_raw);
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int nwarps = (blockDim.x >> 5) - 1;
+    const int g = lane / L, l = lane % L;
+    const int64_t first = (int64_t)blockIdx.x * nwarps * NI;
+    const int64_t remaining = a.mm.count - first;
+    const int live_warps = (int)(remaining >= (int64_t)nwarps * NI ? nwarps : (remaining + NI - 1) / NI);
+    const int64_t ind = first + (int64_t)warp * NI + g;
+    const bool live = ind < a.mm.count;
+    const int64_t T = a.T;
+    const int64_t nrounds = (T + ROUND_BARS - 1) / ROUND_BARS;
+    const int N = (ROUND_BARS + burn) / 2;                           // steps of each chain in a whole round
+
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int s = 0; s < 2; ++s) { mbar_init(&sm.full[s], 1); mbar_init(&sm.rec_full[s], live_warps); }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+
+    if (warp == nwarps) {
+        // ===== TMA producer of the round buffers and the fp64 half of the env step (as in rollout_kernel_h32) =====
+        const int64_t indj = first + lane;
+        const bool livej = lane < live_warps * NI && indj < a.mm.count;
+        const double tick = a.tick, fee = a.fee;
+        const PenaltyTable pen = penalty_table(a.phi);
+        double total = 0.0;
+        int ntr = 0, inv = 0;
+        auto load = [&](int64_t r) {
+            if (lane == 0) {
+                const int s = (int)(r & 1);
+                const int64_t tl = r * ROUND_BARS;
+                const uint32_t nb = (uint32_t)(T - tl < ROUND_BARS ? T - tl : ROUND_BARS);
+                mbar_arrive_expect_tx(&sm.full[s], nb * (uint32_t)(sizeof(BarSig) + sizeof(BarPx)));
+                tma_bulk_g2s(&sm.sig[s][0], a.sig + tl, nb * (uint32_t)sizeof(BarSig), &sm.full[s]);
+                tma_bulk_g2s(&sm.px[s][0], a.px + tl, nb * (uint32_t)sizeof(BarPx), &sm.full[s]);
+            }
+        };
+        for (int64_t r = 0; r < nrounds && r < 2; ++r) load(r);
+        for (int64_t r = 0; r < nrounds; ++r) {
+            const int s = (int)(r & 1);
+            mbar_wait(&sm.rec_full[s], (uint32_t)((r >> 1) & 1));
+            const int64_t t0 = r * ROUND_BARS;
+            const int n = (int)(T - t0 < ROUND_BARS ? T - t0 : ROUND_BARS);
+            const BarPx* pxs = &sm.px[s][0];
+#pragma unroll 4
+            for (int i = 0; i < n; ++i) {
+                const uint64_t code = sm.rec[s][i][lane];
+                int ka = (int)(uint32_t)code, kb = (int)(uint32_t)(code >> 32);
+                const bool fs = ka != SGMM_CODE_NOFILL_F, fb = kb != SGMM_CODE_NOFILL_F;
+                inv += (fb ? 1 : 0) - (fs ? 1 : 0);                      // market_env.py:45,51
+                const int ai = inv < 0 ? -inv : inv;
+                const bool traded = fb || fs;
+                ntr += traded ? 1 : 0;                                   // drl_engine.py:60-61
+                double pnl = 0.0;                                        // market_env.py:40
+                if (__any_sync(0xffffffffu, traded)) {
+                    const double2 ab = *reinterpret_cast<const double2*>(&pxs[i].ask);
+                    const double mid = pxs[i].mid_next;
+                    ka = __float2int_rn(__int_as_float(ka)); kb = __float2int_rn(__int_as_float(kb));   // drl_engine.py:39
+                    const double my_ask = quote_ask(ab.x, ka, tick), my_bid = quote_bid(ab.y, kb, tick);      // market_env.py:30-31
+                    const double leg_b = buy_leg<FEE>(my_bid, mid, fee), leg_s = sell_leg<FEE>(my_ask, mid, fee);
+                    pnl = fb ? add_rn(pnl, leg_b) : pnl;
+                    pnl = fs ? add_rn(pnl, leg_s) : pnl;
+                }
+                total = add_rn(total, sub_rn(pnl, penalty(pen, ai)));                   // market_env.py:58, drl_engine.py:54
+            }
+            __syncwarp();
+            if (r + 2 < nrounds) load(r + 2);                            // both buffers of round r are free again
+        }
+        if (livej) { a.fitness[indj] = episode_fitness(total, ntr); a.trades[indj] = ntr; }
+        return;
+    }
+    if (warp >= live_warps) return;
+
+    // ---- weights into registers (models/model.py:31-36 layout) ---------------------------------
+    const PopArgs mmp = resolve(a.mm);
+    const GenomeSource src = make_source(mmp, live ? ind : 0, G);
+    H32Regs<U> w;
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const int j = l + L * u;
+        if (live) {
+            w.w1x[u] = src.at(3 * j + 0); w.w1y[u] = src.at(3 * j + 1); w.w1i[u] = src.at(3 * j + 2);
+            w.b1[u] = src.at(3 * H + j);
+            w.b2[u] = src.at(4 * H + H * H + j);
+            w.w3a[u] = src.at(5 * H + H * H + j);
+            w.w3b[u] = src.at(6 * H + H * H + j);
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+                float v[4]; src.at4(4 * H + (int64_t)j * H + 4 * c, v);
+                w.w2[u][2 * c] = make_float2(v[0], v[1]);
+                w.w2[u][2 * c + 1] = make_float2(v[2], v[3]);
+            }
+        } else {
+            w.w1x[u] = w.w1y[u] = w.w1i[u] = w.b1[u] = w.b2[u] = w.w3a[u] = w.w3b[u] = 0.0f;
+#pragma unroll
+            for (int c = 0; c < 16; ++c) w.w2[u][c] = make_float2(0.0f, 0.0f);
+        }
+    }
+    w.b3a = live ? src.at(7 * H + H * H) : 0.0f;
+    w.b3b = live ? src.at(7 * H + H * H + 1) : 0.0f;
+
+    float* const hA = &sm.hbuf[0][warp][0];
+    float* const hB = &sm.hbuf[1][warp][0];
+    float* const rA = &sm.rbuf[0][warp][0];
+    float* const rB = &sm.rbuf[1][warp][0];
+    const int slotj = warp * NI + g;                                 // this individual's lane in the accounting warp
+    float inv2 = 0.0f;                                               // inventory / 2.0 (drl_engine.py:35), exact
+
+    // one step of a lone chain on chain A's buffers (partial rounds and repairs); returns the step record
+    auto step1 = [&](const BarSig* sg, float& iv) -> float2 {
+        float h[U];
+        h32_layer1<U>(w, *reinterpret_cast<const float2*>(&sg->z1), iv, h);
+        h32_put_h1<U>(hA, g, l, h);
+        __syncwarp();
+        float4 h4[8];
+        h32_get_h1<U>(hA, g, h4);
+        float2 p = h32_layer23<U>(w, h4);
+        if (U == 4) {
+            h32_put_partial(rA, g, l, p);
+            __syncwarp();
+            float4 pr[4];
+            h32_get_partials(rA, g, pr);
+            p = h32_tree(pr);
+        }
+        return h32_decide(p, w.b3a, w.b3b, *reinterpret_cast<const float2*>(&sg->tha), iv);
+    };
+
+    for (int64_t r = 0; r < nrounds; ++r) {
+        const int s = (int)(r & 1);
+        mbar_wait(&sm.full[s], (uint32_t)((r >> 1) & 1));               // also: round r - 2 is accounted
+        __syncwarp();
+        const BarSig* const sigs = &sm.sig[s][0];
+        float2* const recs = reinterpret_cast<float2*>(&sm.rec[s][0][slotj]);   // bar i at recs[32 * i]
+        const int64_t t0 = r * ROUND_BARS;
+        const int n = (int)(T - t0 < ROUND_BARS ? T - t0 : ROUND_BARS);
+
+        if (n < ROUND_BARS) {
+#pragma unroll 1
+            for (int i = 0; i < n; ++i) recs[32 * i] = step1(&sigs[i], inv2);
+        } else {
+            // ---- two chains.  B runs half a step behind A: each half-step overlaps one chain's layer-2 burst with
+            // the other's reduction, fill decision and next layer 1; all loads of a half come first in program order,
+            // its stores last, so that ptxas can interleave the two chains' arithmetic.
+            const BarSig* const sigB = sigs + (N - burn);
+            float2* const recB = recs + 32 * (N - burn);     // burn-in records land on bars chain A rewrites later
+            float inv2B = 0.0f, inv2Bent = 0.0f;           // B's inventory; B's inventory entering bar N
+            float2 pA, pB;
+            {
+                float h[U];
+                h32_layer1<U>(w, *reinterpret_cast<const float2*>(&sigs[0].z1), inv2, h);
+                h32_put_h1<U>(hA, g, l, h);
+                h32_layer1<U>(w, *reinterpret_cast<const float2*>(&sigB[0].z1), inv2B, h);
+                h32_put_h1<U>(hB, g, l, h);
+                __syncwarp();
+                float4 h4[8];
+                h32_get_h1<U>(hB, g, h4);
+                pB = h32_layer23<U>(w, h4);
+                if (U == 4) h32_put_partial(rB, g, l, pB);
+            }
+#pragma unroll 1
+            for (int i = 0; i < N; ++i) {
+                const int ibn = N - burn + i + 1 < ROUND_BARS ? i + 1 : i;   // B's next bar (the last one is not used)
+                // -- half 1: A's layer 2 of bar i | B's decision of its bar i and layer 1 of the next
+                __syncwarp();
+                {
+                    float4 h4[8];
+                    h32_get_h1<U>(hA, g, h4);
+                    float2 qB = pB;
+                    if (U == 4) { float4 pr[4]; h32_get_partials(rB, g, pr); qB = h32_tree(pr); }
+                    const float2 thB = *reinterpret_cast<const float2*>(&sigB[i].tha);
+                    const float2 zB = *reinterpret_cast<const float2*>(&sigB[ibn].z1);
+                    const float2 cB = h32_decide(qB, w.b3a, w.b3b, thB, inv2B);
+                    inv2Bent = i == burn - 1 ? inv2B : inv2Bent;
+                    float h[U];
+                    h32_layer1<U>(w, zB, inv2B, h);
+                    pA = h32_layer23<U>(w, h4);
+                    recB[32 * i] = cB;
+                    h32_put_h1<U>(hB, g, l, h);
+                    if (U == 4) h32_put_partial(rA, g, l, pA);
+                }
+                // -- half 2: B's layer 2 of its next bar | A's decision of bar i and layer 1 of bar i + 1
+                __syncwarp();
+                {
+                    float4 h4[8];
+                    h32_get_h1<U>(hB, g, h4);
+                    float2 qA = pA;
+                    if (U == 4) { float4 pr[4]; h32_get_partials(rA, g, pr); qA = h32_tree(pr); }
+                    const float2 thA = *reinterpret_cast<const float2*>(&sigs[i].tha);
+                    const float2 zA = *reinterpret_cast<const float2*>(&sigs[i + 1].z1);    // i + 1 <= N < ROUND_BARS
+                    const float2 cA = h32_decide(qA, w.b3a, w.b3b, thA, inv2);
+                    float h[U];
+                    h32_layer1<U>(w, zA, inv2, h);
+                    pB = h32_layer23<U>(w, h4);
+                    recs[32 * i] = cA;
+                    h32_put_h1<U>(hA, g, l, h);
+                    if (U == 4) h32_put_partial(rB, g, l, pB);
+                }
+            }
+            __syncwarp();
+            // ---- stitch: where B entered bar N with another inventory than A left it, step B's block again from the
+            // true state until the two inventories meet (from there on the records are the same) or the block ends.
+            // B's own inventory entering each bar comes from the record about to be overwritten.
+            bool fix = live && inv2 != inv2Bent;
+            float inv2R = inv2, inv2O = inv2Bent;
+#pragma unroll 1
+            for (int j = N; j < ROUND_BARS && __any_sync(0xffffffffu, fix); ++j) {
+                const float2 old = recs[32 * j];                                // read before step1's __syncwarp
+                const float2 c = step1(&sigs[j], inv2R);
+                inv2O = __fadd_rn(inv2O, h32_record_move(old));
+                recs[32 * j] = fix ? c : old;
+                fix = fix && inv2R != inv2O;
+            }
+            inv2 = fix ? inv2R : inv2B;                                         // the state entering the next round
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&sm.rec_full[s]);
+    }
+}
+
+template <int U, bool FEE>
+static int launch_variant2(const RolloutArgs& args, int warps, int burn, cudaStream_t st)
+{
+    auto kern = rollout2_kernel_h32<U, FEE>;
+    static std::atomic<uint64_t> configured{0};   // per instantiation, one bit per device
+    const size_t smem = sizeof(Ring2Smem);
+    if (int rc = opt_in_smem(kern, smem, configured, "cudaFuncSetAttribute(smem)")) return rc;
+    const int64_t per_cta = (int64_t)warps * U;
+    const int64_t blocks = (args.mm.count + per_cta - 1) / per_cta;
+    kern<<<(unsigned)blocks, (warps + 1) * 32, smem, st>>>(args, burn);   // + the producer warp
+    return check_cuda(cudaGetLastError(), "rollout2_kernel_h32 launch");
+}
+
+template <int U>
+static int launch_u2(const RolloutArgs& args, bool fee, int warps, int burn, cudaStream_t st)
+{
+    return fee ? launch_variant2<U, true>(args, warps, burn, st) : launch_variant2<U, false>(args, warps, burn, st);
+}
+
 int launch_rollout(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int hidden,
                    double phi, double fee, int units_per_lane, int warps_per_cta,
                    double* fitness, int32_t* trades, cudaStream_t st)
@@ -536,6 +923,16 @@ int launch_rollout(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, 
     args.fitness = fitness; args.trades = trades;
     args.codes = nullptr;
     const bool has_fee = (fee != 0.0);
+    // without the adversary: two time blocks per warp (rollout2_kernel_h32) unless SGMM_ROLLOUT_CHAINS=1; the burn-in of
+    // the second block from SGMM_ROLLOUT_BURN_IN (even, 0 .. ROUND_BARS - 2; 0 makes the stitch repair almost every round)
+    static const int chains = [] { const char* e = getenv("SGMM_ROLLOUT_CHAINS"); return e && atoi(e) == 1 ? 1 : 2; }();
+    static const int burn = [] {
+        const char* e = getenv("SGMM_ROLLOUT_BURN_IN");
+        const int v = e ? atoi(e) : ROLLOUT_BURN_IN;
+        return (v < 0 ? 0 : (v > ROUND_BARS - 2 ? ROUND_BARS - 2 : v)) & ~1;
+    }();
+    // (U = 2, only when pinned by the caller, stays single-chain: 5.49 against 5.35 ms at P = 4096 x 14 400 bars)
+    if (!adv && chains == 2 && U != 2) return U == 1 ? launch_u2<1>(args, has_fee, W, burn, st) : launch_u2<4>(args, has_fee, W, burn, st);
     switch (U) {
         case 1: return launch_u<1>(args, adv != nullptr, has_fee, W, st);
         case 2: return launch_u<2>(args, adv != nullptr, has_fee, W, st);
