@@ -139,6 +139,9 @@ SIGNATURES = {
     "sgmm_ga_set_parents": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "sgmm_ga_run_parents_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_ga_parents_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sgmm_ga_set_es": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p]),
+    "sgmm_ga_run_es_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sgmm_ga_es_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_bundle_windows": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_bundle_windows_host": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,

@@ -5,7 +5,8 @@
 //             (master, sigma, seed, generation, i) with the counter-based noise of sgmm_rng.cuh
 //   tell      argmax with numpy's semantics (first maximum, a NaN wins) -> master <- that child
 //             (model.py:73-76); the adversary is told -fitness (drl_engine.py:123-125).  After sgmm_ga_set_parents:
-//             the mu best children (device top-k) recombined into master + sigma * sum_k w_k eps_k instead
+//             the mu best children (device top-k) recombined into master + sigma * sum_k w_k eps_k instead; after
+//             sgmm_ga_set_es: centered-rank utilities of every child, g = sum_i u_i eps_i / (lambda sigma), an Adam step
 //   validate  rollout of the new master (== best child, drl_engine.py:129-140) with no adversary
 //   select    keep-best-on-validation snapshot (:144-150), sigma halving after `patience` stale
 //             generations (:155-160), history (:163-167)
@@ -317,6 +318,164 @@ __global__ void __launch_bounds__(RECOMBINE_THREADS) ga_recombine_kernel(const G
         if (4 * q + i < n) m[4 * q + i] = __fadd_rn(m[4 * q + i], __fmul_rn(acc[i], sigma));
 }
 
+// ---- natural-gradient evolution strategy (sgmm_ga_set_es): centered-rank utilities of all lambda children, the noise-
+// weighted sum g = sum_i u_i eps_i / (lambda sigma) in a fixed order, and an Adam ascent step on the master.
+//   rank      r_i = child i's position in ga_select_kernel's order (NaN first, then descending fitness -- the adversary's
+//             ascending --, ties to the lower index, -0.0 == +0.0);  u_i = fl(fl((float)(lambda-1-r_i) / (float)(lambda-1)) - 0.5f)
+//   sum       index order, segments of ES_SEGMENT children: acc = u_i*eps_i for a segment's first child, then fmaf(u_i, eps_i,
+//             acc); the segment sums are combined by a pairwise tree ((s0+s1), (s2+s3), ...; an odd last one moves up)
+//   gradient  g = fl(S * fl(1 / fl((float)lambda * sigma))), sigma the run's device sigma of this generation
+//   Adam      p1 *= b1, p2 *= b2 (running products from 1, once per generation);  m = b1*m + (1-b1)*g;  v = b2*v + (1-b2)*g*g;
+//             theta += lr * ((m / (1-p1)) / (sqrt(v / (1-p2)) + eps)), every operation one binary32 rounding
+// The segment length is part of the definition, not of the launch.
+constexpr int ES_SEGMENT = 256;
+constexpr int ES_RANK_THREADS = 256;
+constexpr int ES_GRAD_THREADS = 256;
+constexpr int ES_GRAD_QUADS = 16;                                   // quads (64 elements) per gradient block
+constexpr int ES_GRAD_CHUNK = 64;                                   // children per noise chunk of a gradient block
+constexpr int ES_ADAM_THREADS = 256;
+constexpr float ES_B1 = 0.9f, ES_B2 = 0.999f, ES_EPS = 1e-8f;
+
+// Block (run, t) ranks run r's children t*256 .. t*256+255 in one direction by counting the children ranked before each
+// (every key above it, and the equal keys of lower index), reading all the run's keys tile by tile through for_children.
+template <int SIGN>
+__device__ int64_t es_rank(const Gather& f, int64_t first, int64_t n, int64_t i, uint64_t* s_key, int64_t* s_j0)
+{
+    const uint64_t ki = i < n ? rank_key<SIGN>(f.fit(first + i)) : 0ull;
+    int64_t before = 0;
+    for_children<SIGN>(f, first, n, [&](int64_t j, uint64_t key, bool valid) {
+        s_key[threadIdx.x] = key;                                   // the tile: children j0 .. j0+cnt-1 (a valid prefix)
+        if (threadIdx.x == 0) *s_j0 = j;
+        const int cnt = __syncthreads_count(valid);
+        const int64_t j0 = *s_j0;
+        const int lim = (int)max((int64_t)0, min((int64_t)cnt, i - j0));   // tile entries of lower index than i
+        int c = 0;
+        for (int k = 0; k < lim; ++k) c += s_key[k] >= ki ? 1 : 0;
+        for (int k = lim; k < cnt; ++k) c += s_key[k] > ki ? 1 : 0;
+        before += c;
+        __syncthreads();
+    });
+    return before;
+}
+
+__device__ __forceinline__ float es_utility(int64_t r, int64_t n)
+{
+    return __fsub_rn(__fdiv_rn((float)(n - 1 - r), (float)(n - 1)), 0.5f);
+}
+
+// Grid (runs, ceil(lambda/256)): utilities u[runs][lambda] (and adv_u under use_arl), the best child's state as
+// ga_select_kernel records it, and the run's Adam powers (block 0).
+__global__ void __launch_bounds__(ES_RANK_THREADS) es_rank_kernel(GaDev* runs, const Gather fit, int64_t pop, float* u,
+                                                                   float* adv_u, float* pows, int use_arl)
+{
+    __shared__ uint64_t s_key[ES_RANK_THREADS];
+    __shared__ int64_t s_j0;
+    const int64_t run = blockIdx.x, first = run * pop;
+    const int64_t i = (int64_t)blockIdx.y * blockDim.x + threadIdx.x;
+    GaDev* st = runs + run;
+    const int64_t r = es_rank<+1>(fit, first, pop, i, s_key, &s_j0);
+    if (i < pop) {
+        u[run * pop + i] = es_utility(r, pop);
+        if (r == 0) {
+            st->best_idx = i;
+            st->train_f = fit.fit(first + i); st->train_trades = fit.trd(first + i);
+            if (!use_arl) st->adv_best_idx = 0;
+        }
+    }
+    if (use_arl) {
+        const int64_t ra = es_rank<-1>(fit, first, pop, i, s_key, &s_j0);
+        if (i < pop) {
+            adv_u[run * pop + i] = es_utility(ra, pop);
+            if (ra == 0) st->adv_best_idx = i;
+        }
+    }
+    if (blockIdx.y == 0 && threadIdx.x == 0) {
+        pows[2 * run] = __fmul_rn(pows[2 * run], ES_B1);
+        pows[2 * run + 1] = __fmul_rn(pows[2 * run + 1], ES_B2);
+    }
+}
+
+// Grid (runs, quad blocks, segments): block (r, b, s) owns ES_GRAD_QUADS element quads of one master (quad blocks
+// [0, mm_blocks) the market maker's G elements, the rest the adversary's 1250) and segment s of run r's children.  Its
+// threads regenerate the noise of ES_GRAD_CHUNK children at a time into shared memory; thread e < 64 then chains element
+// e's fmaf over those children in index order.  The segment sum goes to part[r][s][element].
+__global__ void __launch_bounds__(ES_GRAD_THREADS) es_grad_kernel(const GaDev* runs, int64_t pop, const float* u,
+                                                                   const float* adv_u, float* part, float* adv_part,
+                                                                   int64_t G, int mm_blocks)
+{
+    __shared__ float4 s_eps[ES_GRAD_CHUNK][ES_GRAD_QUADS];
+    __shared__ float s_u[ES_GRAD_CHUNK];
+    const int64_t run = blockIdx.x, seg = blockIdx.z, nseg = gridDim.z;
+    const GaDev* st = runs + run;
+    const bool adv = (int)blockIdx.y >= mm_blocks;
+    const int64_t n = adv ? 1250 : G;
+    const int64_t q0 = (int64_t)(adv ? blockIdx.y - mm_blocks : blockIdx.y) * ES_GRAD_QUADS;
+    const float* ur = (adv ? adv_u : u) + run * pop;
+    const uint64_t seed = adv ? st->seed ^ ADV_SEED_FLIP : st->seed, gen = (uint64_t)st->generation;
+    const int64_t c0 = seg * ES_SEGMENT, c1 = min(pop, c0 + ES_SEGMENT);
+    const int e = threadIdx.x;
+    const int64_t elem = 4 * q0 + e;
+    float acc = 0.0f;
+    for (int64_t cb = c0; cb < c1; cb += ES_GRAD_CHUNK) {
+        const int nc = (int)min((int64_t)ES_GRAD_CHUNK, c1 - cb);
+        for (int t = threadIdx.x; t < ES_GRAD_CHUNK * ES_GRAD_QUADS; t += blockDim.x) {
+            const int c = t / ES_GRAD_QUADS, qi = t % ES_GRAD_QUADS;
+            const int64_t q = q0 + qi;
+            if (c < nc && 4 * q < n) {
+                float z[4]; normal4(seed, gen, (uint64_t)(cb + c), (uint32_t)q, z);
+                s_eps[c][qi] = make_float4(z[0], z[1], z[2], z[3]);
+            }
+        }
+        if (threadIdx.x < nc) s_u[threadIdx.x] = ur[cb + threadIdx.x];
+        __syncthreads();
+        if (e < 4 * ES_GRAD_QUADS) {
+            const float* col = reinterpret_cast<const float*>(&s_eps[0][0]) + e;
+            for (int c = 0; c < nc; ++c) {
+                const float x = col[c * 4 * ES_GRAD_QUADS], w = s_u[c];
+                acc = (cb + c == c0) ? __fmul_rn(w, x) : __fmaf_rn(w, x, acc);
+            }
+        }
+        __syncthreads();
+    }
+    if (e < 4 * ES_GRAD_QUADS && elem < n) (adv ? adv_part + run * nseg * 1250 : part + run * nseg * G)[seg * n + elem] = acc;
+}
+
+// Grid (runs, element blocks): thread (r, e) combines element e's segment sums of run r by the pairwise tree (in place in
+// part[r][.][e]), scales them into the gradient and takes the Adam step on the master (blocks [0, mm_blocks) the market
+// maker's G elements, the rest the adversary's 1250, from its own utilities and adv_sigma).
+__global__ void __launch_bounds__(ES_ADAM_THREADS) es_adam_kernel(const GaDev* runs, int64_t pop, int nseg, float lr,
+                                                                   const float* pows, float* part, float* adv_part,
+                                                                   float* grad, float* adv_grad, float* mom, float* adv_mom,
+                                                                   float* vel, float* adv_vel, float* mm_masters,
+                                                                   float* adv_masters, int64_t G, int mm_blocks)
+{
+    const int64_t run = blockIdx.x;
+    const GaDev* st = runs + run;
+    const bool adv = (int)blockIdx.y >= mm_blocks;
+    const int64_t n = adv ? 1250 : G;
+    const int64_t e = (int64_t)(adv ? blockIdx.y - mm_blocks : blockIdx.y) * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    float* p = (adv ? adv_part + run * (int64_t)nseg * 1250 : part + run * (int64_t)nseg * G) + e;
+    for (int len = nseg; len > 1; len = (len + 1) >> 1) {
+        for (int k = 0; 2 * k + 1 < len; ++k) p[k * n] = __fadd_rn(p[2 * k * n], p[(2 * k + 1) * n]);
+        if (len & 1) p[(len >> 1) * n] = p[(len - 1) * n];
+    }
+    const float sigma = adv ? st->adv_sigma : st->sigma;
+    const float g = __fmul_rn(p[0], __fdiv_rn(1.0f, __fmul_rn((float)pop, sigma)));
+    const int64_t o = run * n + e;
+    float* m = (adv ? adv_mom : mom) + o;
+    float* v = (adv ? adv_vel : vel) + o;
+    float* th = (adv ? adv_masters : mm_masters) + o;
+    (adv ? adv_grad : grad)[o] = g;
+    const float p1 = pows[2 * run], p2 = pows[2 * run + 1];
+    const float mn = __fadd_rn(__fmul_rn(ES_B1, *m), __fmul_rn(__fsub_rn(1.0f, ES_B1), g));
+    const float vn = __fadd_rn(__fmul_rn(ES_B2, *v), __fmul_rn(__fsub_rn(1.0f, ES_B2), __fmul_rn(g, g)));
+    const float mh = __fdiv_rn(mn, __fsub_rn(1.0f, p1));
+    const float vh = __fdiv_rn(vn, __fsub_rn(1.0f, p2));
+    *m = mn; *v = vn;
+    *th = __fadd_rn(*th, __fmul_rn(lr, __fdiv_rn(mh, __fadd_rn(__fsqrt_rn(vh), ES_EPS))));
+}
+
 }  // namespace sgmm
 
 using namespace sgmm;
@@ -339,6 +498,15 @@ struct sgmm_ga {
     int32_t parents = 1;
     float* weights = nullptr;                                               // [parents]
     int64_t* mm_parents = nullptr; int64_t* adv_parents = nullptr;          // [runs][parents]
+    // evolution strategy (sgmm_ga_set_es): es_lr > 0 selects es_rank_kernel + es_grad_kernel + es_adam_kernel
+    float es_lr = 0.0f;
+    int32_t es_nseg = 0;                                                    // ceil(lambda / ES_SEGMENT)
+    float* es_u = nullptr; float* es_adv_u = nullptr;                       // [runs][lambda]
+    float* es_part = nullptr; float* es_adv_part = nullptr;                 // [runs][nseg][G], [runs][nseg][1250]
+    float* es_grad = nullptr; float* es_adv_grad = nullptr;                 // [runs][G], [runs][1250]
+    float* es_m = nullptr; float* es_adv_m = nullptr;                       // Adam moments, as the gradients
+    float* es_v = nullptr; float* es_adv_v = nullptr;
+    float* es_pow = nullptr;                                                // [runs][2]: b1^t, b2^t
     bool started = false;                                                   // a generation phase has been enqueued
 };
 
@@ -393,6 +561,14 @@ int single_run(const sgmm_ga* ga, const char* what)
     set_error("%s: this GA is a sweep of %d runs; use the per-run entry sgmm_ga_run_%s", what, (int)ga->runs,
               what + sizeof("sgmm_ga_") - 1);
     return SGMM_ERR_INVALID;
+}
+
+void es_free(sgmm_ga* ga)
+{
+    float** bufs[] = {&ga->es_u, &ga->es_adv_u, &ga->es_part, &ga->es_adv_part, &ga->es_grad, &ga->es_adv_grad,
+                      &ga->es_m, &ga->es_adv_m, &ga->es_v, &ga->es_adv_v, &ga->es_pow};
+    for (float** b : bufs) { cudaFree(*b); *b = nullptr; }
+    ga->es_lr = 0.0f; ga->es_nseg = 0;
 }
 
 int check_run(const sgmm_ga* ga, int32_t run)
@@ -485,6 +661,7 @@ int sgmm_ga_destroy(sgmm_ga* ga)
         cudaFree(ga->st); cudaFree(ga->h_train_f); cudaFree(ga->h_val_f); cudaFree(ga->h_train_t);
         cudaFree(ga->h_val_t); cudaFree(ga->h_sigma);
         cudaFree(ga->weights); cudaFree(ga->mm_parents); cudaFree(ga->adv_parents);
+        es_free(ga);
     }
     delete ga;
     return SGMM_OK;
@@ -535,7 +712,23 @@ int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
     cudaStream_t st = (cudaStream_t)stream;
     const sgmm_ga_config& c = ga->cfg;
     ga->started = true;
-    if (!ga->weights) {
+    if (ga->es_lr > 0.0f) {
+        const int64_t lam = c.pop_size;
+        es_rank_kernel<<<dim3((unsigned)ga->runs, (unsigned)((lam + ES_RANK_THREADS - 1) / ES_RANK_THREADS)), ES_RANK_THREADS, 0, st>>>(
+            ga->st, ga->gather, lam, ga->es_u, ga->es_adv_u, ga->es_pow, c.use_arl);
+        if (int rc = check_cuda(cudaGetLastError(), "es_rank_kernel launch")) return rc;
+        const int64_t quads = 4 * ES_GRAD_QUADS;
+        const int mm_blocks = (int)((ga->G + quads - 1) / quads), adv_blocks = c.use_arl ? (int)((1250 + quads - 1) / quads) : 0;
+        es_grad_kernel<<<dim3((unsigned)ga->runs, (unsigned)(mm_blocks + adv_blocks), (unsigned)ga->es_nseg), ES_GRAD_THREADS, 0, st>>>(
+            ga->st, lam, ga->es_u, ga->es_adv_u, ga->es_part, ga->es_adv_part, ga->G, mm_blocks);
+        if (int rc = check_cuda(cudaGetLastError(), "es_grad_kernel launch")) return rc;
+        const int mm_eblocks = (int)((ga->G + ES_ADAM_THREADS - 1) / ES_ADAM_THREADS);
+        const int adv_eblocks = c.use_arl ? (1250 + ES_ADAM_THREADS - 1) / ES_ADAM_THREADS : 0;
+        es_adam_kernel<<<dim3((unsigned)ga->runs, (unsigned)(mm_eblocks + adv_eblocks)), ES_ADAM_THREADS, 0, st>>>(
+            ga->st, lam, ga->es_nseg, ga->es_lr, ga->es_pow, ga->es_part, ga->es_adv_part, ga->es_grad, ga->es_adv_grad,
+            ga->es_m, ga->es_adv_m, ga->es_v, ga->es_adv_v, ga->mm_master, ga->adv_master, ga->G, mm_eblocks);
+        if (int rc = check_cuda(cudaGetLastError(), "es_adam_kernel launch")) return rc;
+    } else if (!ga->weights) {
         ga_tell_kernel<<<(unsigned)ga->runs, 256, 0, st>>>(ga->st, ga->gather, c.pop_size, ga->mm_master, ga->G,
                                                            ga->adv_master, c.use_arl);
         if (int rc = check_cuda(cudaGetLastError(), "ga_tell_kernel launch")) return rc;
@@ -650,6 +843,10 @@ int sgmm_ga_set_parents(sgmm_ga* ga, int32_t parents, const float* weights, void
         set_error("sgmm_ga_set_parents: a generation of this GA has already been enqueued; set the parents right after create");
         return SGMM_ERR_INVALID;
     }
+    if (ga->es_lr > 0.0f) {
+        set_error("sgmm_ga_set_parents: this GA runs the evolution strategy (sgmm_ga_set_es); the two updates exclude each other");
+        return SGMM_ERR_INVALID;
+    }
     if (parents < 1 || parents > SGMM_MAX_PARENTS || parents > ga->cfg.pop_size) {
         set_error("parents=%d: need 1 <= parents <= min(pop_size=%lld, %d)", (int)parents, (long long)ga->cfg.pop_size,
                   SGMM_MAX_PARENTS);
@@ -714,6 +911,69 @@ int sgmm_ga_parents_host(sgmm_ga* ga, int32_t n, int64_t* mm_index, int64_t* adv
     if (!ga || n < 0) { set_error("bad argument"); return SGMM_ERR_INVALID; }
     if (int rc = single_run(ga, "sgmm_ga_parents_host")) return rc;
     return sgmm_ga_run_parents_host(ga, 0, n, mm_index, adv_index, stream);
+}
+
+int sgmm_ga_set_es(sgmm_ga* ga, float lr, void* stream)
+{
+    if (!ga) { set_error("ga is NULL"); return SGMM_ERR_INVALID; }
+    if (ga->started) {
+        set_error("sgmm_ga_set_es: a generation of this GA has already been enqueued; set the evolution strategy right after create");
+        return SGMM_ERR_INVALID;
+    }
+    if (!std::isfinite(lr) || !(lr > 0.0f)) { set_error("lr=%g: the Adam step size must be finite and > 0", (double)lr); return SGMM_ERR_INVALID; }
+    if (ga->weights) {
+        set_error("sgmm_ga_set_es: this GA runs truncation selection (sgmm_ga_set_parents); the two updates exclude each other");
+        return SGMM_ERR_INVALID;
+    }
+    const int64_t lam = ga->cfg.pop_size;
+    if (lam < 2) { set_error("pop_size=%lld: centered-rank utilities need lambda >= 2", (long long)lam); return SGMM_ERR_INVALID; }
+    if (lam > (int64_t)65535 * ES_RANK_THREADS) {
+        set_error("pop_size=%lld: the evolution strategy ranks at most %lld children per run", (long long)lam,
+                  (long long)65535 * ES_RANK_THREADS);
+        return SGMM_ERR_INVALID;
+    }
+    DeviceGuard guard(ga->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    es_free(ga);                                                    // a second call before the first generation
+    const size_t R = (size_t)ga->runs, G = (size_t)ga->G, L = (size_t)lam, S = (size_t)((lam + ES_SEGMENT - 1) / ES_SEGMENT);
+    struct { float** p; size_t n; } bufs[] = {
+        {&ga->es_u, R * L}, {&ga->es_adv_u, R * L}, {&ga->es_part, R * S * G}, {&ga->es_adv_part, R * S * 1250},
+        {&ga->es_grad, R * G}, {&ga->es_adv_grad, R * 1250}, {&ga->es_m, R * G}, {&ga->es_adv_m, R * 1250},
+        {&ga->es_v, R * G}, {&ga->es_adv_v, R * 1250}, {&ga->es_pow, R * 2}};
+    int rc = SGMM_OK;
+    for (auto& b : bufs) {
+        if (!rc) rc = check_cuda(cudaMalloc(b.p, b.n * sizeof(float)), "cudaMalloc");
+        if (!rc) rc = check_cuda(cudaMemsetAsync(*b.p, 0, b.n * sizeof(float), st), "memset");
+    }
+    std::vector<float> ones(2 * R, 1.0f);                           // b1^0, b2^0
+    if (!rc) rc = check_cuda(cudaMemcpyAsync(ga->es_pow, ones.data(), 2 * R * sizeof(float), cudaMemcpyHostToDevice, st), "H2D es powers");
+    if (!rc) rc = check_cuda(cudaStreamSynchronize(st), "ga_set_es");
+    if (rc) { es_free(ga); return rc; }                             // back to the (1,lambda) GA
+    ga->es_lr = lr; ga->es_nseg = (int32_t)S;
+    return SGMM_OK;
+}
+
+int sgmm_ga_run_es_host(sgmm_ga* ga, int32_t run, float* utilities, float* grad, float* adv_utilities, float* adv_grad,
+                        void* stream)
+{
+    if (!ga) { set_error("ga is NULL"); return SGMM_ERR_INVALID; }
+    if (int rc = check_run(ga, run)) return rc;
+    if (!(ga->es_lr > 0.0f)) { set_error("sgmm_ga_run_es_host: this GA does not run the evolution strategy (sgmm_ga_set_es)"); return SGMM_ERR_INVALID; }
+    DeviceGuard guard(ga->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t L = (size_t)ga->cfg.pop_size, G = (size_t)ga->G, r = (size_t)run;
+    if (utilities) if (int rc = check_cuda(cudaMemcpyAsync(utilities, ga->es_u + r * L, L * sizeof(float), cudaMemcpyDeviceToHost, st), "D2H es")) return rc;
+    if (grad) if (int rc = check_cuda(cudaMemcpyAsync(grad, ga->es_grad + r * G, G * sizeof(float), cudaMemcpyDeviceToHost, st), "D2H es")) return rc;
+    if (adv_utilities) if (int rc = check_cuda(cudaMemcpyAsync(adv_utilities, ga->es_adv_u + r * L, L * sizeof(float), cudaMemcpyDeviceToHost, st), "D2H es")) return rc;
+    if (adv_grad) if (int rc = check_cuda(cudaMemcpyAsync(adv_grad, ga->es_adv_grad + r * 1250, 1250 * sizeof(float), cudaMemcpyDeviceToHost, st), "D2H es")) return rc;
+    return check_cuda(cudaStreamSynchronize(st), "ga_es");
+}
+
+int sgmm_ga_es_host(sgmm_ga* ga, float* utilities, float* grad, float* adv_utilities, float* adv_grad, void* stream)
+{
+    if (!ga) { set_error("ga is NULL"); return SGMM_ERR_INVALID; }
+    if (int rc = single_run(ga, "sgmm_ga_es_host")) return rc;
+    return sgmm_ga_run_es_host(ga, 0, utilities, grad, adv_utilities, adv_grad, stream);
 }
 
 }  // extern "C"

@@ -448,8 +448,46 @@ def _parent_weights(parents, weights, pop_size):
     return w
 
 
+def _es_lr(es_lr, parents, weights, pop_size):
+    """Checks the evolution-strategy arguments (``sgmm_ga_set_es``) without touching a device.  Returns the Adam step size
+    as a float, or ``None`` when the GA keeps its (1,lambda) or truncation-selection update."""
+    if es_lr is None:
+        return None
+    if isinstance(es_lr, bool) or not isinstance(es_lr, (int, float, np.floating, np.integer)):
+        raise ValueError(f"es_lr must be a number, got {es_lr!r}")
+    lr = float(np.float32(es_lr))
+    if not np.isfinite(lr) or not lr > 0:
+        raise ValueError(f"es_lr={es_lr!r}: the Adam step size must be finite and > 0")
+    if parents != 1 or weights is not None:
+        raise ValueError("es_lr (evolution strategy) and parents / weights (truncation selection) exclude each other")
+    if int(pop_size) < 2:
+        raise ValueError(f"pop_size={pop_size}: the evolution strategy's centered ranks need pop_size >= 2")
+    return lr
+
+
 class _GAHandle:
     """What every ``sgmm_ga`` handle offers: the generation phases, graph capture, the per-run read-backs and close."""
+
+    def _set_es(self, lr):
+        """After create: switch to the evolution strategy with Adam step size ``lr`` (from :func:`_es_lr`)."""
+        self.es_lr = lr
+        if lr is None:
+            return
+        try:
+            _lib.check(_lib.lib().sgmm_ga_set_es(self._h, lr, _stream(self.device)))
+        except Exception:
+            self.close()
+            raise
+
+    def es_state(self, run=0):
+        """The evolution strategy's last generation of run ``run``: ``{"utilities", "adv_utilities"}`` float32[lambda] in
+        child-index order and ``{"grad", "adv_grad"}`` float32[G] / [1250] (the adversary's read 0 without use_arl)."""
+        lam = self.pop_size
+        u, au = np.zeros(lam, np.float32), np.zeros(lam, np.float32)
+        g, ag = np.zeros(self.G, np.float32), np.zeros(1250, np.float32)
+        _lib.check(_lib.lib().sgmm_ga_run_es_host(self._h, int(run), u.ctypes.data, g.ctypes.data, au.ctypes.data,
+                                                  ag.ctypes.data, _stream(self.device)))
+        return {"utilities": u, "grad": g, "adv_utilities": au, "adv_grad": ag}
 
     def _set_parents(self, parents, w):
         """After create: switch to truncation selection of ``parents`` parents (``w``: from :func:`_parent_weights`)."""
@@ -530,11 +568,17 @@ class DeviceGA(_GAHandle):
 
     ``parents`` (mu) > 1 or ``weights`` switch the (1,lambda) rule to truncation selection (``sgmm_ga_set_parents``): the
     mu best children in rank order are recombined into the new master ``master + sigma * sum_k weights[k] * eps_k``
-    (``weights`` float[mu], used as given; default ``1/mu`` each).  ``parents()`` reads the last generation's parents."""
+    (``weights`` float[mu], used as given; default ``1/mu`` each).  ``parents()`` reads the last generation's parents.
+
+    ``es_lr`` switches it to a natural-gradient evolution strategy (``sgmm_ga_set_es``): centered-rank utilities of all
+    lambda children, ``g = sum_i u_i eps_i / (lambda sigma)`` and an Adam ascent step of size ``es_lr`` on the master
+    (the adversary's on -fitness).  ``es_state()`` reads the last generation's utilities and gradients."""
 
     def __init__(self, mm_master, adv_master=None, *, pop_size, sigma, phi, fee_rate, use_arl, seed,
-                 max_generations, patience=15, hidden=32, device=None, shard=None, precision=None, parents=1, weights=None):
+                 max_generations, patience=15, hidden=32, device=None, shard=None, precision=None, parents=1, weights=None,
+                 es_lr=None):
         w = _parent_weights(parents, weights, pop_size)
+        lr = _es_lr(es_lr, parents, weights, pop_size)
         self.device = torch.cuda.current_device() if device is None else int(device)
         first, count, stride = (0, pop_size, 0) if shard is None else shard
         cfg = _lib.GaConfig(hidden, int(bool(use_arl)), pop_size, first, count, stride, float(sigma), patience,
@@ -551,6 +595,7 @@ class DeviceGA(_GAHandle):
                                              None if a is None else a.ctypes.data, self.device,
                                              _stream(self.device)))
         self._set_parents(parents, w)
+        self._set_es(lr)
 
     def parents(self):
         """``(mm_index, adv_index)`` int64[mu]: the last generation's parents in rank order (global child indices)."""
@@ -585,11 +630,13 @@ class DeviceGASweep(_GAHandle):
     every run), ``adv_masters`` likewise when ``use_arl``.  ``pop_size`` is lambda PER RUN.  Run r is bit-identical to
     ``DeviceGA(masters[r], adv_masters[r], precision="exact", **runs[r])``.  Hidden width 32, exact precision, one
     device.  Read-backs take the run: ``status(r)``, ``masters(r)``, ``history(r)``, ``parents(r)``.  ``parents`` /
-    ``weights`` select truncation selection as for :class:`DeviceGA`, one setting for every run."""
+    ``weights`` select truncation selection and ``es_lr`` the evolution strategy as for :class:`DeviceGA`, one setting
+    for every run; ``es_state(r)`` reads run r's last utilities and gradients."""
 
     def __init__(self, masters, adv_masters=None, *, runs, pop_size, use_arl, max_generations, device=None, parents=1,
-                 weights=None):
+                 weights=None, es_lr=None):
         w = _parent_weights(parents, weights, pop_size)
+        lr = _es_lr(es_lr, parents, weights, pop_size)
         self.device = torch.cuda.current_device() if device is None else int(device)
         K = len(runs)
         if K == 0:
@@ -627,6 +674,7 @@ class DeviceGASweep(_GAHandle):
         _lib.check(_lib.lib().sgmm_ga_create_sweep(C.byref(self._h), C.byref(cfg), K, arr, m.ctypes.data,
                                                    None if a is None else a.ctypes.data, self.device, _stream(self.device)))
         self._set_parents(parents, w)
+        self._set_es(lr)
 
     def parents(self, run=0):
         """``(mm_index, adv_index)`` int64[mu] of run ``run``: its last generation's parents in rank order (indices within
@@ -668,13 +716,19 @@ class DRLEngine:
       keep the (1,lambda) rule.  With mu > 1 the master is no longer a child: ``val_f`` in the history, the
       keep-best-on-validation choice and the checkpoint all belong to the recombined master; ``train_f`` /
       ``train_trades`` stay those of the best child.
+    * ``es_lr`` replaces it by a natural-gradient evolution strategy (OpenAI-ES: centered-rank utilities of every child,
+      ``g = sum_i u_i eps_i / (lambda sigma)``, an Adam ascent step of size ``es_lr``; see :class:`DeviceGA`), in
+      ``train`` (solo and sharded) and ``train_sweep``.  It excludes ``parents`` > 1 / ``parent_weights``.  As with
+      truncation selection, ``val_f``, keep-best and the checkpoint belong to the updated master, ``train_f`` /
+      ``train_trades`` to the best child.
     """
 
     def __init__(self, pop_size=50, sigma=0.05, phi=0.01, tick_size=0.01, fee_rate=0.0, use_arl=False,
                  save_dir="checkpoints/drl", seed=None, device=None, patience=15, precision=None, hidden_dim=32,
-                 group=None, parents=1, parent_weights=None):
+                 group=None, parents=1, parent_weights=None, es_lr=None):
         _parent_weights(parents, parent_weights, pop_size)            # argument errors before any side effect
-        self.parents, self.parent_weights = parents, parent_weights
+        _es_lr(es_lr, parents, parent_weights, pop_size)
+        self.parents, self.parent_weights, self.es_lr = parents, parent_weights, es_lr
         self.precision = precision
         self.phi = phi
         self.tick_size = tick_size
@@ -725,7 +779,7 @@ class DRLEngine:
                             fee_rate=self.fee_rate, use_arl=self.use_arl, seed=seed,
                             max_generations=max(1, generations), patience=self.patience, device=dev,
                             precision=self.precision, hidden=self.hidden_dim, shard=shard,
-                            parents=self.parents, weights=self.parent_weights)
+                            parents=self.parents, weights=self.parent_weights, es_lr=self.es_lr)
         if sharded:
             from .dist import ShardedGA
             runner = ShardedGA(make, pop, group=self.group)
@@ -825,7 +879,7 @@ class DRLEngine:
                            self.adv_evolver.master_policy.get_weights() if self.use_arl else None,
                            runs=runs, pop_size=self.mm_evolver.pop_size, use_arl=self.use_arl,
                            max_generations=max(1, generations), device=dev, parents=self.parents,
-                           weights=self.parent_weights)
+                           weights=self.parent_weights, es_lr=self.es_lr)
         save_paths = [os.path.join(self.save_dir, f"{output_prefix}_run{r}_best_val_{phi_r[r]}.pth") for r in range(K)]
         saved_val = [-np.inf] * K
 

@@ -417,6 +417,34 @@ int sgmm_ga_run_parents_host(sgmm_ga* ga, int32_t run, int32_t n, int64_t* mm_in
 int sgmm_ga_parents_host(sgmm_ga* ga, int32_t n, int64_t* mm_index, int64_t* adv_index, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Natural-gradient evolution strategy (OpenAI-ES with Adam), on any GA handle (solo, sharded or sweep; one lr for every
+ * run).  Each generation every child of a run contributes, by its centered-rank utility:
+ *     r_i  = child i's position in the rank order of sgmm_ga_set_parents (NaN first, then descending fitness -- the
+ *            adversary's ascending --, ties to the lower index, -0.0 == +0.0), 0 = best
+ *     u_i  = fl(fl((float)(lambda-1-r_i) / (float)(lambda-1)) - 0.5f)
+ *     S    = sum of u_i*eps_i in index order, in segments of 256 children: acc = u_i*eps_i for a segment's first child,
+ *            then acc = fmaf(u_i, eps_i, acc); the segment sums combined by a pairwise tree ((s0+s1), (s2+s3), ...; an odd
+ *            last one moves up unchanged).  eps_i is child i's noise, as the rollouts regenerate it.
+ *     g    = fl(S * fl(1 / fl((float)lambda * sigma)))   (sigma: the run's sigma of this generation, before any decay)
+ *     Adam ascent, b1 = 0.9f, b2 = 0.999f, eps = 1e-8f, powers p1 = p1*b1, p2 = p2*b2 from 1 once per generation:
+ *            m = b1*m + (1-b1)*g;  v = b2*v + (1-b2)*(g*g);  theta = theta + lr*((m/(1-p1)) / (sqrt(v/(1-p2)) + eps))
+ * every operation one binary32 rounding.  The adversary (use_arl) takes the same step from its own utilities, noise
+ * (seed ^ 1<<63) and adv_sigma, so it ascends -fitness.  History train_f / train_trades and status.last_best_index are
+ * the best child's; validation, keep-best-on-validation and sigma decay act on the updated master.
+ *   lr   the Adam step size: finite and > 0.
+ * Refused (SGMM_ERR_INVALID): after the first evaluate / select / generation of the handle, lambda (pop_size per run)
+ * < 2, together with sgmm_ga_set_parents (in either order).  Call it right after create; the buffers it allocates are
+ * never reallocated by a generation, so captured generations stay valid.  Synchronises the stream.  Sharded GAs need no
+ * extra exchange: every rank computes the same update from the one all-gather of fitness. */
+int sgmm_ga_set_es(sgmm_ga* ga, float lr, void* stream);
+/* synchronising read-back of the last generation of run `run`: utilities float[lambda] (index order), the gradient
+ * float[G], and the adversary's utilities float[lambda] and gradient float[1250] (zeros without use_arl); any pointer may
+ * be NULL.  SGMM_ERR_INVALID without sgmm_ga_set_es.  Before the first generation every array reads 0. */
+int sgmm_ga_run_es_host(sgmm_ga* ga, int32_t run, float* utilities, float* grad, float* adv_utilities, float* adv_grad,
+                        void* stream);
+int sgmm_ga_es_host(sgmm_ga* ga, float* utilities, float* grad, float* adv_utilities, float* adv_grad, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Upstream of the rollout: the per-day window loop of load_signals_bundle
  * (pipeline/agent_trainer.py:47-73).  Inputs are one day's event frame columns (loader2.event_df:
  * askprice1, bidprice1, p_buy_max, p_sell_min; n_events rows, NaN allowed in the last two) and
