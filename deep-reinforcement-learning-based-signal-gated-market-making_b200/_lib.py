@@ -13,6 +13,8 @@ LIB_PATH = os.path.join(HERE, "libsgmm_b200.so")
 
 OK, ERR_INVALID, ERR_CUDA, ERR_NOMEM, ERR_UNSUPPORTED = 0, -1, -2, -3, -4
 MAX_PARENTS = 1024          # SGMM_MAX_PARENTS
+# training objectives (SGMM_OBJECTIVE_*): the reference's total reward, or a StrategyAnalytics column of the episode
+OBJECTIVES = {"reward": 0, "pnl": 1, "pnl_map": 2, "sharpe": 3}
 
 
 class SgmmLibraryError(RuntimeError):
@@ -97,6 +99,8 @@ SIGNATURES = {
     "sgmm_bundle_destroy": (C.c_int, [C.c_void_p]),
     "sgmm_rollout_population": (C.c_int, [C.c_void_p, C.POINTER(Population), C.POINTER(Population),
                                           C.POINTER(RolloutParams), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sgmm_rollout_objective": (C.c_int, [C.c_void_p, C.POINTER(Population), C.POINTER(Population),
+                                         C.POINTER(RolloutParams), C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_rollout_population_host": (C.c_int, [C.c_void_p, C.POINTER(Population), C.POINTER(Population),
                                                C.POINTER(RolloutParams), C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_rollout_population_host_async": (C.c_int, [C.c_void_p, C.POINTER(Population), C.POINTER(Population),
@@ -142,6 +146,7 @@ SIGNATURES = {
     "sgmm_ga_set_es": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p]),
     "sgmm_ga_run_es_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_ga_es_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sgmm_ga_set_objective": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
     "sgmm_bundle_windows": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sgmm_bundle_windows_host": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,

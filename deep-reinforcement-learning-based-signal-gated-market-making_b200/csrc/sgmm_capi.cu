@@ -60,9 +60,16 @@ static int fill_pop(const sgmm_population* p, const char* name, PopArgs& out)
 static int tc32_mode_of(int precision) { return precision == SGMM_PRECISION_TF32 ? 1 : (precision == SGMM_PRECISION_F16 ? 2 : 0); }
 
 int launch_population(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int hidden, int precision, double phi, double fee,
-                      int units_per_lane, int warps_per_cta, double* fitness, int32_t* trades, cudaStream_t st)
+                      int units_per_lane, int warps_per_cta, double* fitness, int32_t* trades, cudaStream_t st, int objective)
 {
     if (precision == SGMM_PRECISION_EXACT && hidden == 32) precision = SGMM_PRECISION_F32;     // EXACT at H = 32 is the F32 route
+    if (objective != SGMM_OBJECTIVE_REWARD) {                       // StrategyAnalytics objectives: the policy-table walk
+        if (hidden == 32 && precision == SGMM_PRECISION_F32) return launch_rollout_small(b, mm, adv, phi, fee, fitness, trades, st, objective);
+        if (hidden == 256 && precision == SGMM_PRECISION_EXACT) return launch_exact256(b, mm, adv, phi, fee, fitness, trades, st, objective);
+        set_error("objective %d: training objectives run in SGMM-F32 order only (precision SGMM_PRECISION_F32 / SGMM_PRECISION_EXACT); "
+                  "the tensor-core paths compute the reward", objective);
+        return SGMM_ERR_UNSUPPORTED;
+    }
     if (hidden == 256 && precision == SGMM_PRECISION_EXACT)         // bit-exact H = 256: policy tables + walks, in batches
         return launch_exact256(b, mm, adv, phi, fee, fitness, trades, st);
     if (hidden == 256 && adv && precision == SGMM_PRECISION_BF16)   // spec256 q tables + walk_account_kernel<Walk20>, in batches
@@ -239,6 +246,20 @@ int sgmm_rollout_population(const sgmm_bundle* bundle, const sgmm_population* mm
     DeviceGuard guard(bundle->device);
     return launch_population(bundle, pm, adv ? &pa : nullptr, mm->hidden, params->precision, params->phi, params->fee_rate,
                              params->units_per_lane, params->warps_per_cta, fitness, trades, (cudaStream_t)stream);
+}
+
+int sgmm_rollout_objective(const sgmm_bundle* bundle, const sgmm_population* mm, const sgmm_population* adv,
+                           const sgmm_rollout_params* params, int32_t objective, double* fitness, int32_t* trades, void* stream)
+{
+    if (objective < SGMM_OBJECTIVE_REWARD || objective > SGMM_OBJECTIVE_SHARPE) { set_error("unknown objective %d", (int)objective); return SGMM_ERR_INVALID; }
+    if (objective == SGMM_OBJECTIVE_REWARD) return sgmm_rollout_population(bundle, mm, adv, params, fitness, trades, stream);
+    if (int rc = check_rollout_args(bundle, mm, adv, params, fitness, trades)) return rc;
+    PopArgs pm, pa;
+    if (int rc = fill_pop(mm, "mm", pm)) return rc;
+    if (adv) if (int rc = fill_pop(adv, "adv", pa)) return rc;
+    DeviceGuard guard(bundle->device);
+    return launch_population(bundle, pm, adv ? &pa : nullptr, mm->hidden, params->precision, params->phi, params->fee_rate,
+                             params->units_per_lane, params->warps_per_cta, fitness, trades, (cudaStream_t)stream, objective);
 }
 
 int sgmm_rollout_tc_audit(const sgmm_bundle* bundle, const sgmm_population* mm, const sgmm_population* adv,

@@ -268,7 +268,7 @@ bool needs_stage(const PopArgs& mm) { return mm.genomes == nullptr || (reinterpr
 // genomes,) policy table, walk (table_walk_batches).  The table ([n][T] x 48 B) and the staged genomes ([n] x 269 KB; seeded
 // children, or explicit rows not 8-byte aligned) live in the bundle's code buffer.
 int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
-                    cudaStream_t st)
+                    cudaStream_t st, int objective)
 {
     using namespace x256;
     const bool stage = b->T > 0 && needs_stage(mm);
@@ -280,7 +280,7 @@ int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv,
             rows = reinterpret_cast<float*>(s.extra);
         }
         return launch_table(b, rows, pm.count, adv ? 1 : 0, s.code, s.next, st);
-    });
+    }, objective);
 }
 
 // raw policy outputs (before x5) of ONE explicit genome for every (bar, inventory): out = float2[T][5].  `stage_buf` holds

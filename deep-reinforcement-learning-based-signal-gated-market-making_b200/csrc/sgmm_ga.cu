@@ -507,6 +507,8 @@ struct sgmm_ga {
     float* es_m = nullptr; float* es_adv_m = nullptr;                       // Adam moments, as the gradients
     float* es_v = nullptr; float* es_adv_v = nullptr;
     float* es_pow = nullptr;                                                // [runs][2]: b1^t, b2^t
+    // training objective (sgmm_ga_set_objective): what the population and validation rollouts write as fitness
+    int32_t objective = SGMM_OBJECTIVE_REWARD;
     bool started = false;                                                   // a generation phase has been enqueued
 };
 
@@ -692,7 +694,8 @@ int sgmm_ga_evaluate(sgmm_ga* ga, const sgmm_bundle* train, void* stream)
         const SweepPop mm{ga->mm_master, ga->st, c.pop_size, 0, (int64_t)ga->runs * c.pop_size, 0};
         SweepPop adv = mm;
         adv.master = ga->adv_master; adv.adv = 1;
-        return launch_sweep_population(train, mm, c.use_arl ? &adv : nullptr, ga->my_fit(), ga->my_trd(), (cudaStream_t)stream);
+        return launch_sweep_population(train, mm, c.use_arl ? &adv : nullptr, ga->my_fit(), ga->my_trd(), (cudaStream_t)stream,
+                                       ga->objective);
     }
     PopArgs mm{};
     mm.genomes = nullptr; mm.master = ga->mm_master; mm.sigma = c.sigma; mm.sigma_dev = &ga->st->sigma;
@@ -701,7 +704,7 @@ int sgmm_ga_evaluate(sgmm_ga* ga, const sgmm_bundle* train, void* stream)
     PopArgs adv = mm;
     adv.master = ga->adv_master; adv.sigma_dev = &ga->st->adv_sigma; adv.seed = c.seed ^ ADV_SEED_FLIP;
     return launch_population(train, mm, c.use_arl ? &adv : nullptr, c.hidden, c.precision, c.phi, c.fee_rate, 0, 0,
-                             ga->my_fit(), ga->my_trd(), (cudaStream_t)stream);
+                             ga->my_fit(), ga->my_trd(), (cudaStream_t)stream, ga->objective);
 }
 
 int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
@@ -743,7 +746,7 @@ int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
         if (int rc = check_cuda(cudaGetLastError(), "ga_recombine_kernel launch")) return rc;
     }
     if (ga->sweep) {                                                // the new masters (best children, or recombined): [runs] rows
-        if (int rc = launch_sweep_validation(val, ga->mm_master, ga->st, ga->runs, ga->val_fit, ga->val_trd, st)) return rc;
+        if (int rc = launch_sweep_validation(val, ga->mm_master, ga->st, ga->runs, ga->val_fit, ga->val_trd, st, ga->objective)) return rc;
     } else {
         PopArgs one{};
         one.genomes = ga->mm_master; one.master = nullptr; one.count = 1;      // the new master (best child, or recombined)
@@ -751,7 +754,8 @@ int sgmm_ga_select(sgmm_ga* ga, const sgmm_bundle* val, void* stream)
         // adversary off, so launch_rollout takes the small-population path of sgmm_one.cu (policy for every (bar, inventory)
         // in parallel, automaton scan, reference-order sum; bit-identical to the sequential kernel)
         const int val_precision = c.hidden == 32 ? SGMM_PRECISION_F32 : c.precision;
-        if (int rc = launch_population(val, one, nullptr, c.hidden, val_precision, c.phi, c.fee_rate, 0, 0, ga->val_fit, ga->val_trd, st)) return rc;
+        if (int rc = launch_population(val, one, nullptr, c.hidden, val_precision, c.phi, c.fee_rate, 0, 0, ga->val_fit, ga->val_trd, st,
+                                       ga->objective)) return rc;
     }
     ga_update_kernel<<<(unsigned)ga->runs, 256, 0, st>>>(ga->st, ga->val_fit, ga->val_trd, ga->mm_master, ga->best_master, ga->G,
                                                          c.use_arl, c.max_generations, ga->h_train_f, ga->h_val_f,
@@ -950,6 +954,26 @@ int sgmm_ga_set_es(sgmm_ga* ga, float lr, void* stream)
     if (!rc) rc = check_cuda(cudaStreamSynchronize(st), "ga_set_es");
     if (rc) { es_free(ga); return rc; }                             // back to the (1,lambda) GA
     ga->es_lr = lr; ga->es_nseg = (int32_t)S;
+    return SGMM_OK;
+}
+
+int sgmm_ga_set_objective(sgmm_ga* ga, int32_t objective, void* stream)
+{
+    if (!ga) { set_error("ga is NULL"); return SGMM_ERR_INVALID; }
+    if (ga->started) {
+        set_error("sgmm_ga_set_objective: a generation of this GA has already been enqueued; set the objective right after create");
+        return SGMM_ERR_INVALID;
+    }
+    if (objective < SGMM_OBJECTIVE_REWARD || objective > SGMM_OBJECTIVE_SHARPE) { set_error("unknown objective %d", (int)objective); return SGMM_ERR_INVALID; }
+    const int p = ga->cfg.precision;
+    if (objective != SGMM_OBJECTIVE_REWARD && p != SGMM_PRECISION_F32 && p != SGMM_PRECISION_EXACT) {
+        set_error("objective %d: training objectives run in SGMM-F32 order only; this GA has the tensor-core precision %d "
+                  "(create it with SGMM_PRECISION_EXACT)", (int)objective, p);
+        return SGMM_ERR_UNSUPPORTED;
+    }
+    DeviceGuard guard(ga->device);
+    if (int rc = check_cuda(cudaStreamSynchronize((cudaStream_t)stream), "ga_set_objective")) return rc;
+    ga->objective = objective;
     return SGMM_OK;
 }
 

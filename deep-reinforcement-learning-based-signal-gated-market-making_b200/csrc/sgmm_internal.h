@@ -161,8 +161,9 @@ int launch_rollout(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, 
 // small populations, fast (sgmm_one.cu): policy table for every (bar, inventory) + automaton scan + reference-order sum
 constexpr int64_t SMALL_POP_MAX = 400;      // measured break-even against the sequential kernel: ~420 individuals (profiles/r2_small_population_path.log)
 constexpr int64_t SMALL_POP_MAX_ADV = 148;  // with the adversary (one 512-thread CTA per individual and SM)
+// objective: SGMM_OBJECTIVE_* (sgmm.h); a non-REWARD objective takes this route at every population size
 int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
-                         cudaStream_t st);
+                         cudaStream_t st, int objective = SGMM_OBJECTIVE_REWARD);
 // the policy table of the small-population path for mm.count individuals (sgmm_one.cu), in the format of `mode`: 0 step code
 // + next inventory, 1 q = raw*5 per (bar, inventory) (adversary walk), 2 raw outputs per (bar, inventory) (population trace,
 // PopArgs only).  Pop: PopArgs, or SweepPop (the children of a GA sweep).
@@ -170,10 +171,11 @@ template <class Pop>
 int launch_policy_table(const sgmm_bundle* b, const Pop& mm, int mode, float2* code, uint8_t* next, cudaStream_t st);
 // the walk + fp64 half of the policy-table path over tables code [P][T][5] / next [P][T][8] (sgmm_one.cu).  CTA i walks
 // individual i of `pop`: with `adv` pop holds the adversaries (the 20-state walk over q tables; next unused); a SweepPop
-// gives every CTA its run's phi and fee, a PopArgs takes phi / fee (and is not read without the adversary).
+// gives every CTA its run's phi and fee, a PopArgs takes phi / fee (and is not read without the adversary).  objective:
+// SGMM_OBJECTIVE_* (sgmm.h); SHARPE needs obj_scratch [P][T] doubles, the others take nullptr.
 template <class Pop>
 int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const Pop& pop, bool adv, double phi,
-                double fee, double* fitness, int32_t* trades, cudaStream_t st);
+                double fee, double* fitness, int32_t* trades, int objective, double* obj_scratch, cudaStream_t st);
 // the market maker's offsets before the adversary's displacement along the Walk20 walk of q tables [P][T][5] (audit, sgmm_one.cu)
 int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, const PopArgs& adv, int32_t* act_trace, cudaStream_t st);
 
@@ -232,34 +234,37 @@ int for_each_batch(const Pop& mm, const Pop* adv, int64_t nb, int64_t G, Fn fn)
 }
 // The scratch of one table-and-walk batch of n individuals: the policy table code [n][T][5], the next-inventory bytes
 // [n][T][8] of the 5-state walk (nullptr when the table kind has none), then `extra` words per individual for the table
-// callback (staged genomes).
+// callback (staged genomes), then the walk's objective scratch [n][T] (SGMM_OBJECTIVE_SHARPE only, else nullptr).
 struct BatchScratch {
     float2* code;
     uint8_t* next;
     uint64_t* extra;
+    double* obj;
 };
 // Episodes of mm.count individuals of genome length G as batches of policy table + walk in the bundle's code buffer
 // (ScratchLease::reserve_in_batches).  table(pm, pa, b0, s) enqueues into s the table of individuals b0 .. b0+n-1, pm / pa being
 // those individuals of mm / adv (pa nullptr without the adversary); the walk then writes their fitness / trades: over the
 // adversaries pa, or else with individuals b0 .. b0+n-1 of `walk` as its CTAs' population -- mm itself, or the runs of a
-// GA sweep whose phi and fee the CTAs take (launch_walk).
+// GA sweep whose phi and fee the CTAs take (launch_walk).  objective: what the walk writes as fitness (SGMM_OBJECTIVE_*);
+// SHARPE adds T words per individual to the batch's scratch.
 template <class Pop, class WalkPop, class Table>
 int table_walk_batches(const sgmm_bundle* b, const Pop& mm, const Pop* adv, const WalkPop& walk, int64_t G, bool with_next,
-                       int64_t extra, double phi, double fee, double* fitness, int32_t* trades, cudaStream_t st, Table table)
+                       int64_t extra, double phi, double fee, double* fitness, int32_t* trades, cudaStream_t st, Table table,
+                       int objective = SGMM_OBJECTIVE_REWARD)
 {
     if (mm.count == 0) return SGMM_OK;
-    const int64_t T = b->T, table_words = (with_next ? 6 : 5) * T;
+    const int64_t T = b->T, table_words = (with_next ? 6 : 5) * T, obj_words = objective == SGMM_OBJECTIVE_SHARPE ? T : 0;
     ScratchLease lease(b, st);
     int64_t nb = 0;
     uint64_t* buf = nullptr;
-    if (int rc = lease.reserve_in_batches(mm.count, table_words + extra, &nb, &buf)) return rc;
+    if (int rc = lease.reserve_in_batches(mm.count, table_words + extra + obj_words, &nb, &buf)) return rc;
     const BatchScratch s{reinterpret_cast<float2*>(buf), with_next ? reinterpret_cast<uint8_t*>(buf + nb * T * 5) : nullptr,
-                         buf + nb * table_words};
+                         buf + nb * table_words, obj_words ? reinterpret_cast<double*>(buf + nb * (table_words + extra)) : nullptr};
     const int rc = for_each_batch(mm, adv, nb, G, [&](const Pop& pm, const Pop* pa, int64_t b0) {
         if (int rc = table(pm, pa, b0, s)) return rc;
-        if (pa) return launch_walk(b, pm.count, s.code, nullptr, *pa, true, phi, fee, fitness + b0, trades + b0, st);
+        if (pa) return launch_walk(b, pm.count, s.code, nullptr, *pa, true, phi, fee, fitness + b0, trades + b0, objective, s.obj, st);
         return launch_walk(b, pm.count, s.code, s.next, batch_of(walk, b0, pm.count, G), false, phi, fee, fitness + b0,
-                           trades + b0, st);
+                           trades + b0, objective, s.obj, st);
     });
     if (rc) return rc;
     return lease.done();
@@ -267,13 +272,14 @@ int table_walk_batches(const sgmm_bundle* b, const Pop& mm, const Pop* adv, cons
 // GA sweeps at H = 32, exact (sgmm_one.cu).  launch_sweep_population: the mm.count seeded children of mm (and adv) on the
 // policy-table path at every size, in batches (table_walk_batches); every walk CTA takes its run's phi and fee.
 // launch_sweep_validation: K explicit masters [K][1250] (adversary off), walk CTA r with run r's phi and fee.
+// objective: SGMM_OBJECTIVE_* of both (sgmm.h).
 int launch_sweep_population(const sgmm_bundle* b, const SweepPop& mm, const SweepPop* adv, double* fitness, int32_t* trades,
-                            cudaStream_t st);
+                            cudaStream_t st, int objective);
 int launch_sweep_validation(const sgmm_bundle* b, const float* masters, const GaDev* runs, int64_t K, double* fitness,
-                            int32_t* trades, cudaStream_t st);
+                            int32_t* trades, cudaStream_t st, int objective);
 // bit-exact H = 256 (sgmm_exact256.cu): batches of policy table + walk; and the raw-output table of one genome for the trace
 int launch_exact256(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
-                    cudaStream_t st);
+                    cudaStream_t st, int objective = SGMM_OBJECTIVE_REWARD);
 namespace x256 {
 // the exact H = 256 policy table of `count` 8-byte aligned genome rows (modes as launch_policy_table), and the staging of
 // seeded children or unaligned rows into such rows (sgmm_exact256.cu)
@@ -296,9 +302,12 @@ int launch_spec256_adv(const sgmm_bundle* b, const PopArgs& mm, const PopArgs& a
 int launch_tc32(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, int group, double* fitness, int32_t* trades,
                 float* raw_table, int32_t* act_trace, cudaStream_t st, int mode = 0);   // mode: 0 bf16, 1 tf32, 2 f16
 // the rollout of a population on the kernel that serves (hidden, precision, adversary) (sgmm_capi.cu); units_per_lane is
-// the tensor-core group size at H = 32 in BF16 / TF32 / F16.  The arguments are checked by the caller.
+// the tensor-core group size at H = 32 in BF16 / TF32 / F16.  The arguments are checked by the caller.  A non-REWARD
+// objective (SGMM_OBJECTIVE_*) takes the policy-table route (H = 32 F32 / EXACT, H = 256 EXACT); with a tensor-core
+// precision it is SGMM_ERR_UNSUPPORTED.
 int launch_population(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, int hidden, int precision, double phi, double fee,
-                      int units_per_lane, int warps_per_cta, double* fitness, int32_t* trades, cudaStream_t st);
+                      int units_per_lane, int warps_per_cta, double* fitness, int32_t* trades, cudaStream_t st,
+                      int objective = SGMM_OBJECTIVE_REWARD);
 int launch_tc32_prologue(sgmm_bundle* b, cudaStream_t st);
 int launch_account(const sgmm_bundle* b, const uint64_t* codes, int64_t count, double phi, double fee, double* fitness,
                    int32_t* trades, cudaStream_t st, bool float_offsets = false);

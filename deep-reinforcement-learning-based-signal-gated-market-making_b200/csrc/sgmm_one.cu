@@ -26,6 +26,7 @@
 #include "sgmm_adversary.cuh"
 #include "sgmm_step_core.h"
 #include "sgmm_walk.cuh"
+#include "sgmm_np_sum.cuh"
 
 namespace sgmm {
 
@@ -183,8 +184,9 @@ struct Walk5 {
     struct Step { float2 q; bool fb, fs; uint32_t next; };
     const float2* code;                    // this individual's [T][5] q of each side that filled, NaN marker otherwise
     const uint8_t* next;                   // [T][8] next inventory index
-    template <class Pop>
-    __device__ Walk5(const BarSig*, const float2* code_all, const uint8_t* next_all, const Pop&, int64_t ind, int64_t T)
+    template <class Pop, int OBJ>
+    __device__ Walk5(const BarSig*, const float2* code_all, const uint8_t* next_all, const Pop&, int64_t ind, int64_t T,
+                     std::integral_constant<int, OBJ>)
         : code(code_all + ind * T * 5), next(next_all + ind * T * 8) {}
     __device__ static Map identity() { return MAP_ID; }
     __device__ static Map then(Map f, Map g) { return map_then(f, g); }
@@ -212,8 +214,11 @@ struct Walk20 {
     const BarSig* sig;
     const float2* code;                    // this individual's [T][5] raw q = raw*5
     uint32_t at0, at1, at2;                // displacement table (sgmm_adversary.cuh)
-    template <class Pop>
-    __device__ Walk20(const BarSig* sig_, const float2* code_all, const uint8_t*, const Pop& adv_in, int64_t ind, int64_t T)
+    // OBJ (the walk's objective) only gives each kernel its own s_adv: a table that two kernels share moves out of the
+    // kernel to module scope, which shifts the shared-memory layout (and the code) of the reward kernel
+    template <class Pop, int OBJ>
+    __device__ Walk20(const BarSig* sig_, const float2* code_all, const uint8_t*, const Pop& adv_in, int64_t ind, int64_t T,
+                      std::integral_constant<int, OBJ>)
         : sig(sig_), code(code_all + ind * T * 5)
     {
         __shared__ uint32_t s_adv[3];
@@ -248,15 +253,116 @@ __device__ __forceinline__ double cta_fee(const SweepPop& p, double) { return ct
 template <class Pop> constexpr int walk_ctas_per_sm() { return 3; }
 template <> constexpr int walk_ctas_per_sm<SweepPop>() { return 2; }
 
+// Phase 3 of walk_account_kernel for a StrategyAnalytics objective (sgmm.h, SGMM_OBJECTIVE_*), chunk by chunk of OBJ_CHUNK
+// bars: every thread steps its own bars and stages the two cash terms (my_bid + fee, my_ask - fee) in s_buf (both halves
+// of the reward kernel's s_rew), the fill bits and the inventory after the bar; one thread runs the cash chain in bar
+// order (buy leg, then sell leg, as env_step); then wealth = cash + inventory * mid_next in parallel, the expression of
+// sgmm_trace_pop.cu.  Total PnL needs the first and last wealth, MAP the sum of |inventory| (an integer: any order), the
+// Sharpe the wealth differences of consecutive trade rows, which one thread appends in bar order to `scratch` before the
+// two pairwise passes of analytics_kernel (trade_sharpe).  Every thread of the CTA calls it.
+constexpr int OBJ_CHUNK = SUM_CHUNK / 2;
+
+template <class A, int WALK_THREADS, int OBJ>
+__device__ __forceinline__ void walk_objective(const A& w, uint32_t st, int64_t t_lo, int64_t t_hi, int64_t T,
+                                               const BarPx* __restrict__ px, double tick, double fee, double* s_buf,
+                                               int* s_trades, double* __restrict__ obj_scratch, double* __restrict__ fitness,
+                                               int32_t* __restrict__ trades)
+{
+    __shared__ uint8_t s_out[OBJ_CHUNK];                    // fill_buy | fill_sell << 1 | inventory index after the bar << 2
+    __shared__ unsigned long long s_abs;
+    __shared__ double s_w0, s_wl;
+    double* s_cb = s_buf;                                   // cash term of the buy leg, then the cash after the bar
+    double* s_cs = s_buf + OBJ_CHUNK;                       // cash term of the sell leg, then (SHARPE) the wealth
+    const int tid = threadIdx.x;
+    if (tid == 0) { s_abs = 0ull; s_w0 = 0.0; s_wl = 0.0; }
+    double* scratch = OBJ == SGMM_OBJECTIVE_SHARPE ? obj_scratch + (int64_t)blockIdx.x * T : nullptr;
+    int ntr = 0, abs_inv = 0;
+    double cash = 0.0, prev = 0.0;                          // thread 0: the cash chain, the last trade row's wealth
+    int64_t m = 0;                                          // thread 0: wealth differences written
+    bool seen = false;                                      // thread 0: a trade row has been met
+    for (int64_t c0 = 0; c0 < T; c0 += OBJ_CHUNK) {
+        const int64_t c1 = c0 + OBJ_CHUNK < T ? c0 + OBJ_CHUNK : T;
+        const int n = (int)(c1 - c0);
+        const int64_t a = t_lo > c0 ? t_lo : c0, b = t_hi < c1 ? t_hi : c1;
+        for (int64_t t = a; t < b; ++t) {
+            const typename A::Step r = w.step(st, t);
+            const int iv = A::inventory_index(r.next);
+            ntr += (r.fb || r.fs) ? 1 : 0;                                         // drl_engine.py:60-61
+            abs_inv += iv > 2 ? iv - 2 : 2 - iv;                                   // mm_analyzer.py:27
+            double cb = 0.0, cs = 0.0;
+            if (r.fb || r.fs) {
+                const BarPx p = px[t];
+                const int2 k = A::offsets(r);
+                const double my_ask = quote_ask(p.ask, k.x, tick), my_bid = quote_bid(p.bid, k.y, tick);     // market_env.py:30-31
+                cb = add_rn(my_bid, mul_rn(my_bid, fee));                                                    // :47
+                cs = sub_rn(my_ask, mul_rn(my_ask, fee));                                                    // :53
+            }
+            s_cb[t - c0] = cb; s_cs[t - c0] = cs;
+            s_out[t - c0] = (uint8_t)((r.fb ? 1 : 0) | (r.fs ? 2 : 0) | (iv << 2));
+            st = r.next;
+        }
+        __syncthreads();
+        if (tid == 0) {
+            for (int i = 0; i < n; ++i) {
+                const int f = s_out[i];
+                if (f & 1) cash = sub_rn(cash, s_cb[i]);
+                if (f & 2) cash = add_rn(cash, s_cs[i]);
+                s_cb[i] = cash;
+            }
+        }
+        __syncthreads();
+        for (int i = tid; i < n; i += WALK_THREADS) {
+            const int64_t t = c0 + i;
+            if (OBJ == SGMM_OBJECTIVE_SHARPE || t == 0 || t == T - 1) {
+                const double wl = add_rn(s_cb[i], mul_rn((double)((s_out[i] >> 2) - 2), px[t].mid_next));   // Env/recorder.py:46
+                if (t == 0) s_w0 = wl;
+                if (t == T - 1) s_wl = wl;
+                if (OBJ == SGMM_OBJECTIVE_SHARPE) s_cs[i] = wl;
+            }
+        }
+        if constexpr (OBJ == SGMM_OBJECTIVE_SHARPE) {
+            __syncthreads();
+            if (tid == 0) {
+                for (int i = 0; i < n; ++i) {
+                    if (s_out[i] & 3) {                                            // mm_analyzer.py:10,39
+                        const double wl = s_cs[i];
+                        if (seen) scratch[m++] = sub_rn(wl, prev);
+                        prev = wl; seen = true;
+                    }
+                }
+            }
+        }
+        __syncthreads();
+    }
+    if (ntr) atomicAdd(s_trades, ntr);
+    if (abs_inv) atomicAdd(&s_abs, (unsigned long long)abs_inv);
+    __syncthreads();
+    if (tid == 0) {
+        const int nt = *s_trades;
+        const double total = sub_rn(s_wl, s_w0);                                   // mm_analyzer.py:15
+        double v;
+        if constexpr (OBJ == SGMM_OBJECTIVE_PNL) v = total;
+        else if constexpr (OBJ == SGMM_OBJECTIVE_PNL_MAP) {
+            const double map = T > 0 ? __ddiv_rn((double)s_abs, (double)T) : 0.0;    // :27
+            v = map == 0.0 ? 0.0 : __ddiv_rn(total, map);
+        } else v = trade_sharpe(scratch, m, nt);
+        fitness[blockIdx.x] = objective_fitness(v, nt); trades[blockIdx.x] = nt;
+    }
+}
+
 // One CTA per individual.  WALK_THREADS = 1024 (one individual per SM: shortest latency, populations up to the SM count) or
 // 512 (three per SM without the adversary: the serial reward sum of one individual hides behind the others).
 // Pop: PopArgs (phi_arg / fee_arg apply to every CTA), or SweepPop (a GA sweep: CTA i walks individual adv.first + i of the
 // sweep with its run's phi and fee; with the adversary, adv gives the individual's seeded adversary).
-template <class A, int WALK_THREADS, class Pop>
-__global__ void __launch_bounds__(WALK_THREADS, (WALK_THREADS == 1024 || A::STATES == 20) ? 1 : walk_ctas_per_sm<Pop>())
+// OBJ: the training objective (SGMM_OBJECTIVE_*).  REWARD sums the reference's rewards; the others run the cash chain
+// instead and reduce wealth to the StrategyAnalytics column (phase 3 below).  SHARPE writes the wealth differences of
+// consecutive trade rows of CTA i to obj_scratch[i][0 .. trades-1) (T doubles per CTA).  An objective CTA keeps the cash
+// chain, the first and last wealth and the Sharpe state in registers: two CTAs per SM at 512 threads, 64 registers.
+template <class A, int WALK_THREADS, class Pop, int OBJ = SGMM_OBJECTIVE_REWARD>
+__global__ void __launch_bounds__(WALK_THREADS, (WALK_THREADS == 1024 || A::STATES == 20) ? 1 : (OBJ != SGMM_OBJECTIVE_REWARD ? 2 : walk_ctas_per_sm<Pop>()))
 walk_account_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px, int64_t T, const float2* __restrict__ code_all,
                     const uint8_t* __restrict__ next_all, const Pop adv, double tick, double phi_arg, double fee_arg,
-                    double* __restrict__ fitness, int32_t* __restrict__ trades)
+                    double* __restrict__ fitness, int32_t* __restrict__ trades, double* __restrict__ obj_scratch)
 {
     using Map = typename A::Map;
     __shared__ Map s_warp[32];                              // (WALK_THREADS / 32 entries used)
@@ -264,7 +370,7 @@ walk_account_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px
     __shared__ double s_rew[SUM_CHUNK];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) s_trades = 0;
-    const A w(sig, code_all, next_all, adv, blockIdx.x, T);
+    const A w(sig, code_all, next_all, adv, blockIdx.x, T, std::integral_constant<int, OBJ>{});
     // ---- 1. every thread composes the maps of its contiguous segment of bars ----
     const int64_t L = (T + WALK_THREADS - 1) / WALK_THREADS;
     const int64_t t_lo = (int64_t)tid * L < T ? (int64_t)tid * L : T, t_hi = t_lo + L < T ? t_lo + L : T;
@@ -293,6 +399,11 @@ walk_account_kernel(const BarSig* __restrict__ sig, const BarPx* __restrict__ px
     if (lane == 0) before = A::identity();
     if (warp > 0) before = A::then(s_warp[warp - 1], before);
     uint32_t st = A::at(before, 2u);                        // flat, no previous fills: state 2 (market_env.py:17, drl_engine.py:29)
+    if constexpr (OBJ != SGMM_OBJECTIVE_REWARD) {
+        walk_objective<A, WALK_THREADS, OBJ>(w, st, t_lo, t_hi, T, px, tick, cta_fee(adv, fee_arg), s_rew, &s_trades,
+                                             obj_scratch, fitness, trades);
+        return;
+    }
     // ---- 3. the fp64 half for the visited states, chunk by chunk; one thread sums each chunk in bar order ----
     const PenaltyTable pen = penalty_table(cta_phi(adv, phi_arg));
     int ntr = 0;
@@ -398,52 +509,68 @@ int launch_policy_table(const sgmm_bundle* b, const Pop& mm, int mode, float2* c
     return check_cuda(cudaGetLastError(), "policy_table_kernel launch");
 }
 
+namespace one {
+template <int OBJ, class Pop>
+static void launch_walk_as(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const Pop& pop, bool adv,
+                           double phi, double fee, double* fitness, int32_t* trades, double* obj_scratch, cudaStream_t st)
+{
+    const int64_t T = b->T;
+    if (adv) walk_account_kernel<Walk20, 512, Pop, OBJ><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, nullptr, pop, b->tick, phi, fee, fitness, trades, obj_scratch);
+    else if (P <= sm_count(b->device)) walk_account_kernel<Walk5, 1024, Pop, OBJ><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, T, code, next, pop, b->tick, phi, fee, fitness, trades, obj_scratch);
+    else walk_account_kernel<Walk5, 512, Pop, OBJ><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, next, pop, b->tick, phi, fee, fitness, trades, obj_scratch);
+}
+}  // namespace one
+
 template <class Pop>
 int launch_walk(const sgmm_bundle* b, int64_t P, const float2* code, const uint8_t* next, const Pop& pop, bool adv, double phi,
-                double fee, double* fitness, int32_t* trades, cudaStream_t st)
+                double fee, double* fitness, int32_t* trades, int objective, double* obj_scratch, cudaStream_t st)
 {
     using namespace one;
-    const int64_t T = b->T;
-    if (adv) walk_account_kernel<Walk20, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, nullptr, pop, b->tick, phi, fee, fitness, trades);
-    else if (P <= sm_count(b->device)) walk_account_kernel<Walk5, 1024><<<(unsigned)P, 1024, 0, st>>>(b->sig, b->px, T, code, next, pop, b->tick, phi, fee, fitness, trades);
-    else walk_account_kernel<Walk5, 512><<<(unsigned)P, 512, 0, st>>>(b->sig, b->px, T, code, next, pop, b->tick, phi, fee, fitness, trades);
+    switch (objective) {
+        case SGMM_OBJECTIVE_PNL: launch_walk_as<SGMM_OBJECTIVE_PNL>(b, P, code, next, pop, adv, phi, fee, fitness, trades, obj_scratch, st); break;
+        case SGMM_OBJECTIVE_PNL_MAP: launch_walk_as<SGMM_OBJECTIVE_PNL_MAP>(b, P, code, next, pop, adv, phi, fee, fitness, trades, obj_scratch, st); break;
+        case SGMM_OBJECTIVE_SHARPE: launch_walk_as<SGMM_OBJECTIVE_SHARPE>(b, P, code, next, pop, adv, phi, fee, fitness, trades, obj_scratch, st); break;
+        default: launch_walk_as<SGMM_OBJECTIVE_REWARD>(b, P, code, next, pop, adv, phi, fee, fitness, trades, obj_scratch, st); break;
+    }
     return check_cuda(cudaGetLastError(), "walk_account_kernel launch");
 }
 
 template int launch_policy_table<PopArgs>(const sgmm_bundle*, const PopArgs&, int, float2*, uint8_t*, cudaStream_t);
 template int launch_policy_table<SweepPop>(const sgmm_bundle*, const SweepPop&, int, float2*, uint8_t*, cudaStream_t);
 template int launch_walk<PopArgs>(const sgmm_bundle*, int64_t, const float2*, const uint8_t*, const PopArgs&, bool, double, double,
-                                  double*, int32_t*, cudaStream_t);
+                                  double*, int32_t*, int, double*, cudaStream_t);
 template int launch_walk<SweepPop>(const sgmm_bundle*, int64_t, const float2*, const uint8_t*, const SweepPop&, bool, double, double,
-                                   double*, int32_t*, cudaStream_t);
+                                   double*, int32_t*, int, double*, cudaStream_t);
 
 // Episodes of a small population on `b` (H = 32, exact SGMM-F32 order, with or without the adversary) through the kernels
 // above.  The policy table ([count][T] x 48 B) lives in the bundle's code buffer, as batches of table_walk_batches: one
-// batch at the default budget.
+// batch at the default budget.  A non-REWARD objective takes this route at every population size.
 int launch_rollout_small(const sgmm_bundle* b, const PopArgs& mm, const PopArgs* adv, double phi, double fee, double* fitness, int32_t* trades,
-                         cudaStream_t st)
+                         cudaStream_t st, int objective)
 {
-    return table_walk_batches(b, mm, adv, mm, genome_len(32), true, 0, phi, fee, fitness, trades, st, one::policy_tables(b, st));
+    return table_walk_batches(b, mm, adv, mm, genome_len(32), true, 0, phi, fee, fitness, trades, st, one::policy_tables(b, st), objective);
 }
 
 // The K*lambda children of a GA sweep take the policy-table path whatever their number (a solo GA of more than
 // SMALL_POP_MAX children runs rollout_kernel_h32, which gives the same bits).  The table ([n][T] x 48 B) lives in the
 // bundle's code buffer, in batches of n individuals; a batch may start inside a run.  phi / fee are the runs'.
 int launch_sweep_population(const sgmm_bundle* b, const SweepPop& mm, const SweepPop* adv, double* fitness, int32_t* trades,
-                            cudaStream_t st)
+                            cudaStream_t st, int objective)
 {
-    return table_walk_batches(b, mm, adv, mm, genome_len(32), true, 0, 0.0, 0.0, fitness, trades, st, one::policy_tables(b, st));
+    return table_walk_batches(b, mm, adv, mm, genome_len(32), true, 0, 0.0, 0.0, fitness, trades, st, one::policy_tables(b, st),
+                              objective);
 }
 
 // The K masters of a sweep, contiguous [K][1250] rows, as one explicit population (adversary off, as the validation of a
 // solo GA); the walk's CTA r takes run r's phi and fee
 int launch_sweep_validation(const sgmm_bundle* b, const float* masters, const GaDev* runs, int64_t K, double* fitness,
-                            int32_t* trades, cudaStream_t st)
+                            int32_t* trades, cudaStream_t st, int objective)
 {
     PopArgs pm{};
     pm.genomes = masters; pm.count = K;
     const SweepPop all{nullptr, runs, 1, 0, K, 0};
-    return table_walk_batches(b, pm, (const PopArgs*)nullptr, all, genome_len(32), true, 0, 0.0, 0.0, fitness, trades, st, one::policy_tables(b, st));
+    return table_walk_batches(b, pm, (const PopArgs*)nullptr, all, genome_len(32), true, 0, 0.0, 0.0, fitness, trades, st,
+                              one::policy_tables(b, st), objective);
 }
 
 int launch_adv_offsets(const sgmm_bundle* b, int64_t P, const float2* code, const PopArgs& adv, int32_t* act_trace, cudaStream_t st)

@@ -79,6 +79,9 @@ SGMM_HD double penalty(const PenaltyTable& pen, int abs_inventory)
 
 // drl_engine.py:64-65 -- an episode without a single trade loses 50
 SGMM_HD double episode_fitness(double total, int trades) { return trades == 0 ? sub_rn(total, 50.0) : total; }
+// the fitness of a StrategyAnalytics objective value v (sgmm.h, SGMM_OBJECTIVE_*): the same -50 without trades, and a NaN
+// objective (the Sharpe of exactly two trades) is -50 too, since the GA's ranking would put it first
+SGMM_HD double objective_fitness(double v, int trades) { return trades == 0 ? sub_rn(v, 50.0) : (v != v ? -50.0 : v); }
 
 // market_env.py:22-67.  off_a/off_b already include the adversary's displacement (:25-28).  Off = int64_t or double.
 template <typename Off>

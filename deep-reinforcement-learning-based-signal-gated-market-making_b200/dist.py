@@ -81,15 +81,21 @@ def all_gather_packed(fit, trd, pop_size: int, stride: int, group=None):
 class ShardedGA:
     """One process per GPU: evaluate the local shard, ONE in-place all-gather of this rank's (fitness, trades) block
     into the library's rank-blocked gather buffer, select locally (identical on every rank).  Replaces the
-    ``Pool.starmap`` fan-out / result list of Env/drl_engine.py:104-125 across the GPUs of one box."""
+    ``Pool.starmap`` fan-out / result list of Env/drl_engine.py:104-125 across the GPUs of one box.
 
-    def __init__(self, make_ga, pop_size, group=None):
+    ``objective`` (``"reward"``, ``"pnl"``, ``"pnl_map"``, ``"sharpe"``; None = whatever ``make_ga`` set) is set on the
+    rank's GA before its first generation (``sgmm_ga_set_objective``).  Every rank must pass the same one; the objective
+    is per child, so the exchange is unchanged."""
+
+    def __init__(self, make_ga, pop_size, group=None, objective=None):
         self.group = group
         self.world = dist.get_world_size(group)
         self.rank = dist.get_rank(group)
         self.pop_size = pop_size
         self.first, self.count, self.stride = shard_bounds(pop_size, self.world, self.rank)
         self.ga = make_ga((self.first, self.count, self.stride))
+        if objective is not None:
+            self.ga.set_objective(objective)
         _, _, base, block_bytes, n_blocks, my_block = self.ga.buffers()
         assert n_blocks <= self.world and block_bytes == block_layout(self.stride)[0]
         dev = self.ga.device

@@ -57,6 +57,30 @@ def _params(phi, fee_rate, units_per_lane=0, warps_per_cta=0, hidden=32, precisi
     return _lib.RolloutParams(float(phi), float(fee_rate), prec, 0, int(units_per_lane), int(warps_per_cta))
 
 
+def _objective(objective, precision, hidden):
+    """Checks a training objective (``"reward"``, ``"pnl"``, ``"pnl_map"``, ``"sharpe"``) against the precision without
+    touching a device; returns its ``SGMM_OBJECTIVE_*`` code."""
+    if not isinstance(objective, str) or objective not in _lib.OBJECTIVES:
+        raise ValueError(f"unknown objective {objective!r}: one of {', '.join(repr(k) for k in _lib.OBJECTIVES)}")
+    code = _lib.OBJECTIVES[objective]
+    if code and _precision(precision, hidden) not in (PRECISION_F32, PRECISION_EXACT):
+        hint = " (hidden 256 defaults to the tensor-core path)" if hidden == 256 and precision is None else ""
+        raise ValueError(f"objective={objective!r} is computed in SGMM-F32 order only: pass precision='exact'{hint}; "
+                         f"the tensor-core precisions train on the reward")
+    return code
+
+
+def _launch_population(bundle, mm, advp, prm, objective, fit, trd):
+    """``sgmm_rollout_population`` for the reward, ``sgmm_rollout_objective`` for any other objective code."""
+    L = _lib.lib()
+    if objective:
+        _lib.check(L.sgmm_rollout_objective(bundle.handle, C.byref(mm), advp, C.byref(prm), objective, fit.data_ptr(),
+                                            trd.data_ptr(), _stream(bundle.device)))
+    else:
+        _lib.check(L.sgmm_rollout_population(bundle.handle, C.byref(mm), advp, C.byref(prm), fit.data_ptr(), trd.data_ptr(),
+                                             _stream(bundle.device)))
+
+
 def _as_f32_matrix(x, width):
     """Accept a list of 1-D tensors (NeuroEvolution.ask), a 2-D tensor or ndarray."""
     if isinstance(x, (list, tuple)):
@@ -94,20 +118,32 @@ def _as_adv_matrix(x):
 
 
 def rollout_population(bundle: Bundle, genomes, adv_genomes=None, *, phi, fee_rate=0.0, hidden=32,
-                       units_per_lane=0, warps_per_cta=0, precision=None):
+                       units_per_lane=0, warps_per_cta=0, precision=None, objective="reward"):
     """One episode per individual (the reference's ``pool.starmap(evaluate_individual, ...)``).
 
     ``genomes``: [P, G] float32 -- CUDA tensor (device path, returns CUDA tensors, no sync) or
     CPU tensor / ndarray / list of tensors (end-to-end path through ``sgmm_rollout_population_host``:
     H2D, kernel, D2H, returns numpy arrays).  ``adv_genomes``: optional [P, 1250] (use_arl).
+    ``objective``: what ``fitness`` measures (``sgmm_rollout_objective``): ``"reward"`` (the reference's total reward,
+    the default), or the StrategyAnalytics ``"pnl"`` (Total PnL), ``"pnl_map"`` (PnL / MAP) or ``"sharpe"`` (trade
+    Sharpe) of each episode, -50 without trades and -50 for a NaN value; exact precision only.
     Returns ``(fitness float64[P], trades int32[P])``.
     """
+    obj = _objective(objective, precision, hidden)
     G = genome_len(hidden)
     g = _as_f32_matrix(genomes, G)
     P = g.shape[0]
     a = None if adv_genomes is None else _as_adv_matrix(adv_genomes)
     if a is not None and a.shape[0] != P:
         raise ValueError("adversary population size differs from the market-maker population")
+    if obj and not g.is_cuda:                   # no host entry for the objectives: through the device and back
+        if a is not None and a.is_cuda:
+            raise ValueError("mixing CPU market-maker genomes with CUDA adversary genomes")
+        dev = f"cuda:{bundle.device}"
+        fit, trd = rollout_population(bundle, g.to(dev), None if a is None else a.to(dev), phi=phi, fee_rate=fee_rate,
+                                      hidden=hidden, units_per_lane=units_per_lane, warps_per_cta=warps_per_cta,
+                                      precision=precision, objective=objective)
+        return fit.cpu().numpy(), trd.cpu().numpy()
     L = _lib.lib()
     mm = _lib.Population(hidden, 0, P, g.data_ptr(), None, 0.0, 0.0, 0, 0, 0)
     adv = None if a is None else _lib.Population(32, 0, P, a.data_ptr(), None, 0.0, 0.0, 0, 0, 0)
@@ -118,8 +154,7 @@ def rollout_population(bundle: Bundle, genomes, adv_genomes=None, *, phi, fee_ra
             raise ValueError("genomes must live on the bundle's device")
         fit = torch.empty(P, dtype=torch.float64, device=g.device)
         trd = torch.empty(P, dtype=torch.int32, device=g.device)
-        _lib.check(L.sgmm_rollout_population(bundle.handle, C.byref(mm), advp, C.byref(prm),
-                                             fit.data_ptr(), trd.data_ptr(), _stream(bundle.device)))
+        _launch_population(bundle, mm, advp, prm, obj, fit, trd)
         return fit, trd
     if a is not None and a.is_cuda:
         raise ValueError("mixing CPU market-maker genomes with CUDA adversary genomes")
@@ -176,11 +211,12 @@ def rollout_population_async(bundle: Bundle, genomes, adv_genomes=None, *, phi, 
 
 def rollout_seeded(bundle: Bundle, master, *, count, sigma, seed, generation, first_index=0,
                    adv_master=None, adv_sigma=None, phi, fee_rate=0.0, hidden=32,
-                   units_per_lane=0, warps_per_cta=0, precision=None):
+                   units_per_lane=0, warps_per_cta=0, precision=None, objective="reward"):
     """Evaluate children ``first_index .. first_index+count-1`` of ``master`` without ever storing
     them: child i = master + sigma*N(0,1)[Philox(seed, generation, i)] is generated inside the
     kernel (device-resident ``ask``, models/model.py:65-71).  ``master`` (and ``adv_master``) are
-    CUDA float32 tensors; returns CUDA tensors."""
+    CUDA float32 tensors; returns CUDA tensors.  ``objective`` as :func:`rollout_population`."""
+    obj = _objective(objective, precision, hidden)
     G = genome_len(hidden)
     m = torch.as_tensor(master, dtype=torch.float32, device=f"cuda:{bundle.device}").contiguous()
     if m.numel() != G:
@@ -196,8 +232,7 @@ def rollout_seeded(bundle: Bundle, master, *, count, sigma, seed, generation, fi
                               0.0, int(seed) ^ ADV_SEED_FLIP, int(generation), int(first_index))
         advp = C.byref(adv)
     prm = _params(phi, fee_rate, units_per_lane, warps_per_cta, hidden, precision)
-    _lib.check(_lib.lib().sgmm_rollout_population(bundle.handle, C.byref(mm), advp, C.byref(prm),
-                                                  fit.data_ptr(), trd.data_ptr(), _stream(bundle.device)))
+    _launch_population(bundle, mm, advp, prm, obj, fit, trd)
     return fit, trd
 
 
@@ -468,6 +503,26 @@ def _es_lr(es_lr, parents, weights, pop_size):
 class _GAHandle:
     """What every ``sgmm_ga`` handle offers: the generation phases, graph capture, the per-run read-backs and close."""
 
+    objective = "reward"
+
+    def set_objective(self, objective):
+        """Train on ``objective`` (``"reward"``, ``"pnl"``, ``"pnl_map"``, ``"sharpe"``; ``sgmm_ga_set_objective``) from
+        the first generation on.  Call it before the first generation; the handle's precision must be exact for any
+        objective but the reward."""
+        _objective(objective, self.precision, 32 if self.G == genome_len(32) else 256)
+        _lib.check(_lib.lib().sgmm_ga_set_objective(self._h, _lib.OBJECTIVES[objective], _stream(self.device)))
+        self.objective = objective
+
+    def _set_objective(self, objective):
+        """After create: the objective checked by :func:`_objective`; the reward needs no call."""
+        if objective == "reward":
+            return
+        try:
+            self.set_objective(objective)
+        except Exception:
+            self.close()
+            raise
+
     def _set_es(self, lr):
         """After create: switch to the evolution strategy with Adam step size ``lr`` (from :func:`_es_lr`)."""
         self.es_lr = lr
@@ -572,13 +627,22 @@ class DeviceGA(_GAHandle):
 
     ``es_lr`` switches it to a natural-gradient evolution strategy (``sgmm_ga_set_es``): centered-rank utilities of all
     lambda children, ``g = sum_i u_i eps_i / (lambda sigma)`` and an Adam ascent step of size ``es_lr`` on the master
-    (the adversary's on -fitness).  ``es_state()`` reads the last generation's utilities and gradients."""
+    (the adversary's on -fitness).  ``es_state()`` reads the last generation's utilities and gradients.
+
+    ``objective`` is what the GA maximises (``sgmm_ga_set_objective``): ``"reward"`` (the reference's total reward, the
+    default), or the StrategyAnalytics ``"pnl"`` (Total PnL), ``"pnl_map"`` (PnL / MAP) or ``"sharpe"`` (trade Sharpe)
+    of each episode, -50 without trades and -50 for a NaN value.  The children's fitness and the validation both measure
+    it, so the history's ``train_f`` / ``val_f``, ``best_val``, keep-best-on-validation and sigma decay follow it; the
+    adversary minimises it.  It composes with ``parents`` / ``weights`` and ``es_lr``.  Exact precision only: the H = 32
+    population then takes the policy-table route at every size."""
 
     def __init__(self, mm_master, adv_master=None, *, pop_size, sigma, phi, fee_rate, use_arl, seed,
                  max_generations, patience=15, hidden=32, device=None, shard=None, precision=None, parents=1, weights=None,
-                 es_lr=None):
+                 es_lr=None, objective="reward"):
         w = _parent_weights(parents, weights, pop_size)
         lr = _es_lr(es_lr, parents, weights, pop_size)
+        _objective(objective, precision, hidden)
+        self.precision = precision
         self.device = torch.cuda.current_device() if device is None else int(device)
         first, count, stride = (0, pop_size, 0) if shard is None else shard
         cfg = _lib.GaConfig(hidden, int(bool(use_arl)), pop_size, first, count, stride, float(sigma), patience,
@@ -596,6 +660,7 @@ class DeviceGA(_GAHandle):
                                              _stream(self.device)))
         self._set_parents(parents, w)
         self._set_es(lr)
+        self._set_objective(objective)
 
     def parents(self):
         """``(mm_index, adv_index)`` int64[mu]: the last generation's parents in rank order (global child indices)."""
@@ -631,12 +696,15 @@ class DeviceGASweep(_GAHandle):
     ``DeviceGA(masters[r], adv_masters[r], precision="exact", **runs[r])``.  Hidden width 32, exact precision, one
     device.  Read-backs take the run: ``status(r)``, ``masters(r)``, ``history(r)``, ``parents(r)``.  ``parents`` /
     ``weights`` select truncation selection and ``es_lr`` the evolution strategy as for :class:`DeviceGA`, one setting
-    for every run; ``es_state(r)`` reads run r's last utilities and gradients."""
+    for every run; ``es_state(r)`` reads run r's last utilities and gradients.  ``objective`` selects the training
+    objective as for :class:`DeviceGA`, one for every run."""
 
     def __init__(self, masters, adv_masters=None, *, runs, pop_size, use_arl, max_generations, device=None, parents=1,
-                 weights=None, es_lr=None):
+                 weights=None, es_lr=None, objective="reward"):
         w = _parent_weights(parents, weights, pop_size)
         lr = _es_lr(es_lr, parents, weights, pop_size)
+        _objective(objective, "exact", 32)
+        self.precision = "exact"
         self.device = torch.cuda.current_device() if device is None else int(device)
         K = len(runs)
         if K == 0:
@@ -675,6 +743,7 @@ class DeviceGASweep(_GAHandle):
                                                    None if a is None else a.ctypes.data, self.device, _stream(self.device)))
         self._set_parents(parents, w)
         self._set_es(lr)
+        self._set_objective(objective)
 
     def parents(self, run=0):
         """``(mm_index, adv_index)`` int64[mu] of run ``run``: its last generation's parents in rank order (indices within
@@ -721,14 +790,21 @@ class DRLEngine:
       ``train`` (solo and sharded) and ``train_sweep``.  It excludes ``parents`` > 1 / ``parent_weights``.  As with
       truncation selection, ``val_f``, keep-best and the checkpoint belong to the updated master, ``train_f`` /
       ``train_trades`` to the best child.
+    * ``objective`` (``"reward"``, the default, or ``"pnl"`` / ``"pnl_map"`` / ``"sharpe"``: the StrategyAnalytics Total
+      PnL, PnL-to-MAP or trade Sharpe of each episode, -50 without trades and for a NaN value) is what ``train`` (solo and
+      sharded) and ``train_sweep`` maximise: ``train_f`` / ``val_f`` in the history, the keep-best-on-validation choice,
+      the checkpoint and sigma decay all follow it (see :class:`DeviceGA`).  Any objective but the reward needs the exact
+      path: at ``hidden_dim=256`` pass ``precision="exact"``.
     """
 
     def __init__(self, pop_size=50, sigma=0.05, phi=0.01, tick_size=0.01, fee_rate=0.0, use_arl=False,
                  save_dir="checkpoints/drl", seed=None, device=None, patience=15, precision=None, hidden_dim=32,
-                 group=None, parents=1, parent_weights=None, es_lr=None):
+                 group=None, parents=1, parent_weights=None, es_lr=None, objective="reward"):
         _parent_weights(parents, parent_weights, pop_size)            # argument errors before any side effect
         _es_lr(es_lr, parents, parent_weights, pop_size)
+        _objective(objective, precision, hidden_dim)
         self.parents, self.parent_weights, self.es_lr = parents, parent_weights, es_lr
+        self.objective = objective
         self.precision = precision
         self.phi = phi
         self.tick_size = tick_size
@@ -779,7 +855,8 @@ class DRLEngine:
                             fee_rate=self.fee_rate, use_arl=self.use_arl, seed=seed,
                             max_generations=max(1, generations), patience=self.patience, device=dev,
                             precision=self.precision, hidden=self.hidden_dim, shard=shard,
-                            parents=self.parents, weights=self.parent_weights, es_lr=self.es_lr)
+                            parents=self.parents, weights=self.parent_weights, es_lr=self.es_lr,
+                            objective=self.objective)
         if sharded:
             from .dist import ShardedGA
             runner = ShardedGA(make, pop, group=self.group)
@@ -879,7 +956,7 @@ class DRLEngine:
                            self.adv_evolver.master_policy.get_weights() if self.use_arl else None,
                            runs=runs, pop_size=self.mm_evolver.pop_size, use_arl=self.use_arl,
                            max_generations=max(1, generations), device=dev, parents=self.parents,
-                           weights=self.parent_weights, es_lr=self.es_lr)
+                           weights=self.parent_weights, es_lr=self.es_lr, objective=self.objective)
         save_paths = [os.path.join(self.save_dir, f"{output_prefix}_run{r}_best_val_{phi_r[r]}.pth") for r in range(K)]
         saved_val = [-np.inf] * K
 

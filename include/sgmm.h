@@ -176,6 +176,37 @@ int sgmm_rollout_population_host(const sgmm_bundle* bundle, const sgmm_populatio
                                  const sgmm_population* adv, const sgmm_rollout_params* params,
                                  double* fitness, int32_t* trades, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Training objectives: what fitness[i] measures.  REWARD is the reference's total reward; the others are columns of
+ * StrategyAnalytics (analytics/mm_analyzer.py:5-56, analytics.KEYS) of the same episode, computed inside the walk of the
+ * policy-table route without per-bar trace columns.
+ * For an episode with trace columns wealth = cash + inventory * mid_next (the cash chain applies the buy leg, then the
+ * sell leg, as the env step does) and is_trade = fill_buy | fill_sell, let v be the StrategyAnalytics value evaluated
+ * with exactly the operations of sgmm_trace_analytics:
+ *   PNL      wealth[T-1] - wealth[0]                                           (0 for T = 0)
+ *   PNL_MAP  map == 0 ? 0 : total / map,  map = sum |inventory| / T
+ *   SHARPE   pairwise (numpy order) mean / ddof = 1 std of the wealth differences between consecutive trade rows:
+ *            0 below two trades, NaN with exactly two (one difference), 0 when the std is 0
+ * Then  fitness = trades == 0 ? v - 50 : (v is NaN ? -50 : v)   and trades is unchanged.  The -50 keeps the reference's
+ * pressure against idle agents (Env/drl_engine.py:64-65); a NaN objective becomes -50 because the GA's ranking puts NaN
+ * first (numpy argmax), so it would win every selection.  Every non-REWARD objective is bit-identical to that
+ * post-processing of sgmm_trace_analytics over sgmm_rollout_trace_population's columns.
+ * ------------------------------------------------------------------------------------------- */
+#define SGMM_OBJECTIVE_REWARD   0   /* the reference: total reward, -50 without trades (today's fitness, the default) */
+#define SGMM_OBJECTIVE_PNL      1   /* StrategyAnalytics "Total PnL"     (analytics.KEYS[0]) */
+#define SGMM_OBJECTIVE_PNL_MAP  2   /* StrategyAnalytics "PnLMAP (Eff)"  (analytics.KEYS[2]) */
+#define SGMM_OBJECTIVE_SHARPE   3   /* StrategyAnalytics "Sharpe", the trade Sharpe (analytics.KEYS[4]) */
+
+/* sgmm_rollout_population with a training objective (DEVICE pointers, the code-buffer rules of sgmm_rollout_population).
+ * SGMM_OBJECTIVE_REWARD is exactly sgmm_rollout_population.  Any other objective takes the policy-table route at every
+ * population size (H = 32 F32 / EXACT, with or without the adversary; H = 256 EXACT), whose table lives in the bundle's
+ * code buffer in batches under SGMM_EXACT256_BATCH_BYTES; SHARPE adds 8 B per individual and bar to a batch's scratch.
+ * The tensor-core precisions (BF16 / TF32 / F16) with a non-REWARD objective: SGMM_ERR_UNSUPPORTED.  An unknown
+ * objective: SGMM_ERR_INVALID. */
+int sgmm_rollout_objective(const sgmm_bundle* bundle, const sgmm_population* mm, const sgmm_population* adv,
+                           const sgmm_rollout_params* params, int32_t objective, double* fitness, int32_t* trades,
+                           void* stream);
+
 /* Pipelined variant of the host-buffer entry for callers that evaluate batch after batch (a population service, or
  * independent populations such as a phi sweep): enqueues H2D + kernel + D2H of this batch on one of two internal streams
  * of the bundle and returns at once, so the upload of batch k+1 overlaps the kernel of batch k.  The HOST buffers
@@ -443,6 +474,17 @@ int sgmm_ga_set_es(sgmm_ga* ga, float lr, void* stream);
 int sgmm_ga_run_es_host(sgmm_ga* ga, int32_t run, float* utilities, float* grad, float* adv_utilities, float* adv_grad,
                         void* stream);
 int sgmm_ga_es_host(sgmm_ga* ga, float* utilities, float* grad, float* adv_utilities, float* adv_grad, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Training objective (SGMM_OBJECTIVE_*, see sgmm_rollout_objective) of any GA handle (solo, sharded or sweep; one
+ * objective for every run).  It changes only the fitness values the GA ranks: the population evaluation and the
+ * validation rollout both measure the objective, so train_f / val_f, best_val, keep-best-on-validation and sigma decay
+ * follow it, and the adversary (use_arl) still receives -fitness, so it minimises the objective.  It composes with
+ * sgmm_ga_set_parents and sgmm_ga_set_es.  A non-REWARD objective moves the H = 32 population to the policy-table route
+ * at every size.  SGMM_OBJECTIVE_REWARD gives the same bits as no call.
+ * Refused: after the first evaluate / select / generation of the handle, or an unknown objective (SGMM_ERR_INVALID); a
+ * non-REWARD objective with a tensor-core precision (SGMM_ERR_UNSUPPORTED).  Synchronises the stream. */
+int sgmm_ga_set_objective(sgmm_ga* ga, int32_t objective, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Upstream of the rollout: the per-day window loop of load_signals_bundle
