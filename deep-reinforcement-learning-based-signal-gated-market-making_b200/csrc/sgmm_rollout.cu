@@ -152,10 +152,270 @@ int launch_prologue(sgmm_bundle* b, const float* z1, const float* z2, const doub
 }
 
 // ---------------------------------------------------------------------------------------------
-// the rollout kernel (H = 32)
+// the pieces of the rollout kernels (H = 32)
 // ---------------------------------------------------------------------------------------------
 // compute warps per CTA (one more warp is the producer): bounded by the register file
 __host__ __device__ constexpr int max_compute_warps(int U) { return U == 4 ? 7 : (U == 2 ? 15 : MAX_WARPS); }
+
+// where a thread sits: a CTA has nwarps compute warps of U individuals each (L = 32 / U lanes per individual) and, last,
+// the producer / accounting warp
+template <int U>
+struct H32Cta {
+    int warp, lane, nwarps;
+    int g, l;                 // the lane's individual within the warp, and its lane within the individual
+    int live_warps;           // compute warps with at least one individual < count
+    int64_t first, ind;       // the CTA's first individual, the lane's individual
+    bool live;                // ind < count
+
+    __device__ __forceinline__ explicit H32Cta(const int64_t& count)
+    {
+        warp = threadIdx.x >> 5; lane = threadIdx.x & 31;
+        nwarps = (blockDim.x >> 5) - 1;
+        g = lane / (32 / U); l = lane % (32 / U);
+        first = (int64_t)blockIdx.x * nwarps * U;
+        const int64_t remaining = count - first;
+        live_warps = (int)(remaining >= (int64_t)nwarps * U ? nwarps : (remaining + U - 1) / U);
+        ind = first + (int64_t)warp * U + g;
+        live = ind < count;
+    }
+};
+
+// one bar of the accounting warp: the fp64 half of the env step of this lane's individual from its step record `code`
+// (the offset of each side that filled, or a no-fill marker; without the adversary the offsets travel as the fp32 q = raw*5)
+template <bool ADV, bool FEE>
+__device__ __forceinline__ void account_bar(uint64_t code, const BarPx* pxs, int i, double tick, double fee,
+                                            const PenaltyTable& pen, int& inv, int& ntr, double& total)
+{
+    int ka = (int)(uint32_t)code, kb = (int)(uint32_t)(code >> 32);
+    const bool fs = ka != (ADV ? SGMM_CODE_NOFILL : SGMM_CODE_NOFILL_F), fb = kb != (ADV ? SGMM_CODE_NOFILL : SGMM_CODE_NOFILL_F);
+    inv += (fb ? 1 : 0) - (fs ? 1 : 0);                      // market_env.py:45,51
+    const int ai = inv < 0 ? -inv : inv;
+    const bool traded = fb || fs;
+    ntr += traded ? 1 : 0;                                   // drl_engine.py:60-61
+    double pnl = 0.0;                                        // market_env.py:40
+    if (__any_sync(0xffffffffu, traded)) {
+        const double2 ab = *reinterpret_cast<const double2*>(&pxs[i].ask);
+        const double mid = pxs[i].mid_next;
+        if (!ADV) { ka = __float2int_rn(__int_as_float(ka)); kb = __float2int_rn(__int_as_float(kb)); }   // drl_engine.py:39
+        const double my_ask = quote_ask(ab.x, ka, tick), my_bid = quote_bid(ab.y, kb, tick);      // market_env.py:30-31
+        const double leg_b = buy_leg<FEE>(my_bid, mid, fee), leg_s = sell_leg<FEE>(my_ask, mid, fee);
+        pnl = fb ? add_rn(pnl, leg_b) : pnl;
+        pnl = fs ? add_rn(pnl, leg_s) : pnl;
+    }
+    total = add_rn(total, sub_rn(pnl, penalty(pen, ai)));                   // market_env.py:58, drl_engine.py:54
+}
+
+// the lane's weights in registers (models/model.py:31-36 layout): hidden units l, l + L, ... of W1 / b1 / b2 / W2 rows / W3,
+// and b3; zeros for a lane without an individual
+template <int U>
+struct H32Regs {
+    float w1x[U], w1y[U], w1i[U], b1[U], b2[U], w3a[U], w3b[U];
+    float2 w2[U][16];
+    float b3a, b3b;
+};
+
+template <int U>
+__device__ __forceinline__ void h32_load_weights(const PopArgs& mm, const H32Cta<U>& cta, H32Regs<U>& w)
+{
+    constexpr int H = 32, L = 32 / U;
+    const GenomeSource src = make_source(resolve(mm), cta.live ? cta.ind : 0, (int64_t)H * H + 7 * H + 2);
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const int j = cta.l + L * u;
+        if (cta.live) {
+            w.w1x[u] = src.at(3 * j + 0); w.w1y[u] = src.at(3 * j + 1); w.w1i[u] = src.at(3 * j + 2);
+            w.b1[u] = src.at(3 * H + j);
+            w.b2[u] = src.at(4 * H + H * H + j);
+            w.w3a[u] = src.at(5 * H + H * H + j);
+            w.w3b[u] = src.at(6 * H + H * H + j);
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+                float v[4]; src.at4(4 * H + (int64_t)j * H + 4 * c, v);
+                w.w2[u][2 * c] = make_float2(v[0], v[1]);
+                w.w2[u][2 * c + 1] = make_float2(v[2], v[3]);
+            }
+        } else {
+            w.w1x[u] = w.w1y[u] = w.w1i[u] = w.b1[u] = w.b2[u] = w.w3a[u] = w.w3b[u] = 0.0f;
+#pragma unroll
+            for (int c = 0; c < 16; ++c) w.w2[u][c] = make_float2(0.0f, 0.0f);
+        }
+    }
+    w.b3a = cta.live ? src.at(7 * H + H * H) : 0.0f;
+    w.b3b = cta.live ? src.at(7 * H + H * H + 1) : 0.0f;
+}
+
+// the adversary's displacement table of the lane's individual (drl_engine.py:42-48, models/model.py:40-50): 4 bits for
+// each of the 20 states in t[0..2]; the L lanes of an individual split the states, then gather the whole table
+template <int U>
+__device__ __forceinline__ void h32_adv_table(const PopArgs& adv, const H32Cta<U>& cta, uint32_t t[3])
+{
+    constexpr int L = 32 / U;
+    const GenomeSource asrc = make_source(resolve(adv), cta.live ? cta.ind : 0, (int64_t)1250);
+    t[0] = t[1] = t[2] = 0u;
+    for (int s = cta.l; s < 20; s += L) {
+        const uint32_t e = cta.live ? adversary_entry(asrc, s) : 5u;
+        t[s >> 3] |= e << ((s & 7) * 4);
+    }
+#pragma unroll
+    for (int m = L / 2; m >= 1; m >>= 1) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) t[k] |= __shfl_xor_sync(0xffffffffu, t[k], m);
+    }
+}
+
+// layer 1 of one bar: the bar part w1x*z1 + w1y*z2 + b1 (inventory-independent), then the inventory term and the ReLU
+template <int U>
+__device__ __forceinline__ void h32_layer1_bar(const H32Regs<U>& w, float2 z, float a1[U])
+{
+#pragma unroll
+    for (int u = 0; u < U; ++u) a1[u] = __fmaf_rn(w.w1y[u], z.y, __fmaf_rn(w.w1x[u], z.x, w.b1[u]));
+}
+template <int U>
+__device__ __forceinline__ void h32_layer1_inv(const H32Regs<U>& w, const float a1[U], float inv2, float h[U])
+{
+#pragma unroll
+    for (int u = 0; u < U; ++u) h[u] = fmaxf(__fmaf_rn(w.w1i[u], inv2, a1[u]), 0.0f);
+}
+template <int U>
+__device__ __forceinline__ void h32_layer1(const H32Regs<U>& w, float2 z, float inv2, float h[U])
+{
+    float a1[U];
+    h32_layer1_bar<U>(w, z, a1);
+    h32_layer1_inv<U>(w, a1, inv2, h);
+}
+// h1 through the warp's shared buffer: U individuals x 32 activations, 16-B interleaved
+template <int U>
+__device__ __forceinline__ void h32_put_h1(float* hb, int g, int l, const float h[U])
+{
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const int j = l + (32 / U) * u;
+        hb[((j >> 2) * U + g) * 4 + (j & 3)] = h[u];
+    }
+}
+template <int U>
+__device__ __forceinline__ void h32_get_h1(const float* hb, int g, float4 h4[8])
+{
+#pragma unroll
+    for (int k = 0; k < 8; ++k) h4[k] = *reinterpret_cast<const float4*>(&hb[(k * U + g) * 4]);
+}
+// layers 2 and 3 up to the lane's partial outputs: U rows x 32 as packed FFMA2, four chains per row (the two halves of
+// P and Q are the four interleaved chains of the SGMM-F32 order), then the products and the local tree; for U < 4 the
+// cross-lane butterfly too (shuffles)
+template <int U>
+__device__ __forceinline__ float2 h32_layer23(const H32Regs<U>& w, const float4 h4[8])
+{
+    constexpr int L = 32 / U;
+    float2 P[U], Q[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) { P[u] = make_float2(w.b2[u], 0.0f); Q[u] = make_float2(0.0f, 0.0f); }
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+        const float2 hlo = make_float2(h4[k].x, h4[k].y), hhi = make_float2(h4[k].z, h4[k].w);
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            P[u] = __ffma2_rn(w.w2[u][2 * k], hlo, P[u]);
+            Q[u] = __ffma2_rn(w.w2[u][2 * k + 1], hhi, Q[u]);
+        }
+    }
+    float pa[U], pb[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const float2 S = __fadd2_rn(P[u], Q[u]);                 // (a0+a2, a1+a3)
+        const float h2 = fmaxf(__fadd_rn(S.x, S.y), 0.0f);
+        pa[u] = __fmul_rn(w.w3a[u], h2);
+        pb[u] = __fmul_rn(w.w3b[u], h2);
+    }
+    float ra, rb;
+    if (U == 4) {
+        ra = __fadd_rn(__fadd_rn(pa[0], pa[2 % U]), __fadd_rn(pa[1 % U], pa[3 % U]));
+        rb = __fadd_rn(__fadd_rn(pb[0], pb[2 % U]), __fadd_rn(pb[1 % U], pb[3 % U]));
+    } else {
+        if (U == 2) { ra = __fadd_rn(pa[0], pa[1 % U]); rb = __fadd_rn(pb[0], pb[1 % U]); }
+        else { ra = pa[0]; rb = pb[0]; }
+#pragma unroll
+        for (int m = L / 2; m >= 1; m >>= 1) {
+            ra = __fadd_rn(ra, __shfl_xor_sync(0xffffffffu, ra, m));
+            rb = __fadd_rn(rb, __shfl_xor_sync(0xffffffffu, rb, m));
+        }
+    }
+    return make_float2(ra, rb);
+}
+// U = 4: the butterfly over the 8 lanes of the individual, evaluated by every lane from the 8 partials exchanged through
+// shared memory (the same tree, one round trip instead of 3 shuffles)
+__device__ __forceinline__ void h32_put_partial(float* rbw, int g, int l, float2 r)
+{
+    *reinterpret_cast<float2*>(&rbw[g * 20 + l * 2]) = r;
+}
+__device__ __forceinline__ void h32_get_partials(const float* rbw, int g, float4 r[4])
+{
+#pragma unroll
+    for (int k = 0; k < 4; ++k) r[k] = *reinterpret_cast<const float4*>(&rbw[g * 20 + 4 * k]);
+}
+__device__ __forceinline__ float2 h32_tree(const float4 r[4])
+{
+    const float2 t04 = __fadd2_rn(make_float2(r[0].x, r[0].y), make_float2(r[2].x, r[2].y));
+    const float2 t15 = __fadd2_rn(make_float2(r[0].z, r[0].w), make_float2(r[2].z, r[2].w));
+    const float2 t26 = __fadd2_rn(make_float2(r[1].x, r[1].y), make_float2(r[3].x, r[3].y));
+    const float2 t37 = __fadd2_rn(make_float2(r[1].z, r[1].w), make_float2(r[3].z, r[3].w));
+    return __fadd2_rn(__fadd2_rn(t04, t26), __fadd2_rn(t15, t37));
+}
+// layers 2 and 3 of one chain from the h1 it published: the individual's raw outputs before b3
+template <int U>
+__device__ __forceinline__ float2 h32_output(const H32Regs<U>& w, const float* hb, float* rbw, int g, int l)
+{
+    float4 h4[8];
+    h32_get_h1<U>(hb, g, h4);
+    float2 p = h32_layer23<U>(w, h4);
+    if (U == 4) {
+        h32_put_partial(rbw, g, l, p);
+        __syncwarp();
+        float4 pr[4];
+        h32_get_partials(rbw, g, pr);
+        p = h32_tree(pr);
+    }
+    return p;
+}
+
+// the fill decision: q = raw*5 (drl_engine.py:39), and the inventory move (in halves, exact) of the fills
+__device__ __forceinline__ float2 h32_q(float2 r, float b3a, float b3b)
+{
+    return make_float2(__fmul_rn(__fadd_rn(r.x, b3a), 5.0f), __fmul_rn(__fadd_rn(r.y, b3b), 5.0f));
+}
+__device__ __forceinline__ float h32_move(bool fb, bool fs) { return fb ? (fs ? 0.0f : 0.5f) : (fs ? -0.5f : 0.0f); }   // market_env.py:45,51
+// without the adversary: the rounding is folded into the bar's float thresholds th = (tha, thb), so there is no
+// conversion on the critical path; moves inv2 and returns the step record (the q of each side that filled)
+__device__ __forceinline__ float2 h32_decide(float2 r, float b3a, float b3b, float2 th, float& inv2)
+{
+    const float2 q = h32_q(r, b3a, b3b);
+    const bool fb = (inv2 < 1.0f) && (q.y < th.y);                 // market_env.py:34,37
+    const bool fs = (inv2 > -1.0f) && (q.x < th.x);                // :35,:38
+    inv2 = __fadd_rn(inv2, h32_move(fb, fs));
+    return make_float2(fs ? q.x : __int_as_float(SGMM_CODE_NOFILL_F), fb ? q.y : __int_as_float(SGMM_CODE_NOFILL_F));
+}
+// with the adversary (drl_engine.py:42-48): integer offsets, clamped and displaced by the table entry of the state
+// (previous fills, inventory), against the bar's integer thresholds k1 = (ka1, kb1); moves the state and returns the step
+// record (the offset of each side that filled)
+__device__ __forceinline__ int2 h32_decide_adv(float2 r, float b3a, float b3b, int2 k1, const uint32_t t[3], int& inv,
+                                               int& fbp, int& fsp, float& inv2)
+{
+    const float2 q = h32_q(r, b3a, b3b);
+    int ka = __float2int_rn(q.x), kb = __float2int_rn(q.y);        // np.round(...).astype(int)
+    const uint32_t e = table_lookup(t[0], t[1], t[2], fsp * 10 + fbp * 5 + inv + 2);
+    ka = max(min(ka, K_CLAMP), -K_CLAMP) + (int)(e & 3u) - 1;      // market_env.py:26-28
+    kb = max(min(kb, K_CLAMP), -K_CLAMP) + (int)(e >> 2) - 1;
+    const bool fb = (inv2 < 1.0f) && (kb < k1.y);                  // :34,:37
+    const bool fs = (inv2 > -1.0f) && (ka < k1.x);                 // :35,:38
+    fbp = fb ? 1 : 0; fsp = fs ? 1 : 0;                            // drl_engine.py:57-58
+    inv2 = __fadd_rn(inv2, h32_move(fb, fs));
+    inv += (fb ? 1 : 0) - (fs ? 1 : 0);
+    return make_int2(fs ? ka : SGMM_CODE_NOFILL, fb ? kb : SGMM_CODE_NOFILL);
+}
+// the inventory move (in halves) a step record of h32_decide encodes
+__device__ __forceinline__ float h32_record_move(float2 c)
+{
+    return h32_move(__float_as_int(c.y) != SGMM_CODE_NOFILL_F, __float_as_int(c.x) != SGMM_CODE_NOFILL_F);
+}
 
 struct RingSmem {
     uint64_t full[RING_STAGES];
@@ -168,43 +428,29 @@ struct RingSmem {
     uint64_t rec_full[REC_STAGES];
     uint64_t rec_empty[REC_STAGES];
     uint64_t rec[REC_STAGES][CHUNK_BARS][32];
-#ifdef SGMM_ROLLOUT_TRACE
-    long long trace[2][64][3];
-#endif
 };
 
 template <int U, bool ADV, bool FEE>
 __global__ void __launch_bounds__((max_compute_warps(U) + 1) * 32, 1)
 rollout_kernel_h32(const RolloutArgs a)
 {
-    constexpr int H = 32;
-    constexpr int NI = U;                // individuals per warp
-    constexpr int L = 32 / U;            // lanes per individual
-    constexpr int64_t G = (int64_t)H * H + 7 * H + 2;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     RingSmem& sm = *reinterpret_cast<RingSmem*>(smem_raw);
 
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int nwarps = (blockDim.x >> 5) - 1;          // compute warps; the last warp is the TMA producer
-    const int g = lane / L, l = lane % L;
-    const int64_t first = (int64_t)blockIdx.x * nwarps * NI;
-    const int64_t remaining = a.mm.count - first;
-    const int live_warps = (int)(remaining >= (int64_t)nwarps * NI ? nwarps : (remaining + NI - 1) / NI);
-    const int64_t ind = first + (int64_t)warp * NI + g;
-    const bool live = ind < a.mm.count;
+    const H32Cta<U> cta(a.mm.count);
     const int64_t T = a.T;
     const int64_t nchunks = (T + CHUNK_BARS - 1) / CHUNK_BARS;
 
     if (threadIdx.x == 0) {
 #pragma unroll
-        for (int s = 0; s < RING_STAGES; ++s) { mbar_init(&sm.full[s], 1); mbar_init(&sm.empty[s], live_warps); }
+        for (int s = 0; s < RING_STAGES; ++s) { mbar_init(&sm.full[s], 1); mbar_init(&sm.empty[s], cta.live_warps); }
 #pragma unroll
-        for (int r = 0; r < REC_STAGES; ++r) { mbar_init(&sm.rec_full[r], live_warps); mbar_init(&sm.rec_empty[r], 1); }
+        for (int r = 0; r < REC_STAGES; ++r) { mbar_init(&sm.rec_full[r], cta.live_warps); mbar_init(&sm.rec_empty[r], 1); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
 
-    if (warp == nwarps) {
+    if (cta.warp == cta.nwarps) {
         // ===== the CTA's last warp: TMA producer of the bar ring AND the fp64 half of the env step =====
         // The compute warps do the policy and the INTEGER half of the step and hand one 8-byte record per bar and
         // individual through shared memory; here lane j accounts individual first + j: quotes, P&L legs, penalty and
@@ -212,8 +458,9 @@ rollout_kernel_h32(const RolloutArgs a)
         // warp instruction per fp64 operation for ALL individuals of the CTA -- in the step loop the same arithmetic
         // was issued once per compute warp (22 of 217 instructions, two of them conversions on the XU pipe, plus the
         // fp64 live ranges in a 254-register kernel) and cost 16 % of the loop.
-        const int64_t indj = first + lane;
-        const bool livej = lane < live_warps * NI && indj < a.mm.count;
+        const int lane = cta.lane;
+        const int64_t indj = cta.first + lane;
+        const bool livej = lane < cta.live_warps * U && indj < a.mm.count;
         const double tick = a.tick, fee = a.fee;
         const PenaltyTable pen = penalty_table(a.phi);
         double total = 0.0;                                              // drl_engine.py:26
@@ -243,24 +490,7 @@ rollout_kernel_h32(const RolloutArgs a)
             const BarPx* pxs = &sm.px[c % RING_STAGES][0];
 #pragma unroll 4
             for (int i = 0; i < n; ++i) {
-                const uint64_t code = sm.rec[r][i][lane];
-                int ka = (int)(uint32_t)code, kb = (int)(uint32_t)(code >> 32);
-                const bool fs = ka != (ADV ? SGMM_CODE_NOFILL : SGMM_CODE_NOFILL_F), fb = kb != (ADV ? SGMM_CODE_NOFILL : SGMM_CODE_NOFILL_F);
-                inv += (fb ? 1 : 0) - (fs ? 1 : 0);                      // market_env.py:45,51
-                const int ai = inv < 0 ? -inv : inv;
-                const bool traded = fb || fs;
-                ntr += traded ? 1 : 0;                                   // drl_engine.py:60-61
-                double pnl = 0.0;                                        // market_env.py:40
-                if (__any_sync(0xffffffffu, traded)) {
-                    const double2 ab = *reinterpret_cast<const double2*>(&pxs[i].ask);
-                    const double mid = pxs[i].mid_next;
-                    if (!ADV) { ka = __float2int_rn(__int_as_float(ka)); kb = __float2int_rn(__int_as_float(kb)); }   // drl_engine.py:39
-                    const double my_ask = quote_ask(ab.x, ka, tick), my_bid = quote_bid(ab.y, kb, tick);      // market_env.py:30-31
-                    const double leg_b = buy_leg<FEE>(my_bid, mid, fee), leg_s = sell_leg<FEE>(my_ask, mid, fee);
-                    pnl = fb ? add_rn(pnl, leg_b) : pnl;
-                    pnl = fs ? add_rn(pnl, leg_s) : pnl;
-                }
-                total = add_rn(total, sub_rn(pnl, penalty(pen, ai)));                   // market_env.py:58, drl_engine.py:54
+                account_bar<ADV, FEE>(sm.rec[r][i][lane], pxs, i, tick, fee, pen, inv, ntr, total);
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(&sm.rec_empty[r]);
@@ -268,67 +498,24 @@ rollout_kernel_h32(const RolloutArgs a)
         if (livej) { a.fitness[indj] = episode_fitness(total, ntr); a.trades[indj] = ntr; }
         return;
     }
-    if (warp >= live_warps) return;
+    if (cta.warp >= cta.live_warps) return;
 
-    // ---- weights into registers (models/model.py:31-36 layout) ---------------------------------
-    const PopArgs mmp = resolve(a.mm);
-    const GenomeSource src = make_source(mmp, live ? ind : 0, G);
-    float w1x[U], w1y[U], w1i[U], b1[U], b2[U], w3a[U], w3b[U];
-    float2 w2[U][16];
-    float b3a = 0.0f, b3b = 0.0f;
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-        const int j = l + L * u;
-        if (live) {
-            w1x[u] = src.at(3 * j + 0); w1y[u] = src.at(3 * j + 1); w1i[u] = src.at(3 * j + 2);
-            b1[u] = src.at(3 * H + j);
-            b2[u] = src.at(4 * H + H * H + j);
-            w3a[u] = src.at(5 * H + H * H + j);
-            w3b[u] = src.at(6 * H + H * H + j);
-#pragma unroll
-            for (int c = 0; c < 8; ++c) {
-                float v[4]; src.at4(4 * H + (int64_t)j * H + 4 * c, v);
-                w2[u][2 * c] = make_float2(v[0], v[1]);
-                w2[u][2 * c + 1] = make_float2(v[2], v[3]);
-            }
-        } else {
-            w1x[u] = w1y[u] = w1i[u] = b1[u] = b2[u] = w3a[u] = w3b[u] = 0.0f;
-#pragma unroll
-            for (int c = 0; c < 16; ++c) w2[u][c] = make_float2(0.0f, 0.0f);
-        }
-    }
-    if (live) { b3a = src.at(7 * H + H * H); b3b = src.at(7 * H + H * H + 1); }
+    H32Regs<U> w;
+    h32_load_weights<U>(a.mm, cta, w);
+    uint32_t adv_t[3] = {0u, 0u, 0u};
+    if (ADV) h32_adv_table<U>(a.adv, cta, adv_t);
 
-    uint32_t adv_t0 = 0x55555555u, adv_t1 = 0x55555555u, adv_t2 = 0x55555555u;   // all (0,0)
-    if (ADV) {
-        const PopArgs advp = resolve(a.adv);
-        const GenomeSource asrc = make_source(advp, live ? ind : 0, (int64_t)1250);
-        // the L lanes of an individual split the 20 states, then gather the whole table
-        uint32_t mine[3] = {0u, 0u, 0u};
-        for (int s = l; s < 20; s += L) {
-            const uint32_t e = live ? adversary_entry(asrc, s) : 5u;
-            mine[s >> 3] |= e << ((s & 7) * 4);
-        }
-#pragma unroll
-        for (int m = L / 2; m >= 1; m >>= 1) {
-#pragma unroll
-            for (int k = 0; k < 3; ++k) mine[k] |= __shfl_xor_sync(0xffffffffu, mine[k], m);
-        }
-        adv_t0 = mine[0]; adv_t1 = mine[1]; adv_t2 = mine[2];
-    }
-
-    float* hb = &sm.hbuf[warp][0];
-    float* rbw = &sm.rbuf[warp][0];
-    int inv = 0, fbp = 0, fsp = 0;
+    float* const hb = &sm.hbuf[cta.warp][0];
+    float* const rbw = &sm.rbuf[cta.warp][0];
+    int inv = 0, fbp = 0, fsp = 0;                                   // the adversary's state
     float inv2 = 0.0f;                                               // inventory / 2.0 (drl_engine.py:35), exact
 
     // The step loop does the INTEGER half of the env step (offsets, fills, inventory) and hands one 8-byte record per
-    // bar to the accounting warp (above): the offset of each side that filled, or a no-fill marker.  Without the
-    // adversary the offsets travel as the fp32 q = raw*5 they are rounded from (no conversion in this loop).
-    const int slotj = warp * NI + g;                                 // this individual's lane in the accounting warp
+    // bar to the accounting warp (above).
+    const int slotj = cta.warp * U + cta.g;                          // this individual's lane in the accounting warp
 
     // Two compute warps share a scheduler (warps w and w + 4).  Measured (profiles/r2_exact_phase_trace_*.log, a clock64 trace of
-    // both from the SGMM_ROLLOUT_TRACE build): their steps lock at a relative phase of 0.19 whatever the start offset, and
+    // both from a trace build, removed after 2e97c64): their steps lock at a relative phase of 0.19 whatever the start offset, and
     // forcing strict alternation of the layer-2 bursts with named barriers is SLOWER (4.88 vs 4.66 ms): the FMA pipe's time
     // per pair of warp-steps (2 x ~200 cycles, FFMA2 with three register operands issues every 2.34 cycles) is conserved
     // whatever the interleaving; both experiments were removed again.
@@ -343,134 +530,35 @@ rollout_kernel_h32(const RolloutArgs a)
         const int n = (int)(T - t0 < CHUNK_BARS ? T - t0 : CHUNK_BARS);
         const BarSig* sigs = &sm.sig[s][0];
 
-        // bar 0 of the chunk: signals, thresholds and the inventory-independent part of layer 1
+        // bar 0 of the chunk: signals, thresholds and the bar part of layer 1
         float4 sg = *reinterpret_cast<const float4*>(&sigs[0]);                     // z1, z2, tha, thb
         int2 kth = *reinterpret_cast<const int2*>(&sigs[0].ka1);
-        float A1[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) A1[u] = __fmaf_rn(w1y[u], sg.y, __fmaf_rn(w1x[u], sg.x, b1[u]));
-
-#ifdef SGMM_ROLLOUT_TRACE
-        const bool trc = blockIdx.x == 0 && (warp & 3) == 0 && lane == 0 && c == 4;
-#endif
+        float a1[U];
+        h32_layer1_bar<U>(w, make_float2(sg.x, sg.y), a1);
 #pragma unroll 1
         for (int i = 0; i < n; ++i) {
-#ifdef SGMM_ROLLOUT_TRACE
-            if (trc && i < 64) { long long t; asm volatile("mov.u64 %0, %%clock64; // %1" : "=l"(t) : "f"(inv2)); sm.trace[warp >> 2][i][0] = t; }
-#endif
-            // ---- layer 1 (inventory term) + ReLU, publish h1 ------------------------------------
-#pragma unroll
-            for (int u = 0; u < U; ++u) {
-                const int j = l + L * u;
-                hb[((j >> 2) * NI + g) * 4 + (j & 3)] = fmaxf(__fmaf_rn(w1i[u], inv2, A1[u]), 0.0f);
-            }
+            float h[U];
+            h32_layer1_inv<U>(w, a1, inv2, h);
+            h32_put_h1<U>(hb, cta.g, cta.l, h);
             __syncwarp();
-            const float tha = sg.z, thb = sg.w;
-            const int ka1 = kth.x, kb1 = kth.y;
-            // ---- prefetch bar i+1 and its layer-1 partial (off the critical path) --------------
+            const float2 th = make_float2(sg.z, sg.w);
+            const int2 k1 = kth;
+            const float2 p = h32_output<U>(w, hb, rbw, cta.g, cta.l);
+            // prefetch bar i+1 and the bar part of its layer 1 (off the critical path)
             const int inext = i + 1 < CHUNK_BARS ? i + 1 : CHUNK_BARS - 1;
             sg = *reinterpret_cast<const float4*>(&sigs[inext]);
             if (ADV) kth = *reinterpret_cast<const int2*>(&sigs[inext].ka1);
-            float A1n[U];
-#pragma unroll
-            for (int u = 0; u < U; ++u) A1n[u] = __fmaf_rn(w1y[u], sg.y, __fmaf_rn(w1x[u], sg.x, b1[u]));
-            // ---- layer 2: U rows x 32, packed FFMA2, four chains per row -----------------------
-            float2 P[U], Q[U];
-#pragma unroll
-            for (int u = 0; u < U; ++u) { P[u] = make_float2(b2[u], 0.0f); Q[u] = make_float2(0.0f, 0.0f); }
-#pragma unroll
-            for (int k = 0; k < 8; ++k) {
-                const float4 h4 = *reinterpret_cast<const float4*>(&hb[(k * NI + g) * 4]);
-                const float2 hlo = make_float2(h4.x, h4.y), hhi = make_float2(h4.z, h4.w);
-#pragma unroll
-                for (int u = 0; u < U; ++u) {
-#ifdef SGMM_ROLLOUT_SCALAR_FMA       // A/B switch: 128 scalar FFMA instead of 64 FFMA2 -- 4.74 instead of 4.51 ms at P = 4096 (same results)
-                    P[u].x = __fmaf_rn(w2[u][2 * k].x, hlo.x, P[u].x); P[u].y = __fmaf_rn(w2[u][2 * k].y, hlo.y, P[u].y);
-                    Q[u].x = __fmaf_rn(w2[u][2 * k + 1].x, hhi.x, Q[u].x); Q[u].y = __fmaf_rn(w2[u][2 * k + 1].y, hhi.y, Q[u].y);
-#else
-                    P[u] = __ffma2_rn(w2[u][2 * k], hlo, P[u]);
-                    Q[u] = __ffma2_rn(w2[u][2 * k + 1], hhi, Q[u]);
-#endif
-                }
-            }
-#ifdef SGMM_ROLLOUT_TRACE
-            if (trc && i < 64) { long long t; asm volatile("mov.u64 %0, %%clock64; // %1 %2" : "=l"(t) : "f"(Q[U - 1].y), "f"(P[0].x)); sm.trace[warp >> 2][i][1] = t; }
-#endif
-            // ---- layer 3: products, local tree, then the cross-lane tree ------------------------
-            float pa[U], pb[U];
-#pragma unroll
-            for (int u = 0; u < U; ++u) {
-                const float2 S = __fadd2_rn(P[u], Q[u]);                 // (a0+a2, a1+a3)
-                const float h2 = fmaxf(__fadd_rn(S.x, S.y), 0.0f);
-                pa[u] = __fmul_rn(w3a[u], h2);
-                pb[u] = __fmul_rn(w3b[u], h2);
-            }
-            float ra, rb;
-            if (U == 4) {
-                ra = __fadd_rn(__fadd_rn(pa[0], pa[2 % U]), __fadd_rn(pa[1 % U], pa[3 % U]));
-                rb = __fadd_rn(__fadd_rn(pb[0], pb[2 % U]), __fadd_rn(pb[1 % U], pb[3 % U]));
-                // butterfly over the 8 lanes of the individual, evaluated by every lane from the 8
-                // partials exchanged through shared memory (same tree, 1 round trip instead of 3 shuffles)
-                *reinterpret_cast<float2*>(&rbw[g * 20 + l * 2]) = make_float2(ra, rb);
-                __syncwarp();
-                const float4 r01 = *reinterpret_cast<const float4*>(&rbw[g * 20 + 0]);
-                const float4 r23 = *reinterpret_cast<const float4*>(&rbw[g * 20 + 4]);
-                const float4 r45 = *reinterpret_cast<const float4*>(&rbw[g * 20 + 8]);
-                const float4 r67 = *reinterpret_cast<const float4*>(&rbw[g * 20 + 12]);
-                const float2 t04 = __fadd2_rn(make_float2(r01.x, r01.y), make_float2(r45.x, r45.y));
-                const float2 t15 = __fadd2_rn(make_float2(r01.z, r01.w), make_float2(r45.z, r45.w));
-                const float2 t26 = __fadd2_rn(make_float2(r23.x, r23.y), make_float2(r67.x, r67.y));
-                const float2 t37 = __fadd2_rn(make_float2(r23.z, r23.w), make_float2(r67.z, r67.w));
-                const float2 e = __fadd2_rn(__fadd2_rn(t04, t26), __fadd2_rn(t15, t37));
-                ra = e.x; rb = e.y;
+            h32_layer1_bar<U>(w, make_float2(sg.x, sg.y), a1);
+            if (ADV) {
+                const int2 code = h32_decide_adv(p, w.b3a, w.b3b, k1, adv_t, inv, fbp, fsp, inv2);
+                if (cta.l == 0) *reinterpret_cast<int2*>(recs + i * 32) = code;
             } else {
-                if (U == 2) { ra = __fadd_rn(pa[0], pa[1 % U]); rb = __fadd_rn(pb[0], pb[1 % U]); }
-                else { ra = pa[0]; rb = pb[0]; }
-#pragma unroll
-                for (int m = L / 2; m >= 1; m >>= 1) {
-                    ra = __fadd_rn(ra, __shfl_xor_sync(0xffffffffu, ra, m));
-                    rb = __fadd_rn(rb, __shfl_xor_sync(0xffffffffu, rb, m));
-                }
+                const float2 code = h32_decide(p, w.b3a, w.b3b, th, inv2);
+                if (cta.l == 0) *reinterpret_cast<float2*>(recs + i * 32) = code;
             }
-#ifdef SGMM_ROLLOUT_TRACE
-            if (trc && i < 64) { long long t; asm volatile("mov.u64 %0, %%clock64; // %1" : "=l"(t) : "f"(ra)); sm.trace[warp >> 2][i][2] = t; }
-#endif
-            // ---- quantise + fill decision -------------------------------------------------------
-            const float qa = __fmul_rn(__fadd_rn(ra, b3a), 5.0f);           // raw*5.0 (drl_engine.py:39)
-            const float qb = __fmul_rn(__fadd_rn(rb, b3b), 5.0f);
-            int ka = 0, kb = 0;
-            bool fb, fs;
-            if (ADV) {                                                       // drl_engine.py:42-48
-                ka = __float2int_rn(qa);                                     // np.round(...).astype(int)
-                kb = __float2int_rn(qb);
-                const uint32_t e = table_lookup(adv_t0, adv_t1, adv_t2, fsp * 10 + fbp * 5 + inv + 2);
-                ka = max(min(ka, K_CLAMP), -K_CLAMP) + (int)(e & 3u) - 1;    // market_env.py:26-28
-                kb = max(min(kb, K_CLAMP), -K_CLAMP) + (int)(e >> 2) - 1;
-                fb = (inv2 < 1.0f) && (kb < kb1);                            // :34,:37
-                fs = (inv2 > -1.0f) && (ka < ka1);                           // :35,:38
-                fbp = fb ? 1 : 0; fsp = fs ? 1 : 0;                          // drl_engine.py:57-58
-            } else {
-                // rounding folded into the per-bar float threshold: no conversion on the critical path
-                fb = (inv2 < 1.0f) && (qb < thb);
-                fs = (inv2 > -1.0f) && (qa < tha);
-            }
-            inv2 = __fadd_rn(inv2, fb ? (fs ? 0.0f : 0.5f) : (fs ? -0.5f : 0.0f));   // :45,:51 (exact)
-            inv += (fb ? 1 : 0) - (fs ? 1 : 0);
-            // ---- step code: the offset of each side that filled -------------------------------
-            if (l == 0) {
-                if (ADV) *reinterpret_cast<int2*>(recs + i * 32) = make_int2(fs ? ka : SGMM_CODE_NOFILL, fb ? kb : SGMM_CODE_NOFILL);
-                else *reinterpret_cast<float2*>(recs + i * 32) = make_float2(fs ? qa : __int_as_float(SGMM_CODE_NOFILL_F), fb ? qb : __int_as_float(SGMM_CODE_NOFILL_F));
-            }
-#pragma unroll
-            for (int u = 0; u < U; ++u) A1[u] = A1n[u];
         }
         __syncwarp();
-        if (lane == 0) { mbar_arrive(&sm.empty[s]); mbar_arrive(&sm.rec_full[r]); }
-#ifdef SGMM_ROLLOUT_TRACE
-        if (trc) for (int i = 0; i < 64; ++i)
-            printf("w%d step %2d top %6lld burst_end %6lld reduced %6lld\n", warp, i, sm.trace[warp >> 2][i][0] - sm.trace[0][0][0],
-                   sm.trace[warp >> 2][i][1] - sm.trace[0][0][0], sm.trace[warp >> 2][i][2] - sm.trace[0][0][0]);
-#endif
+        if (cta.lane == 0) { mbar_arrive(&sm.empty[s]); mbar_arrive(&sm.rec_full[r]); }
     }
 }
 
@@ -529,144 +617,30 @@ struct Ring2Smem {
     uint64_t rec[2][ROUND_BARS][32];      // one 8-byte step record per (bar of the round, individual of the CTA)
 };
 
-template <int U>
-struct H32Regs {
-    float w1x[U], w1y[U], w1i[U], b1[U], b2[U], w3a[U], w3b[U];
-    float2 w2[U][16];
-    float b3a, b3b;
-};
-
-// layer 1 (bar part + inventory term) + ReLU of one bar, in rollout_kernel_h32's op order
-template <int U>
-__device__ __forceinline__ void h32_layer1(const H32Regs<U>& w, float2 z, float inv2, float h[U])
-{
-#pragma unroll
-    for (int u = 0; u < U; ++u) h[u] = fmaxf(__fmaf_rn(w.w1i[u], inv2, __fmaf_rn(w.w1y[u], z.y, __fmaf_rn(w.w1x[u], z.x, w.b1[u]))), 0.0f);
-}
-template <int U>
-__device__ __forceinline__ void h32_put_h1(float* hb, int g, int l, const float h[U])
-{
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-        const int j = l + (32 / U) * u;
-        hb[((j >> 2) * U + g) * 4 + (j & 3)] = h[u];
-    }
-}
-template <int U>
-__device__ __forceinline__ void h32_get_h1(const float* hb, int g, float4 h4[8])
-{
-#pragma unroll
-    for (int k = 0; k < 8; ++k) h4[k] = *reinterpret_cast<const float4*>(&hb[(k * U + g) * 4]);
-}
-// layers 2 and 3 up to the lane's partial outputs; for U < 4 the cross-lane butterfly too (shuffles)
-template <int U>
-__device__ __forceinline__ float2 h32_layer23(const H32Regs<U>& w, const float4 h4[8])
-{
-    constexpr int L = 32 / U;
-    float2 P[U], Q[U];
-#pragma unroll
-    for (int u = 0; u < U; ++u) { P[u] = make_float2(w.b2[u], 0.0f); Q[u] = make_float2(0.0f, 0.0f); }
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        const float2 hlo = make_float2(h4[k].x, h4[k].y), hhi = make_float2(h4[k].z, h4[k].w);
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            P[u] = __ffma2_rn(w.w2[u][2 * k], hlo, P[u]);
-            Q[u] = __ffma2_rn(w.w2[u][2 * k + 1], hhi, Q[u]);
-        }
-    }
-    float pa[U], pb[U];
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-        const float2 S = __fadd2_rn(P[u], Q[u]);
-        const float h2 = fmaxf(__fadd_rn(S.x, S.y), 0.0f);
-        pa[u] = __fmul_rn(w.w3a[u], h2);
-        pb[u] = __fmul_rn(w.w3b[u], h2);
-    }
-    float ra, rb;
-    if (U == 4) {
-        ra = __fadd_rn(__fadd_rn(pa[0], pa[2 % U]), __fadd_rn(pa[1 % U], pa[3 % U]));
-        rb = __fadd_rn(__fadd_rn(pb[0], pb[2 % U]), __fadd_rn(pb[1 % U], pb[3 % U]));
-    } else {
-        if (U == 2) { ra = __fadd_rn(pa[0], pa[1 % U]); rb = __fadd_rn(pb[0], pb[1 % U]); }
-        else { ra = pa[0]; rb = pb[0]; }
-#pragma unroll
-        for (int m = L / 2; m >= 1; m >>= 1) {
-            ra = __fadd_rn(ra, __shfl_xor_sync(0xffffffffu, ra, m));
-            rb = __fadd_rn(rb, __shfl_xor_sync(0xffffffffu, rb, m));
-        }
-    }
-    return make_float2(ra, rb);
-}
-// U = 4: the 8 lanes' partials through shared memory, the same tree as rollout_kernel_h32
-__device__ __forceinline__ void h32_put_partial(float* rbw, int g, int l, float2 r)
-{
-    *reinterpret_cast<float2*>(&rbw[g * 20 + l * 2]) = r;
-}
-__device__ __forceinline__ void h32_get_partials(const float* rbw, int g, float4 r[4])
-{
-#pragma unroll
-    for (int k = 0; k < 4; ++k) r[k] = *reinterpret_cast<const float4*>(&rbw[g * 20 + 4 * k]);
-}
-__device__ __forceinline__ float2 h32_tree(const float4 r[4])
-{
-    const float2 t04 = __fadd2_rn(make_float2(r[0].x, r[0].y), make_float2(r[2].x, r[2].y));
-    const float2 t15 = __fadd2_rn(make_float2(r[0].z, r[0].w), make_float2(r[2].z, r[2].w));
-    const float2 t26 = __fadd2_rn(make_float2(r[1].x, r[1].y), make_float2(r[3].x, r[3].y));
-    const float2 t37 = __fadd2_rn(make_float2(r[1].z, r[1].w), make_float2(r[3].z, r[3].w));
-    return __fadd2_rn(__fadd2_rn(t04, t26), __fadd2_rn(t15, t37));
-}
-// quantise + fill decision against the bar's float thresholds (tha, thb); moves inv2 and returns the step record
-__device__ __forceinline__ float2 h32_decide(float2 r, float b3a, float b3b, float2 th, float& inv2)
-{
-    const float qa = __fmul_rn(__fadd_rn(r.x, b3a), 5.0f);           // raw*5.0 (drl_engine.py:39)
-    const float qb = __fmul_rn(__fadd_rn(r.y, b3b), 5.0f);
-    const bool fb = (inv2 < 1.0f) && (qb < th.y);
-    const bool fs = (inv2 > -1.0f) && (qa < th.x);
-    inv2 = __fadd_rn(inv2, fb ? (fs ? 0.0f : 0.5f) : (fs ? -0.5f : 0.0f));
-    return make_float2(fs ? qa : __int_as_float(SGMM_CODE_NOFILL_F), fb ? qb : __int_as_float(SGMM_CODE_NOFILL_F));
-}
-// the inventory move (in halves) a step record encodes
-__device__ __forceinline__ float h32_record_move(float2 c)
-{
-    const bool fs = __float_as_int(c.x) != SGMM_CODE_NOFILL_F, fb = __float_as_int(c.y) != SGMM_CODE_NOFILL_F;
-    return fb ? (fs ? 0.0f : 0.5f) : (fs ? -0.5f : 0.0f);
-}
-
 template <int U, bool FEE>
 __global__ void __launch_bounds__((max_compute_warps(U) + 1) * 32, 1)
 rollout2_kernel_h32(const RolloutArgs a, const int burn)
 {
-    constexpr int H = 32;
-    constexpr int NI = U;
-    constexpr int L = 32 / U;
-    constexpr int64_t G = (int64_t)H * H + 7 * H + 2;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Ring2Smem& sm = *reinterpret_cast<Ring2Smem*>(smem_raw);
 
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int nwarps = (blockDim.x >> 5) - 1;
-    const int g = lane / L, l = lane % L;
-    const int64_t first = (int64_t)blockIdx.x * nwarps * NI;
-    const int64_t remaining = a.mm.count - first;
-    const int live_warps = (int)(remaining >= (int64_t)nwarps * NI ? nwarps : (remaining + NI - 1) / NI);
-    const int64_t ind = first + (int64_t)warp * NI + g;
-    const bool live = ind < a.mm.count;
+    const H32Cta<U> cta(a.mm.count);
     const int64_t T = a.T;
     const int64_t nrounds = (T + ROUND_BARS - 1) / ROUND_BARS;
     const int N = (ROUND_BARS + burn) / 2;                           // steps of each chain in a whole round
 
     if (threadIdx.x == 0) {
 #pragma unroll
-        for (int s = 0; s < 2; ++s) { mbar_init(&sm.full[s], 1); mbar_init(&sm.rec_full[s], live_warps); }
+        for (int s = 0; s < 2; ++s) { mbar_init(&sm.full[s], 1); mbar_init(&sm.rec_full[s], cta.live_warps); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
 
-    if (warp == nwarps) {
+    if (cta.warp == cta.nwarps) {
         // ===== TMA producer of the round buffers and the fp64 half of the env step (as in rollout_kernel_h32) =====
-        const int64_t indj = first + lane;
-        const bool livej = lane < live_warps * NI && indj < a.mm.count;
+        const int lane = cta.lane;
+        const int64_t indj = cta.first + lane;
+        const bool livej = lane < cta.live_warps * U && indj < a.mm.count;
         const double tick = a.tick, fee = a.fee;
         const PenaltyTable pen = penalty_table(a.phi);
         double total = 0.0;
@@ -690,24 +664,7 @@ rollout2_kernel_h32(const RolloutArgs a, const int burn)
             const BarPx* pxs = &sm.px[s][0];
 #pragma unroll 4
             for (int i = 0; i < n; ++i) {
-                const uint64_t code = sm.rec[s][i][lane];
-                int ka = (int)(uint32_t)code, kb = (int)(uint32_t)(code >> 32);
-                const bool fs = ka != SGMM_CODE_NOFILL_F, fb = kb != SGMM_CODE_NOFILL_F;
-                inv += (fb ? 1 : 0) - (fs ? 1 : 0);                      // market_env.py:45,51
-                const int ai = inv < 0 ? -inv : inv;
-                const bool traded = fb || fs;
-                ntr += traded ? 1 : 0;                                   // drl_engine.py:60-61
-                double pnl = 0.0;                                        // market_env.py:40
-                if (__any_sync(0xffffffffu, traded)) {
-                    const double2 ab = *reinterpret_cast<const double2*>(&pxs[i].ask);
-                    const double mid = pxs[i].mid_next;
-                    ka = __float2int_rn(__int_as_float(ka)); kb = __float2int_rn(__int_as_float(kb));   // drl_engine.py:39
-                    const double my_ask = quote_ask(ab.x, ka, tick), my_bid = quote_bid(ab.y, kb, tick);      // market_env.py:30-31
-                    const double leg_b = buy_leg<FEE>(my_bid, mid, fee), leg_s = sell_leg<FEE>(my_ask, mid, fee);
-                    pnl = fb ? add_rn(pnl, leg_b) : pnl;
-                    pnl = fs ? add_rn(pnl, leg_s) : pnl;
-                }
-                total = add_rn(total, sub_rn(pnl, penalty(pen, ai)));                   // market_env.py:58, drl_engine.py:54
+                account_bar<false, FEE>(sm.rec[s][i][lane], pxs, i, tick, fee, pen, inv, ntr, total);
             }
             __syncwarp();
             if (r + 2 < nrounds) load(r + 2);                            // both buffers of round r are free again
@@ -715,60 +672,25 @@ rollout2_kernel_h32(const RolloutArgs a, const int burn)
         if (livej) { a.fitness[indj] = episode_fitness(total, ntr); a.trades[indj] = ntr; }
         return;
     }
-    if (warp >= live_warps) return;
+    if (cta.warp >= cta.live_warps) return;
 
-    // ---- weights into registers (models/model.py:31-36 layout) ---------------------------------
-    const PopArgs mmp = resolve(a.mm);
-    const GenomeSource src = make_source(mmp, live ? ind : 0, G);
     H32Regs<U> w;
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-        const int j = l + L * u;
-        if (live) {
-            w.w1x[u] = src.at(3 * j + 0); w.w1y[u] = src.at(3 * j + 1); w.w1i[u] = src.at(3 * j + 2);
-            w.b1[u] = src.at(3 * H + j);
-            w.b2[u] = src.at(4 * H + H * H + j);
-            w.w3a[u] = src.at(5 * H + H * H + j);
-            w.w3b[u] = src.at(6 * H + H * H + j);
-#pragma unroll
-            for (int c = 0; c < 8; ++c) {
-                float v[4]; src.at4(4 * H + (int64_t)j * H + 4 * c, v);
-                w.w2[u][2 * c] = make_float2(v[0], v[1]);
-                w.w2[u][2 * c + 1] = make_float2(v[2], v[3]);
-            }
-        } else {
-            w.w1x[u] = w.w1y[u] = w.w1i[u] = w.b1[u] = w.b2[u] = w.w3a[u] = w.w3b[u] = 0.0f;
-#pragma unroll
-            for (int c = 0; c < 16; ++c) w.w2[u][c] = make_float2(0.0f, 0.0f);
-        }
-    }
-    w.b3a = live ? src.at(7 * H + H * H) : 0.0f;
-    w.b3b = live ? src.at(7 * H + H * H + 1) : 0.0f;
+    h32_load_weights<U>(a.mm, cta, w);
 
-    float* const hA = &sm.hbuf[0][warp][0];
-    float* const hB = &sm.hbuf[1][warp][0];
-    float* const rA = &sm.rbuf[0][warp][0];
-    float* const rB = &sm.rbuf[1][warp][0];
-    const int slotj = warp * NI + g;                                 // this individual's lane in the accounting warp
+    float* const hA = &sm.hbuf[0][cta.warp][0];
+    float* const hB = &sm.hbuf[1][cta.warp][0];
+    float* const rA = &sm.rbuf[0][cta.warp][0];
+    float* const rB = &sm.rbuf[1][cta.warp][0];
+    const int slotj = cta.warp * U + cta.g;                         // this individual's lane in the accounting warp
     float inv2 = 0.0f;                                               // inventory / 2.0 (drl_engine.py:35), exact
 
     // one step of a lone chain on chain A's buffers (partial rounds and repairs); returns the step record
     auto step1 = [&](const BarSig* sg, float& iv) -> float2 {
         float h[U];
         h32_layer1<U>(w, *reinterpret_cast<const float2*>(&sg->z1), iv, h);
-        h32_put_h1<U>(hA, g, l, h);
+        h32_put_h1<U>(hA, cta.g, cta.l, h);
         __syncwarp();
-        float4 h4[8];
-        h32_get_h1<U>(hA, g, h4);
-        float2 p = h32_layer23<U>(w, h4);
-        if (U == 4) {
-            h32_put_partial(rA, g, l, p);
-            __syncwarp();
-            float4 pr[4];
-            h32_get_partials(rA, g, pr);
-            p = h32_tree(pr);
-        }
-        return h32_decide(p, w.b3a, w.b3b, *reinterpret_cast<const float2*>(&sg->tha), iv);
+        return h32_decide(h32_output<U>(w, hA, rA, cta.g, cta.l), w.b3a, w.b3b, *reinterpret_cast<const float2*>(&sg->tha), iv);
     };
 
     for (int64_t r = 0; r < nrounds; ++r) {
@@ -794,14 +716,14 @@ rollout2_kernel_h32(const RolloutArgs a, const int burn)
             {
                 float h[U];
                 h32_layer1<U>(w, *reinterpret_cast<const float2*>(&sigs[0].z1), inv2, h);
-                h32_put_h1<U>(hA, g, l, h);
+                h32_put_h1<U>(hA, cta.g, cta.l, h);
                 h32_layer1<U>(w, *reinterpret_cast<const float2*>(&sigB[0].z1), inv2B, h);
-                h32_put_h1<U>(hB, g, l, h);
+                h32_put_h1<U>(hB, cta.g, cta.l, h);
                 __syncwarp();
                 float4 h4[8];
-                h32_get_h1<U>(hB, g, h4);
+                h32_get_h1<U>(hB, cta.g, h4);
                 pB = h32_layer23<U>(w, h4);
-                if (U == 4) h32_put_partial(rB, g, l, pB);
+                if (U == 4) h32_put_partial(rB, cta.g, cta.l, pB);
             }
 #pragma unroll 1
             for (int i = 0; i < N; ++i) {
@@ -810,9 +732,9 @@ rollout2_kernel_h32(const RolloutArgs a, const int burn)
                 __syncwarp();
                 {
                     float4 h4[8];
-                    h32_get_h1<U>(hA, g, h4);
+                    h32_get_h1<U>(hA, cta.g, h4);
                     float2 qB = pB;
-                    if (U == 4) { float4 pr[4]; h32_get_partials(rB, g, pr); qB = h32_tree(pr); }
+                    if (U == 4) { float4 pr[4]; h32_get_partials(rB, cta.g, pr); qB = h32_tree(pr); }
                     const float2 thB = *reinterpret_cast<const float2*>(&sigB[i].tha);
                     const float2 zB = *reinterpret_cast<const float2*>(&sigB[ibn].z1);
                     const float2 cB = h32_decide(qB, w.b3a, w.b3b, thB, inv2B);
@@ -821,16 +743,16 @@ rollout2_kernel_h32(const RolloutArgs a, const int burn)
                     h32_layer1<U>(w, zB, inv2B, h);
                     pA = h32_layer23<U>(w, h4);
                     recB[32 * i] = cB;
-                    h32_put_h1<U>(hB, g, l, h);
-                    if (U == 4) h32_put_partial(rA, g, l, pA);
+                    h32_put_h1<U>(hB, cta.g, cta.l, h);
+                    if (U == 4) h32_put_partial(rA, cta.g, cta.l, pA);
                 }
                 // -- half 2: B's layer 2 of its next bar | A's decision of bar i and layer 1 of bar i + 1
                 __syncwarp();
                 {
                     float4 h4[8];
-                    h32_get_h1<U>(hB, g, h4);
+                    h32_get_h1<U>(hB, cta.g, h4);
                     float2 qA = pA;
-                    if (U == 4) { float4 pr[4]; h32_get_partials(rA, g, pr); qA = h32_tree(pr); }
+                    if (U == 4) { float4 pr[4]; h32_get_partials(rA, cta.g, pr); qA = h32_tree(pr); }
                     const float2 thA = *reinterpret_cast<const float2*>(&sigs[i].tha);
                     const float2 zA = *reinterpret_cast<const float2*>(&sigs[i + 1].z1);    // i + 1 <= N < ROUND_BARS
                     const float2 cA = h32_decide(qA, w.b3a, w.b3b, thA, inv2);
@@ -838,15 +760,15 @@ rollout2_kernel_h32(const RolloutArgs a, const int burn)
                     h32_layer1<U>(w, zA, inv2, h);
                     pB = h32_layer23<U>(w, h4);
                     recs[32 * i] = cA;
-                    h32_put_h1<U>(hA, g, l, h);
-                    if (U == 4) h32_put_partial(rB, g, l, pB);
+                    h32_put_h1<U>(hA, cta.g, cta.l, h);
+                    if (U == 4) h32_put_partial(rB, cta.g, cta.l, pB);
                 }
             }
             __syncwarp();
             // ---- stitch: where B entered bar N with another inventory than A left it, step B's block again from the
             // true state until the two inventories meet (from there on the records are the same) or the block ends.
             // B's own inventory entering each bar comes from the record about to be overwritten.
-            bool fix = live && inv2 != inv2Bent;
+            bool fix = cta.live && inv2 != inv2Bent;
             float inv2R = inv2, inv2O = inv2Bent;
 #pragma unroll 1
             for (int j = N; j < ROUND_BARS && __any_sync(0xffffffffu, fix); ++j) {
@@ -859,7 +781,7 @@ rollout2_kernel_h32(const RolloutArgs a, const int burn)
             inv2 = fix ? inv2R : inv2B;                                         // the state entering the next round
         }
         __syncwarp();
-        if (lane == 0) mbar_arrive(&sm.rec_full[s]);
+        if (cta.lane == 0) mbar_arrive(&sm.rec_full[s]);
     }
 }
 
